@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload reddit|wikipedia|mooc|lastfm|scaled]
     python bench.py --impl reference ...      # the CPU restatement of the reference path (oracle/), host cores
+    python bench.py --dump-outputs DIR ...    # + the last timed step's results as DIR/<name>.npy (float32)
 
 One step = one batch of 200 events through the whole fused path: temporal neighbor finder ->
 involved/outdated compaction -> lazy restart -> pending-message gather + GRU -> temporal
@@ -72,7 +73,22 @@ def parse_args():
     p.add_argument('--train-steps', type=int, default=100,
                    help='infer mode: also time this many training steps (fwd + bwd + all-reduce + Adam) of the same '
                         'configuration and report them under "train_step" (0 = off)')
-    return p.parse_args()
+    p.add_argument('--dump-outputs', metavar='DIR', default=None,
+                   help='write what the last timed step computed (scores, loss, embeddings, memories) to '
+                        'DIR/<name>.npy as float32, so that two builds can be compared output for output')
+    args = p.parse_args()
+    if args.dump_outputs and (args.micro or args.impl != 'b200' or args.mode != 'infer' or args.api != 'engine'):
+        p.error('--dump-outputs covers the default path (--impl b200 --mode infer --api engine) only')
+    if args.steps < 1:
+        p.error('--steps must be at least 1')
+    if args.dump_outputs:
+        # the engine runs with the CPU arm's parameters when there is one: random_weights(seed) for the oracle port
+        # (the same as without an arm), but the reference's own init_model where oracle/_ref is vendored - pinned to
+        # the port, so that a dump depends on the arguments only
+        if args.cpu_kind == 'reference':
+            p.error('--dump-outputs runs with the seeded random_weights: --cpu-kind reference does not apply')
+        args.cpu_kind = 'port'
+    return args
 
 
 def pick_restarter(args, shape):
@@ -293,16 +309,12 @@ def run_reference(args):
         return
     shape, st, neg = load_workload(args, with_efeats=True, cpu_only=True)
     lo, avail = batch_window(args, st.n_events, 0, max(world, 1))
-    budget_s = 200.0
-    W = min(args.warmup, max(avail - 1, 0), 5)
-    K = min(args.steps, avail - W)
+    W, K = args.warmup, args.steps
+    if W + K > avail:
+        raise SystemExit(f'--warmup {W} + --steps {K} exceed the {avail} batches of the stream window')
     arm = CpuArm(args, shape, st, neg, lo, W + K, kind=args.cpu_kind, mode=args.mode)
-    t0 = time.perf_counter()
     for i in range(W):
         arm.step(i)
-    per = (time.perf_counter() - t0) / max(W, 1)
-    if per > 0 and K * per > budget_s:
-        K = max(3, int(budget_s / per))
     t0 = time.perf_counter()
     for i in range(W, W + K):
         arm.step(i)
@@ -443,6 +455,30 @@ class DeviceWorkload:
         torch.cuda.synchronize()
 
 
+DUMP_BYTES = 60 << 20      # --dump-outputs: array bytes, leaves room for the .npy headers under 64 MB
+
+
+def dump_outputs(out_dir, eng, out_buf):
+    """Writes one step's results as float32 .npy files: the link scores and loss (`out_buf`, the step's [pos | neg |
+    loss] buffer), the [src | dst | neg] embeddings, and the left / right memories with their update times after the
+    step.  Memories larger than the DUMP_BYTES budget keep a fixed sample of rows (RandomState(0), ascending node
+    ids), the same rows in every run."""
+    import torch
+    B, N, d = eng.B, eng.N, eng.d
+    res = out_buf.cpu().numpy()
+    arrays = {'pos_scores': res[:B], 'neg_scores': res[B:2 * B], 'loss': res[2 * B:], 'embeddings': eng.emb.cpu().numpy()}
+    per_row = 2 * (d + 1) * 4
+    n_rows = min(N, (DUMP_BYTES - sum(a.nbytes for a in arrays.values())) // per_row)
+    rows = None if n_rows == N else torch.from_numpy(
+        np.sort(np.random.RandomState(0).choice(N, n_rows, replace=False))).to(eng.device)
+    for name, t in (('left_memory', eng.left_vals), ('left_memory_ts', eng.left_ts),
+                    ('right_memory', eng.right_vals), ('right_memory_ts', eng.right_ts)):
+        arrays[name] = (t if rows is None else t[rows]).cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + '.npy'), a.astype(np.float32))
+
+
 def run_b200(args):
     import torch
     import torch.distributed as dist
@@ -472,7 +508,7 @@ def run_b200(args):
         j = i % avail
         if j == 0 and i > 0:
             eng.reset()           # epoch boundary (train_self_supervised.py:127-128): the window wraps
-        runner.submit_device(dev_in[j])
+        return runner.submit_device(dev_in[j])
 
     barrier = wl.barrier
     Wm, K = args.warmup, args.steps
@@ -483,12 +519,14 @@ def run_b200(args):
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     ev0.record()
     for i in range(Wm, Wm + K):
-        device_step(i)
+        slot = device_step(i)
     runner.join()             # the last batch's link scorer runs on the copy-out stream
     ev1.record()
     barrier()
     ms = ev0.elapsed_time(ev1)
     eng.check_errors()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, eng, runner.d_out[slot])
     ms = max_over_ranks(ms, world, dev)
     value = world * K * B / (ms * 1e-3)
 
@@ -1193,7 +1231,9 @@ def run_dropin(args):
     if wl.world > 1:
         raise SystemExit('--api dropin is a single-process loop')
     st, neg, shape, rst, dev, lo, B = wl.st, wl.neg, wl.shape, wl.rst, wl.dev, wl.lo, BATCH
-    Wm, K = args.warmup, min(args.steps, wl.avail - args.warmup)
+    Wm, K = args.warmup, args.steps
+    if Wm + K > wl.avail:
+        raise SystemExit(f'--warmup {Wm} + --steps {K} exceed the {wl.avail} batches of the stream window')
     graph = Graph.from_csr(wl.csr)
     torch.manual_seed(args.seed)
     model = build_model(None, wl.efeats, graph, wl.N, st.n_events, dev, dim=shape.dim, n_layers=1, n_heads=N_HEAD,

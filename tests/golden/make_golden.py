@@ -1,8 +1,7 @@
 """Generate the golden fixtures in this directory by running the UNMODIFIED reference
-(yzhang1918/www2023tiger at /root/reference, read-only) on small seeded synthetic
-streams.  Runs only in the build container (the GPU box has no /root/reference):
+(a read-only checkout of yzhang1918/www2023tiger) on small seeded synthetic streams:
 
-    python tests/golden/make_golden.py
+    TIGER_REFERENCE=<reference checkout> python tests/golden/make_golden.py
 
 Workarounds (SURVEY.md §8(c)): torch_scatter is replaced by tests/golden/_shim
 (CPU tie rule of torch_scatter), and load_jodie_data (broken on Python >= 3.11) is
@@ -19,7 +18,10 @@ import torch
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, os.path.join(HERE, '_shim'))
-sys.path.insert(0, '/root/reference')
+REFERENCE = os.environ.get('TIGER_REFERENCE', '')
+if not os.path.isdir(os.path.join(REFERENCE, 'tiger')):
+    sys.exit('set TIGER_REFERENCE to a checkout of the reference (the directory that holds tiger/)')
+sys.path.insert(0, REFERENCE)
 sys.path.insert(0, ROOT)
 
 from init_utils import init_model                                   # noqa: E402  (reference)

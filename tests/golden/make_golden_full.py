@@ -1,15 +1,15 @@
-"""Full-dimension golden fixtures: the UNMODIFIED reference (/root/reference, read-only) at the dimensions of the
-BASELINE.json configs - d / d_e / K / hist_len / batch = the config values, on the BASELINE-shaped synthetic streams
-themselves (not on toy streams).  Runs only in the build container:
+"""Full-dimension golden fixtures: the UNMODIFIED reference (a read-only checkout of yzhang1918/www2023tiger) at the
+dimensions of the BASELINE.json configs - d / d_e / K / hist_len / batch = the config values, on the BASELINE-shaped
+synthetic streams themselves (not on toy streams):
 
-    python tests/golden/make_golden_full.py
+    TIGER_REFERENCE=<reference checkout> python tests/golden/make_golden_full.py
 
 The streams and the parameters are NOT stored: both are regenerated bit-identically from seeds by
 `www2023tiger_b200.synthetic.make_stream` and `www2023tiger_b200.init.random_weights` (+ `perturb_biases`), which
 the generator loads into the reference model with `load_state_dict`.  Stored per recorded batch: the complete
 integer results (neighbor tables, involved / restart / pending node lists, argmax-by-timestamp winners), the scores
 and losses, and for the wide float tensors (embeddings, restarter outputs, the three state tables) a fixed sample
-of complete rows plus float64 row / table sums of everything, so that a fixture stays ~1 MB.
+of complete rows plus float64 row / table sums of everything, so that a fixture stays under 1 MB.
 
 Protocol per case (eval_utils.py:29-46 with restart_mode=True): reset at event `start`, WARM lazy-restart batches,
 then REC recorded batches; afterwards the restarter on the collated batch + the mutual loss (tiger.py:574-590).
@@ -23,7 +23,10 @@ import torch
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, os.path.join(HERE, '_shim'))
-sys.path.insert(0, '/root/reference')
+REFERENCE = os.environ.get('TIGER_REFERENCE', '')
+if not os.path.isdir(os.path.join(REFERENCE, 'tiger')):
+    sys.exit('set TIGER_REFERENCE to a checkout of the reference (the directory that holds tiger/)')
+sys.path.insert(0, REFERENCE)
 sys.path.insert(0, ROOT)
 
 from init_utils import init_model                                   # noqa: E402  (reference)
@@ -35,16 +38,16 @@ from www2023tiger_b200.synthetic import SHAPES, NegativeSampler, make_stream   #
 
 B, K, H, HIST = 200, 10, 2, 40
 WARM, REC = 5, 5
-N_ROWS = 96          # embedding rows kept in full (48 src + 48 dst positions)
 N_NODES_KEPT = 16    # state-table rows kept in full per batch
 WEIGHT_SEED = 3
 
-# name: (BASELINE shape, restarter, first event of the window)
+# name: (BASELINE shape, restarter, first event of the window, embedding rows kept in full (half src, half dst
+# positions), restarter output rows kept in full); the 172-wide cases keep fewer rows to stay under 1 MB
 CASES = {
-    'full_wikipedia_seq': ('wikipedia', 'seq', 60000),
-    'full_reddit_static': ('reddit', 'static', 100000),
-    'full_mooc_seq_right_right': ('mooc', 'seq', 60000),
-    'full_lastfm_seq_noefeat': ('lastfm', 'seq', 100000),
+    'full_wikipedia_seq': ('wikipedia', 'seq', 60000, 48, 16),
+    'full_reddit_static': ('reddit', 'static', 100000, 48, 16),
+    'full_mooc_seq_right_right': ('mooc', 'seq', 60000, 96, 32),
+    'full_lastfm_seq_noefeat': ('lastfm', 'seq', 100000, 96, 32),
 }
 
 
@@ -64,7 +67,7 @@ def case_weights(st, restarter):
                                          seed=WEIGHT_SEED, nonzero_static=True))
 
 
-def run_case(name, shape_name, restarter, start):
+def run_case(name, shape_name, restarter, start, n_rows, n_restart_rows):
     shape = SHAPES[shape_name]
     st = make_stream(shape, seed=0)
     neg = NegativeSampler(st.src, st.dst, seed=0).pre_sample_neg_dsts(st.n_events, B)
@@ -99,9 +102,9 @@ def run_case(name, shape_name, restarter, start):
     model.reset()
     out = {'meta_shape': shape_name, 'meta_restarter': restarter, 'meta_start': start, 'meta_warm': WARM,
            'meta_rec': REC, 'meta_bs': B, 'meta_n_neighbors': K, 'meta_n_heads': H, 'meta_hist_len': HIST,
-           'meta_weight_seed': WEIGHT_SEED, 'meta_n_rows': N_ROWS, 'meta_dim': model.nfeat_dim}
+           'meta_weight_seed': WEIGHT_SEED, 'meta_n_rows': n_rows, 'meta_dim': model.nfeat_dim}
     i32 = lambda a: np.asarray(a).astype(np.int32)
-    rows_kept = np.concatenate([np.arange(N_ROWS // 2), B + np.arange(N_ROWS // 2)])
+    rows_kept = np.concatenate([np.arange(n_rows // 2), B + np.arange(n_rows // 2)])
     uptodate = set()
     with torch.no_grad():
         for ib in range(WARM + REC):
@@ -115,7 +118,7 @@ def run_case(name, shape_name, restarter, start):
             p = f'b{ib - WARM}_'
             if rec and len(r_nids):
                 hl, hr, pt = model.restarter_fn(r_nids, r_ts)
-                keep = min(32, len(r_nids))
+                keep = min(n_restart_rows, len(r_nids))
                 out[p + 'restart_hl'], out[p + 'restart_hr'] = t2n(hl[:keep]), t2n(hr[:keep])
                 out[p + 'restart_hl_rowsum'] = t2n(hl.double().sum(1))
                 out[p + 'restart_hr_rowsum'] = t2n(hr.double().sum(1))

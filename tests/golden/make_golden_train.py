@@ -1,10 +1,10 @@
 """Golden fixtures of the TRAINING step: losses and parameter gradients of the UNMODIFIED reference
-(/root/reference, read-only) for the loop body of train_self_supervised.py:143-171 (zero_grad ->
+(a read-only checkout of yzhang1918/www2023tiger) for the loop body of train_self_supervised.py:143-171 (zero_grad ->
 contrast_and_mutual_learning -> (contrast + mutual).backward()), on the toy streams of make_golden.py, in train()
 mode with dropout = 0 (dropout masks are not reproducible across implementations), no optimizer step (the
 parameters stay at their initial values so that every recorded batch is comparable on its own).
 
-    python tests/golden/make_golden_train.py
+    TIGER_REFERENCE=<reference checkout> python tests/golden/make_golden_train.py
 """
 import os
 import sys
@@ -15,7 +15,10 @@ import torch
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, os.path.join(HERE, '_shim'))
-sys.path.insert(0, '/root/reference')
+REFERENCE = os.environ.get('TIGER_REFERENCE', '')
+if not os.path.isdir(os.path.join(REFERENCE, 'tiger')):
+    sys.exit('set TIGER_REFERENCE to a checkout of the reference (the directory that holds tiger/)')
+sys.path.insert(0, REFERENCE)
 sys.path.insert(0, ROOT)
 
 from init_utils import init_model                                   # noqa: E402  (reference)

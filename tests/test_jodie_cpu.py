@@ -1,36 +1,20 @@
 """f4: the on-disk format.  `load_jodie_data` of the drop-in package (rewritten for Python >= 3.11, where the
-reference's own `random.sample(set, k)` raises) against the reference's loader run in a subprocess with exactly that
-one call made 3.11-safe (random.sample over the SORTED set, which is what the drop-in does)."""
+reference's own `random.sample(set, k)` raises) against the reference's loader with exactly that one call made
+3.11-safe (tests/jodie_utils.py:REFERENCE_LOADER), run live where the reference's sources are vendored in
+oracle/_ref, and against the splits stored in tests/golden/jodie_toy_splits.json, whose `source` field says which
+loader recorded them (tests/golden/make_golden_jodie.py)."""
 import json
 import os
-import subprocess
-import sys
 
 import numpy as np
 import pytest
 
-from jodie_utils import write_toy_dataset
+from jodie_utils import SPLITS, reference_splits, write_toy_dataset
 from www2023tiger_b200.tiger.data.data_loader import load_jodie_data
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = '/root/reference' if os.path.isdir('/root/reference/tiger') else os.path.join(ROOT, 'oracle', '_ref')
-
-REF_SCRIPT = r'''
-import random, sys, json
-import numpy as np
-sys.path.insert(0, sys.argv[1])
-sys.path.insert(0, sys.argv[2])           # torch_scatter shim
-_orig = random.sample
-random.sample = lambda pop, k: _orig(sorted(pop), k)      # the only change: sets are rejected by Python >= 3.11
-from tiger.data.data_loader import load_jodie_data
-out = load_jodie_data('toy', train_seed=5, root=sys.argv[3])
-names = ['full', 'train', 'val', 'test', 'ind_val', 'ind_test']
-res = {'nfeats_shape': list(out[0].shape) if out[0] is not None else None, 'efeats_sum': float(out[1].sum())}
-for n, d in zip(names, out[2:]):
-    res[n] = {'eids': d.eids.tolist(), 'neg': (d.neg_dst.tolist() if d.neg_dst is not None else None), 'eval': bool(d.eval),
-              'seed': d.seed}
-print(json.dumps(res))
-'''
+GOLDEN = os.path.join(ROOT, 'tests', 'golden', 'jodie_toy_splits.json')
+REF = os.path.join(ROOT, 'oracle', '_ref')
 
 
 def test_load_jodie_data_properties(tmp_path):
@@ -57,15 +41,24 @@ def test_load_jodie_data_properties(tmp_path):
 @pytest.mark.skipif(not os.path.isdir(os.path.join(REF, 'tiger')), reason='no reference sources (vendor with tools/vendor_ref.py)')
 def test_load_jodie_data_equals_reference_loader(tmp_path):
     write_toy_dataset(str(tmp_path))
-    shim = os.path.join(ROOT, 'tests', 'golden', '_shim')
-    res = subprocess.run([sys.executable, '-c', REF_SCRIPT, REF, shim, str(tmp_path)], capture_output=True, text=True,
-                         timeout=300)
-    assert res.returncode == 0, res.stderr[-2000:]
-    ref = json.loads(res.stdout.strip().splitlines()[-1])
+    ref = reference_splits(REF, str(tmp_path))
+    assert_same_splits(load_jodie_data('toy', train_seed=5, root=str(tmp_path)), ref)
+
+
+def test_load_jodie_data_equals_recorded_splits(tmp_path):
+    """Against the stored splits.  Recorded from the reference's loader they are the comparison above without its
+    sources; recorded from this package's loader (`source` says so) they only catch changes to it."""
+    write_toy_dataset(str(tmp_path))
+    with open(GOLDEN) as f:
+        ref = json.load(f)
     out = load_jodie_data('toy', train_seed=5, root=str(tmp_path))
-    assert list(out[0].shape) == ref['nfeats_shape'] and abs(float(out[1].sum()) - ref['efeats_sum']) < 1e-3
-    for n, d in zip(['full', 'train', 'val', 'test', 'ind_val', 'ind_test'], out[2:]):
-        r = ref[n]
-        assert d.eids.tolist() == r['eids'], n                       # the same events in every split
-        assert bool(d.eval) == r['eval'] and d.seed == r['seed'], n
-        assert (d.neg_dst.tolist() if d.neg_dst is not None else None) == r['neg'], n   # the same pre-sampled negatives
+    assert_same_splits(out, ref, 'splits recorded by ' + ref['source'])
+
+
+def assert_same_splits(out, ref, what='reference loader'):
+    assert list(out[0].shape) == ref['nfeats_shape'] and abs(float(out[1].sum()) - ref['efeats_sum']) < 1e-3, what
+    for n, d in zip(SPLITS, out[2:]):
+        r, w = ref[n], f'{n} vs {what}'
+        assert d.eids.tolist() == r['eids'], w                       # the same events in every split
+        assert bool(d.eval) == r['eval'] and d.seed == r['seed'], w
+        assert (d.neg_dst.tolist() if d.neg_dst is not None else None) == r['neg'], w   # the same pre-sampled negatives
