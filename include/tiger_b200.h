@@ -363,16 +363,20 @@ int tiger_seq_tail(const float* xbar, const int32_t* count, int64_t n, int d_mod
                    const float* psum, float p_drop, int seed, float* att, float* o, float* hid, float* h_left,
                    float* h_right, void* stream);
 
-/* C[m,n] = act(sum_k A[m,k] * W[n,k] + bias[n]): fp32 FFMA GEMM on row-major A [M,K] and nn.Linear
- * style weights W [N,K] (bias may be NULL; relu != 0 applies max(.,0)).  The row count is
- * min(m_rows, *count * rows_per_count) when count (device) is non-NULL.  Replaces the in/out
- * projections of nn.MultiheadAttention, nn.Linear and MergeLayer on the restarter path
- * (restarters.py:45-50,106-111; basic_modules.py:16-19). */
+/* Dense products on the tensor cores (csrc/gemm.cu: tcgen05, tf32 head / tail split, fp32-accurate).  Two kernels:
+ * tiger_sgemm_nt and tiger_sgemm_ex stage both operands through shared memory; the tiger_sgemm_nt_packed* family
+ * takes the weight as a pre-split pack (tiger_gemm_pack_weight) streamed by TMA.
+ *
+ * C[m,n] = act(sum_k A[m,k] * W[n,k] + bias[n]) on row-major A [M,K] and nn.Linear style weights W [N,K] (bias may
+ * be NULL; relu != 0 applies max(.,0)); tiger_sgemm_ex with trans 0 / 0, alpha 1 and no accumulation.  The row count
+ * is min(m_rows, *count * rows_per_count) when count (device) is non-NULL.  Replaces the in/out projections of
+ * nn.MultiheadAttention, nn.Linear and MergeLayer on the restarter path (restarters.py:45-50,106-111;
+ * basic_modules.py:16-19). */
 int tiger_sgemm_nt(const float* A, int64_t lda, const float* W, int64_t ldw, const float* bias, float* C,
                    int64_t ldc, int64_t m_rows, const int32_t* count, int64_t rows_per_count, int n_cols,
                    int k_dim, int relu, void* stream);
 
-/* General product for the training step (same tensor-core kernel):
+/* General product for the training step (the same staging kernel):
  *   C[m,n] (+)= act(alpha * (sum_k opA[m,k] * opW[n,k] + bias[n]))
  * opA[m,k] = A[m*lda + k] (trans_a = 0) or A[k*lda + m] (trans_a = 1), opW likewise, so that the three products of
  * a linear layer use the tensors as stored: y = x W^T (0,0), dx = dy W (0,1), dW = dy^T x (1,1) - what autograd
@@ -385,20 +389,10 @@ int tiger_sgemm_ex(const float* A, int64_t lda, int trans_a, const float* W, int
                    const int32_t* m_count, const int32_t* k_count, int64_t rows_per_count, float alpha, int relu,
                    int accumulate, int k_parts, void* stream);
 
-/* Batched / extended form: problem b uses A + b*stride_a, W + b*stride_w, bias + b*stride_bias,
- * C + b*stride_c (strides in floats); the result is act(alpha * (A W^T + bias)); rows with
- * row_zero[m] != 0 (may be NULL; shared by all problems) are written as zeros - the
- * masked_fill(invalid_rows, 0) of TemporalAttention.forward (temporal_agg_modules.py:230). */
-int tiger_sgemm_nt_batched(const float* A, int64_t lda, int64_t stride_a, const float* W, int64_t ldw,
-                           int64_t stride_w, const float* bias, int64_t stride_bias, float* C, int64_t ldc,
-                           int64_t stride_c, int batch, int64_t m_rows, const int32_t* count,
-                           int64_t rows_per_count, int n_cols, int k_dim, float alpha, int relu,
-                           const uint8_t* row_zero, void* stream);
-
 /* Pre-split weight packs for the tensor-core GEMM: W [n_rows][k_dim] (row stride ldw) -> tf32 head / tail
  * planes in the shared-memory image of each (column tile of bn rows, k-block) stage, so the kernel loads
  * a stage of W with one TMA bulk copy.  row_map (device int32 [n_tiles*bn], may be NULL) selects the
- * source row of every tile row (-1 = zeros).  bn: multiple of 16, <= 128 (tiger_gemm_pick_bn proposes
+ * source row of every tile row (-1 = zeros).  bn: multiple of 16, <= 64 (tiger_gemm_pick_bn proposes
  * one for an expected row count). */
 int tiger_gemm_pick_bn(int64_t m_rows, int n_cols, int batch);
 int64_t tiger_gemm_pack_bytes(int n_tiles, int k_dim, int bn);
@@ -434,36 +428,14 @@ int tiger_sgemm_nt_packed_scatter(const float* A, int64_t lda, const float* wpac
                                   int64_t ldc, int n_cols0, float* C2, int64_t ldc2, int n_split, int n_cols1,
                                   int64_t m_rows, int k_dim, const tiger_left_writeback_fused* wb, void* stream);
 
-/* Split-K pair for long reductions with few output tiles.  tiger_sgemm_nt_packed_splitk writes
- * tiger_gemm_splitk_parts(k_dim, k_parts) raw partial products A[:, part] Wpack[:, part]^T to
- * C_parts + part * part_stride (no bias / activation); tiger_sgemm_nt_packed_sum consumes such partials as its
- * A operand: A = act(sum_p A_parts[p] + a_bias[k]) is formed while the activations are staged, so no
- * reduction kernel runs in between.  C2 / n_split / n_cols1 as in tiger_sgemm_nt_packed_split (C2 may be NULL). */
-int tiger_gemm_splitk_parts(int k_dim, int k_parts);
-int tiger_sgemm_nt_packed_splitk(const float* A, int64_t lda, const float* wpack, int bn, float* C_parts, int64_t ldc,
-                                 int64_t part_stride, int k_parts, int64_t m_rows, const int32_t* count,
-                                 int64_t rows_per_count, int n_cols, int k_dim, void* stream);
-/* Split-K with the reduction inside the launch: the k_parts (<= 8) CTAs of an output tile form a thread-block
- * cluster, exchange their partial tiles through distributed shared memory, sum them in part order
- * (deterministic) and write act(alpha * (A W^T + bias)) once. */
+/* Split-K for long reductions with few output tiles, the reduction inside the launch: the k_parts (<= 8; fewer
+ * when K has fewer 32-float blocks) CTAs of an output tile form a thread-block cluster, exchange their partial
+ * tiles through distributed shared memory, sum them in part order (deterministic) and write
+ * act(alpha * (A W^T + bias)) once. */
 int tiger_sgemm_nt_packed_splitk_fused(const float* A, int64_t lda, const float* wpack, int bn, const float* bias,
                                        float* C, int64_t ldc, int k_parts, int64_t m_rows, const int32_t* count,
                                        int64_t rows_per_count, int n_cols, int k_dim, float alpha, int relu,
                                        void* stream);
-int tiger_sgemm_nt_packed_sum(const float* A_parts, int64_t lda, int64_t a_part_stride, int a_parts,
-                              const float* a_bias, int a_relu, const float* wpack, int bn, const float* bias,
-                              float* C, int64_t ldc, int n_cols0, float* C2, int64_t ldc2, int n_split, int n_cols1,
-                              int64_t m_rows, const int32_t* count, int64_t rows_per_count, int k_dim, float alpha,
-                              int relu, void* stream);
-
-/* Self-attention weights of SeqRestarter's MHA (restarters.py:106, torch MHA need_weights branch),
- * reduced to what the mean over positions needs: for node i and head h
- *   p_h = softmax_keys((q_h * sqrt(1/hd)) k_h^T + mask)   [len x len], pbar_h = mean over queries,
- *   xbar[i,h,:] = sum_j pbar_h[j] * x[i,j,:]               [d_model]
- * qk [n*len, ld_qk] holds q in columns [0,d_model) and k in [d_model, 2*d_model).  len <= 64. */
-int tiger_seq_attn_pool(const float* qk, int64_t ld_qk, const float* x, const uint8_t* mask,
-                        const int32_t* count, int64_t n, int len, int d_model, int n_head, float* xbar,
-                        void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * Host-side batch pipeline (csrc/pipe.cu; no device code).  Replaces the synchronous per-batch `.to(device)` /

@@ -46,9 +46,6 @@ _SIGNATURES: Dict[str, str] = {
     'tiger_score_fold_cab_offset': 'i',
     'tiger_score_fold': 'pppppip' + 'p',
     'tiger_link_score_folded': 'pli' + 'pppp' + 'i' + 'ppp' + 'ppp' + 'p',
-    'tiger_gemm_splitk_parts': 'ii',
-    'tiger_sgemm_nt_packed_splitk': 'plpi' + 'plli' + 'lpl' + 'ii' + 'p',
-    'tiger_sgemm_nt_packed_sum': 'plli' + 'pi' + 'pi' + 'p' + 'pli' + 'pliil' + 'pl' + 'ifi' + 'p',
     'tiger_sgemm_nt_packed_gather': 'ppi' + 'pplp' + 'pi' + 'ppl' + 'lpl' + 'iifi' + 'p',
     'tiger_sgemm_nt_packed_splitk_fused': 'plpi' + 'ppl' + 'i' + 'lpl' + 'iifi' + 'p',
     'tiger_pipe_capture_begin': 'p',
@@ -93,12 +90,10 @@ _SIGNATURES: Dict[str, str] = {
     'tiger_seq_gate_count': 'pipp' + 'p',
     'tiger_seq_tail': 'ppliii' + 'pppppp' + 'plp' + 'pp' + 'pfi' + 'ppppp' + 'p',
     'tiger_sgemm_ex': 'pli' + 'pli' + 'ppl' + 'lil' + 'ppl' + 'fiii' + 'p',
-    'tiger_sgemm_nt_batched': 'pll' + 'pll' + 'pl' + 'pll' + 'il' + 'pl' + 'ii' + 'fi' + 'p' + 'p',
     'tiger_gemm_pick_bn': 'lii',
     'tiger_gemm_pack_bytes': 'iii',
     'tiger_gemm_pack_weight': 'plpiiiip' + 'p',
     'tiger_sgemm_nt_packed': 'plpippllpliifi' + 'p',
-    'tiger_seq_attn_pool': 'plpp' + 'pli' + 'iip' + 'p',
     'tiger_static_restart': 'ppl' + 'plp' + 'pp' + 'ppi' + 'ppp' + 'ppp' + 'pp' + 'p',
 }
 _KIND = {'p': P, 'l': L, 'i': I, 'f': F}

@@ -32,36 +32,6 @@
 #include <cstdio>
 #endif
 
-extern "C" int tiger_sgemm_nt_batched(const float* A, int64_t lda, int64_t stride_a, const float* W, int64_t ldw,
-                                      int64_t stride_w, const float* bias, int64_t stride_bias, float* C,
-                                      int64_t ldc, int64_t stride_c, int batch, int64_t m_rows,
-                                      const int32_t* count, int64_t rows_per_count, int n_cols, int k_dim,
-                                      float alpha, int relu, const uint8_t* row_zero, void* stream);
-
-extern "C" int64_t tiger_gemm_pack_bytes(int n_tiles, int k_dim, int bn);
-extern "C" int tiger_gemm_pack_weight(const float* W, int64_t ldw, const int32_t* row_map, int n_rows, int k_dim,
-                                      int bn, int n_tiles, float* out, void* stream);
-extern "C" int tiger_sgemm_nt_packed(const float* A, int64_t lda, const float* wpack, int bn, const float* bias,
-                                     float* C, int64_t ldc, int64_t m_rows, const int32_t* count,
-                                     int64_t rows_per_count, int n_cols, int k_dim, float alpha, int relu,
-                                     void* stream);
-
-extern "C" int tiger_gemm_splitk_parts(int k_dim, int k_parts);
-extern "C" int tiger_sgemm_nt_packed_splitk(const float* A, int64_t lda, const float* wpack, int bn, float* C_parts,
-                                            int64_t ldc, int64_t part_stride, int k_parts, int64_t m_rows,
-                                            const int32_t* count, int64_t rows_per_count, int n_cols, int k_dim,
-                                            void* stream);
-extern "C" int tiger_sgemm_nt_packed_sum(const float* A_parts, int64_t lda, int64_t a_part_stride, int a_parts,
-                                         const float* a_bias, int a_relu, const float* wpack, int bn,
-                                         const float* bias, float* C, int64_t ldc, int n_cols0, float* C2,
-                                         int64_t ldc2, int n_split, int n_cols1, int64_t m_rows,
-                                         const int32_t* count, int64_t rows_per_count, int k_dim, float alpha,
-                                         int relu, void* stream);
-extern "C" int tiger_sgemm_nt_packed_split(const float* A, int64_t lda, const float* wpack, int bn, const float* bias,
-                                           float* C, int64_t ldc, int n_cols0, float* C2, int64_t ldc2, int n_split,
-                                           int n_cols1, int64_t m_rows, const int32_t* count,
-                                           int64_t rows_per_count, int k_dim, float alpha, int relu, void* stream);
-
 #define ATT_MAXH 8
 #ifndef ATT_THREADS
 #define ATT_THREADS 256
@@ -701,9 +671,8 @@ static int attention_run(AttArgs& a, const tiger_attn_params* p, float* out, cud
   if (rc != TIGER_OK) return rc;
   // hidden = relu([kvbar | c | live] W2f^T + b1): the long K is split over a cluster of ATT_KPARTS CTAs per tile whose
   // partial tiles are summed through distributed shared memory ; z = hidden W2^T + b2
-  const int kparts = tiger_gemm_splitk_parts(m.off_live + 1, ATT_KPARTS);
-  rc = tiger_sgemm_nt_packed_splitk_fused(a.w.kvc, m.ld_kvc, f.pk_w2f, ATT_BN_D, p->fc1_b, a.w.hid, m.ld_hid, kparts, n,
-                                          nullptr, 1, m.d, m.off_live + 1, 1.0f, 1, s);
+  rc = tiger_sgemm_nt_packed_splitk_fused(a.w.kvc, m.ld_kvc, f.pk_w2f, ATT_BN_D, p->fc1_b, a.w.hid, m.ld_hid,
+                                          ATT_KPARTS, n, nullptr, 1, m.d, m.off_live + 1, 1.0f, 1, s);
   if (rc != TIGER_OK) return rc;
   const bool fold_scorer = p->score_folded != nullptr && p->pq_out != nullptr;
   if (p->left_wb != nullptr && !a.dense) {

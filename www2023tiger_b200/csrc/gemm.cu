@@ -1,5 +1,5 @@
 // fp32-accurate "NT" GEMM on the 5th-generation tensor cores (tcgen05, kind::tf32, tf32x3 split):
-//     C[b][m, n] = act(alpha * (sum_k A[b][m, k] * W[b][n, k] + bias[b][n])),  rows with row_zero[m] != 0 -> 0
+//     C[m, n] = act(alpha * (sum_k A[m, k] * W[n, k] + bias[n]))
 // A row-major [M, K] (lda), W row-major [N, K] (ldw) - the layout of nn.Linear / in_proj weights, so
 // parameters are used as stored (reference: nn.MultiheadAttention in/out projections, nn.Linear and
 // MergeLayer of tiger/model/restarters.py:45-50, temporal_agg_modules.py:203-209, basic_modules.py:5-19).
@@ -10,22 +10,28 @@
 // (error ~2^-22 per product), at 3 MMAs per k-step - still several times the FFMA rate, and the MMAs
 // run asynchronously to the threads that stage the operands.
 //
-// Structure (one CTA = one 128 x BN output tile, BN <= 128, 19 warps):
+// Two kernels:
+//   gemm_tf32x3_kernel     (tiger_sgemm_ex, tiger_sgemm_nt) both operands staged through shared memory by
+//                          the producer warps; either operand may be read transposed
+//   gemm_tf32x3_ts_kernel  (tiger_sgemm_nt_packed*) weights pre-split into a pack (tiger_gemm_pack_weight)
+//                          and streamed by TMA, activations staged in tensor memory
+// Staging kernel (one CTA = one 128 x BN output tile at a time, BN <= 128, 19 warps):
 //   warps 0-15 producers in 4 groups of 4 warps; group g fills stages g, g+4, ...: global (L2) ->
 //              registers -> tf32 split -> shared memory in the canonical K-major UMMA layout
 //              (umma.cuh), 16 floats of K per stage, up to 8 stages, full/empty mbarriers; a group's
 //              next loads are issued before it publishes the current stage, and the four groups keep
 //              four stages of loads in flight, which is what hides the L2 latency;
 //              afterwards the same warps run the epilogue: tcgen05.ld of the partial accumulators
-//              (thread = row, 16 columns at a time), bias / alpha / ReLU / row mask, 16-byte stores
+//              (thread = row, 16 columns at a time), bias / alpha / ReLU, 16-byte stores or atomic adds
 //   warps 16-18 MMA issuers: one elected thread each issues one of the three tf32x3 product streams
 //              into its own TMEM accumulator and commits each stage back to the producers
 //              (tcgen05.commit -> mbarrier); see umma.cuh for why three
+//   warp 19    idle: it only takes part in the block barriers.  The block shape, and with it the register
+//              budget __launch_bounds__ gives every thread, is the one the kernel was tuned and measured at.
 // The row count may live on the device (`count` * rows_per_count), which keeps the restart path free of
 // host syncs: CTAs whose row block starts beyond it exit before touching TMEM.
 #include "common.cuh"
 #include "umma.cuh"
-#include <cstring>
 
 #ifdef TIGER_TRACE
 #include <cstdio>
@@ -39,7 +45,7 @@
 #endif
 
 #define TCG_PRODUCER_WARPS 16
-#define TCG_THREADS ((TCG_PRODUCER_WARPS + UMMA_ISSUERS + 1) * 32)   // + the TMA warp
+#define TCG_THREADS ((TCG_PRODUCER_WARPS + UMMA_ISSUERS + 1) * 32)   // + the idle warp
 #define TCG_BM 128
 #define TCG_GROUPS 4                                    // producer groups, each fills every 4th stage
 #define TCG_GROUP_WARPS (TCG_PRODUCER_WARPS / TCG_GROUPS)
@@ -49,39 +55,43 @@
 #define TCG_NA (TCG_BM / 8 / TCG_GROUP_WARPS)           // A warp-chunks per producer warp
 #define TCG_NW (TCG_MAX_BN / 8 / TCG_GROUP_WARPS)       // W warp-chunks per producer warp at the widest tile
 
+// Kernel arguments.  "both": read by both kernels; "staging": gemm_tf32x3_kernel only; "packed":
+// gemm_tf32x3_ts_kernel only.
 struct GemmArgs {
-  const float* A;
-  const float* W;
-  const float* wpack;    // pre-split weight pack (tiger_gemm_pack_weight) or NULL: convert W in the kernel
-  int64_t stride_wpack;
-  const float* bias;
-  float* C;
-  const uint8_t* row_zero;
-  const int32_t* count;
-  int64_t lda, ldw, ldc;
-  int64_t stride_a, stride_w, stride_bias, stride_c;
-  int64_t M, rows_per_count;
-  int N, K;
-  float alpha;
-  int relu;
-  int vec_a, vec_w, vec_c;  // 16-byte alignment of the rows of A / W / C
-  int bn, tiles_n, stages;
-  uint32_t tmem_cols;
-  // optional split output (packed variant): columns [0, n_lim0) go to C, columns [n_split, n_split + n_lim1) to C2
+  const float* A;        // both (packed: may be NULL with a gathered A)
+  const float* W;        // staging
+  const float* wpack;    // packed: pre-split weight pack (tiger_gemm_pack_weight)
+  const float* bias;     // both, may be NULL
+  float* C;              // both
+  const uint8_t* row_zero;  // staging: always NULL (see the note in gemm_tf32x3_kernel)
+  const int32_t* count;  // both: device row count (times rows_per_count) or NULL
+  int64_t lda, ldw, ldc; // both (ldw: staging)
+  int64_t stride_a, stride_w, stride_bias, stride_c;  // staging: always 0 (see the note in gemm_tf32x3_kernel)
+  int64_t M, rows_per_count;  // both
+  int N, K;              // both
+  float alpha;           // both
+  int relu;              // both
+  int vec_a, vec_w, vec_c;  // both (vec_w: staging): 16-byte alignment of the rows of A / W / C
+  int bn, tiles_n, stages;  // both
+  uint32_t tmem_cols;    // both
+  // staging: either operand may be read transposed (a template parameter of the kernel) - the dgrad / wgrad
+  // products of the training step use the tensors as stored; the reduction length may live on the device
+  // (k_count * k_rows_per_count); with `accumulate`, blockIdx.y splits K into parts of kblk_per_part stages whose
+  // partial tiles are added into C with atomic adds (gradient accumulation)
+  int accumulate;
+  const int32_t* k_count;
+  int64_t k_rows_per_count;
+  int kblk_per_part;
+  // packed, split output: columns [0, n_lim0) go to C, columns [n_split, n_split + n_lim1) to C2 (C2 may be NULL)
   float* C2;
   int64_t ldc2;
   int n_split, n_lim0, n_lim1, vec_c2;
-  // optional split-K (packed variant): blockIdx.y = part, every part writes its raw partial sums to
-  // C + part * c_part_stride (no bias / alpha / activation); and its counterpart on the input side: A is
-  // the sum of a_parts partial matrices (+ a_bias[k], ReLU) - the consumer of a split-K product applies the
-  // producer's epilogue while it stages its activations, so no reduction kernel runs in between
+  // packed, split-K: blockIdx.y = part; with k_parts > 1 the parts of a tile form a thread-block cluster, exchange
+  // their partial tiles through distributed shared memory, sum them in part order (deterministic) and write the
+  // biased / activated tile once
   int k_parts;
-  int64_t c_part_stride;
-  // cluster_reduce: the k_parts CTAs of a tile form a thread-block cluster; partial tiles are exchanged through
-  // distributed shared memory, summed in part order (deterministic), biased / activated and written once
-  int cluster_reduce;
-  int late_trigger;      // programmatic-launch trigger only after this kernel's own dependency wait
-  // optional fused row scatter (tiger_left_writeback_fused): rows m < sc_rows with sc_mask[m] also go to
+  int late_trigger;      // packed: programmatic-launch trigger only after this kernel's own dependency wait
+  // packed, fused row scatter (tiger_left_writeback_fused): rows m < sc_rows with sc_mask[m] also go to
   // sc_table[sc_ids[m]] (columns of the first output), with the row's clock / activity flag
   const int64_t* sc_ids;
   const uint8_t* sc_mask;
@@ -92,40 +102,20 @@ struct GemmArgs {
   uint8_t* sc_active;
   uint32_t* sc_err;
   int vec_sc;
-  int a_parts, a_relu;
-  int64_t a_part_stride;
-  const float* a_bias;
-  // optional gathered input (packed variant): row m of A is row sel[ids[m]] of a_alt when that is >= 0 (or A is
-  // NULL), else row ids[m] of A, plus row ids[m] of a_add - the representation lookup of the embedding module
-  // (csrc/attention.cu resolve_row) done by the producer warps instead of a gather kernel in front of the GEMM
+  // packed, gathered A: row m of A is row sel[ids[m]] of a_alt when that is >= 0 (or A is NULL), else row ids[m] of
+  // A, plus row ids[m] of a_add - the representation lookup of the embedding module (csrc/attention.cu resolve_row)
+  // done by the producer warps instead of a gather kernel in front of the GEMM
   const int64_t* a_ids;
   const void* a_sel;
   int a_sel_i64;
   const float* a_alt;
   const float* a_add;
-  // general form (tiger_sgemm_ex, unpacked kernel): either operand may be read transposed (element (row, k) at
-  // base[k * ld + row]) - the dgrad / wgrad products of the training step use the tensors as stored; the
-  // reduction length may live on the device (k_count * k_rows_per_count); blockIdx.y splits K into parts of
-  // kblk_per_part stages whose partial tiles are accumulated into C with atomic adds (gradient accumulation)
-  int trans_a, trans_w, accumulate;
-  int mn_a, mn_w;        // the transposed operand is 16-byte aligned: vector loads along its rows + quad transposes
-  const int32_t* k_count;
-  int64_t k_rows_per_count;
-  int kblk_per_part;
 };
 
-struct GemmGather {
-  const int64_t* ids;
-  const void* sel;
-  int sel_is_i64;
-  const float* alt;
-  const float* add;
-};
-
-// MODE_A / MODE_W: how the operand is fetched - 0 row-major [rows, K] (vector loads along K), 1 transposed with
-// scalar loads, 2 transposed and 16-byte aligned (vector loads along the rows + in-quad transposes).  Template
-// parameters, not runtime switches: with all three loaders in one body the kernel spilled 1.5 KB per thread.
-template <bool PACKED, int MODE_A, int MODE_W>
+// MODE_A / MODE_W: how the operand is fetched - 0 row-major [rows, K] (vector loads along K), 1 transposed
+// (element (row, k) at base[k * ld + row], scalar loads).  Template parameters, not runtime switches: loaders
+// selected at run time in one body made the kernel spill heavily.
+template <int MODE_A, int MODE_W>
 __global__ void __launch_bounds__(TCG_THREADS, 1) gemm_tf32x3_kernel(const GemmArgs g) {
   extern __shared__ __align__(128) unsigned char tcg_smem[];
   const int BN = g.bn, S = g.stages;
@@ -148,6 +138,10 @@ __global__ void __launch_bounds__(TCG_THREADS, 1) gemm_tf32x3_kernel(const GemmA
   // one (immediately exiting) CTA per capacity tile - at the seq restarter's capacity that was 29k CTAs = 57 us
   const int64_t n_tiles_total = ((g.M + TCG_BM - 1) / TCG_BM) * g.tiles_n;
   if ((int64_t)(blockIdx.x / g.tiles_n) * TCG_BM >= M) return;
+  // Note: row_zero and the four strides are never set; every launch leaves them NULL / 0.  They stay because without
+  // them ptxas allocates this kernel's registers differently: the transposed-W instantiations spill 20-44 more bytes
+  // and the training step measured 0.5-0.7 % slower on a B200 (1000 W power limit).  Drop them together with a change
+  // that retunes the producers, and measure it.
   const int b = g.kblk_per_part > 0 ? 0 : blockIdx.y;
   int K_eff = g.K;
   if (g.k_count != nullptr) {
@@ -169,7 +163,7 @@ __global__ void __launch_bounds__(TCG_THREADS, 1) gemm_tf32x3_kernel(const GemmA
     if (tid == TCG_PRODUCER_WARPS * 32) {
       for (int s = 0; s < S; ++s) {
         if (again) { mbar_inval(full + s); mbar_inval(empty + s); }
-        mbar_init(full + s, TCG_GROUP_WARPS + (PACKED ? 1 : 0));
+        mbar_init(full + s, TCG_GROUP_WARPS);
         mbar_init(empty + s, UMMA_ISSUERS);
       }
       if (again) mbar_inval(done);
@@ -211,9 +205,8 @@ __global__ void __launch_bounds__(TCG_THREADS, 1) gemm_tf32x3_kernel(const GemmA
     // group `grp` fills stages grp, grp + GROUPS, ...: while one group waits for its loads the others
     // convert / publish theirs, so GROUPS stages worth of global loads are always in flight
     const int grp = warp / TCG_GROUP_WARPS, wg = warp % TCG_GROUP_WARPS;
-    constexpr int NW = PACKED ? 1 : TCG_NW;   // the packed variant moves no W chunks (placeholder of 1, never owned)
     UmmaChunks<TCG_NA> ca;
-    UmmaChunks<NW> cw;
+    UmmaChunks<TCG_NW> cw;
     {
       int row, kc;
       umma_chunk_pos(wg, lane, row, kc);          // chunk 0 = warp-chunk wg; chunk i = warp-chunk wg + 4 i
@@ -226,49 +219,39 @@ __global__ void __launch_bounds__(TCG_THREADS, 1) gemm_tf32x3_kernel(const GemmA
       if constexpr (MODE_A == 0) {
         ca.ptr0 = A + (m0 + row) * g.lda + kc * 4;
         ca.step = 32 * g.lda;
-      } else if constexpr (MODE_A == 1) {
-        ca.ptr0 = A + (int64_t)(kc * 4) * g.lda + m0 + row;
-        ca.step = 32;
       } else {
-        ca.ptr0 = A + (int64_t)(kc * 4 + (lane & 3)) * g.lda + m0 + (row & ~3);
+        ca.ptr0 = A + (int64_t)(kc * 4) * g.lda + m0 + row;
         ca.step = 32;
       }
       const int rows_w = g.N - n0;
       cw.rows_valid = rows_w < BN ? rows_w : BN;
       const int wchunks = BN >> 3;                // warp-chunks of the W tile
-      cw.n_own = PACKED ? 0 : (wchunks > wg ? (wchunks - wg + TCG_GROUP_WARPS - 1) / TCG_GROUP_WARPS : 0);
+      cw.n_own = wchunks > wg ? (wchunks - wg + TCG_GROUP_WARPS - 1) / TCG_GROUP_WARPS : 0;
       cw.row0 = row;
       cw.kq = kc * 4;
       cw.soff0 = (kc * BN + row) * 4;
       if constexpr (MODE_W == 0) {
         cw.ptr0 = W + (int64_t)(n0 + row) * g.ldw + kc * 4;
         cw.step = 32 * g.ldw;
-      } else if constexpr (MODE_W == 1) {
-        cw.ptr0 = W + (int64_t)(kc * 4) * g.ldw + n0 + row;
-        cw.step = 32;
       } else {
-        cw.ptr0 = W + (int64_t)(kc * 4 + (lane & 3)) * g.ldw + n0 + (row & ~3);
+        cw.ptr0 = W + (int64_t)(kc * 4) * g.ldw + n0 + row;
         cw.step = 32;
       }
     }
     // two register sets per thread: the loads of this group's next two stages are in flight while the
     // current one is converted and published (the proxy fence would otherwise wait for a stage's loads
     // right after they were issued)
-    float4 va0[TCG_NA], vw0[NW], va1[TCG_NA], vw1[NW];
-    auto load = [&](float4 (&va)[TCG_NA], float4 (&vw)[NW], int blk) {
+    float4 va0[TCG_NA], vw0[TCG_NW], va1[TCG_NA], vw1[TCG_NW];
+    auto load = [&](float4 (&va)[TCG_NA], float4 (&vw)[TCG_NW], int blk) {
       if (blk < n_blocks) {
         const int k0 = (kblk0 + blk) * UMMA_BK;
-        if constexpr (MODE_A == 2) umma_chunks_load_tv(va, ca, k0, K_eff, g.lda, lane);
-        else if constexpr (MODE_A == 1) umma_chunks_load_t(va, ca, k0, K_eff, g.lda);
+        if constexpr (MODE_A == 1) umma_chunks_load_t(va, ca, k0, K_eff, g.lda);
         else umma_chunks_load(va, ca, k0, K_eff, g.vec_a != 0);
-        if constexpr (!PACKED) {
-          if constexpr (MODE_W == 2) umma_chunks_load_tv(vw, cw, k0, K_eff, g.ldw, lane);
-          else if constexpr (MODE_W == 1) umma_chunks_load_t(vw, cw, k0, K_eff, g.ldw);
-          else umma_chunks_load(vw, cw, k0, K_eff, g.vec_w != 0);
-        }
+        if constexpr (MODE_W == 1) umma_chunks_load_t(vw, cw, k0, K_eff, g.ldw);
+        else umma_chunks_load(vw, cw, k0, K_eff, g.vec_w != 0);
       }
     };
-    auto publish = [&](const float4 (&va)[TCG_NA], const float4 (&vw)[NW], int blk) {
+    auto publish = [&](const float4 (&va)[TCG_NA], const float4 (&vw)[TCG_NW], int blk) {
       const int s = blk % S;
       float* a_hi = stage0 + (size_t)s * stage_floats;
       float* a_lo = a_hi + a_plane;
@@ -277,7 +260,7 @@ __global__ void __launch_bounds__(TCG_THREADS, 1) gemm_tf32x3_kernel(const GemmA
       mbar_wait(empty + s, ((blk / S) & 1) ^ 1);
       TRACE_MARK();
       umma_chunks_store(a_hi, a_lo, ca, va);
-      if constexpr (!PACKED) umma_chunks_store(w_hi, w_lo, cw, vw);
+      umma_chunks_store(w_hi, w_lo, cw, vw);
       TRACE_MARK();
       fence_proxy_async_smem();
       __syncwarp();
@@ -337,21 +320,7 @@ __global__ void __launch_bounds__(TCG_THREADS, 1) gemm_tf32x3_kernel(const GemmA
           if (nb + j < g.N) dst[j] = v[j];
       }
     }
-  } else if (warp == TCG_PRODUCER_WARPS + UMMA_ISSUERS) {
-    // ---------------- TMA warp: one bulk copy per stage brings both planes of the weight tile ----------------
-    if (lane == 0 && PACKED) {
-      const uint32_t bytes = (uint32_t)UMMA_PACK_STAGE_FLOATS(BN) * 4u;
-      const float* src = g.wpack + b * g.stride_wpack +
-                         (int64_t)(tile % g.tiles_n) * n_blocks * UMMA_PACK_STAGE_FLOATS(BN);
-      for (int blk = 0; blk < n_blocks; ++blk) {
-        const int s = blk % S;
-        mbar_wait(empty + s, ((blk / S) & 1) ^ 1);
-        mbar_arrive_expect_tx(full + s, bytes);
-        tma_bulk_load(stage0 + (size_t)s * stage_floats + 2 * a_plane, src + (int64_t)blk * UMMA_PACK_STAGE_FLOATS(BN),
-                      bytes, full + s);
-      }
-    }
-  } else {
+  } else if (warp < TCG_PRODUCER_WARPS + UMMA_ISSUERS) {
     // ---------------- MMA issuers (one elected thread per role, see umma.cuh) ----------------
     // The whole warp runs the loop so that every operand stays warp-uniform; only the tcgen05 instructions
     // are issued by the elected lane.
@@ -526,37 +495,12 @@ __global__ void __launch_bounds__(TS_THREADS, 1) gemm_tf32x3_ts_kernel(const Gem
     auto load = [&](int blk) {
       const int k0 = (kb0 + blk) * TS_BK;
       ts_load_row(v, rowp, k0, g.K, vec);
-      if (addp != nullptr) {
+      if (g.a_add != nullptr && g.a_ids != nullptr) {
         float4 t[TS_KCH];
         ts_load_row(t, addp, k0, g.K, vec);
 #pragma unroll
         for (int i = 0; i < TS_KCH; ++i) {
           v[i].x += t[i].x; v[i].y += t[i].y; v[i].z += t[i].z; v[i].w += t[i].w;
-        }
-      }
-      if (g.a_parts > 1 || g.a_bias != nullptr || g.a_relu) {
-        // A = act(sum of the partial matrices + bias[k]): the epilogue of the split-K product that made it
-        for (int part = 1; part < g.a_parts; ++part) {
-          float4 t[TS_KCH];
-          ts_load_row(t, rowp + part * g.a_part_stride, k0, g.K, vec);
-#pragma unroll
-          for (int i = 0; i < TS_KCH; ++i) {
-            v[i].x += t[i].x; v[i].y += t[i].y; v[i].z += t[i].z; v[i].w += t[i].w;
-          }
-        }
-#pragma unroll
-        for (int i = 0; i < TS_KCH; ++i) {
-          const float4 bb = g.a_bias != nullptr ? umma_load_chunk(g.a_bias, k0 + 4 * i, g.K, false)
-                                                : make_float4(0.f, 0.f, 0.f, 0.f);
-          v[i].x += bb.x; v[i].y += bb.y; v[i].z += bb.z; v[i].w += bb.w;
-          if (g.a_relu) {
-            v[i].x = fmaxf(v[i].x, 0.f); v[i].y = fmaxf(v[i].y, 0.f);
-            v[i].z = fmaxf(v[i].z, 0.f); v[i].w = fmaxf(v[i].w, 0.f);
-          }
-          if (k0 + 4 * i + 0 >= g.K) v[i].x = 0.f;   // keep the zero padding of the K tail (bias must not leak in)
-          if (k0 + 4 * i + 1 >= g.K) v[i].y = 0.f;
-          if (k0 + 4 * i + 2 >= g.K) v[i].z = 0.f;
-          if (k0 + 4 * i + 3 >= g.K) v[i].w = 0.f;
         }
       }
     };
@@ -592,7 +536,7 @@ __global__ void __launch_bounds__(TS_THREADS, 1) gemm_tf32x3_ts_kernel(const Gem
 #pragma unroll
         for (int e = 0; e < 16; ++e) o[e] += t[e];
       }
-      if (g.cluster_reduce) {
+      if (g.k_parts > 1) {                              // cluster split-K: partial tile to shared memory
         float* dst = stage0 + row * (BN + 4) + c0;       // the weight ring is idle once `done` has fired
 #pragma unroll
         for (int j = 0; j < 16; j += 4)
@@ -601,19 +545,17 @@ __global__ void __launch_bounds__(TS_THREADS, 1) gemm_tf32x3_ts_kernel(const Gem
       }
       const int nb = n0 + c0;
       if (!row_ok || nb >= g.N) continue;
-      if (g.k_parts == 1) {
 #pragma unroll
-        for (int j = 0; j < 16; ++j) {
-          const int n = nb + j;
-          float x = (o[j] + ((bias != nullptr && n < g.N) ? __ldg(bias + n) : 0.f)) * g.alpha;
-          if (g.relu) x = fmaxf(x, 0.f);
-          o[j] = x;
-        }
+      for (int j = 0; j < 16; ++j) {
+        const int n = nb + j;
+        float x = (o[j] + ((bias != nullptr && n < g.N) ? __ldg(bias + n) : 0.f)) * g.alpha;
+        if (g.relu) x = fmaxf(x, 0.f);
+        o[j] = x;
       }
       // destination of this 16-column chunk (n_split is a multiple of 16, so a chunk never straddles it)
       const bool second = g.C2 != nullptr && nb >= g.n_split;
       const int col = second ? nb - g.n_split : nb, lim = second ? g.n_lim1 : g.n_lim0;
-      float* dst = second ? g.C2 + mr * g.ldc2 + col : C + (int64_t)blockIdx.y * g.c_part_stride + mr * g.ldc + col;
+      float* dst = second ? g.C2 + mr * g.ldc2 + col : C + mr * g.ldc + col;
       if ((second ? g.vec_c2 : g.vec_c) && col + 16 <= lim) {
 #pragma unroll
         for (int j = 0; j < 16; j += 4)
@@ -707,7 +649,7 @@ __global__ void __launch_bounds__(TS_THREADS, 1) gemm_tf32x3_ts_kernel(const Gem
   TRACE_MARK();
   if (warp % TCG_GROUP_WARPS == 0 || warp >= TCG_PRODUCER_WARPS) TRACE_DUMP(warp < TCG_PRODUCER_WARPS ? "producer" : "issuer", warp);
 #endif
-  if (g.cluster_reduce) {
+  if (g.k_parts > 1) {
     __syncwarp();
     if (early && warp >= TCG_PRODUCER_WARPS) pdl_wait();   // these warps store results below
     cluster_sync_all();                       // every part's tile sits in its CTA's shared memory
@@ -818,13 +760,10 @@ static int gemm_sms() {
       ok = ok && cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, TCG_SMEM_BUDGET + 256) ==
                      cudaSuccess;
     };
-    set_smem(gemm_tf32x3_kernel<false, 0, 0>);
-    set_smem(gemm_tf32x3_kernel<false, 0, 1>);
-    set_smem(gemm_tf32x3_kernel<false, 0, 2>);
-    set_smem(gemm_tf32x3_kernel<false, 1, 0>);
-    set_smem(gemm_tf32x3_kernel<false, 1, 1>);
-    set_smem(gemm_tf32x3_kernel<false, 2, 0>);
-    set_smem(gemm_tf32x3_kernel<false, 2, 2>);
+    set_smem(gemm_tf32x3_kernel<0, 0>);
+    set_smem(gemm_tf32x3_kernel<0, 1>);
+    set_smem(gemm_tf32x3_kernel<1, 0>);
+    set_smem(gemm_tf32x3_kernel<1, 1>);
     if (!ok ||
         cudaFuncSetAttribute(gemm_tf32x3_ts_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                              TS_MAX_STAGES * UMMA_PACK_STAGE_FLOATS(TS_MAX_BN) * 4 + 256) != cudaSuccess)
@@ -840,127 +779,111 @@ extern "C" int tiger_gemm_pick_bn(int64_t m_rows, int n_cols, int batch) {
   return gemm_pick_bn(m_rows, n_cols, batch, sms, TS_MAX_BN);
 }
 
-static int gemm_launch(const float* A, int64_t lda, int64_t stride_a, const float* W, int64_t ldw, int64_t stride_w,
-                       const float* wpack, int64_t stride_wpack, int bn_pack, const float* bias, int64_t stride_bias,
-                       float* C, int64_t ldc, int64_t stride_c, int batch, int64_t m_rows, const int32_t* count,
-                       int64_t rows_per_count, int n_cols, int k_dim, float alpha, int relu, const uint8_t* row_zero,
-                       void* stream, float* C2 = nullptr, int64_t ldc2 = 0, int n_split = 0, int n_cols1 = 0,
-                       int k_parts = 1, int64_t c_part_stride = 0, int a_parts = 1, int64_t a_part_stride = 0,
-                       const float* a_bias = nullptr, int a_relu = 0, const GemmGather* gather = nullptr,
-                       int cluster_reduce = 0, const tiger_left_writeback_fused* wb = nullptr) {
-  if (m_rows < 0 || batch <= 0 || n_cols <= 0 || k_dim <= 0 || lda < k_dim || ldc < n_cols) return TIGER_EINVAL;
-  if (gather != nullptr && (wpack == nullptr || gather->ids == nullptr || gather->sel == nullptr ||
-                            gather->alt == nullptr || a_parts > 1))
+// A product on the packed kernel: C = act(alpha * (A Wpack^T + bias)) for a pack of ceil(n_cols / bn) column tiles,
+// plus the options the attention chain uses.  The tiger_sgemm_nt_packed* entry points fill it by field name; the
+// fields they leave out are zero / NULL (or the default given here), which turns every option off.
+struct PackedGemm {
+  const float* A;                 // NULL allowed with a gathered A
+  int64_t lda;
+  const float* wpack;
+  int bn;
+  const float* bias;
+  float* C;
+  int64_t ldc;
+  int n_cols;                     // columns written to C
+  int64_t m_rows;
+  const int32_t* count;
+  int64_t rows_per_count = 1;
+  int k_dim;
+  float alpha = 1.0f;
+  int relu;
+  // split output: pack columns [n_split, n_split + n_cols1) go to C2 (n_split a multiple of 16 >= n_cols)
+  float* C2;
+  int64_t ldc2;
+  int n_split, n_cols1;
+  int k_parts = 1;                // > 1: K split over a thread-block cluster of up to 8 CTAs per tile
+  // gathered A (GemmArgs::a_ids): row m is row sel[ids[m]] of alt when that is >= 0, else row ids[m] of A, + add
+  const int64_t* ids;
+  const void* sel;
+  int sel_is_i64;
+  const float* alt;
+  const float* add;
+  const tiger_left_writeback_fused* wb;   // fused row scatter into the left memory
+};
+
+static int gemm_packed_launch(const PackedGemm& p, void* stream) {
+  if (p.wpack == nullptr || p.m_rows < 0 || p.n_cols <= 0 || p.k_dim <= 0 || p.lda < p.k_dim || p.ldc < p.n_cols)
     return TIGER_EINVAL;
-  if (wpack == nullptr && (W == nullptr || ldw < k_dim)) return TIGER_EINVAL;
-  if (C2 != nullptr && (wpack == nullptr || (n_split & 15) != 0 || n_split < n_cols || n_cols1 <= 0 || ldc2 < n_cols1))
+  if (p.C2 != nullptr && ((p.n_split & 15) != 0 || p.n_split < p.n_cols || p.n_cols1 <= 0 || p.ldc2 < p.n_cols1))
     return TIGER_EINVAL;
-  if (k_parts < 1 || a_parts < 1 || ((k_parts > 1 || a_parts > 1 || a_bias != nullptr || a_relu) && wpack == nullptr) ||
-      (k_parts > 1 && !cluster_reduce && (C2 != nullptr || c_part_stride < m_rows * ldc)) ||
-      (a_parts > 1 && a_part_stride < m_rows * lda) || (cluster_reduce && (C2 != nullptr || k_parts > 8)))
-    return TIGER_EINVAL;
-  if (wpack != nullptr && (bn_pack < 16 || bn_pack > TS_MAX_BN || (bn_pack & 15) != 0 || (((uintptr_t)wpack) & 15) != 0 ||
-                           batch != 1))
-    return TIGER_EINVAL;
-  if (m_rows == 0) return TIGER_OK;
+  if (p.k_parts < 1 || p.k_parts > 8 || (p.k_parts > 1 && p.C2 != nullptr)) return TIGER_EINVAL;
+  if (p.bn < 16 || p.bn > TS_MAX_BN || (p.bn & 15) != 0 || (((uintptr_t)p.wpack) & 15) != 0) return TIGER_EINVAL;
+  if (p.m_rows == 0) return TIGER_OK;
   const int sms = gemm_sms();
   if (sms < 0) return TIGER_ECUDA;
-  GemmArgs g;
-  g.A = A; g.W = W; g.wpack = wpack; g.stride_wpack = stride_wpack;
-  g.bias = bias; g.C = C; g.row_zero = row_zero; g.count = count;
-  g.lda = lda; g.ldw = ldw; g.ldc = ldc;
-  g.stride_a = stride_a; g.stride_w = stride_w; g.stride_bias = stride_bias; g.stride_c = stride_c;
-  g.M = m_rows; g.rows_per_count = rows_per_count > 0 ? rows_per_count : 1;
-  g.N = C2 != nullptr ? n_split + n_cols1 : n_cols;   // columns of the (padded) weight / bias space
-  g.K = k_dim; g.alpha = alpha; g.relu = relu;
-  g.C2 = C2; g.ldc2 = ldc2; g.n_split = n_split; g.n_lim0 = n_cols; g.n_lim1 = n_cols1;
-  g.vec_c2 = (C2 != nullptr && (((uintptr_t)C2) & 15) == 0 && (ldc2 & 3) == 0) ? 1 : 0;
-  const int k_blocks = (k_dim + TS_BK - 1) / TS_BK;
-  g.k_parts = k_parts < k_blocks ? k_parts : k_blocks;              // every part owns at least one k-block
+  GemmArgs g{};
+  g.A = p.A; g.wpack = p.wpack; g.bias = p.bias; g.C = p.C; g.count = p.count;
+  g.lda = p.lda; g.ldc = p.ldc;
+  g.M = p.m_rows; g.rows_per_count = p.rows_per_count > 0 ? p.rows_per_count : 1;
+  g.N = p.C2 != nullptr ? p.n_split + p.n_cols1 : p.n_cols;   // columns of the (padded) weight / bias space
+  g.K = p.k_dim; g.alpha = p.alpha; g.relu = p.relu;
+  g.C2 = p.C2; g.ldc2 = p.ldc2; g.n_split = p.n_split; g.n_lim0 = p.n_cols; g.n_lim1 = p.n_cols1;
+  g.vec_c2 = (p.C2 != nullptr && (((uintptr_t)p.C2) & 15) == 0 && (p.ldc2 & 3) == 0) ? 1 : 0;
+  const int k_blocks = (p.k_dim + TS_BK - 1) / TS_BK;
+  g.k_parts = p.k_parts < k_blocks ? p.k_parts : k_blocks;              // every part owns at least one k-block
   g.k_parts = (k_blocks + ((k_blocks + g.k_parts - 1) / g.k_parts) - 1) / ((k_blocks + g.k_parts - 1) / g.k_parts);
-  g.c_part_stride = cluster_reduce ? 0 : c_part_stride;
-  g.cluster_reduce = (cluster_reduce && g.k_parts > 1) ? 1 : 0;
-  g.late_trigger = gather != nullptr ? 1 : 0;
-  g.sc_table = nullptr; g.sc_ids = nullptr; g.sc_mask = nullptr; g.sc_rows = 0; g.sc_period = 1; g.sc_ld = 0;
-  g.sc_ts = nullptr; g.sc_ts_table = nullptr; g.sc_active = nullptr; g.sc_err = nullptr; g.vec_sc = 0;
-  if (wb != nullptr) {
-    if (wpack == nullptr || k_parts != 1 || wb->pos_ids == nullptr || wb->winner == nullptr || wb->ts == nullptr ||
-        wb->left_vals == nullptr || wb->left_ts == nullptr || wb->n_pos < 0 || wb->n_pos > m_rows || wb->batch <= 0)
+  g.late_trigger = p.ids != nullptr ? 1 : 0;
+  if (p.wb != nullptr) {
+    const tiger_left_writeback_fused* wb = p.wb;
+    if (p.k_parts != 1 || wb->pos_ids == nullptr || wb->winner == nullptr || wb->ts == nullptr ||
+        wb->left_vals == nullptr || wb->left_ts == nullptr || wb->n_pos < 0 || wb->n_pos > p.m_rows || wb->batch <= 0)
       return TIGER_EINVAL;
     g.sc_table = wb->left_vals; g.sc_ids = wb->pos_ids; g.sc_mask = wb->winner; g.sc_rows = wb->n_pos;
-    g.sc_period = wb->batch; g.sc_ld = ldc; g.sc_ts = wb->ts; g.sc_ts_table = wb->left_ts;
+    g.sc_period = wb->batch; g.sc_ld = p.ldc; g.sc_ts = wb->ts; g.sc_ts_table = wb->left_ts;
     g.sc_active = wb->left_active; g.sc_err = wb->err_flags;
-    g.vec_sc = ((((uintptr_t)wb->left_vals) & 15) == 0 && (ldc & 3) == 0) ? 1 : 0;
+    g.vec_sc = ((((uintptr_t)wb->left_vals) & 15) == 0 && (p.ldc & 3) == 0) ? 1 : 0;
   }
-  g.a_parts = a_parts; g.a_part_stride = a_part_stride; g.a_bias = a_bias; g.a_relu = a_relu;
-  g.trans_a = 0; g.trans_w = 0; g.accumulate = 0; g.k_count = nullptr; g.k_rows_per_count = 1; g.kblk_per_part = 0;
-  g.mn_a = 0; g.mn_w = 0;
-  g.a_ids = nullptr; g.a_sel = nullptr; g.a_sel_i64 = 0; g.a_alt = nullptr; g.a_add = nullptr;
-  if (gather != nullptr) {
-    g.a_ids = gather->ids; g.a_sel = gather->sel; g.a_sel_i64 = gather->sel_is_i64;
-    g.a_alt = gather->alt; g.a_add = gather->add;
-  }
-  n_cols = g.N;
-  const bool multi = batch > 1;
-  g.vec_a = ((((uintptr_t)A) & 15) == 0 && (lda & 3) == 0 && (!multi || (stride_a & 3) == 0) &&
-             (a_parts == 1 || (a_part_stride & 3) == 0) &&
-             (gather == nullptr || ((((uintptr_t)gather->alt) | ((uintptr_t)gather->add)) & 15) == 0)) ? 1 : 0;
-  g.vec_w = (wpack == nullptr && (((uintptr_t)W) & 15) == 0 && (ldw & 3) == 0 && (!multi || (stride_w & 3) == 0)) ? 1 : 0;
-  g.vec_c = ((((uintptr_t)C) & 15) == 0 && (ldc & 3) == 0 && (!multi || (stride_c & 3) == 0)) ? 1 : 0;
-  const int64_t tiles_m = (m_rows + TCG_BM - 1) / TCG_BM;
-  g.bn = wpack != nullptr ? bn_pack : gemm_pick_bn(m_rows, n_cols, batch, sms, TCG_MAX_BN);
-  g.tiles_n = (n_cols + g.bn - 1) / g.bn;
-  if (wpack != nullptr) {
-    // activations in tensor memory: 4 accumulators + a ring of 32-column stages must fit 512 columns
-    int stages = (512 - UMMA_ACCS * g.bn) / (2 * TS_BK);
-    stages = stages > TS_MAX_STAGES ? TS_MAX_STAGES : stages;
-    g.stages = stages;
-    g.tmem_cols = tmem_cols_pow2((uint32_t)(UMMA_ACCS * g.bn + stages * 2 * TS_BK));
-    const size_t smem = (size_t)stages * UMMA_PACK_STAGE_FLOATS(g.bn) * 4 + 256;
-    dim3 grid((unsigned)(tiles_m * g.tiles_n), (unsigned)g.k_parts);
-    if (g.cluster_reduce && (size_t)TCG_BM * (g.bn + 4) * 4 > (size_t)stages * UMMA_PACK_STAGE_FLOATS(g.bn) * 4)
-      return TIGER_EINVAL;
-    return tiger_launch_chain(gemm_tf32x3_ts_kernel, grid, dim3(TS_THREADS), smem, as_stream(stream),
-                              dim3(1, g.cluster_reduce ? (unsigned)g.k_parts : 1u, 1), g);
-  }
-  g.tmem_cols = tmem_cols_pow2((uint32_t)(UMMA_ACCS * g.bn));
-  const size_t stage_bytes = (size_t)(2 * UMMA_KCH * TCG_BM * 4 + 2 * UMMA_KCH * g.bn * 4) * sizeof(float);
-  int stages = (int)(TCG_SMEM_BUDGET / stage_bytes);
-  stages = stages > TCG_MAX_STAGES ? TCG_MAX_STAGES : stages;
-  if (stages < 2) return TIGER_EINVAL;
+  g.a_ids = p.ids; g.a_sel = p.sel; g.a_sel_i64 = p.sel_is_i64; g.a_alt = p.alt; g.a_add = p.add;
+  g.vec_a = ((((uintptr_t)p.A) & 15) == 0 && (p.lda & 3) == 0 && ((((uintptr_t)p.alt) | ((uintptr_t)p.add)) & 15) == 0)
+                ? 1 : 0;
+  g.vec_c = ((((uintptr_t)p.C) & 15) == 0 && (p.ldc & 3) == 0) ? 1 : 0;
+  const int64_t tiles_m = (p.m_rows + TCG_BM - 1) / TCG_BM;
+  g.bn = p.bn;
+  g.tiles_n = (g.N + g.bn - 1) / g.bn;
+  // activations in tensor memory: 4 accumulators + a ring of 32-column stages must fit 512 columns
+  int stages = (512 - UMMA_ACCS * g.bn) / (2 * TS_BK);
+  stages = stages > TS_MAX_STAGES ? TS_MAX_STAGES : stages;
   g.stages = stages;
-  const size_t smem = stages * stage_bytes + 256;
-  const int64_t tiles = tiles_m * g.tiles_n;
-  dim3 grid((unsigned)(tiles < sms ? tiles : sms), (unsigned)batch);      // persistent over tiles
-  gemm_tf32x3_kernel<false, 0, 0><<<grid, TCG_THREADS, smem, as_stream(stream)>>>(g);
-  return tiger_launch_status();
-}
-
-extern "C" int tiger_sgemm_nt_batched(const float* A, int64_t lda, int64_t stride_a, const float* W, int64_t ldw,
-                                      int64_t stride_w, const float* bias, int64_t stride_bias, float* C,
-                                      int64_t ldc, int64_t stride_c, int batch, int64_t m_rows,
-                                      const int32_t* count, int64_t rows_per_count, int n_cols, int k_dim,
-                                      float alpha, int relu, const uint8_t* row_zero, void* stream) {
-  return gemm_launch(A, lda, stride_a, W, ldw, stride_w, nullptr, 0, 0, bias, stride_bias, C, ldc, stride_c, batch,
-                     m_rows, count, rows_per_count, n_cols, k_dim, alpha, relu, row_zero, stream);
+  g.tmem_cols = tmem_cols_pow2((uint32_t)(UMMA_ACCS * g.bn + stages * 2 * TS_BK));
+  const size_t smem = (size_t)stages * UMMA_PACK_STAGE_FLOATS(g.bn) * 4 + 256;
+  dim3 grid((unsigned)(tiles_m * g.tiles_n), (unsigned)g.k_parts);
+  // the cluster reduction reuses the weight ring for the partial tile
+  if (g.k_parts > 1 && (size_t)TCG_BM * (g.bn + 4) * 4 > (size_t)stages * UMMA_PACK_STAGE_FLOATS(g.bn) * 4)
+    return TIGER_EINVAL;
+  return tiger_launch_chain(gemm_tf32x3_ts_kernel, grid, dim3(TS_THREADS), smem, as_stream(stream),
+                            dim3(1, (unsigned)g.k_parts, 1), g);
 }
 
 extern "C" int tiger_sgemm_nt_packed(const float* A, int64_t lda, const float* wpack, int bn, const float* bias,
                                      float* C, int64_t ldc, int64_t m_rows, const int32_t* count,
                                      int64_t rows_per_count, int n_cols, int k_dim, float alpha, int relu,
                                      void* stream) {
-  if (wpack == nullptr) return TIGER_EINVAL;
-  return gemm_launch(A, lda, 0, nullptr, 0, 0, wpack, 0, bn, bias, 0, C, ldc, 0, 1, m_rows, count, rows_per_count,
-                     n_cols, k_dim, alpha, relu, nullptr, stream);
+  return gemm_packed_launch({.A = A, .lda = lda, .wpack = wpack, .bn = bn, .bias = bias, .C = C, .ldc = ldc,
+                             .n_cols = n_cols, .m_rows = m_rows, .count = count, .rows_per_count = rows_per_count,
+                             .k_dim = k_dim, .alpha = alpha, .relu = relu},
+                            stream);
 }
 
 extern "C" int tiger_sgemm_nt_packed_split(const float* A, int64_t lda, const float* wpack, int bn, const float* bias,
                                            float* C, int64_t ldc, int n_cols0, float* C2, int64_t ldc2, int n_split,
                                            int n_cols1, int64_t m_rows, const int32_t* count,
                                            int64_t rows_per_count, int k_dim, float alpha, int relu, void* stream) {
-  if (wpack == nullptr || C2 == nullptr) return TIGER_EINVAL;
-  return gemm_launch(A, lda, 0, nullptr, 0, 0, wpack, 0, bn, bias, 0, C, ldc, 0, 1, m_rows, count, rows_per_count,
-                     n_cols0, k_dim, alpha, relu, nullptr, stream, C2, ldc2, n_split, n_cols1);
+  if (C2 == nullptr) return TIGER_EINVAL;
+  return gemm_packed_launch({.A = A, .lda = lda, .wpack = wpack, .bn = bn, .bias = bias, .C = C, .ldc = ldc,
+                             .n_cols = n_cols0, .m_rows = m_rows, .count = count, .rows_per_count = rows_per_count,
+                             .k_dim = k_dim, .alpha = alpha, .relu = relu, .C2 = C2, .ldc2 = ldc2, .n_split = n_split,
+                             .n_cols1 = n_cols1},
+                            stream);
 }
 
 extern "C" int tiger_sgemm_nt_packed_scatter(const float* A, int64_t lda, const float* wpack, int bn, const float* bias,
@@ -971,49 +894,22 @@ extern "C" int tiger_sgemm_nt_packed_scatter(const float* A, int64_t lda, const 
   if (wb->ready_event != nullptr &&
       cudaStreamWaitEvent(as_stream(stream), reinterpret_cast<cudaEvent_t>(wb->ready_event), 0) != cudaSuccess)
     return TIGER_ECUDA;
-  return gemm_launch(A, lda, 0, nullptr, 0, 0, wpack, 0, bn, bias, 0, C, ldc, 0, 1, m_rows, nullptr, 1, n_cols0, k_dim, 1.0f,
-                     0, nullptr, stream, C2, ldc2, C2 != nullptr ? n_split : 0, C2 != nullptr ? n_cols1 : 0, 1, 0, 1, 0,
-                     nullptr, 0, nullptr, 0, wb);
-}
-
-// number of partial products tiger_sgemm_nt_packed_splitk will actually write for this K (<= k_parts)
-extern "C" int tiger_gemm_splitk_parts(int k_dim, int k_parts) {
-  if (k_dim <= 0 || k_parts < 1) return TIGER_EINVAL;
-  const int k_blocks = (k_dim + TS_BK - 1) / TS_BK;
-  int p = k_parts < k_blocks ? k_parts : k_blocks;
-  const int per = (k_blocks + p - 1) / p;
-  return (k_blocks + per - 1) / per;
-}
-
-extern "C" int tiger_sgemm_nt_packed_splitk(const float* A, int64_t lda, const float* wpack, int bn, float* C_parts,
-                                            int64_t ldc, int64_t part_stride, int k_parts, int64_t m_rows,
-                                            const int32_t* count, int64_t rows_per_count, int n_cols, int k_dim,
-                                            void* stream) {
-  if (wpack == nullptr || C_parts == nullptr) return TIGER_EINVAL;
-  return gemm_launch(A, lda, 0, nullptr, 0, 0, wpack, 0, bn, nullptr, 0, C_parts, ldc, 0, 1, m_rows, count,
-                     rows_per_count, n_cols, k_dim, 1.0f, 0, nullptr, stream, nullptr, 0, 0, 0, k_parts, part_stride);
+  return gemm_packed_launch({.A = A, .lda = lda, .wpack = wpack, .bn = bn, .bias = bias, .C = C, .ldc = ldc,
+                             .n_cols = n_cols0, .m_rows = m_rows, .k_dim = k_dim, .C2 = C2,
+                             .ldc2 = ldc2, .n_split = C2 != nullptr ? n_split : 0,
+                             .n_cols1 = C2 != nullptr ? n_cols1 : 0, .wb = wb},
+                            stream);
 }
 
 extern "C" int tiger_sgemm_nt_packed_splitk_fused(const float* A, int64_t lda, const float* wpack, int bn,
                                                   const float* bias, float* C, int64_t ldc, int k_parts,
                                                   int64_t m_rows, const int32_t* count, int64_t rows_per_count,
                                                   int n_cols, int k_dim, float alpha, int relu, void* stream) {
-  if (wpack == nullptr || C == nullptr || k_parts < 1 || k_parts > 8) return TIGER_EINVAL;
-  return gemm_launch(A, lda, 0, nullptr, 0, 0, wpack, 0, bn, bias, 0, C, ldc, 0, 1, m_rows, count, rows_per_count,
-                     n_cols, k_dim, alpha, relu, nullptr, stream, nullptr, 0, 0, 0, k_parts, 0, 1, 0, nullptr, 0,
-                     nullptr, 1);
-}
-
-extern "C" int tiger_sgemm_nt_packed_sum(const float* A_parts, int64_t lda, int64_t a_part_stride, int a_parts,
-                                         const float* a_bias, int a_relu, const float* wpack, int bn,
-                                         const float* bias, float* C, int64_t ldc, int n_cols0, float* C2,
-                                         int64_t ldc2, int n_split, int n_cols1, int64_t m_rows,
-                                         const int32_t* count, int64_t rows_per_count, int k_dim, float alpha,
-                                         int relu, void* stream) {
-  if (wpack == nullptr || A_parts == nullptr) return TIGER_EINVAL;
-  return gemm_launch(A_parts, lda, 0, nullptr, 0, 0, wpack, 0, bn, bias, 0, C, ldc, 0, 1, m_rows, count, rows_per_count,
-                     n_cols0, k_dim, alpha, relu, nullptr, stream, C2, ldc2, n_split, n_cols1, 1, 0, a_parts,
-                     a_part_stride, a_bias, a_relu);
+  if (C == nullptr) return TIGER_EINVAL;
+  return gemm_packed_launch({.A = A, .lda = lda, .wpack = wpack, .bn = bn, .bias = bias, .C = C, .ldc = ldc,
+                             .n_cols = n_cols, .m_rows = m_rows, .count = count, .rows_per_count = rows_per_count,
+                             .k_dim = k_dim, .alpha = alpha, .relu = relu, .k_parts = k_parts},
+                            stream);
 }
 
 extern "C" int tiger_sgemm_nt_packed_gather(const int64_t* ids, const void* sel, int sel_is_i64, const float* rows_a,
@@ -1021,21 +917,15 @@ extern "C" int tiger_sgemm_nt_packed_gather(const int64_t* ids, const void* sel,
                                             const float* wpack, int bn, const float* bias, float* C, int64_t ldc,
                                             int64_t m_rows, const int32_t* count, int64_t rows_per_count,
                                             int n_cols, int k_dim, float alpha, int relu, void* stream) {
-  if (wpack == nullptr) return TIGER_EINVAL;
-  const GemmGather gg = {ids, sel, sel_is_i64, rows_b, add_rows};
-  return gemm_launch(rows_a, ld_rows, 0, nullptr, 0, 0, wpack, 0, bn, bias, 0, C, ldc, 0, 1, m_rows, count,
-                     rows_per_count, n_cols, k_dim, alpha, relu, nullptr, stream, nullptr, 0, 0, 0, 1, 0, 1, 0, nullptr,
-                     0, &gg);
+  if (ids == nullptr || sel == nullptr || rows_b == nullptr) return TIGER_EINVAL;
+  return gemm_packed_launch({.A = rows_a, .lda = ld_rows, .wpack = wpack, .bn = bn, .bias = bias, .C = C, .ldc = ldc,
+                             .n_cols = n_cols, .m_rows = m_rows, .count = count, .rows_per_count = rows_per_count,
+                             .k_dim = k_dim, .alpha = alpha, .relu = relu, .ids = ids, .sel = sel,
+                             .sel_is_i64 = sel_is_i64, .alt = rows_b, .add = add_rows},
+                            stream);
 }
 
-extern "C" int tiger_sgemm_nt(const float* A, int64_t lda, const float* W, int64_t ldw, const float* bias,
-                              float* C, int64_t ldc, int64_t m_rows, const int32_t* count, int64_t rows_per_count,
-                              int n_cols, int k_dim, int relu, void* stream) {
-  return tiger_sgemm_nt_batched(A, lda, 0, W, ldw, 0, bias, 0, C, ldc, 0, 1, m_rows, count, rows_per_count, n_cols,
-                                k_dim, 1.0f, relu, nullptr, stream);
-}
-
-// General product on the unpacked tensor-core kernel:
+// General product on the staging kernel:
 //   C[m, n] (+)= act(alpha * (sum_k opA[m, k] * opW[n, k] + bias[n]))
 // opA[m, k] = A[m * lda + k] (trans_a = 0) or A[k * lda + m] (trans_a = 1), opW likewise.  With the three
 // combinations the training step needs no transposed copies: forward y = x W^T (0, 0), input gradient
@@ -1055,24 +945,16 @@ extern "C" int tiger_sgemm_ex(const float* A, int64_t lda, int trans_a, const fl
   if (m_rows == 0) return TIGER_OK;
   const int sms = gemm_sms();
   if (sms < 0) return TIGER_ECUDA;
-  GemmArgs g;
-  memset(&g, 0, sizeof(g));
+  GemmArgs g{};
   g.A = A; g.W = W; g.bias = bias; g.C = C; g.count = m_count; g.k_count = k_count;
   g.lda = lda; g.ldw = ldw; g.ldc = ldc;
   g.M = m_rows; g.rows_per_count = rows_per_count > 0 ? rows_per_count : 1;
   g.k_rows_per_count = g.rows_per_count;
   g.N = n_cols; g.K = (int)k_dim; g.alpha = alpha; g.relu = relu;
-  g.trans_a = trans_a ? 1 : 0; g.trans_w = trans_w ? 1 : 0; g.accumulate = accumulate ? 1 : 0;
-  g.k_parts = 1; g.a_parts = 1; g.sc_period = 1;
+  g.accumulate = accumulate ? 1 : 0;
   g.vec_a = (!trans_a && (((uintptr_t)A) & 15) == 0 && (lda & 3) == 0) ? 1 : 0;
   g.vec_w = (!trans_w && (((uintptr_t)W) & 15) == 0 && (ldw & 3) == 0) ? 1 : 0;
   g.vec_c = ((((uintptr_t)C) & 15) == 0 && (ldc & 3) == 0) ? 1 : 0;
-  // vector loads along the rows + in-quad transposes (mode 2) measured SLOWER than the scalar transposed loader
-  // (mode 1) on B200 (ncu, weight gradient 344 x 516 x 6000: 185 us vs 93 us - the producers are instruction-bound and
-  // the 4 shuffles + selects per chunk cost more than the 3 extra load instructions), so it is opt-in (TIGER_TV=1)
-  const bool tv = getenv("TIGER_TV") != nullptr;
-  g.mn_a = (tv && trans_a && (((uintptr_t)A) & 15) == 0 && (lda & 3) == 0) ? 1 : 0;
-  g.mn_w = (tv && trans_w && (((uintptr_t)W) & 15) == 0 && (ldw & 3) == 0) ? 1 : 0;
   const int64_t tiles_m = (m_rows + TCG_BM - 1) / TCG_BM;
   g.bn = gemm_pick_bn(m_rows, n_cols, accumulate ? k_parts : 1, sms, TCG_MAX_BN);
   g.tiles_n = (n_cols + g.bn - 1) / g.bn;
@@ -1091,22 +973,15 @@ extern "C" int tiger_sgemm_ex(const float* A, int64_t lda, int trans_a, const fl
   // capacity-sized launch exit at once, the live ones must not queue behind each other
   dim3 grid((unsigned)(tiles < sms ? tiles : sms), (unsigned)parts);
   const size_t smem = stages * stage_bytes + 256;
-  cudaStream_t st = as_stream(stream);
-  // an operand pair mixes the scalar and the vector transposed loader only if exactly one of them is misaligned:
-  // then both take the scalar one (fewer instantiations of a large kernel)
-  int ma = trans_a ? (g.mn_a ? 2 : 1) : 0, mw = trans_w ? (g.mn_w ? 2 : 1) : 0;
-  if (ma == 2 && mw == 1) ma = 1;
-  if (ma == 1 && mw == 2) mw = 1;
-  const int mode = ma * 3 + mw;
-  switch (mode) {
-    case 0: gemm_tf32x3_kernel<false, 0, 0><<<grid, TCG_THREADS, smem, st>>>(g); break;
-    case 1: gemm_tf32x3_kernel<false, 0, 1><<<grid, TCG_THREADS, smem, st>>>(g); break;
-    case 2: gemm_tf32x3_kernel<false, 0, 2><<<grid, TCG_THREADS, smem, st>>>(g); break;
-    case 3: gemm_tf32x3_kernel<false, 1, 0><<<grid, TCG_THREADS, smem, st>>>(g); break;
-    case 4: gemm_tf32x3_kernel<false, 1, 1><<<grid, TCG_THREADS, smem, st>>>(g); break;
-    case 6: gemm_tf32x3_kernel<false, 2, 0><<<grid, TCG_THREADS, smem, st>>>(g); break;
-    case 8: gemm_tf32x3_kernel<false, 2, 2><<<grid, TCG_THREADS, smem, st>>>(g); break;
-    default: return TIGER_EINVAL;
-  }
+  void (*kernel)(GemmArgs) = trans_a ? (trans_w ? gemm_tf32x3_kernel<1, 1> : gemm_tf32x3_kernel<1, 0>)
+                                     : (trans_w ? gemm_tf32x3_kernel<0, 1> : gemm_tf32x3_kernel<0, 0>);
+  kernel<<<grid, TCG_THREADS, smem, as_stream(stream)>>>(g);
   return tiger_launch_status();
+}
+
+extern "C" int tiger_sgemm_nt(const float* A, int64_t lda, const float* W, int64_t ldw, const float* bias,
+                              float* C, int64_t ldc, int64_t m_rows, const int32_t* count, int64_t rows_per_count,
+                              int n_cols, int k_dim, int relu, void* stream) {
+  return tiger_sgemm_ex(A, lda, 0, W, ldw, 0, bias, C, ldc, m_rows, n_cols, k_dim, count, nullptr, rows_per_count, 1.0f,
+                        relu, 0, 1, stream);
 }

@@ -4,8 +4,8 @@
 //   tiger_anonymized_reindex                                                   (select.cu)
 //   tiger_seq_tokens      event tokens [src | dst | anony | edge | time], key-padding mask, prev_ts
 //   tiger_sgemm_nt        packed q,k in-projection of all tokens               (gemm.cu)
-//   tiger_seq_attn_pool   per (node, head): L x L scores, masked softmax, position-mean of the
-//                         attention weights, pooled tokens xbar_h = sum_i pbar_hi x_i
+//   tiger_train_seq_pool  per (node, head): L x L scores, masked softmax, position-mean of the
+//                         attention weights, pooled tokens xbar_h = sum_i pbar_hi x_i  (train_seq.cu, dropout 0)
 //   tiger_sgemm_nt x5     value projection of the pooled tokens (per head), out-proj (+ReLU), out_fn,
 //                         merger fc1 (+ReLU, first d input columns only), merger fc2
 // Folding (exact by linearity, because the reference takes the MEAN over positions of the MHA output
@@ -106,120 +106,6 @@ extern "C" int tiger_seq_tokens(const int64_t* nids, const int32_t* count, int64
   seq_tokens_kernel<<<(unsigned)grid, 256, 0, as_stream(stream)>>>(nids, count, n, len, hist_nids, hist_eids,
                                                                   hist_ts, hist_dirs, anony_ids, nfeats, efeats, d,
                                                                   de, anony_emb, time_w, time_b, x, mask, prev_ts);
-  return tiger_launch_status();
-}
-
-// ------------------------------------------------------------------------------------------
-// per (node, head): scores -> masked softmax -> mean over query positions -> pooled tokens
-// ------------------------------------------------------------------------------------------
-#define POOL_THREADS 256
-#define POOL_CW 32       // head-dim chunk staged in shared memory
-#define POOL_MAXL 64     // hist_len limit (default 40)
-#define POOL_MAXP ((POOL_MAXL * POOL_MAXL + POOL_THREADS - 1) / POOL_THREADS)
-
-__global__ void __launch_bounds__(POOL_THREADS)
-seq_attn_pool_kernel(const float* __restrict__ qk, int64_t ld_qk, const float* __restrict__ x,
-                     const uint8_t* __restrict__ mask, const int32_t* __restrict__ count, int64_t n, int len,
-                     int dm, int n_head, float* __restrict__ xbar) {
-  __shared__ float qs[POOL_MAXL][POOL_CW + 1];
-  __shared__ float ks[POOL_MAXL][POOL_CW + 1];
-  __shared__ float sc[POOL_MAXL][POOL_MAXL + 1];
-  __shared__ float pbar[POOL_MAXL];
-  int64_t total = n;
-  if (count != nullptr) {
-    const int64_t c = *count;
-    total = c < n ? c : n;
-  }
-  total *= n_head;
-  const int tid = threadIdx.x, lane = lane_id(), warp = warp_id_in_block();
-  const int hd = dm / n_head;
-  const float scale = sqrtf(1.0f / (float)hd);
-  const int n_pairs = len * len;
-  for (int64_t item = blockIdx.x; item < total; item += gridDim.x) {
-    const int64_t i = item / n_head;
-    const int h = (int)(item % n_head);
-    const float* qbase = qk + i * len * ld_qk + h * hd;
-    const float* kbase = qbase + dm;
-    float acc[POOL_MAXP];
-#pragma unroll
-    for (int r = 0; r < POOL_MAXP; ++r) acc[r] = 0.f;
-    for (int c0 = 0; c0 < hd; c0 += POOL_CW) {
-      const int cw = (hd - c0) < POOL_CW ? (hd - c0) : POOL_CW;
-      __syncthreads();
-      for (int e = tid; e < len * POOL_CW; e += POOL_THREADS) {
-        const int j = e / POOL_CW, c = e % POOL_CW;
-        float qv = 0.f, kv = 0.f;
-        if (c < cw) {
-          qv = qbase[(int64_t)j * ld_qk + c0 + c] * scale;   // torch scales q before q.k^T
-          kv = kbase[(int64_t)j * ld_qk + c0 + c];
-        }
-        qs[j][c] = qv;
-        ks[j][c] = kv;
-      }
-      __syncthreads();
-#pragma unroll
-      for (int r = 0; r < POOL_MAXP; ++r) {
-        const int p = tid + r * POOL_THREADS;
-        if (p < n_pairs) {
-          const int j = p / len, i2 = p % len;
-          float s = acc[r];
-#pragma unroll 8
-          for (int c = 0; c < POOL_CW; ++c) s = fmaf(qs[j][c], ks[i2][c], s);
-          acc[r] = s;
-        }
-      }
-    }
-    const uint8_t* mrow = mask + i * len;
-#pragma unroll
-    for (int r = 0; r < POOL_MAXP; ++r) {
-      const int p = tid + r * POOL_THREADS;
-      if (p < n_pairs) {
-        const int j = p / len, i2 = p % len;
-        sc[j][i2] = mrow[i2] ? -INFINITY : acc[r];
-      }
-    }
-    __syncthreads();
-    for (int j = warp; j < len; j += POOL_THREADS / 32) {       // softmax over keys, one warp per query row
-      float m = -INFINITY;
-      for (int c = lane; c < len; c += 32) m = fmaxf(m, sc[j][c]);
-      m = warp_max(m);
-      float sum = 0.f;
-      for (int c = lane; c < len; c += 32) {
-        const float e = expf(sc[j][c] - m);
-        sc[j][c] = e;
-        sum += e;
-      }
-      sum = warp_sum(sum);
-      for (int c = lane; c < len; c += 32) sc[j][c] = sc[j][c] / sum;
-    }
-    __syncthreads();
-    if (tid < len) {                                             // mean over ALL query positions (restarters.py:108)
-      float s = 0.f;
-      for (int j = 0; j < len; ++j) s += sc[j][tid];
-      pbar[tid] = s / (float)len;
-    }
-    __syncthreads();
-    const float* xrow = x + i * len * (int64_t)dm;
-    float* orow = xbar + (i * n_head + h) * (int64_t)dm;
-    for (int c = tid; c < dm; c += POOL_THREADS) {
-      float s = 0.f;
-      for (int j = 0; j < len; ++j) s = fmaf(pbar[j], xrow[(int64_t)j * dm + c], s);
-      orow[c] = s;
-    }
-  }
-}
-
-extern "C" int tiger_seq_attn_pool(const float* qk, int64_t ld_qk, const float* x, const uint8_t* mask,
-                                   const int32_t* count, int64_t n, int len, int d_model, int n_head, float* xbar,
-                                   void* stream) {
-  if (n < 0 || len <= 0 || len > POOL_MAXL || d_model <= 0 || n_head <= 0 || d_model % n_head != 0 ||
-      ld_qk < 2 * (int64_t)d_model)
-    return TIGER_EINVAL;
-  if (n == 0) return TIGER_OK;
-  int64_t grid = n * n_head;
-  if (grid > 148 * 4) grid = 148 * 4;
-  seq_attn_pool_kernel<<<(unsigned)grid, POOL_THREADS, 0, as_stream(stream)>>>(qk, ld_qk, x, mask, count, n, len,
-                                                                              d_model, n_head, xbar);
   return tiger_launch_status();
 }
 

@@ -263,7 +263,7 @@ __device__ __forceinline__ float4 umma_load_chunk(const float* row_ptr, int k, i
 // tile-relative row = row0 + 32 i.  Rows at or beyond rows_valid (tile edge / device-side row count) read as zero.
 template <int N>
 struct UmmaChunks {
-  const float* ptr0;   // row-major: &A[row, kq];  transposed: &A[kq (+ q), row (quad start)]
+  const float* ptr0;   // row-major: &A[row, kq];  transposed: &A[kq, row]
   int64_t step;        // row-major: 32 * ld;  transposed: 32
   int soff0;           // (kc * rows + row0) * 4
   int n_own;           // chunks [0, n_own) exist in this tile (narrow W tiles own fewer)
@@ -312,48 +312,6 @@ __device__ __forceinline__ void umma_chunks_load_t(float4 (&v)[N], const UmmaChu
       if (k + 3 < k_end) t.w = __ldg(p + 3 * ld);
     }
     v[i] = t;
-  }
-}
-
-// Transposed operand, 16-byte aligned (element (row, k) at base[k * ld + row], ld % 4 == 0): the chunk geometry of
-// the K-major tile stays (lane & 7 -> row, lane >> 3 -> kc), but the data is fetched with vector loads ALONG THE
-// ROWS and transposed inside quads of lanes: lane (rq = (lane >> 2) & 1, q = lane & 3, kc) loads the float4
-// (k = 4 kc + q, rows 4 rq .. 4 rq + 3), then the four lanes of a quad exchange components with four shuffles so
-// that lane q ends up with (row 4 rq + q, k = 4 kc .. 4 kc + 3) - exactly the K-major chunk it has to store.
-// c.ptr0 = base + (4 kc + q) * ld + first row of the quad.
-template <int N>
-__device__ __forceinline__ void umma_chunks_load_tv(float4 (&v)[N], const UmmaChunks<N>& c, int k0, int k_end,
-                                                    int64_t ld, int lane) {
-  const int q = lane & 3;
-  const bool k_ok = k0 + c.kq + q < k_end;
-#pragma unroll
-  for (int i = 0; i < N; ++i) {
-    float4 t = make_float4(0.f, 0.f, 0.f, 0.f);
-    const int left = c.rows_valid - ((c.row0 + 32 * i) & ~3);     // rows of this quad that exist
-    if (i < c.n_own && k_ok && left > 0) {
-      const float* p = c.ptr0 + i * c.step + (int64_t)k0 * ld;
-      if (left >= 4) {
-        t = __ldg(reinterpret_cast<const float4*>(p));
-      } else {
-        t.x = __ldg(p);
-        if (left > 1) t.y = __ldg(p + 1);
-        if (left > 2) t.z = __ldg(p + 2);
-      }
-    }
-    // 4 x 4 transpose inside the quad: in round j lane q sends its component (q ^ j) to lane q ^ j and receives
-    // that lane's component q = element (row q, k-offset q ^ j)
-    float o[4];
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      const int comp = q ^ j;
-      const float send = comp == 0 ? t.x : (comp == 1 ? t.y : (comp == 2 ? t.z : t.w));
-      const float got = __shfl_xor_sync(0xffffffffu, send, j);
-      if (comp == 0) o[0] = got;
-      else if (comp == 1) o[1] = got;
-      else if (comp == 2) o[2] = got;
-      else o[3] = got;
-    }
-    v[i] = make_float4(o[0], o[1], o[2], o[3]);
   }
 }
 

@@ -448,6 +448,13 @@ def sgemm_nt(a: Tensor, w: Tensor, bias: Optional[Tensor], out: Tensor, *, m_row
     return out
 
 
+def wgrad_k_parts(k: int) -> int:
+    """K split of a weight-gradient product with reduction length k: at most 256 reduction steps per CTA (the tensor
+    core truncates when it adds into its fp32 accumulator, an error that grows with the accumulation length:
+    DESIGN.md, Tensor cores)."""
+    return max(1, min(128, (k + 255) // 256))
+
+
 def sgemm_ex(a: Tensor, w: Tensor, out: Tensor, *, m: int, n: int, k: int, trans_a: bool = False,
              trans_w: bool = False, bias: Optional[Tensor] = None, relu: bool = False, alpha: float = 1.0,
              accumulate: bool = False, k_parts: int = 1, m_count: Optional[Tensor] = None,
@@ -607,19 +614,6 @@ class SeqRestarterOp:
         self.fn_w, self.fn_b = g('out_fn.weight'), g('out_fn.bias')
         self.fc1_w, self.fc1_b = g('merger.fc1.weight'), g('merger.fc1.bias')
         self.fc2_w, self.fc2_b = g('merger.fc2.weight'), g('merger.fc2.bias')
-        # The products on the n pooled rows (value projection per head, out-projection, out_fn, merger) have a handful of
-        # rows and K = d_model: one CTA per tile walks 54 dependent k-steps (33 us each, ncu).  Tried: packed weights with
-        # K split over a cluster of up to 8 CTAs (DSMEM reduction) - measured SLOWER in the captured step (wikipedia
-        # 0.333 -> 0.410 ms, mooc 0.126 -> 0.212 ms): the launch is sized for the row capacity (52 row tiles x column tiles
-        # x 8 cluster CTAs, almost all of which only exit) and cluster launches cost more than plain ones.  Kept behind
-        # TIGER_SEQ_SPLITK=1; the default is the persistent staging kernel.
-        dm, hd, d = self.dm, self.dm // self.H, self.d
-        self._small = os.environ.get('TIGER_SEQ_SPLITK') == '1'
-        if self._small:
-            mk = lambda w: WeightPack(w.contiguous(), m_rows_hint=128)
-            self.pk_v = [mk(self.in_w[2 * dm + h * hd:2 * dm + (h + 1) * hd]) for h in range(self.H)]
-            self.pk_out, self.pk_fn = mk(self.out_w), mk(self.fn_w)
-            self.pk_fc1, self.pk_fc2 = mk(self.fc1_w[:, :d]), mk(self.fc2_w)
 
     def history(self, csr: DeviceCSR, nids: Tensor, q_ts: Tensor, n: int, *, ts_period: int = 0,
                 count: Optional[Tensor] = None):
@@ -641,8 +635,7 @@ class SeqRestarterOp:
              ptr(self.x), ptr(self.mask), ptr(self.prev_ts))
         sgemm_nt(self.x, self.in_w[:2 * dm], self.in_b[:2 * dm], self.qk, m_rows=n * L, count=count,
                  rows_per_count=L)
-        # the register-tiled pooling kernel of the training step with dropout 0 (5x faster than tiger_seq_attn_pool,
-        # which stays as the plain reference kernel of the C ABI)
+        # the register-tiled pooling kernel of the training step, with dropout 0
         call('tiger_train_seq_pool', ptr(self.qk), self.qk.stride(0), ptr(self.x), ptr(self.mask), ptr(count), n, L, dm,
              H, 0.0, 0, ptr(self.P), ptr(self.pbar), ptr(self.psum), ptr(self.xbar))
         if self.tail_rows > 0:
@@ -685,17 +678,6 @@ class SeqRestarterOp:
         """The layers after the pooling kernel as tensor-core products."""
         dm, d, H = self.dm, self.d, self.H
         hd = dm // H
-        if self._small:
-            kw = dict(m_rows=n, count=count)
-            for h in range(H):
-                rows = slice(2 * dm + h * hd, 2 * dm + (h + 1) * hd)
-                sgemm_nt_packed_splitk_fused(self.xbar[:, h * dm:(h + 1) * dm], self.pk_v[h], self.in_b[rows],
-                                             self.att[:, h * hd:(h + 1) * hd], 8, **kw)
-            sgemm_nt_packed_splitk_fused(self.att, self.pk_out, self.out_b, self.o, 8, relu=True, **kw)
-            sgemm_nt_packed_splitk_fused(self.o, self.pk_fn, self.fn_b, self.h_left, 8, **kw)
-            sgemm_nt_packed_splitk_fused(self.h_left, self.pk_fc1, self.fc1_b, self.hid, 2, relu=True, **kw)
-            sgemm_nt_packed_splitk_fused(self.hid, self.pk_fc2, self.fc2_b, self.h_right, 2, **kw)
-            return
         for h in range(H):
             rows = slice(2 * dm + h * hd, 2 * dm + (h + 1) * hd)
             sgemm_nt(self.xbar[:, h * dm:(h + 1) * dm], self.in_w[rows], self.in_b[rows],

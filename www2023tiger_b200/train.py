@@ -135,14 +135,12 @@ def _linear_fwd(x, w, b, out, *, m, relu=False, m_count=None, per=1):
     ops.sgemm_big(x, w, out, m=m, n=w.shape[0], k=w.shape[1], bias=b, relu=relu, m_count=m_count, rows_per_count=per)
 
 
-def _linear_bwd(dy, x, w, gw, gb, dx, *, m, k_parts=None, count=None, per=1, accumulate_dx=False):
+def _linear_bwd(dy, x, w, gw, gb, dx, *, m, count=None, per=1, accumulate_dx=False):
     """dy [m, n], x [m, k], w [n, k]: gw += dy^T x, gb += colsum(dy), dx (=|+=) dy w.  `count` bounds m on the device."""
     n, k = w.shape
-    # K split of the weight gradient: <= 256 reduction steps per CTA (accumulator truncation grows with the length)
-    k_parts = max(1, min(128, (m + 255) // 256))
     if gw is not None:
-        ops.sgemm_big(dy, x, gw, m=n, n=k, k=m, trans_a=True, trans_w=True, accumulate=True, k_parts=k_parts,
-                      k_count=count, rows_per_count=per)
+        ops.sgemm_big(dy, x, gw, m=n, n=k, k=m, trans_a=True, trans_w=True, accumulate=True,
+                      k_parts=ops.wgrad_k_parts(m), k_count=count, rows_per_count=per)
     if gb is not None:
         call('tiger_train_colsum', ptr(dy), dy.stride(0), m, ptr(count), per, n, 1.0, ptr(gb))
     if dx is not None:
@@ -530,30 +528,30 @@ class NativeTrainer:
         call('tiger_train_score_head_bwd', ptr(self.dscore), float(g_contrast), ptr(self.hid_s), ptr(P[s + 'fc2.weight']),
              B, d, ctx['p_score'], ptr(self.dhid_s), ptr(G[s + 'fc2.weight']), ptr(G[s + 'fc2.bias']))
         _linear_bwd(self.dhid_s, self.pair, P[s + 'fc1.weight'], G[s + 'fc1.weight'], G[s + 'fc1.bias'], self.dpair,
-                    m=2 * B, k_parts=4)
+                    m=2 * B)
         call('tiger_train_score_build_bwd', ptr(self.dpair), ptr(self.codes) if ctx['hits'] else None, B, d, ptr(self.dz),
              ptr(G['hit_embedding.weight']) if ctx['hits'] else None)
         # ---- merger (MergeLayer: fc2(relu(fc1([out | c]))))
         _linear_bwd(self.dz, self.hid, P[a + 'merger.fc2.weight'], G[a + 'merger.fc2.weight'], G[a + 'merger.fc2.bias'],
-                    self.dhid, m=nq, k_parts=4)
+                    self.dhid, m=nq)
         call('tiger_train_relu_bwd', ptr(self.dhid), d, ptr(self.hid), d, d, nq, None, 1, 1.0)
         _linear_bwd(self.dhid, self.cat, P[a + 'merger.fc1.weight'], G[a + 'merger.fc1.weight'],
-                    G[a + 'merger.fc1.bias'], self.dcat, m=nq, k_parts=4)
+                    G[a + 'merger.fc1.bias'], self.dcat, m=nq)
         call('tiger_train_zero_rows', ptr(self.dcat), E + d, E, nq, ptr(self.empty))
         # ---- out-projection, attention core
         dout = self.dcat[:, :E]
         _linear_bwd(dout, self.attn, P[a + 'mha_fn.out_proj.weight'], G[a + 'mha_fn.out_proj.weight'],
-                    G[a + 'mha_fn.out_proj.bias'], self.dattn, m=nq, k_parts=4)
+                    G[a + 'mha_fn.out_proj.bias'], self.dattn, m=nq)
         hd = E // H
         call('tiger_train_attn_core_bwd', ptr(self.dattn), E, ptr(self.Qp), E, ptr(self.KV), ptr(self.KV[:, E:]), 2 * E,
              ptr(self.P), ptr(self.keep), nq, K, H, hd, ctx['p_attn'], ptr(self.dQ), ptr(self.dKV), ptr(self.dKV[:, E:]))
         g_in_b = G[a + 'mha_fn.in_proj_bias']
         _linear_bwd(self.dQ, self.q_in, P[a + 'mha_fn.q_proj_weight'], G[a + 'mha_fn.q_proj_weight'], g_in_b[:E],
-                    self.dq_in, m=nq, k_parts=4)
+                    self.dq_in, m=nq)
         _linear_bwd(self.dKV[:, :E], self.kv_in, P[a + 'mha_fn.k_proj_weight'], G[a + 'mha_fn.k_proj_weight'],
-                    g_in_b[E:2 * E], self.dkv_in, m=nq * K, k_parts=16)
+                    g_in_b[E:2 * E], self.dkv_in, m=nq * K)
         _linear_bwd(self.dKV[:, E:], self.kv_in, P[a + 'mha_fn.v_proj_weight'], G[a + 'mha_fn.v_proj_weight'],
-                    g_in_b[2 * E:], self.dkv_in, m=nq * K, k_parts=16, accumulate_dx=True)
+                    g_in_b[2 * E:], self.dkv_in, m=nq * K, accumulate_dx=True)
         if comm is not None:
             comm('attention')
         # ---- representation gradients back onto the GRU rows, TimeEncode gradients
@@ -564,9 +562,9 @@ class NativeTrainer:
         # ---- GRU (inputs are detached messages / memory buffers: weight gradients only)
         call('tiger_train_gru_gates_bwd', ptr(self.dh_new), ptr(self.r), ptr(self.zg), ptr(self.n), ptr(self.Gh),
              ptr(self.Hs), ptr(cnt_o), cap, d, ptr(self.dGi), ptr(self.dGh))
-        _linear_bwd(self.dGi, self.X, P[c + 'weight_ih'], G[c + 'weight_ih'], G[c + 'bias_ih'], None, m=cap, k_parts=16,
+        _linear_bwd(self.dGi, self.X, P[c + 'weight_ih'], G[c + 'weight_ih'], G[c + 'bias_ih'], None, m=cap,
                     count=cnt_o)
-        _linear_bwd(self.dGh, self.Hs, P[c + 'weight_hh'], G[c + 'weight_hh'], G[c + 'bias_hh'], None, m=cap, k_parts=16,
+        _linear_bwd(self.dGh, self.Hs, P[c + 'weight_hh'], G[c + 'weight_hh'], G[c + 'bias_hh'], None, m=cap,
                     count=cnt_o)
         if comm is not None:
             comm('gru')

@@ -12,12 +12,6 @@ from ._lib import call, ptr
 f32, i64, u8 = torch.float32, torch.int64, torch.uint8
 
 
-def _parts(k: int) -> int:
-    """K split of a weight-gradient product: at most 256 reduction steps per CTA (the tensor core truncates when it
-    adds into its fp32 accumulator, an error that grows with the accumulation length: DESIGN.md, Tensor cores)."""
-    return max(1, min(128, (k + 255) // 256))
-
-
 class SeqRestarterTrainer:
     """`cap` rows for forward + backward (the collated unique positives: <= 2B), `cap_fwd` >= cap rows for forward-only
     calls (lazy restart of up to every involved node, in train() mode with the reference's dropout)."""
@@ -112,8 +106,7 @@ class SeqRestarterTrainer:
         hd = dm // H
         P, G, N = self.fp.p, self.fp.g, self._names()
         inv_keep = 1.0 / (1.0 - p) if p > 0 else 1.0
-        kp = _parts(n)
-        wg = dict(trans_a=True, trans_w=True, accumulate=True, k_parts=kp, k_count=count)    # weight gradients
+        wg = dict(trans_a=True, trans_w=True, accumulate=True, k_parts=ops.wgrad_k_parts(n), k_count=count)  # weight gradients
         dg = dict(trans_w=True, m_count=count)                                               # input gradients
         colsum = lambda x, cols, out, scale=1.0, rows=n, per=1: call(
             'tiger_train_colsum', ptr(x), x.stride(0), rows, ptr(count), per, cols, float(scale), ptr(out))
@@ -148,7 +141,7 @@ class SeqRestarterTrainer:
         call('tiger_train_seq_pool_bwd', ptr(self.dxbar), ptr(self.dpsum), ptr(self.X), ptr(self.QK), 2 * dm, ptr(self.P),
              ptr(self.pbar), ptr(count), n, L, dm, H, p, seed, ptr(self.dX), ptr(self.dQK))
         ops.sgemm_big(self.dQK, self.X, g_in_w[:2 * dm], m=2 * dm, n=dm, k=n * L, trans_a=True, trans_w=True,
-                      accumulate=True, k_parts=_parts(n * L), k_count=count, rows_per_count=L)
+                      accumulate=True, k_parts=ops.wgrad_k_parts(n * L), k_count=count, rows_per_count=L)
         colsum(self.dQK, 2 * dm, g_in_b[:2 * dm], rows=n * L, per=L)
         ops.sgemm_big(self.dQK, in_w[:2 * dm], self.dX, m=n * L, n=dm, k=2 * dm, trans_w=True, accumulate=True,
                       m_count=count, rows_per_count=L)
