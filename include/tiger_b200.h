@@ -274,7 +274,7 @@ int tiger_score_fold(const float* score_fc1, const float* score_fc1_b, const flo
 /* bytes of caller-provided, 16-byte aligned workspace for n_query queries */
 int64_t tiger_temporal_attention_work_bytes(int64_t n_query, int k, int d, int de, int n_head);
 
-/* a15 + a16  GraphEmbedding.compute_embedding_with_computation_graph (n_layers=1) +
+/* a15 + a16  one layer of GraphEmbedding.compute_embedding_with_computation_graph +
  * TemporalAttention.forward (temporal_agg_modules.py:29-83,210-235), eval mode: gather (center + K
  * neighbors + edge rows) -> time encoding -> folded single-query attention (score weights through
  * Wqk, masked softmax, pooled keys) -> folded value / out projection + merger MLP on the tensor
@@ -290,6 +290,22 @@ int tiger_temporal_attention(const int64_t* center_nids, const float* q_ts, int6
                              const void* sel, int sel_is_i64, const float* nfeats,
                              const float* efeats, int d, int de, int n_head,
                              const tiger_attn_params* params, float* out, void* work, void* stream);
+
+/* The same layer for any depth of a multi-layer embedding (tiger_temporal_attention is this entry point with
+ * ts_group = 1 and key_rows = NULL):
+ *   query q reads q_ts[(q / ts_group) % ts_period]: the depth-1 queries of n_layers = 2 are the K neighbors
+ *     of each of the 3B batch nodes at the parent event's time, ts_group = K, ts_period = B
+ *     (repeat_interleave(ts.repeat(3), K)).
+ *   key_rows [n_query * K][d] (NULL: the rows above): slot (q, j) takes its node representation from
+ *     key_rows[q * K + j] with no node features added - the lower layer's output for the depth-2 queries.
+ *     Padding slots (neigh_nids == 0) stay masked.  key_rows is gathered before the kernel's programmatic
+ *     dependency wait, so its producer must be the previous launch sequence on the same stream. */
+int tiger_temporal_attention_ex(const int64_t* center_nids, const float* q_ts, int64_t n_query,
+                                int64_t ts_period, int64_t ts_group, const int64_t* neigh_nids,
+                                const int64_t* neigh_eids, const float* neigh_ts, int k, const float* rows_a,
+                                const float* rows_b, const float* key_rows, const void* sel, int sel_is_i64,
+                                const float* nfeats, const float* efeats, int d, int de, int n_head,
+                                const tiger_attn_params* params, float* out, void* work, void* stream);
 
 /* Same operator with the dense argument list of TemporalAttention.forward
  * (temporal_agg_modules.py:210-235): qx [n,d], qt [n,d], kx [n,K,d], ky [n,K,de], kt [n,K,d],

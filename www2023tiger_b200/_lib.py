@@ -41,6 +41,7 @@ _SIGNATURES: Dict[str, str] = {
     'tiger_attn_fold': 'piii' + 'p',
     'tiger_temporal_attention_work_bytes': 'liiii',
     'tiger_temporal_attention': 'ppll' + 'pppi' + 'pppi' + 'pp' + 'iii' + 'ppp' + 'p',
+    'tiger_temporal_attention_ex': 'pplll' + 'pppi' + 'ppppi' + 'pp' + 'iii' + 'ppp' + 'p',
     'tiger_temporal_attention_dense': 'pppppp' + 'li' + 'iii' + 'ppp' + 'p',
     'tiger_score_fold_bytes': 'i',
     'tiger_score_fold_cab_offset': 'i',

@@ -1,4 +1,4 @@
-// K3  temporal graph attention (n_layers = 1), eval mode.
+// K3  temporal graph attention (one layer per launch sequence; n_layers = 2 chains two of them), eval mode.
 // Reference: GraphEmbedding.compute_embedding_with_computation_graph
 // (tiger/model/temporal_agg_modules.py:29-83) + TemporalAttention.forward (:210-235) + torch
 // F.multi_head_attention_forward (need_weights branch) + MergeLayer (basic_modules.py:16-19).
@@ -286,13 +286,15 @@ extern "C" int tiger_score_fold(const float* score_fc1, const float* score_fc1_b
 struct AttArgs {
   // gather mode
   const int64_t* center_nids;
-  const float* q_ts;
+  const float* q_ts;     // query q reads q_ts[(q / ts_group) % ts_period]
   int64_t ts_period;
+  int64_t ts_group;
   const int64_t* neigh_nids;
   const int64_t* neigh_eids;
   const float* neigh_ts;
   const float* rows_a;
   const float* rows_b;
+  const float* key_rows;   // [n_query * K][d] or NULL: slot (q, j) takes its node row from key_rows[q * K + j]
   const void* sel;
   int sel_is_i64;
   const float* nfeats;
@@ -386,9 +388,13 @@ __global__ void __launch_bounds__(ATT_THREADS, 5) attn_score_pool_kernel(const A
 #endif
   SP_MARK();
   // Everything up to the scores reads what kernels BEFORE the Wqk product wrote (finder tables, GRU rows,
-  // memories) - the Wqk product (graph path) releases its dependents only after its own dependency wait, so
-  // those writes are complete when this CTA starts, and the gathers / time codes below overlap that product.
-  // The dense path's Wqk product triggers at its start: there the wait comes first.
+  // memories, and with key_rows the lower layer's output) - the Wqk product (graph path) releases its dependents
+  // only after its own dependency wait, so those writes are complete when this CTA starts, and the gathers / time
+  // codes below overlap that product.  The dense path's Wqk product triggers at its start: there the wait comes
+  // first.  For key_rows this holds only while the lower layer's last product is launched before this layer's
+  // Wqk product on the same programmatic-dependent chain (same stream, nothing reordered in between): forking the
+  // upper layer's Wqk product onto another stream, or issuing it ahead of the lower layer's last product, needs
+  // the key_rows gather moved behind pdl_wait().
   pdl_trigger();
   if (a.dense) pdl_wait();
   const float* qkf = a.w.qkf + q * a.dm.ld_qkf;
@@ -406,10 +412,14 @@ __global__ void __launch_bounds__(ATT_THREADS, 5) attn_score_pool_kernel(const A
     } else {
       const int64_t u = a.neigh_nids[o];
       if (u != 0) {
-        rp = resolve_row(a, u);
-        nf = a.nfeats != nullptr ? a.nfeats + u * d : nullptr;
+        if (a.key_rows != nullptr) {
+          rp = a.key_rows + o * d;   // the lower layer's embedding of this slot: no node features on top
+        } else {
+          rp = resolve_row(a, u);
+          nf = a.nfeats != nullptr ? a.nfeats + u * d : nullptr;
+        }
         ef = a.efeats != nullptr ? a.efeats + a.neigh_eids[o] * de : nullptr;
-        dt = a.q_ts[q % a.ts_period] - a.neigh_ts[o];
+        dt = a.q_ts[(q / a.ts_group) % a.ts_period] - a.neigh_ts[o];
       }
     }
     s_row[tid] = rp;
@@ -426,8 +436,8 @@ __global__ void __launch_bounds__(ATT_THREADS, 5) attn_score_pool_kernel(const A
   float* out = a.w.kvc + q * a.dm.ld_kvc;
   // ---- gather: node rows (+ node features) and edge-feature rows of all slots ----
   const bool vec = (d & 3) == 0 && (de & 3) == 0 && (Cp & 3) == 0 &&
-                   ((((uintptr_t)a.rows_a | (uintptr_t)a.rows_b | (uintptr_t)a.nfeats | (uintptr_t)a.efeats |
-                      (uintptr_t)a.kx | (uintptr_t)a.ky) & 15) == 0);
+                   ((((uintptr_t)a.rows_a | (uintptr_t)a.rows_b | (uintptr_t)a.key_rows | (uintptr_t)a.nfeats |
+                      (uintptr_t)a.efeats | (uintptr_t)a.kx | (uintptr_t)a.ky) & 15) == 0);
   const float inv_d = 1.0f / (float)d, inv_de = 1.0f / (float)de;
   if (vec) {
     const int d4 = d >> 2, de4 = de >> 2;
@@ -706,20 +716,32 @@ static int attention_entry(AttArgs& a, int k, int d, int de, int n_head, const t
   return attention_run(a, params, out, as_stream(stream));
 }
 
+extern "C" int tiger_temporal_attention_ex(const int64_t* center_nids, const float* q_ts, int64_t n_query,
+                                           int64_t ts_period, int64_t ts_group, const int64_t* neigh_nids,
+                                           const int64_t* neigh_eids, const float* neigh_ts, int k, const float* rows_a,
+                                           const float* rows_b, const float* key_rows, const void* sel, int sel_is_i64,
+                                           const float* nfeats, const float* efeats, int d, int de, int n_head,
+                                           const tiger_attn_params* params, float* out, void* work, void* stream) {
+  if (rows_b == nullptr || sel == nullptr || ts_group <= 0) return TIGER_EINVAL;
+  AttArgs a = {};
+  a.center_nids = center_nids; a.q_ts = q_ts; a.ts_period = ts_period > 0 ? ts_period : n_query;
+  a.ts_group = ts_group;
+  a.neigh_nids = neigh_nids; a.neigh_eids = neigh_eids; a.neigh_ts = neigh_ts;
+  a.rows_a = rows_a; a.rows_b = rows_b; a.key_rows = key_rows; a.sel = sel; a.sel_is_i64 = sel_is_i64;
+  a.nfeats = nfeats; a.efeats = efeats; a.dense = 0;
+  a.n_query = n_query;
+  return attention_entry(a, k, d, de, n_head, params, out, work, stream);
+}
+
 extern "C" int tiger_temporal_attention(const int64_t* center_nids, const float* q_ts, int64_t n_query,
                                         int64_t ts_period, const int64_t* neigh_nids, const int64_t* neigh_eids,
                                         const float* neigh_ts, int k, const float* rows_a, const float* rows_b,
                                         const void* sel, int sel_is_i64, const float* nfeats, const float* efeats,
                                         int d, int de, int n_head, const tiger_attn_params* params, float* out,
                                         void* work, void* stream) {
-  if (rows_b == nullptr || sel == nullptr) return TIGER_EINVAL;
-  AttArgs a = {};
-  a.center_nids = center_nids; a.q_ts = q_ts; a.ts_period = ts_period > 0 ? ts_period : n_query;
-  a.neigh_nids = neigh_nids; a.neigh_eids = neigh_eids; a.neigh_ts = neigh_ts;
-  a.rows_a = rows_a; a.rows_b = rows_b; a.sel = sel; a.sel_is_i64 = sel_is_i64;
-  a.nfeats = nfeats; a.efeats = efeats; a.dense = 0;
-  a.n_query = n_query;
-  return attention_entry(a, k, d, de, n_head, params, out, work, stream);
+  return tiger_temporal_attention_ex(center_nids, q_ts, n_query, ts_period, 1, neigh_nids, neigh_eids, neigh_ts, k,
+                                     rows_a, rows_b, nullptr, sel, sel_is_i64, nfeats, efeats, d, de, n_head, params,
+                                     out, work, stream);
 }
 
 extern "C" int tiger_temporal_attention_dense(const float* qx, const float* qt, const float* kx, const float* ky,
@@ -728,6 +750,7 @@ extern "C" int tiger_temporal_attention_dense(const float* qx, const float* qt, 
                                               void* work, void* stream) {
   AttArgs a = {};
   a.qx = qx; a.qt = qt; a.kx = kx; a.ky = ky; a.kt = kt; a.pad = padding_mask; a.dense = 1; a.ts_period = 1;
+  a.ts_group = 1;
   a.n_query = n_query;
   return attention_entry(a, k, d, de, n_head, params, out, work, stream);
 }

@@ -3,7 +3,8 @@
 `TigerEngine` owns the device state of TIGE/TIGER (both memories, the last-message store, the
 pending / up-to-date flags) and runs TIGE.contrast_learning (reference tiger/model/tiger.py:174-290)
 as a fixed sequence of kernel launches (13 per batch) whose data-dependent sizes (involved U, outdated O, restarted R) stay on
-the device.  `StreamRunner` adds the device neighbor finder in front, captures the sequence in a
+the device.  `n_layers=2` (the reference's keyword default) adds the second neighbor hop to the finder and a depth-1
+attention chain in front of the batch nodes' one.  `StreamRunner` adds the device neighbor finder in front, captures the sequence in a
 CUDA graph and feeds it from pinned host buffers.
 
 Launch sequence of one batch (B events, K neighbors):
@@ -17,6 +18,14 @@ Launch sequence of one batch (B events, K neighbors):
   8 tiger_store_messages     build + store the new raw messages   (step 5)
   9 tiger_left_writeback     persist h(t-) of positives           (step 6)
  10 tiger_link_score         hit flags, scorer, BCE loss          (step 7)
+
+With n_layers = 2 (GraphEmbedding.compute_embedding_with_computation_graph, temporal_agg_modules.py:79-104):
+  1  tiger_find_recent hop 1 as above, then the hop-1 times widened to float64 and tiger_find_recent hop 2: the K
+     neighbors of each of the 3B*K hop-1 neighbors at that neighbor's own event time (the collator's two calls);
+     both mark the involved bitmap, so U, O, R, the GRU and the lazy restart cover the 2-hop nodes
+  5a tiger_temporal_attention_ex, fns.1, 3B*K depth-1 queries (center = hop-1 neighbor, time = its parent event's)
+     over the hop-2 table -> emb1 [3B*K, d]
+  5b tiger_temporal_attention_ex, fns.0, the 3B batch nodes over the hop-1 table, slot (q, j) keyed by emb1[q*K + j]
 """
 from typing import Dict, Optional
 
@@ -41,7 +50,9 @@ class TigerEngine:
                  efeats: Optional[Tensor], nfeats: Optional[Tensor] = None, n_neighbors: int = 10,
                  n_head: int = 2, batch_size: int = 200, msg_src: str = 'left', upd_src: str = 'right',
                  restarter: Optional[str] = None, hist_len: int = 40, hit_type: str = 'bin',
-                 lazy_restart: bool = False, want_restarter_targets: bool = False, device='cuda'):
+                 lazy_restart: bool = False, want_restarter_targets: bool = False, n_layers: int = 1, device='cuda'):
+        if n_layers not in (1, 2):
+            raise NotImplementedError(f'n_layers={n_layers}: the engine runs one or two attention layers')
         if msg_src not in ('left', 'right') or upd_src not in ('left', 'right'):
             raise ValueError(f'Invalid msg_src={msg_src} / upd_src={upd_src}')   # tiger.py:156-160
         if hit_type not in ('bin', 'none'):
@@ -51,6 +62,7 @@ class TigerEngine:
         dev = torch.device(device)
         self.device, self.csr = dev, csr
         self.N, self.K, self.H, self.B = n_nodes, n_neighbors, n_head, batch_size
+        self.n_layers = n_layers
         self.efeats = efeats
         self.nfeats = nfeats
         self.d = nfeats.shape[1] if nfeats is not None else dim              # feature_getter.py:76-77
@@ -67,7 +79,9 @@ class TigerEngine:
         self.msg_vals, self.msg_ts, self.has_msg = z(N, self.M), z(N), z(N, dt=u8)
         self.uptodate = z(N, dt=u8)
         # ---- per-batch scratch (fixed capacity) ----
-        self.cap = 3 * B * (K + 1)
+        # involved-node capacity: every query node and its K neighbors (collate_memory_nodes); with the second hop
+        # the 3B*K hop-1 neighbors are queries too, and no list can hold more than the N distinct nodes
+        self.cap = 3 * B * (K + 1) if n_layers == 1 else min((3 * B + 3 * B * K) * (K + 1), N)
         self.bitmap = z(ops.bitmap_words(N), dt=i32)
         self.involved, self.outdated, self.restart_nodes = z(self.cap, dt=i64), z(self.cap, dt=i64), z(self.cap, dt=i64)
         self.gru_row = torch.full((N,), -1, dtype=i32, device=dev)
@@ -76,6 +90,12 @@ class TigerEngine:
         self.neigh_nids, self.neigh_eids = z(3 * B, K, dt=i64), z(3 * B, K, dt=i64)
         self.neigh_ts = z(3 * B, K)
         self.ts32 = z(B)
+        if n_layers == 2:
+            # second hop: the hop-1 table's times as float64 queries, the [3BK, K] table, the depth-1 embeddings
+            self.neigh_ts64 = z(3 * B * K, dt=f64)
+            self.neigh2_nids, self.neigh2_eids = z(3 * B * K, K, dt=i64), z(3 * B * K, K, dt=i64)
+            self.neigh2_ts = z(3 * B * K, K)
+            self.emb1 = z(3 * B * K, d)
         self.h_new = z(self.cap, d)
         self.emb = z(3 * B, d)
         self.winner = z(2 * B, dt=u8)
@@ -93,6 +113,7 @@ class TigerEngine:
         self._ev_fork0, self._ev_rst = torch.cuda.Event(), torch.cuda.Event()
         self.gru_pack = None
         self.attn_pack = ops.AttnPack(self.d, self.de, dev, n_head)
+        self.attn_pack1 = ops.AttnPack(self.d, self.de, dev, n_head) if n_layers == 2 else None   # fns.1 (depth 1)
         self.score_pack = ops.ScorePack(self.d, dev)
         self.score_fold = ops.ScoreFold(self.d, dev)
         self.pq = torch.zeros(3 * batch_size, 2 * self.d, dtype=f32, device=dev)   # [W1a z | W1b z] per query row
@@ -112,11 +133,14 @@ class TigerEngine:
             self.gru_pack.refresh(*args)
         a = 'temporal_embedding_fn.fns.0.'
         self.time_w, self.time_b = g('time_encoder.basis_freq'), g('time_encoder.phase')
-        self.attn_pack.refresh(g(a + 'mha_fn.q_proj_weight'), g(a + 'mha_fn.k_proj_weight'),
-                               g(a + 'mha_fn.v_proj_weight'), g(a + 'mha_fn.in_proj_bias'),
-                               g(a + 'mha_fn.out_proj.weight'), g(a + 'mha_fn.out_proj.bias'),
-                               g(a + 'merger.fc1.weight'), g(a + 'merger.fc1.bias'),
-                               g(a + 'merger.fc2.weight'), g(a + 'merger.fc2.bias'), self.time_w, self.time_b)
+        # fns.0 embeds the batch nodes (depth n_layers), fns.1 their neighbors (depth 1); the time encoder is shared
+        for pack, fa in ((self.attn_pack, a), (self.attn_pack1, 'temporal_embedding_fn.fns.1.')):
+            if pack is not None:
+                pack.refresh(g(fa + 'mha_fn.q_proj_weight'), g(fa + 'mha_fn.k_proj_weight'),
+                             g(fa + 'mha_fn.v_proj_weight'), g(fa + 'mha_fn.in_proj_bias'),
+                             g(fa + 'mha_fn.out_proj.weight'), g(fa + 'mha_fn.out_proj.bias'),
+                             g(fa + 'merger.fc1.weight'), g(fa + 'merger.fc1.bias'),
+                             g(fa + 'merger.fc2.weight'), g(fa + 'merger.fc2.bias'), self.time_w, self.time_b)
         s = 'score_fn.'
         self.score_pack.refresh(g(s + 'fc1.weight'), g(s + 'fc1.bias'), g(s + 'fc2.weight'), g(s + 'fc2.bias'),
                                 g('hit_embedding.weight') if self.hit_type == 'bin' else None)
@@ -166,6 +190,12 @@ class TigerEngine:
         ops.find_recent(self.csr, self.batch_nids, self.ts64, self.K, ts_period=self.B, want_dirs=False,
                         ts32_out=self.ts32, bitmap=self.bitmap,
                         out=(self.neigh_nids, self.neigh_eids, self.neigh_ts, None))
+        if self.n_layers == 2:
+            # collate_memory_nodes' second call: each hop-1 neighbor queried at its own float32 event time, widened
+            # to float64 (an exact conversion), marking the same bitmap
+            self.neigh_ts64.copy_(self.neigh_ts.view(-1))
+            ops.find_recent(self.csr, self.neigh_nids.view(-1), self.neigh_ts64, self.K, want_dirs=False,
+                            bitmap=self.bitmap, out=(self.neigh2_nids, self.neigh2_eids, self.neigh2_ts, None))
 
     def launch_model(self, with_scorer: bool = True):
         d, B = self.d, self.B
@@ -234,13 +264,25 @@ class TigerEngine:
             self._ev_side.record(side1)
         if self.lazy_restart:
             main.wait_event(self._ev_rst)
+        key_rows = None
+        if self.n_layers == 2:
+            # depth 1 (fns.1): one query per entry of the batch nodes' neighbor table, at the parent event's time
+            # (repeat_interleave(ts.repeat(3), K)), over the second hop.  It reads node rows through resolve_row only,
+            # like depth 2, so the side branch may overlap it (DESIGN.md, "Why the post-GRU branches may overlap").
+            # It must stay on this stream right in front of depth 2: depth 2 gathers emb1 before its dependency wait
+            # (csrc/attention.cu, attn_score_pool_kernel).
+            ops.temporal_attention(self.attn_pack1, self.H, self.neigh_nids.view(-1), self.ts32, self.neigh2_nids,
+                                   self.neigh2_eids, self.neigh2_ts, rows_a=self.right_vals, rows_b=self.h_new,
+                                   sel=self.gru_row, nfeats=self.nfeats, efeats=self.efeats, out=self.emb1,
+                                   ts_group=self.K)
+            key_rows = self.emb1
         # update_left_memory is fused into the last attention product, which first waits for the side branch (the
         # message builder reads the OLD left-memory rows, and `winner` comes from the selection kernel)
         self.attn_pack.attach_left_writeback(self.pos, self.winner, self.ts32, self.left_vals, self.left_ts,
                                              self.left_active, self.err_flags, ready_event=self._ev_side)
         ops.temporal_attention(self.attn_pack, self.H, self.batch_nids, self.ts32, self.neigh_nids, self.neigh_eids,
                                self.neigh_ts, rows_a=self.right_vals, rows_b=self.h_new, sel=self.gru_row,
-                               nfeats=self.nfeats, efeats=self.efeats, out=self.emb)
+                               nfeats=self.nfeats, efeats=self.efeats, out=self.emb, key_rows=key_rows)
         # the link scorer reads the projections `pq` of the embeddings and changes no state: in the pipelined replay
         # it is a separate graph on the copy-out stream (launch_scorer), beside the next batch's model kernels
         if with_scorer:
@@ -273,19 +315,27 @@ class TigerEngine:
         self.scores, self.loss = out_buf[:2 * B], out_buf[2 * B:]
 
     def finder_buffers(self, fresh: bool = False):
-        """The finder's outputs (neighbor tables, float32 batch times, involved-node bitmap).  They depend on the
-        static graph and the batch only, not on the memory state, so the finder of batch i+1 may run while batch
-        i is still in its model kernels - provided it writes its own set (`fresh=True` allocates one)."""
+        """The finder's outputs (neighbor tables, float32 batch times, involved-node bitmap; with n_layers=2 also the
+        float64 hop-1 times and the hop-2 tables).  They depend on the static graph and the batch only, not on the
+        memory state, so the finder of batch i+1 may run while batch i is still in its model kernels - provided it
+        writes its own set (`fresh=True` allocates one)."""
+        bufs = (self.neigh_nids, self.neigh_eids, self.neigh_ts, self.ts32, self.bitmap)
+        if self.n_layers == 2:
+            bufs += (self.neigh_ts64, self.neigh2_nids, self.neigh2_eids, self.neigh2_ts)
         if not fresh:
-            return self.neigh_nids, self.neigh_eids, self.neigh_ts, self.ts32, self.bitmap
-        return tuple(torch.zeros_like(t) for t in
-                     (self.neigh_nids, self.neigh_eids, self.neigh_ts, self.ts32, self.bitmap))
+            return bufs
+        return tuple(torch.zeros_like(t) for t in bufs)
 
     def bind_finder(self, bufs):
-        self.neigh_nids, self.neigh_eids, self.neigh_ts, self.ts32, self.bitmap = bufs
+        self.neigh_nids, self.neigh_eids, self.neigh_ts, self.ts32, self.bitmap = bufs[:5]
+        if self.n_layers == 2:
+            self.neigh_ts64, self.neigh2_nids, self.neigh2_eids, self.neigh2_ts = bufs[5:]
 
     def launches_per_step(self) -> int:
         n = sum(KERNELS_PER_STEP.values())
+        if self.n_layers == 2:
+            # hop-2 finder + the float64 widening of the hop-1 times (a torch copy) + the depth-1 attention chain
+            n += 2 + KERNELS_PER_STEP['temporal_attention']
         if self.lazy_restart:
             n += 1 if self.restarter == 'static' else ops.SeqRestarterOp.LAUNCHES + 2
         if self.want_targets:

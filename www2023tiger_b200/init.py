@@ -15,7 +15,7 @@ def time_basis(d: int) -> torch.Tensor:
 
 
 def random_weights(d: int, de: int, *, n_nodes: int = 0, restarter: Optional[str] = None, hist_len: int = 40,
-                   seed: int = 0, nonzero_static: bool = False) -> Dict[str, torch.Tensor]:
+                   seed: int = 0, nonzero_static: bool = False, n_layers: int = 1) -> Dict[str, torch.Tensor]:
     g = torch.Generator().manual_seed(seed)
     E, C, M = 2 * d, 2 * d + de, 3 * d + de
 
@@ -42,14 +42,16 @@ def random_weights(d: int, de: int, *, n_nodes: int = 0, restarter: Optional[str
     k = 1 / math.sqrt(d)
     W[c + 'weight_ih'], W[c + 'weight_hh'] = uniform((3 * d, M), k), uniform((3 * d, d), k)
     W[c + 'bias_ih'], W[c + 'bias_hh'] = uniform((3 * d,), k), uniform((3 * d,), k)
-    a = 'temporal_embedding_fn.fns.0.'
-    W[a + 'mha_fn.q_proj_weight'] = xavier_uniform((E, E))
-    W[a + 'mha_fn.k_proj_weight'] = xavier_uniform((E, C))
-    W[a + 'mha_fn.v_proj_weight'] = xavier_uniform((E, C))
-    W[a + 'mha_fn.in_proj_bias'] = torch.zeros(3 * E)
-    linear(E, E, a + 'mha_fn.out_proj.', W)
-    W[a + 'mha_fn.out_proj.bias'] = torch.zeros(E)
-    merge_layer(E, d, d, d, a + 'merger.', W)
+    def attention_layer(a, W):
+        W[a + 'mha_fn.q_proj_weight'] = xavier_uniform((E, E))
+        W[a + 'mha_fn.k_proj_weight'] = xavier_uniform((E, C))
+        W[a + 'mha_fn.v_proj_weight'] = xavier_uniform((E, C))
+        W[a + 'mha_fn.in_proj_bias'] = torch.zeros(3 * E)
+        linear(E, E, a + 'mha_fn.out_proj.', W)
+        W[a + 'mha_fn.out_proj.bias'] = torch.zeros(E)
+        merge_layer(E, d, d, d, a + 'merger.', W)
+
+    attention_layer('temporal_embedding_fn.fns.0.', W)
     W['hit_embedding.weight'] = torch.randn((2, d), generator=g)
     merge_layer(d, d, d, 1, 'score_fn.', W)
     r = 'restarter_fn.'
@@ -71,6 +73,9 @@ def random_weights(d: int, de: int, *, n_nodes: int = 0, restarter: Optional[str
         W[r + 'mha_fn.out_proj.bias'] = torch.zeros(dm)
         linear(d, dm, r + 'out_fn.', W)
         merge_layer(d, dm - d, d, d, r + 'merger.', W)
+    # the lower layers' attention (n_layers > 1) is drawn last, so the weights above do not depend on n_layers
+    for i in range(1, n_layers):
+        attention_layer(f'temporal_embedding_fn.fns.{i}.', W)
     return W
 
 

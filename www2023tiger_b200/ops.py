@@ -267,7 +267,9 @@ class LeftWritebackFusedC(ctypes.Structure):
 
 class AttnPack:
     """TemporalAttention parameters for the kernels: the reference's tensors as stored plus the folded
-    weights (tiger_attn_fold: Wqk, bqk, W2f), and a workspace that grows on demand."""
+    weights (tiger_attn_fold: Wqk, bqk, W2f), and a workspace that grows on demand.  A multi-layer embedding
+    keeps one pack per layer (temporal_embedding_fn.fns.i); the score fold and the fused left write-back attach
+    only to the pack of the batch-node layer, whose result they read."""
 
     def __init__(self, d: int, de: int, device, n_head: int = 2):
         self.d, self.de, self.n_head = d, de, n_head
@@ -337,16 +339,19 @@ class AttnPack:
 def temporal_attention(pack: AttnPack, n_head: int, center_nids: Tensor, q_ts: Tensor, neigh_nids: Tensor,
                        neigh_eids: Tensor, neigh_ts: Tensor, *, rows_a: Optional[Tensor], rows_b: Tensor,
                        sel: Tensor, nfeats: Optional[Tensor], efeats: Optional[Tensor],
-                       out: Optional[Tensor] = None) -> Tensor:
-    """a15+a16 (gather form).  q_ts may be shorter than center_nids (ts.repeat semantics)."""
-    check_cuda(center_nids, q_ts, neigh_nids, neigh_eids, neigh_ts, rows_a, rows_b, sel, nfeats, efeats)
+                       out: Optional[Tensor] = None, key_rows: Optional[Tensor] = None, ts_group: int = 1) -> Tensor:
+    """a15+a16 (gather form).  Query q uses q_ts[(q // ts_group) % len(q_ts)] (ts.repeat semantics; ts_group = K
+    gives repeat_interleave(ts.repeat(3), K), the depth-1 queries of n_layers = 2).  key_rows [n * K, d]: slot
+    (q, j) takes the lower layer's output row q * K + j as its node representation, without node features."""
+    check_cuda(center_nids, q_ts, neigh_nids, neigh_eids, neigh_ts, rows_a, rows_b, sel, nfeats, efeats, key_rows)
     n, k = neigh_nids.shape
     if out is None:
         out = _empty((n, pack.d), f32, rows_b)
     assert sel.dtype in (i32, i64) and n_head == pack.n_head
-    call('tiger_temporal_attention', ptr(center_nids), ptr(q_ts), n, q_ts.numel(), ptr(neigh_nids), ptr(neigh_eids),
-         ptr(neigh_ts), k, ptr(rows_a), ptr(rows_b), ptr(sel), int(sel.dtype == i64), ptr(nfeats), ptr(efeats),
-         pack.d, pack.de, n_head, pack.byref(), ptr(out), ptr(pack.work(n, k)))
+    assert key_rows is None or (key_rows.dtype == f32 and key_rows.numel() >= n * k * pack.d)
+    call('tiger_temporal_attention_ex', ptr(center_nids), ptr(q_ts), n, q_ts.numel(), ts_group, ptr(neigh_nids),
+         ptr(neigh_eids), ptr(neigh_ts), k, ptr(rows_a), ptr(rows_b), ptr(key_rows), ptr(sel), int(sel.dtype == i64),
+         ptr(nfeats), ptr(efeats), pack.d, pack.de, n_head, pack.byref(), ptr(out), ptr(pack.work(n, k)))
     return out
 
 

@@ -57,12 +57,14 @@ class _NativeStep(torch.autograd.Function):
 
 
 class _Workspace:
-    """Per-batch device scratch of the fused route (sized for batch B, K neighbors)."""
+    """Per-batch device scratch of the fused route (sized for batch B, K neighbors, n_layers hops)."""
 
-    def __init__(self, n_nodes, d, B, K, dev):
+    def __init__(self, n_nodes, d, B, K, dev, n_layers=1):
         z = lambda *s, dt=torch.float32: torch.zeros(*s, dtype=dt, device=dev)
-        self.B, self.K = B, K
-        self.cap = 3 * B * (K + 1)
+        self.B, self.K, self.n_layers = B, K, n_layers
+        # capacity of the involved / outdated lists as in collate_memory_nodes (the 3BK hop-1 neighbors are queries
+        # of the second hop), bounded by the number of nodes
+        self.cap = 3 * B * (K + 1) if n_layers == 1 else min((3 * B + 3 * B * K) * (K + 1), n_nodes)
         self.bitmap = z(ops.bitmap_words(n_nodes), dt=torch.int32)
         self.involved, self.outdated = z(self.cap, dt=torch.int64), z(self.cap, dt=torch.int64)
         self.gru_row = torch.full((n_nodes,), -1, dtype=torch.int32, device=dev)
@@ -148,14 +150,14 @@ class TIGE(nn.Module):
     # ------------------------------------------------------------------ fused no-grad route
     def _fusable(self) -> bool:
         return (isinstance(self.msg_transform_fn, IdentityMessageFunction)
-                and isinstance(self.right_mem_updater, GRUUpdater) and self.n_layers == 1
+                and isinstance(self.right_mem_updater, GRUUpdater) and self.n_layers in (1, 2)
                 and self.hit_type in ('bin', 'none') and self.left_memory.vals.is_cuda)
 
     def _workspace(self, B: int, K: int) -> _Workspace:
         dev = self.device
         ws = self._ws
-        if ws is None or ws.B < B or ws.K != K or ws.bitmap.device != dev:
-            ws = self._ws = _Workspace(self.n_nodes, self.memory_dim, B, K, dev)
+        if ws is None or ws.B < B or ws.K != K or ws.n_layers != self.n_layers or ws.bitmap.device != dev:
+            ws = self._ws = _Workspace(self.n_nodes, self.memory_dim, B, K, dev, self.n_layers)
         return ws
 
     def _scorer(self) -> ops.ScorePack:
@@ -174,8 +176,9 @@ class TIGE(nn.Module):
 
     def _contrast_learning_fused(self, src_ids, dst_ids, neg_dst_ids, ts, eids, cg):
         B, d, N = len(src_ids), self.memory_dim, self.n_nodes
-        nn_, ne_, nt_ = cg.layers[1]
-        ws = self._workspace(B, nn_.shape[1])
+        nn_, ne_, nt_ = cg.layers[self.n_layers]          # the batch nodes' neighbors (hit flags, scorer)
+        K = nn_.shape[1]
+        ws = self._workspace(B, K)
         dev = self.device
         err = self._err.get(dev)
         left, right, store = self.left_memory, self.right_memory, self.msg_store
@@ -192,10 +195,20 @@ class TIGE(nn.Module):
                        msg_ts=store.node_msg_ts, check_mem_ts=self.msg_memory.update_ts,
                        check_equal=(self.msg_src == 'left'), err_flags=err)
         # step 3: temporal attention over the sampled neighbors (tiger.py:225-227)
-        fn = self.temporal_embedding_fn.fns[0]
+        fns = self.temporal_embedding_fn.fns
+        key_rows = None
+        if self.n_layers == 2:
+            # depth 1 (fns.1): the batch nodes' 3B*K neighbors at their parent event's time over the second hop
+            # cg.layers[1]; their embeddings key the batch nodes' slots (temporal_agg_modules.py:95-104)
+            n2, e2, t2 = cg.layers[1]
+            key_rows = ops.temporal_attention(fns[1].packed(self.time_encoder), fns[1].n_head,
+                                              nn_.reshape(-1).contiguous(), ts, n2, e2, t2, rows_a=right.vals,
+                                              rows_b=ws.h_new, sel=ws.gru_row, nfeats=fg.nfeats, efeats=fg.efeats,
+                                              ts_group=K)
+        fn = fns[0]
         emb = ops.temporal_attention(fn.packed(self.time_encoder), fn.n_head, batch_nids, ts, nn_, ne_, nt_,
                                      rows_a=right.vals, rows_b=ws.h_new, sel=ws.gru_row, nfeats=fg.nfeats,
-                                     efeats=fg.efeats)
+                                     efeats=fg.efeats, key_rows=key_rows)
         # steps 4-6 (tiger.py:230-255)
         winner = ws.winner[:2 * B]
         ops.select_latest(pos, ts, want_unique=False, winner=winner, want_count=False)
@@ -378,7 +391,7 @@ class TIGER(TIGE):
         TIGER_AUTOGRAD_ROUTE=1, the comparison route of the tests) trains through the torch-op route below."""
         import os
         from .restarters import SeqRestarter, StaticRestarter
-        return (torch.is_grad_enabled() and self.training and self._fusable()
+        return (torch.is_grad_enabled() and self.training and self._fusable() and self.n_layers == 1
                 and isinstance(self.restarter_fn, (SeqRestarter, StaticRestarter))
                 and os.environ.get('TIGER_AUTOGRAD_ROUTE') != '1')
 
