@@ -479,8 +479,9 @@ int tiger_pipe_join(void* pipe, void* stream);
  * train_self_supervised.py:165-171 and train_self_supervised_ddp.py:203-208 run through autograd.  Dense products
  * go through tiger_sgemm_ex; gradients accumulate into caller-owned buffers that tiger_train_adam zeroes.
  *   gather_pending / gru_gates[_bwd]   compute_messages + GRUUpdater (tiger.py:292-356, update_modules.py:30-37)
- *   attn_build[_bwd] / attn_core[_bwd] compute_embedding_with_computation_graph + TemporalAttention with dropout
- *                                      (temporal_agg_modules.py:29-83,210-235), TimeEncode gradients
+ *   attn_build[_bwd][_ex] / attn_core[_bwd] compute_embedding_with_computation_graph + TemporalAttention with
+ *                                      dropout (temporal_agg_modules.py:29-104,210-235), either depth of n_layers = 2,
+ *                                      TimeEncode gradients
  *   score_build[_bwd] / score_head[_bwd] hit embedding + score_fn + BCE (tiger.py:259-288)
  *   mse                                 mutual loss over valid rows (tiger.py:583-590)
  *   colsum / relu_bwd / zero_rows / scatter_add_rows   bias gradients, ReLU, masked rows, nn.Embedding gradients
@@ -490,9 +491,19 @@ int tiger_train_gather_pending(const int64_t* ids, const int32_t* count, int64_t
 int tiger_train_gru_gates(const float* Gi, const float* Gh, const float* H, const int32_t* count, int64_t cap, int d, float* h_new, float* r_out, float* z_out, float* n_out, void* stream);
 int tiger_train_gru_gates_bwd(const float* dh, const float* r_in, const float* z_in, const float* n_in, const float* Gh, const float* H, const int32_t* count, int64_t cap, int d, float* dGi, float* dGh, void* stream);
 int tiger_train_attn_build(const int64_t* center, int64_t n_q, const float* ts, int64_t batch, const int64_t* neigh_nids, const int64_t* neigh_eids, const float* neigh_ts, int k, const float* rows_a, const float* rows_b, const int32_t* sel, const float* nfeats, const float* efeats, int d, int de, const float* time_w, const float* time_b, float* q_in, float* kv_in, float* cat, int64_t ld_cat, int cat_off, void* stream);
+/* attn_build[_bwd]_ex: the same builders for either depth of n_layers = 2 (attn_build[_bwd] are these with ts_group = 1
+ * and key_rows / d_key_rows = NULL), the training twins of tiger_temporal_attention_ex:
+ *   query i's time is ts[(i / ts_group) % batch] (depth 1: ts_group = K, repeat_interleave(ts.repeat(3), K));
+ *   key_rows [n_q * K][d] (NULL: the rows above): slot r takes key_rows[r] as its node part, no node features added
+ *     (depth 2: the depth-1 output);
+ *   d_key_rows [n_q * K][d] (NULL: onto dh_new through sel): the slots' node-part gradients are STORED there, zeros
+ *     for padding slots (neigh_nids == 0).  Query / merger-input gradients still go onto dh_new, and both kinds of
+ *     time code accumulate into the TimeEncode gradients. */
+int tiger_train_attn_build_ex(const int64_t* center, int64_t n_q, const float* ts, int64_t batch, int64_t ts_group, const int64_t* neigh_nids, const int64_t* neigh_eids, const float* neigh_ts, int k, const float* rows_a, const float* rows_b, const float* key_rows, const int32_t* sel, const float* nfeats, const float* efeats, int d, int de, const float* time_w, const float* time_b, float* q_in, float* kv_in, float* cat, int64_t ld_cat, int cat_off, void* stream);
 int tiger_train_attn_core(const float* Q, int64_t ldq, const float* Kp, const float* Vp, int64_t ldkv, const int64_t* neigh_nids, int64_t n_q, int k, int n_head, int head_dim, float p_drop, int seed, float* attn, int64_t ld_attn, float* P, uint32_t* keep_bits, uint8_t* empty, void* stream);
 int tiger_train_attn_core_bwd(const float* dattn, int64_t ld_attn, const float* Q, int64_t ldq, const float* Kp, const float* Vp, int64_t ldkv, const float* P, const uint32_t* keep_bits, int64_t n_q, int k, int n_head, int head_dim, float p_drop, float* dQ, float* dKp, float* dVp, void* stream);
 int tiger_train_attn_build_bwd(const float* dkv_in, const float* dq_in, const float* dcat, int64_t ld_cat, int cat_off, const int64_t* center, int64_t n_q, const float* ts, int64_t batch, const int64_t* neigh_nids, const float* neigh_ts, int k, const int32_t* sel, int d, int de, const float* time_w, const float* time_b, float* dh_new, float* g_time_w, float* g_time_b, void* stream);
+int tiger_train_attn_build_bwd_ex(const float* dkv_in, const float* dq_in, const float* dcat, int64_t ld_cat, int cat_off, const int64_t* center, int64_t n_q, const float* ts, int64_t batch, int64_t ts_group, const int64_t* neigh_nids, const float* neigh_ts, int k, const int32_t* sel, int d, int de, const float* time_w, const float* time_b, float* dh_new, float* d_key_rows, float* g_time_w, float* g_time_b, void* stream);
 int tiger_train_zero_rows(float* buf, int64_t ld, int cols, int64_t n_rows, const uint8_t* flag, void* stream);
 int tiger_train_relu_bwd(float* dy, int64_t ld_dy, const float* y, int64_t ld_y, int cols, int64_t n_rows, const int32_t* count, int64_t rows_per_count, float scale, void* stream);
 int tiger_train_colsum(const float* X, int64_t ld, int64_t n_rows, const int32_t* count, int64_t rows_per_count, int cols, float scale, float* out, void* stream);

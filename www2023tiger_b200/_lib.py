@@ -64,9 +64,11 @@ _SIGNATURES: Dict[str, str] = {
     'tiger_train_gru_gates': 'pppplippppp',
     'tiger_train_gru_gates_bwd': 'ppppppplippp',
     'tiger_train_attn_build': 'plplpppipppppiippppplip',
+    'tiger_train_attn_build_ex': 'plpll' + 'pppi' + 'ppppp' + 'p' + 'ii' + 'pp' + 'ppp' + 'li' + 'p',
     'tiger_train_attn_core': 'plpplpliiifiplpppp',
     'tiger_train_attn_core_bwd': 'plplpplppliiifpppp',
     'tiger_train_attn_build_bwd': 'pppliplplppipiipppppp',
+    'tiger_train_attn_build_bwd_ex': 'pppli' + 'plpll' + 'ppi' + 'pii' + 'pp' + 'pppp' + 'p',
     'tiger_train_zero_rows': 'plilpp',
     'tiger_train_relu_bwd': 'plplilplfp',
     'tiger_train_colsum': 'pllplifpp',

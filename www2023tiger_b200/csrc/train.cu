@@ -172,11 +172,13 @@ __device__ __forceinline__ const float* resolve_repr(int64_t nid, const float* r
 
 // One warp per row.  Rows [0, n_q*K): kv_in[i*K+j] = [repr(nb_ij) + nf | ef(e_ij) | cos((t_i - tau_ij) w + b)];
 // rows [n_q*K, n_q*K + n_q): q_in[i] = [repr(center_i) + nf | cos(b)] and the same center row into cat[i, E:E+d]
-// (the second input of the merger).
+// (the second input of the merger).  Query i's time is ts[(i / ts_group) % batch]; with key_rows (the lower layer's
+// output, [n_q*K, d]) slot r takes key_rows[r] as its node part, with no node features added.
 __global__ void __launch_bounds__(256)
 train_attn_build_kernel(const int64_t* __restrict__ center, int64_t n_q, const float* __restrict__ ts, int64_t batch,
-                        const int64_t* __restrict__ nn, const int64_t* __restrict__ ne, const float* __restrict__ nt,
-                        int K, const float* __restrict__ rows_a, const float* __restrict__ rows_b,
+                        int64_t ts_group, const int64_t* __restrict__ nn, const int64_t* __restrict__ ne,
+                        const float* __restrict__ nt, int K, const float* __restrict__ rows_a,
+                        const float* __restrict__ rows_b, const float* __restrict__ key_rows,
                         const int32_t* __restrict__ sel, const float* __restrict__ nfeats,
                         const float* __restrict__ efeats, int d, int de, const float* __restrict__ time_w,
                         const float* __restrict__ time_b, float* __restrict__ q_in, float* __restrict__ kv_in,
@@ -190,18 +192,23 @@ train_attn_build_kernel(const int64_t* __restrict__ center, int64_t n_q, const f
       const int64_t i = r / K;
       const int64_t nid = nn[r];
       float* row = kv_in + r * C;
-      const float* src = resolve_repr(nid, rows_a, rows_b, sel, d);
-      if (nfeats != nullptr) {
-        for (int c = lane; c < d; c += 32) row[c] = src[c] + nfeats[nid * d + c];
+      if (key_rows != nullptr) {
+        for (int c = lane; c < d; c += 32) row[c] = key_rows[r * d + c];
       } else {
-        for (int c = lane; c < d; c += 32) row[c] = src[c] + 0.0f;
+        const float* src = resolve_repr(nid, rows_a, rows_b, sel, d);
+        if (nfeats != nullptr) {
+          for (int c = lane; c < d; c += 32) row[c] = src[c] + nfeats[nid * d + c];
+        } else {
+          for (int c = lane; c < d; c += 32) row[c] = src[c] + 0.0f;
+        }
       }
       if (efeats != nullptr) {
         warp_copy_row(row + d, efeats + ne[r] * de, de, lane);
       } else {
         for (int c = lane; c < de; c += 32) row[d + c] = 0.f;
       }
-      const float dt = ts[i % batch] - nt[r];
+      // (ts_group 1, the one-layer step, skips the 64-bit division)
+      const float dt = ts[(ts_group == 1 ? i : i / ts_group) % batch] - nt[r];
       for (int c = lane; c < d; c += 32) row[d + de + c] = time_enc(dt, time_w[c], time_b[c]);
     } else {
       const int64_t i = r - n_kv;
@@ -219,23 +226,35 @@ train_attn_build_kernel(const int64_t* __restrict__ center, int64_t n_q, const f
   }
 }
 
+extern "C" int tiger_train_attn_build_ex(const int64_t* center, int64_t n_q, const float* ts, int64_t batch,
+                                         int64_t ts_group, const int64_t* neigh_nids, const int64_t* neigh_eids,
+                                         const float* neigh_ts, int k, const float* rows_a, const float* rows_b,
+                                         const float* key_rows, const int32_t* sel, const float* nfeats,
+                                         const float* efeats, int d, int de, const float* time_w, const float* time_b,
+                                         float* q_in, float* kv_in, float* cat, int64_t ld_cat, int cat_off,
+                                         void* stream) {
+  if (center == nullptr || ts == nullptr || neigh_nids == nullptr || rows_a == nullptr || rows_b == nullptr ||
+      sel == nullptr || q_in == nullptr || kv_in == nullptr || cat == nullptr || n_q < 0 || batch <= 0 ||
+      ts_group <= 0 || k <= 0 || d <= 0 || de <= 0)
+    return TIGER_EINVAL;
+  if (n_q == 0) return TIGER_OK;
+  int64_t grid = (n_q * (k + 1) + 7) / 8;
+  if (grid > 148 * 8) grid = 148 * 8;
+  train_attn_build_kernel<<<(unsigned)grid, 256, 0, as_stream(stream)>>>(
+      center, n_q, ts, batch, ts_group, neigh_nids, neigh_eids, neigh_ts, k, rows_a, rows_b, key_rows, sel, nfeats,
+      efeats, d, de, time_w, time_b, q_in, kv_in, cat, ld_cat, cat_off);
+  return tiger_launch_status();
+}
+
 extern "C" int tiger_train_attn_build(const int64_t* center, int64_t n_q, const float* ts, int64_t batch,
                                       const int64_t* neigh_nids, const int64_t* neigh_eids, const float* neigh_ts,
                                       int k, const float* rows_a, const float* rows_b, const int32_t* sel,
                                       const float* nfeats, const float* efeats, int d, int de, const float* time_w,
                                       const float* time_b, float* q_in, float* kv_in, float* cat, int64_t ld_cat,
                                       int cat_off, void* stream) {
-  if (center == nullptr || ts == nullptr || neigh_nids == nullptr || rows_a == nullptr || rows_b == nullptr ||
-      sel == nullptr || q_in == nullptr || kv_in == nullptr || cat == nullptr || n_q < 0 || batch <= 0 || k <= 0 ||
-      d <= 0 || de <= 0)
-    return TIGER_EINVAL;
-  if (n_q == 0) return TIGER_OK;
-  int64_t grid = (n_q * (k + 1) + 7) / 8;
-  if (grid > 148 * 8) grid = 148 * 8;
-  train_attn_build_kernel<<<(unsigned)grid, 256, 0, as_stream(stream)>>>(
-      center, n_q, ts, batch, neigh_nids, neigh_eids, neigh_ts, k, rows_a, rows_b, sel, nfeats, efeats, d, de, time_w,
-      time_b, q_in, kv_in, cat, ld_cat, cat_off);
-  return tiger_launch_status();
+  return tiger_train_attn_build_ex(center, n_q, ts, batch, 1, neigh_nids, neigh_eids, neigh_ts, k, rows_a, rows_b,
+                                   nullptr, sel, nfeats, efeats, d, de, time_w, time_b, q_in, kv_in, cat, ld_cat,
+                                   cat_off, stream);
 }
 
 #define ATT_MAXK 32
@@ -429,16 +448,17 @@ extern "C" int tiger_train_attn_core_bwd(const float* dattn, int64_t ld_attn, co
 
 // Gradients of the builder's inputs: representation columns of dkv_in / dq_in (+ the merger's second input) are
 // added onto the GRU row of the node they were read from (nodes without a pending message read the memory table,
-// a buffer: no gradient); the time-code columns give the TimeEncode gradients
+// a buffer: no gradient); with d_key_rows the slots' node parts are stored there instead (zeros for padding slots),
+// the gradient of the lower layer's output.  The time-code columns give the TimeEncode gradients
 //   d/dw_c = -sin(dt w_c + b_c) dt g,  d/db_c = -sin(dt w_c + b_c) g      (time_encoding.py:16-27)
 __global__ void __launch_bounds__(256)
 train_attn_build_bwd_kernel(const float* __restrict__ dkv_in, const float* __restrict__ dq_in,
                             const float* __restrict__ dcat, int64_t ld_cat, int cat_off,
                             const int64_t* __restrict__ center, int64_t n_q, const float* __restrict__ ts, int64_t batch,
-                            const int64_t* __restrict__ nn, const float* __restrict__ nt, int K,
+                            int64_t ts_group, const int64_t* __restrict__ nn, const float* __restrict__ nt, int K,
                             const int32_t* __restrict__ sel, int d, int de, const float* __restrict__ time_w,
-                            const float* __restrict__ time_b, float* __restrict__ dh_new, float* __restrict__ g_w,
-                            float* __restrict__ g_b) {
+                            const float* __restrict__ time_b, float* __restrict__ dh_new,
+                            float* __restrict__ d_key_rows, float* __restrict__ g_w, float* __restrict__ g_b) {
   extern __shared__ float acc_smem[];          // [2][d]: block partial sums of g_w, g_b
   float* s_w = acc_smem;
   float* s_b = acc_smem + d;
@@ -452,12 +472,17 @@ train_attn_build_bwd_kernel(const float* __restrict__ dkv_in, const float* __res
     if (r < n_kv) {
       const int64_t i = r / K;
       const int64_t nid = nn[r];
-      if (nid == 0) continue;               // padding slot: probability 0, no gradient (and no time gradient)
       const float* g = dkv_in + r * C;
-      const int32_t row = sel[nid];
-      if (row >= 0)
-        for (int c = lane; c < d; c += 32) atomicAdd(dh_new + (int64_t)row * d + c, g[c]);
-      const float dt = ts[i % batch] - nt[r];
+      if (d_key_rows != nullptr) {
+        for (int c = lane; c < d; c += 32) d_key_rows[r * d + c] = nid == 0 ? 0.f : g[c];
+      }
+      if (nid == 0) continue;               // padding slot: probability 0, no gradient (and no time gradient)
+      if (d_key_rows == nullptr) {
+        const int32_t row = sel[nid];
+        if (row >= 0)
+          for (int c = lane; c < d; c += 32) atomicAdd(dh_new + (int64_t)row * d + c, g[c]);
+      }
+      const float dt = ts[(ts_group == 1 ? i : i / ts_group) % batch] - nt[r];
       for (int c = lane; c < d; c += 32) {
         const float v = -sin_reduced(__fadd_rn(__fmul_rn(dt, time_w[c]), time_b[c])) * g[d + de + c];
         atomicAdd(s_w + c, v * dt);
@@ -482,22 +507,34 @@ train_attn_build_bwd_kernel(const float* __restrict__ dkv_in, const float* __res
   }
 }
 
-extern "C" int tiger_train_attn_build_bwd(const float* dkv_in, const float* dq_in, const float* dcat, int64_t ld_cat,
-                                          int cat_off, const int64_t* center, int64_t n_q, const float* ts,
-                                          int64_t batch, const int64_t* neigh_nids, const float* neigh_ts, int k,
-                                          const int32_t* sel, int d, int de, const float* time_w, const float* time_b,
-                                          float* dh_new, float* g_time_w, float* g_time_b, void* stream) {
+extern "C" int tiger_train_attn_build_bwd_ex(const float* dkv_in, const float* dq_in, const float* dcat,
+                                             int64_t ld_cat, int cat_off, const int64_t* center, int64_t n_q,
+                                             const float* ts, int64_t batch, int64_t ts_group,
+                                             const int64_t* neigh_nids, const float* neigh_ts, int k,
+                                             const int32_t* sel, int d, int de, const float* time_w,
+                                             const float* time_b, float* dh_new, float* d_key_rows, float* g_time_w,
+                                             float* g_time_b, void* stream) {
   if (dkv_in == nullptr || dq_in == nullptr || dcat == nullptr || center == nullptr || ts == nullptr ||
       neigh_nids == nullptr || neigh_ts == nullptr || sel == nullptr || dh_new == nullptr || g_time_w == nullptr ||
-      g_time_b == nullptr || n_q < 0 || batch <= 0 || k <= 0 || d <= 0 || de <= 0)
+      g_time_b == nullptr || n_q < 0 || batch <= 0 || ts_group <= 0 || k <= 0 || d <= 0 || de <= 0)
     return TIGER_EINVAL;
   if (n_q == 0) return TIGER_OK;
   int64_t grid = (n_q * (k + 1) + 7) / 8;
   if (grid > 148 * 2) grid = 148 * 2;
   train_attn_build_bwd_kernel<<<(unsigned)grid, 256, 2 * d * sizeof(float), as_stream(stream)>>>(
-      dkv_in, dq_in, dcat, ld_cat, cat_off, center, n_q, ts, batch, neigh_nids, neigh_ts, k, sel, d, de, time_w, time_b,
-      dh_new, g_time_w, g_time_b);
+      dkv_in, dq_in, dcat, ld_cat, cat_off, center, n_q, ts, batch, ts_group, neigh_nids, neigh_ts, k, sel, d, de,
+      time_w, time_b, dh_new, d_key_rows, g_time_w, g_time_b);
   return tiger_launch_status();
+}
+
+extern "C" int tiger_train_attn_build_bwd(const float* dkv_in, const float* dq_in, const float* dcat, int64_t ld_cat,
+                                          int cat_off, const int64_t* center, int64_t n_q, const float* ts,
+                                          int64_t batch, const int64_t* neigh_nids, const float* neigh_ts, int k,
+                                          const int32_t* sel, int d, int de, const float* time_w, const float* time_b,
+                                          float* dh_new, float* g_time_w, float* g_time_b, void* stream) {
+  return tiger_train_attn_build_bwd_ex(dkv_in, dq_in, dcat, ld_cat, cat_off, center, n_q, ts, batch, 1, neigh_nids,
+                                       neigh_ts, k, sel, d, de, time_w, time_b, dh_new, nullptr, g_time_w, g_time_b,
+                                       stream);
 }
 
 // ------------------------------------------------------------------------------------------

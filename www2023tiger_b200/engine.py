@@ -191,11 +191,8 @@ class TigerEngine:
                         ts32_out=self.ts32, bitmap=self.bitmap,
                         out=(self.neigh_nids, self.neigh_eids, self.neigh_ts, None))
         if self.n_layers == 2:
-            # collate_memory_nodes' second call: each hop-1 neighbor queried at its own float32 event time, widened
-            # to float64 (an exact conversion), marking the same bitmap
-            self.neigh_ts64.copy_(self.neigh_ts.view(-1))
-            ops.find_recent(self.csr, self.neigh_nids.view(-1), self.neigh_ts64, self.K, want_dirs=False,
-                            bitmap=self.bitmap, out=(self.neigh2_nids, self.neigh2_eids, self.neigh2_ts, None))
+            ops.find_second_hop(self.csr, self.neigh_nids, self.neigh_ts, self.K, ts64=self.neigh_ts64,
+                                bitmap=self.bitmap, out=(self.neigh2_nids, self.neigh2_eids, self.neigh2_ts))
 
     def launch_model(self, with_scorer: bool = True):
         d, B = self.d, self.B

@@ -73,6 +73,15 @@ def find_recent(csr: DeviceCSR, q_nids: Tensor, q_ts: Tensor, k: int, *, ts_peri
     return o_n, o_e, o_t, o_d
 
 
+def find_second_hop(csr: DeviceCSR, nn1: Tensor, nt1: Tensor, k: int, *, ts64: Tensor, bitmap: Tensor,
+                    out: Tuple[Tensor, Tensor, Tensor]):
+    """collate_memory_nodes' second neighbor call for n_layers = 2: the K most recent neighbors of each hop-1 neighbor
+    nn1 [n, K] at its own float32 event time nt1, widened to float64 (an exact conversion) in `ts64` [n*K]; marks the
+    same involved-node bitmap as the first hop."""
+    ts64.copy_(nt1.view(-1))
+    find_recent(csr, nn1.view(-1), ts64, k, want_dirs=False, bitmap=bitmap, out=(*out, None))
+
+
 def hit_window(center: Tensor, neigh: Tensor) -> Tensor:
     check_cuda(center, neigh)
     n, k = neigh.shape

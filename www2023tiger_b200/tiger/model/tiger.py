@@ -391,7 +391,7 @@ class TIGER(TIGE):
         TIGER_AUTOGRAD_ROUTE=1, the comparison route of the tests) trains through the torch-op route below."""
         import os
         from .restarters import SeqRestarter, StaticRestarter
-        return (torch.is_grad_enabled() and self.training and self._fusable() and self.n_layers == 1
+        return (torch.is_grad_enabled() and self.training and self._fusable()
                 and isinstance(self.restarter_fn, (SeqRestarter, StaticRestarter))
                 and os.environ.get('TIGER_AUTOGRAD_ROUTE') != '1')
 

@@ -16,6 +16,9 @@ Step (B events, K neighbors; all data-dependent counts stay on the device):
             -> message build + store, left write-back
   backward  scorer -> merger -> out-projection -> attention core -> q / k / v products -> scatter onto the GRU rows
             and TimeEncode gradients -> GRU gates -> GRU weight gradients; restarter backward
+With n_layers = 2 the attention is two chains (temporal_agg_modules.py:79-104): depth 1 (fns.1) embeds the 3BK hop-1
+neighbors over the second hop, depth 2 (fns.0) the 3B batch nodes over the first hop with its slots keyed by the depth-1
+output.  Backward runs depth 2 (slot gradients into the depth-1 output's gradient), then depth 1, then the GRU.
   update    [gradient all-reduce] -> Adam (zeroes the gradient buffer for the next step)
 Dense products: ops.sgemm_ex (tcgen05, tf32x3): y = x W^T, dx = dy W, dW += dy^T x on the tensors as stored.
 """
@@ -135,6 +138,18 @@ def _linear_fwd(x, w, b, out, *, m, relu=False, m_count=None, per=1):
     ops.sgemm_big(x, w, out, m=m, n=w.shape[0], k=w.shape[1], bias=b, relu=relu, m_count=m_count, rows_per_count=per)
 
 
+class _AttnLayer:
+    """Activations (kept for backward) and gradients of one attention chain of the step: nq queries, K slots each."""
+
+    def __init__(self, nq: int, K: int, H: int, d: int, E: int, C: int, z):
+        self.q_in, self.kv_in, self.cat = z(nq, E), z(nq * K, C), z(nq, E + d)
+        self.Qp, self.KV, self.attn = z(nq, E), z(nq * K, 2 * E), z(nq, E)
+        self.P, self.keep, self.empty = z(nq * H * K), z(nq * H, dt=i32), z(nq, dt=u8)
+        self.hid, self.z = z(nq, d), z(nq, d)
+        self.dz, self.dhid, self.dcat, self.dattn = z(nq, d), z(nq, d), z(nq, E + d), z(nq, E)
+        self.dQ, self.dKV, self.dkv_in, self.dq_in = z(nq, E), z(nq * K, 2 * E), z(nq * K, C), z(nq, E)
+
+
 def _linear_bwd(dy, x, w, gw, gb, dx, *, m, count=None, per=1, accumulate_dx=False):
     """dy [m, n], x [m, k], w [n, k]: gw += dy^T x, gb += colsum(dy), dx (=|+=) dy w.  `count` bounds m on the device."""
     n, k = w.shape
@@ -154,9 +169,9 @@ class NativeTrainer:
         # reference's drivers see it) and as `www2023tiger_b200.tiger`
         kind = lambda o: type(o).__name__
         if not (kind(model.msg_transform_fn) == 'IdentityMessageFunction' and kind(model.right_mem_updater) == 'GRUUpdater'
-                and model.n_layers == 1 and model.hit_type in ('bin', 'none')):
+                and model.n_layers in (1, 2) and model.hit_type in ('bin', 'none')):
             raise NotImplementedError('native training covers the default operator variants '
-                                      '(tsfm_fn id, upd_fn gru, n_layers 1, hit_type bin|none)')
+                                      '(tsfm_fn id, upd_fn gru, n_layers 1|2, hit_type bin|none)')
         self.model = model
         # a static restarter owns a time encoder it never uses (restarters.py:17-33,254-277): never stepped (group 3)
         static = type(model.restarter_fn).__name__ == 'StaticRestarter'
@@ -172,9 +187,12 @@ class NativeTrainer:
         self.p_attn = float(fn.dropout)
         self.p_score = float(model.score_fn.dropout.p)
         B, K, d, E, C, M = self.B, self.K, self.d, self.E, self.C, self.M
-        self.cap = cap = 3 * B * (K + 1)
-        z = lambda *s, dt=f32: torch.zeros(*s, dtype=dt, device=dev)
         N = model.n_nodes
+        self.n_layers = model.n_layers
+        # involved-node capacity as in TigerEngine / _Workspace: with the second hop the 3BK hop-1 neighbors are
+        # queries too, and no list holds more than the N distinct nodes
+        self.cap = cap = 3 * B * (K + 1) if self.n_layers == 1 else min((3 * B + 3 * B * K) * (K + 1), N)
+        z = lambda *s, dt=f32: torch.zeros(*s, dtype=dt, device=dev)
         # --- compaction scratch
         self.bitmap = z(ops.bitmap_words(N), dt=i32)
         self.involved, self.outdated = z(cap, dt=i64), z(cap, dt=i64)
@@ -186,14 +204,9 @@ class NativeTrainer:
         self.Gi, self.Gh, self.dGi, self.dGh = z(cap, 3 * d), z(cap, 3 * d), z(cap, 3 * d), z(cap, 3 * d)
         self.h_new, self.dh_new = z(cap, d), z(cap, d)
         self.r, self.zg, self.n = z(cap, d), z(cap, d), z(cap, d)
-        # --- attention
-        nq = 3 * B
-        self.q_in, self.kv_in, self.cat = z(nq, E), z(nq * K, C), z(nq, E + d)
-        self.Qp, self.KV, self.attn = z(nq, E), z(nq * K, 2 * E), z(nq, E)
-        self.P, self.keep, self.empty = z(nq * self.H * K), z(nq * self.H, dt=i32), z(nq, dt=u8)
-        self.hid, self.z = z(nq, d), z(nq, d)
-        self.dz, self.dhid, self.dcat, self.dattn = z(nq, d), z(nq, d), z(nq, E + d), z(nq, E)
-        self.dQ, self.dKV, self.dkv_in, self.dq_in = z(nq, E), z(nq * K, 2 * E), z(nq * K, C), z(nq, E)
+        # --- attention: fns.0 over the batch nodes; with two layers fns.1 over their 3BK neighbors (depth 1)
+        self.att = _AttnLayer(3 * B, K, self.H, d, E, C, z)
+        self.att1 = _AttnLayer(3 * B * K, K, self.H, d, E, C, z) if self.n_layers == 2 else None
         # --- steps 4-6
         self.winner = z(2 * B, dt=u8)
         self.hprev_left, self.hprev_right = z(2 * B, d), z(2 * B, d)
@@ -241,7 +254,8 @@ class NativeTrainer:
         m = self.model
         B = len(src)
         assert B <= self.B
-        nn_, ne_, nt_ = cg.layers[1]
+        nn_, ne_, nt_ = cg.layers[self.n_layers]        # the batch nodes' neighbors
+        hop2 = cg.layers[1] if self.n_layers == 2 else None
         batch_nids = torch.cat([src, dst, neg]).contiguous()
         ts = ts.to(f32).contiguous()
         # pending set of the involved nodes (tiger.py:206-209)
@@ -257,13 +271,14 @@ class NativeTrainer:
                 hist = tuple(t.contiguous() for t in (rd.hist_nids, rd.hist_eids, rd.hist_ts, rd.hist_dirs,
                                                       rd.anonymized_ids))
             targets = dict(nids=rd.nids.contiguous(), index=rd.index.contiguous(), n=rd.nids.numel(), count=None, hist=hist)
-        return self._core(B, batch_nids, ts, eids.contiguous(), nn_, ne_, nt_, hits=hits, hits_from_table=False,
+        return self._core(B, batch_nids, ts, eids.contiguous(), nn_, ne_, nt_, hop2, hits=hits, hits_from_table=False,
                           targets=targets, train=train)
 
-    def _core(self, B, batch_nids, ts, eids, nn_, ne_, nt_, *, hits, hits_from_table, targets, train):
-        """Steps 1-7 of TIGE.contrast_learning + the restarter targets, after the involved / pending compaction."""
+    def _core(self, B, batch_nids, ts, eids, nn_, ne_, nt_, hop2, *, hits, hits_from_table, targets, train):
+        """Steps 1-7 of TIGE.contrast_learning + the restarter targets, after the involved / pending compaction.
+        hop2: (nids, eids, ts) [3BK, K] of the second hop with n_layers = 2, else None."""
         m = self.model
-        K, H, d, de, E, C, M, cap = self.K, self.H, self.d, self.de, self.E, self.C, self.M, self.cap
+        K, d, de, M, cap = self.K, self.d, self.de, self.M, self.cap
         nq = 3 * B
         P = self.fp.p
         self.n_steps += 1
@@ -284,23 +299,17 @@ class NativeTrainer:
         _linear_fwd(self.Hs, P[c + 'weight_hh'], P[c + 'bias_hh'], self.Gh, m=cap, m_count=cnt_o)
         call('tiger_train_gru_gates', ptr(self.Gi), ptr(self.Gh), ptr(self.Hs), ptr(cnt_o), cap, d, ptr(self.h_new),
              ptr(self.r), ptr(self.zg), ptr(self.n))
-        # ---- step 3: temporal attention (temporal_agg_modules.py:29-83,210-235)
-        a = 'temporal_embedding_fn.fns.0.'
+        # ---- step 3: temporal attention (temporal_agg_modules.py:29-104,210-235)
         tw, tb = P['time_encoder.basis_freq'], P['time_encoder.phase']
-        call('tiger_train_attn_build', ptr(batch_nids), nq, ptr(ts), B, ptr(nn_), ptr(ne_), ptr(nt_), K, ptr(right.vals),
-             ptr(self.h_new), ptr(self.gru_row), ptr(fg.nfeats), ptr(fg.efeats), d, de, ptr(tw), ptr(tb), ptr(self.q_in),
-             ptr(self.kv_in), ptr(self.cat), E + d, E)
-        in_b = P[a + 'mha_fn.in_proj_bias']
-        _linear_fwd(self.q_in, P[a + 'mha_fn.q_proj_weight'], in_b[:E], self.Qp, m=nq)
-        _linear_fwd(self.kv_in, P[a + 'mha_fn.k_proj_weight'], in_b[E:2 * E], self.KV[:, :E], m=nq * K)
-        _linear_fwd(self.kv_in, P[a + 'mha_fn.v_proj_weight'], in_b[2 * E:], self.KV[:, E:], m=nq * K)
-        hd = E // H
-        call('tiger_train_attn_core', ptr(self.Qp), E, ptr(self.KV), ptr(self.KV[:, E:]), 2 * E, ptr(nn_), nq, K, H, hd,
-             p_attn, seed, ptr(self.attn), E, ptr(self.P), ptr(self.keep), ptr(self.empty))
-        _linear_fwd(self.attn, P[a + 'mha_fn.out_proj.weight'], P[a + 'mha_fn.out_proj.bias'], self.cat[:, :E], m=nq)
-        call('tiger_train_zero_rows', ptr(self.cat), E + d, E, nq, ptr(self.empty))
-        _linear_fwd(self.cat, P[a + 'merger.fc1.weight'], P[a + 'merger.fc1.bias'], self.hid, m=nq, relu=True)
-        _linear_fwd(self.hid, P[a + 'merger.fc2.weight'], P[a + 'merger.fc2.bias'], self.z, m=nq)
+        key_rows = None
+        if hop2 is not None:
+            # depth 1 (fns.1): the 3BK hop-1 neighbors at their parent event's time over the second hop; its own
+            # dropout seed (stream 2 of the seed_stream convention, stream 1 is the lazy restart's)
+            n2, e2, t2 = hop2
+            self._attn_fwd(self.att1, 1, nn_, nq * K, ts, B, K, n2, e2, t2, None, p_attn,
+                           (seed + 7919 * 2) & 0x7fffffff)
+            key_rows = self.att1.z
+        self._attn_fwd(self.att, 0, batch_nids, nq, ts, B, 1, nn_, ne_, nt_, key_rows, p_attn, seed)
         # ---- step 4 + restarter targets (tiger.py:230-251), no grad
         winner = self.winner[:2 * B]
         ops.select_latest(pos, ts, want_unique=False, winner=winner, want_count=False)
@@ -308,7 +317,7 @@ class NativeTrainer:
                             store.node_msg_ts, store.has_msg, left.vals, self.hprev_left, self.hprev_right, self.err)
         # ---- step 7: link scorer (tiger.py:259-288)
         use_hits = hits is not None or hits_from_table
-        call('tiger_train_score_build', ptr(self.z), ptr(hits), ptr(nn_) if hits_from_table else None,
+        call('tiger_train_score_build', ptr(self.att.z), ptr(hits), ptr(nn_) if hits_from_table else None,
              ptr(batch_nids) if hits_from_table else None, K, ptr(P['hit_embedding.weight']) if use_hits else None, B, d,
              ptr(self.pair), ptr(self.codes) if use_hits else None)
         s = 'score_fn.'
@@ -333,10 +342,31 @@ class NativeTrainer:
         ops.store_messages(batch_nids[:B], batch_nids[B:2 * B], eids, ts, winner, msg_mem.vals, msg_mem.update_ts,
                            fg.nfeats, fg.efeats, d, de, tw, tb, store.node_msg_vals, store.node_msg_ts, store.has_msg,
                            self.err)
-        ops.left_writeback(pos, B, winner, self.z, d, ts, left.vals, left.update_ts, left.active_mask, self.err)
-        self._ctx = dict(B=B, batch_nids=batch_nids, ts=ts, nn=nn_, nt=nt_, hits=use_hits, targets=targets,
+        ops.left_writeback(pos, B, winner, self.att.z, d, ts, left.vals, left.update_ts, left.active_mask, self.err)
+        self._ctx = dict(B=B, batch_nids=batch_nids, ts=ts, nn=nn_, nt=nt_, hop2=hop2, hits=use_hits, targets=targets,
                          p_attn=p_attn, p_score=p_score, seed=seed, keepalive=(ne_, hits, eids))
         return self.closs, self.mloss
+
+    def _attn_fwd(self, L: _AttnLayer, fn: int, center, nq, ts, B, ts_group, nn_, ne_, nt_, key_rows, p_attn, seed):
+        """One TemporalAttention (temporal_embedding_fn.fns.<fn>) of nq queries with dropout p_attn."""
+        m, P = self.model, self.fp.p
+        K, H, d, de, E = self.K, self.H, self.d, self.de, self.E
+        fg = m.raw_feat_getter
+        a = f'temporal_embedding_fn.fns.{fn}.'
+        call('tiger_train_attn_build_ex', ptr(center), nq, ptr(ts), B, ts_group, ptr(nn_), ptr(ne_), ptr(nt_), K,
+             ptr(m.right_memory.vals), ptr(self.h_new), ptr(key_rows), ptr(self.gru_row), ptr(fg.nfeats),
+             ptr(fg.efeats), d, de, ptr(P['time_encoder.basis_freq']), ptr(P['time_encoder.phase']), ptr(L.q_in),
+             ptr(L.kv_in), ptr(L.cat), E + d, E)
+        in_b = P[a + 'mha_fn.in_proj_bias']
+        _linear_fwd(L.q_in, P[a + 'mha_fn.q_proj_weight'], in_b[:E], L.Qp, m=nq)
+        _linear_fwd(L.kv_in, P[a + 'mha_fn.k_proj_weight'], in_b[E:2 * E], L.KV[:, :E], m=nq * K)
+        _linear_fwd(L.kv_in, P[a + 'mha_fn.v_proj_weight'], in_b[2 * E:], L.KV[:, E:], m=nq * K)
+        call('tiger_train_attn_core', ptr(L.Qp), E, ptr(L.KV), ptr(L.KV[:, E:]), 2 * E, ptr(nn_), nq, K, H, E // H,
+             p_attn, seed, ptr(L.attn), E, ptr(L.P), ptr(L.keep), ptr(L.empty))
+        _linear_fwd(L.attn, P[a + 'mha_fn.out_proj.weight'], P[a + 'mha_fn.out_proj.bias'], L.cat[:, :E], m=nq)
+        call('tiger_train_zero_rows', ptr(L.cat), E + d, E, nq, ptr(L.empty))
+        _linear_fwd(L.cat, P[a + 'merger.fc1.weight'], P[a + 'merger.fc1.bias'], L.hid, m=nq, relu=True)
+        _linear_fwd(L.hid, P[a + 'merger.fc2.weight'], P[a + 'merger.fc2.bias'], L.z, m=nq)
 
     # ------------------------------------------------------------------ device-resident stream (bench / DDP loop)
     def attach_stream(self, csr: ops.DeviceCSR, hist_len: int = 40):
@@ -348,6 +378,10 @@ class NativeTrainer:
         z = lambda *s, dt=f32: torch.zeros(*s, dtype=dt, device=dev)
         self.csr, self.L = csr, hist_len
         self.nn_, self.ne_, self.nt_ = z(3 * B, K, dt=i64), z(3 * B, K, dt=i64), z(3 * B, K)
+        self.hop2 = None
+        if self.n_layers == 2:        # the second hop: float64 query times of the hop-1 neighbors, the [3BK, K] table
+            self.nt64 = z(3 * B * K, dt=torch.float64)
+            self.hop2 = (z(3 * B * K, K, dt=i64), z(3 * B * K, K, dt=i64), z(3 * B * K, K))
         self.ts32 = z(B)
         self.uptodate = z(m.n_nodes, dt=u8)
         self.restart_nodes = z(cap, dt=i64)
@@ -377,6 +411,8 @@ class NativeTrainer:
         #      restart sets) ----
         ops.find_recent(self.csr, batch_nids, ts64, K, ts_period=B, want_dirs=False, ts32_out=self.ts32,
                         bitmap=self.bitmap, out=(self.nn_, self.ne_, self.nt_, None))
+        if self.hop2 is not None:
+            ops.find_second_hop(self.csr, self.nn_, self.nt_, K, ts64=self.nt64, bitmap=self.bitmap, out=self.hop2)
         ops.compact_involved(self.bitmap, m.n_nodes, self.involved, self.counts, has_msg=store.has_msg,
                              uptodate=self.uptodate if lazy_restart else None, outdated=self.outdated,
                              gru_row=self.gru_row, restart_nodes=self.restart_nodes if lazy_restart else None,
@@ -417,7 +453,7 @@ class NativeTrainer:
             ops.anonymized_reindex(hn, out=an, count=self.t_count)
             hist = self.t_hist
         targets = dict(nids=self.t_uniq, index=self.t_index, n=2 * B, count=self.t_count, hist=hist)
-        return self._core(B, batch_nids, self.ts32, eids, self.nn_, self.ne_, self.nt_, hits=None,
+        return self._core(B, batch_nids, self.ts32, eids, self.nn_, self.ne_, self.nt_, self.hop2, hits=None,
                           hits_from_table=(m.hit_type == 'bin'), targets=targets, train=train)
 
     # ------------------------------------------------------------------ CUDA-graph replay of the stream step
@@ -508,11 +544,11 @@ class NativeTrainer:
         ctx = self._ctx
         assert ctx is not None, 'backward() needs a forward()'
         self._ctx = None
-        B, K, H, d, de, E, C, M, cap = ctx['B'], self.K, self.H, self.d, self.de, self.E, self.C, self.M, self.cap
+        B, K, d, cap = ctx['B'], self.K, self.d, self.cap
         nq = 3 * B
         P, G = self.fp.p, self.fp.g
         cnt_o = self.counts[1:]
-        s, a, c = 'score_fn.', 'temporal_embedding_fn.fns.0.', 'right_mem_updater.cell.'
+        s, c = 'score_fn.', 'right_mem_updater.cell.'
         # ---- restarter
         tg = ctx['targets']
         if tg is not None and g_mutual != 0.0:
@@ -529,36 +565,23 @@ class NativeTrainer:
              B, d, ctx['p_score'], ptr(self.dhid_s), ptr(G[s + 'fc2.weight']), ptr(G[s + 'fc2.bias']))
         _linear_bwd(self.dhid_s, self.pair, P[s + 'fc1.weight'], G[s + 'fc1.weight'], G[s + 'fc1.bias'], self.dpair,
                     m=2 * B)
-        call('tiger_train_score_build_bwd', ptr(self.dpair), ptr(self.codes) if ctx['hits'] else None, B, d, ptr(self.dz),
-             ptr(G['hit_embedding.weight']) if ctx['hits'] else None)
-        # ---- merger (MergeLayer: fc2(relu(fc1([out | c]))))
-        _linear_bwd(self.dz, self.hid, P[a + 'merger.fc2.weight'], G[a + 'merger.fc2.weight'], G[a + 'merger.fc2.bias'],
-                    self.dhid, m=nq)
-        call('tiger_train_relu_bwd', ptr(self.dhid), d, ptr(self.hid), d, d, nq, None, 1, 1.0)
-        _linear_bwd(self.dhid, self.cat, P[a + 'merger.fc1.weight'], G[a + 'merger.fc1.weight'],
-                    G[a + 'merger.fc1.bias'], self.dcat, m=nq)
-        call('tiger_train_zero_rows', ptr(self.dcat), E + d, E, nq, ptr(self.empty))
-        # ---- out-projection, attention core
-        dout = self.dcat[:, :E]
-        _linear_bwd(dout, self.attn, P[a + 'mha_fn.out_proj.weight'], G[a + 'mha_fn.out_proj.weight'],
-                    G[a + 'mha_fn.out_proj.bias'], self.dattn, m=nq)
-        hd = E // H
-        call('tiger_train_attn_core_bwd', ptr(self.dattn), E, ptr(self.Qp), E, ptr(self.KV), ptr(self.KV[:, E:]), 2 * E,
-             ptr(self.P), ptr(self.keep), nq, K, H, hd, ctx['p_attn'], ptr(self.dQ), ptr(self.dKV), ptr(self.dKV[:, E:]))
-        g_in_b = G[a + 'mha_fn.in_proj_bias']
-        _linear_bwd(self.dQ, self.q_in, P[a + 'mha_fn.q_proj_weight'], G[a + 'mha_fn.q_proj_weight'], g_in_b[:E],
-                    self.dq_in, m=nq)
-        _linear_bwd(self.dKV[:, :E], self.kv_in, P[a + 'mha_fn.k_proj_weight'], G[a + 'mha_fn.k_proj_weight'],
-                    g_in_b[E:2 * E], self.dkv_in, m=nq * K)
-        _linear_bwd(self.dKV[:, E:], self.kv_in, P[a + 'mha_fn.v_proj_weight'], G[a + 'mha_fn.v_proj_weight'],
-                    g_in_b[2 * E:], self.dkv_in, m=nq * K, accumulate_dx=True)
-        if comm is not None:
-            comm('attention')
-        # ---- representation gradients back onto the GRU rows, TimeEncode gradients
-        call('tiger_train_attn_build_bwd', ptr(self.dkv_in), ptr(self.dq_in), ptr(self.dcat), E + d, E,
-             ptr(ctx['batch_nids']), nq, ptr(ctx['ts']), B, ptr(ctx['nn']), ptr(ctx['nt']), K, ptr(self.gru_row), d, de,
-             ptr(P['time_encoder.basis_freq']), ptr(P['time_encoder.phase']), ptr(self.dh_new),
-             ptr(G['time_encoder.basis_freq']), ptr(G['time_encoder.phase']))
+        call('tiger_train_score_build_bwd', ptr(self.dpair), ptr(self.codes) if ctx['hits'] else None, B, d,
+             ptr(self.att.dz), ptr(G['hit_embedding.weight']) if ctx['hits'] else None)
+        # ---- attention weight gradients, then the representation gradients back onto the GRU rows (+ TimeEncode
+        #      gradients).  Two layers: depth 2's slot gradients are depth 1's output gradient, and the attention slice
+        #      of the gradient buffer is complete only after depth 1's weight gradients
+        hop2 = ctx['hop2']
+        self._attn_bwd(self.att, 0, nq, ctx['p_attn'])
+        if hop2 is None:
+            if comm is not None:
+                comm('attention')
+            self._build_bwd(self.att, ctx['batch_nids'], nq, ctx['ts'], B, 1, ctx['nn'], ctx['nt'], None)
+        else:
+            self._build_bwd(self.att, ctx['batch_nids'], nq, ctx['ts'], B, 1, ctx['nn'], ctx['nt'], self.att1.dz)
+            self._attn_bwd(self.att1, 1, nq * K, ctx['p_attn'])
+            if comm is not None:
+                comm('attention')
+            self._build_bwd(self.att1, ctx['nn'], nq * K, ctx['ts'], B, K, hop2[0], hop2[2], None)
         # ---- GRU (inputs are detached messages / memory buffers: weight gradients only)
         call('tiger_train_gru_gates_bwd', ptr(self.dh_new), ptr(self.r), ptr(self.zg), ptr(self.n), ptr(self.Gh),
              ptr(self.Hs), ptr(cnt_o), cap, d, ptr(self.dGi), ptr(self.dGh))
@@ -568,6 +591,39 @@ class NativeTrainer:
                     count=cnt_o)
         if comm is not None:
             comm('gru')
+
+    def _attn_bwd(self, L: _AttnLayer, fn: int, nq: int, p_attn: float):
+        """Backward of one TemporalAttention from L.dz: merger (MergeLayer: fc2(relu(fc1([out | c])))),
+        out-projection, core, q / k / v products -> weight gradients, L.dq_in, L.dkv_in, L.dcat."""
+        K, H, d, E = self.K, self.H, self.d, self.E
+        P, G = self.fp.p, self.fp.g
+        a = f'temporal_embedding_fn.fns.{fn}.'
+        _linear_bwd(L.dz, L.hid, P[a + 'merger.fc2.weight'], G[a + 'merger.fc2.weight'], G[a + 'merger.fc2.bias'],
+                    L.dhid, m=nq)
+        call('tiger_train_relu_bwd', ptr(L.dhid), d, ptr(L.hid), d, d, nq, None, 1, 1.0)
+        _linear_bwd(L.dhid, L.cat, P[a + 'merger.fc1.weight'], G[a + 'merger.fc1.weight'], G[a + 'merger.fc1.bias'],
+                    L.dcat, m=nq)
+        call('tiger_train_zero_rows', ptr(L.dcat), E + d, E, nq, ptr(L.empty))
+        _linear_bwd(L.dcat[:, :E], L.attn, P[a + 'mha_fn.out_proj.weight'], G[a + 'mha_fn.out_proj.weight'],
+                    G[a + 'mha_fn.out_proj.bias'], L.dattn, m=nq)
+        call('tiger_train_attn_core_bwd', ptr(L.dattn), E, ptr(L.Qp), E, ptr(L.KV), ptr(L.KV[:, E:]), 2 * E, ptr(L.P),
+             ptr(L.keep), nq, K, H, E // H, p_attn, ptr(L.dQ), ptr(L.dKV), ptr(L.dKV[:, E:]))
+        g_in_b = G[a + 'mha_fn.in_proj_bias']
+        _linear_bwd(L.dQ, L.q_in, P[a + 'mha_fn.q_proj_weight'], G[a + 'mha_fn.q_proj_weight'], g_in_b[:E], L.dq_in,
+                    m=nq)
+        _linear_bwd(L.dKV[:, :E], L.kv_in, P[a + 'mha_fn.k_proj_weight'], G[a + 'mha_fn.k_proj_weight'],
+                    g_in_b[E:2 * E], L.dkv_in, m=nq * K)
+        _linear_bwd(L.dKV[:, E:], L.kv_in, P[a + 'mha_fn.v_proj_weight'], G[a + 'mha_fn.v_proj_weight'],
+                    g_in_b[2 * E:], L.dkv_in, m=nq * K, accumulate_dx=True)
+
+    def _build_bwd(self, L: _AttnLayer, center, nq, ts, B, ts_group, nn_, nt_, d_key_rows):
+        """Row-builder backward: representation gradients onto dh_new (slots into d_key_rows when given), TimeEncode
+        gradients."""
+        P, G, d, E = self.fp.p, self.fp.g, self.d, self.E
+        call('tiger_train_attn_build_bwd_ex', ptr(L.dkv_in), ptr(L.dq_in), ptr(L.dcat), E + d, E, ptr(center), nq,
+             ptr(ts), B, ts_group, ptr(nn_), ptr(nt_), self.K, ptr(self.gru_row), d, self.de,
+             ptr(P['time_encoder.basis_freq']), ptr(P['time_encoder.phase']), ptr(self.dh_new), ptr(d_key_rows),
+             ptr(G['time_encoder.basis_freq']), ptr(G['time_encoder.phase']))
 
     # ------------------------------------------------------------------ whole step
     def step(self, src, dst, neg, ts, eids, cg, *, mutual_coef: float = 1.0, contrast_only: bool = False,
