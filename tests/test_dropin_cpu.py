@@ -81,3 +81,22 @@ def test_ap_and_auc_equal_sklearn():
             label, score = label[keep], score[keep]
         assert abs(average_precision_score(label, score) - metrics.average_precision_score(label, score)) < 1e-12
         assert abs(roc_auc_score(label, score) - metrics.roc_auc_score(label, score)) < 1e-12
+
+
+@pytest.mark.parametrize('K,restarter,hist_len,match', [(40, 'static', 8, 'at most 32 neighbors'),
+                                                        (10, 'seq', 70, 'at most 64 events'),
+                                                        (33, 'seq', 8, 'n_neighbors=33')])
+def test_native_trainer_refuses_sizes_past_its_kernels(K, restarter, hist_len, match):
+    """The attention core keeps one dropout bit per slot in 32 bits and the seq pool stages at most 64 positions:
+    NativeTrainer refuses such models at construction (before it allocates anything), and the drop-in's route
+    choice sends them to the torch-op route."""
+    from www2023tiger_b200.init import build_model
+    from www2023tiger_b200.train import NativeTrainer, native_limit_error
+    model = build_model(None, torch.zeros(50, 6), None, 40, 49, torch.device('cpu'), dim=None, n_neighbors=K,
+                        restarter_type=restarter, hist_len=hist_len)
+    assert match in native_limit_error(model)
+    with pytest.raises(NotImplementedError, match=match):
+        NativeTrainer(model, 10)
+    ok = build_model(None, torch.zeros(50, 6), None, 40, 49, torch.device('cpu'), dim=None, n_neighbors=32,
+                     restarter_type=restarter, hist_len=64)
+    assert native_limit_error(ok) is None

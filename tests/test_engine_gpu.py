@@ -132,6 +132,35 @@ def test_engine_matches_oracle_on_stream(gu, shape, msg_src, upd_src, lazy, rest
                 shape.name + ' final ')
 
 
+@pytest.mark.parametrize('K', [20, 40])
+def test_engine_matches_oracle_at_wide_neighborhoods(gu, K):
+    """K = 20 (the keyword default of TIGE / TIGER) and K = 40 (past one softmax value per lane), eager steps."""
+    B, H, n_batches, start = 100, 2, 8, 1500
+    st = make_stream(StreamShape('k', 300, 60, 4000, 16, None), seed=K)
+    neg = NegativeSampler(st.src, st.dst, seed=0).pre_sample_neg_dsts(st.n_events)
+    N, d = st.n_nodes, st.dim
+    W = perturb_biases(random_weights(d, d, n_nodes=N, restarter='static', nonzero_static=True, seed=1))
+    graph, model = gu.oracle_from(W, st.src, st.dst, st.ts, st.eids, N=N, dim=d, efeats=st.efeats, nfeats=None,
+                                  K=K, H=H, msg_src='left', upd_src='right', restarter='static')
+    outs = run_oracle(model, graph, st, neg, B, K, n_batches, True, start)
+    csr = gu.device_csr(st.src, st.dst, st.ts, st.eids, N)
+    e = gu.engine_from(W, csr, N=N, dim=d, efeats=st.efeats, nfeats=None, K=K, H=H, B=B, msg_src='left',
+                       upd_src='right', restarter='static', lazy_restart=True)
+    for ib in range(n_batches):
+        lo = start + ib * B
+        e.set_batch(st.src[lo:lo + B], st.dst[lo:lo + B], neg[lo:lo + B], st.ts[lo:lo + B], st.eids[lo:lo + B])
+        e.step()
+        o, what = outs[ib], f'K={K} batch {ib} '
+        assert_close(gu.cpu(e.scores[:B]), o['pos_scores'].numpy(), TOL, what + 'pos')
+        assert_close(gu.cpu(e.scores[B:]), o['neg_scores'].numpy(), TOL, what + 'neg')
+        assert_close(gu.cpu(e.loss).reshape(1), o['loss'].reshape(1).numpy(), TOL, what + 'loss')
+        assert_close(gu.cpu(e.emb), o['h_left_with_negs'].numpy(), TOL, what + 'emb')
+    e.check_errors()
+    check_state(gu, e, model.left_vals.numpy(), model.right_vals.numpy(), model.left_ts.numpy(),
+                model.right_ts.numpy(), model.msg_vals.numpy(), model.msg_ts.numpy(), np.nonzero(model.has_msg)[0],
+                f'K={K} final ')
+
+
 def test_invariant_flags_raise_like_the_reference(gu):
     st = make_stream(StreamShape('e', 100, 20, 2000, 8, None, horizon=1000.), seed=4)
     N, d, B, K = st.n_nodes, 8, 50, 5

@@ -7,6 +7,7 @@ import torch
 from oracle import tiger_oracle as O
 from golden_utils import CASES, Golden, assert_close
 from www2023tiger_b200 import ops
+from www2023tiger_b200._lib import TigerLibraryError
 from www2023tiger_b200.init import perturb_biases, random_weights
 from www2023tiger_b200.synthetic import StreamShape, make_stream
 
@@ -249,6 +250,45 @@ def test_temporal_attention_dense_matches_oracle(gu, d, de, n, k, H):
     got = ops.temporal_attention_dense(pack, H, gu.dev(qx), gu.dev(qt), gu.dev(kx), gu.dev(ky), gu.dev(kt),
                                        gu.dev(mask))
     assert_close(gu.cpu(got), want.numpy(), TOL, f'attention dense d={d} de={de} n={n}')
+
+
+def _dense_attention(gu, d, de, n, k, H, seed):
+    W = perturb_biases(random_weights(d, de, seed=seed))
+    g = torch.Generator().manual_seed(seed)
+    qx, qt = torch.randn(n, d, generator=g), torch.randn(n, d, generator=g)
+    kx, ky, kt = torch.randn(n, k, d, generator=g), torch.randn(n, k, de, generator=g), torch.randn(n, k, d, generator=g)
+    mask = torch.rand(n, k, generator=g) < 0.3
+    mask[::7] = True
+    mask[1::7, :-1] = True
+    mask[2::7, 1:] = True                # only the first slot live
+    p = 'temporal_embedding_fn.fns.0.'
+    pack = ops.AttnPack(d, de, 'cuda', H)
+    m = p + 'mha_fn.'
+    pack.refresh(*(gu.dev(W[x]) for x in (m + 'q_proj_weight', m + 'k_proj_weight', m + 'v_proj_weight',
+                                            m + 'in_proj_bias', m + 'out_proj.weight', m + 'out_proj.bias',
+                                            p + 'merger.fc1.weight', p + 'merger.fc1.bias', p + 'merger.fc2.weight',
+                                            p + 'merger.fc2.bias', 'time_encoder.basis_freq', 'time_encoder.phase')))
+    got = lambda: ops.temporal_attention_dense(pack, H, gu.dev(qx), gu.dev(qt), gu.dev(kx), gu.dev(ky), gu.dev(kt),
+                                               gu.dev(mask))
+    return got, lambda: O.temporal_attention(W, p, H, qx, qt, kx, ky, kt, mask)
+
+
+@pytest.mark.parametrize('H,d,de', [(1, 16, 6), (2, 16, 6), (4, 16, 6), (3, 12, 8)])
+@pytest.mark.parametrize('k', [1, 20, 32, 33, 64])
+def test_temporal_attention_dense_matches_oracle_at_every_k(gu, k, H, d, de):
+    """K up to ATT_MAXK = 64 (past 32 the softmax holds two values per lane); H = 3 is the generic (HT = 0) launch."""
+    got, want = _dense_attention(gu, d, de, 90, k, H, seed=k * 10 + H)
+    assert_close(gu.cpu(got()), want().numpy(), TOL, f'attention dense k={k} H={H}')
+
+
+def test_temporal_attention_dense_at_k64_baseline_width_and_k65_refusal(gu):
+    """d = de = 172 at K = 64: the largest shared-memory footprint the kernel takes (about 135 KB, under its 200 KB
+    refusal); K = 65 is refused."""
+    got, want = _dense_attention(gu, 172, 172, 40, 64, 2, seed=5)
+    assert_close(gu.cpu(got()), want().numpy(), TOL, 'attention dense k=64 d=172')
+    got, _ = _dense_attention(gu, 16, 6, 10, 65, 2, seed=6)
+    with pytest.raises(TigerLibraryError, match='invalid argument'):
+        got()
 
 
 # ------------------------------------------------------------------ step 7: scorer

@@ -385,3 +385,78 @@ def test_stream_step_graph_replay_matches_eager_launches(restarter):
     tc.reset_stream()
     lc = np.array([[float(x) for x in tc.step_stream(rec[i], mutual_coef=1.0, grad_scale=1.0)] for i in range(rec.shape[0])])
     assert np.abs(lc - la).max() > 10 * np.abs(lb - la).max()
+
+
+# ------------------------------------------------------------------------------------------
+# neighborhoods and head counts past the goldens', and the sizes the native step refuses
+# ------------------------------------------------------------------------------------------
+def synthetic_setup(K, H, restarter, hist_len=8):
+    from www2023tiger_b200.synthetic import NegativeSampler, StreamShape, make_stream
+    st = make_stream(StreamShape('kh', 200, 40, 3000, 16, None, horizon=3000.), seed=K + H)
+    neg = NegativeSampler(st.src, st.dst, seed=0).pre_sample_neg_dsts(st.n_events)
+    full = InteractionData(st.src, st.dst, st.ts, st.eids, np.zeros_like(st.src), seed=0, eval=True, neg_dst=neg)
+    graph = Graph.from_data(full, strategy='recent_edges', seed=0, max_node_id=st.n_nodes - 1)
+    coll = GraphCollator(graph, K, 1, restarter=restarter, hist_len=hist_len)
+
+    def make():
+        m = D.init_model(None, st.efeats, graph, st.n_nodes, st.n_events, DEV, dim=None, n_layers=1, n_heads=H,
+                         n_neighbors=K, hit_type='bin', dropout=0.0, restarter_type=restarter, hist_len=hist_len,
+                         msg_src='left', upd_src='right')
+        m.train()
+        return m
+    batch = lambda lo, B: to_dev(coll([full[i] for i in range(lo, lo + B)]))
+    return make, batch
+
+
+@pytest.mark.parametrize('restarter', ['seq', 'static'])
+@pytest.mark.parametrize('K,H', [(20, 2), (7, 4), (32, 1)])
+def test_native_step_matches_autograd_route_at_other_k_and_heads(K, H, restarter, monkeypatch):
+    """K = 20 (the keyword default of TIGE / TIGER) runs its own attention-core instantiation, K = 7 and 32 the generic
+    one (32: every bit of keep_bits), with 1, 2 and 4 heads."""
+    torch.manual_seed(K + H)
+    make, batch = synthetic_setup(K, H, restarter)
+    native, ref = make(), make()
+    ref.load_state_dict(native.state_dict())
+    native.reset(), ref.reset()
+    B = 80
+    for ib in range(4):
+        b = batch(1200 + ib * B, B)
+        native.zero_grad(set_to_none=True)
+        c1, m1 = native.contrast_and_mutual_learning(*b)
+        assert type(c1.grad_fn).__name__.startswith('_NativeStep')
+        (c1 + m1).backward()
+        monkeypatch.setenv('TIGER_AUTOGRAD_ROUTE', '1')
+        ref.zero_grad(set_to_none=True)
+        c2, m2 = ref.contrast_and_mutual_learning(*b)
+        (c2 + m2).backward()
+        monkeypatch.delenv('TIGER_AUTOGRAD_ROUTE')
+        what = f'K={K} H={H} {restarter} b{ib}'
+        assert_close(cpu(c1).reshape(1), cpu(c2).reshape(1), 1e-5, what + ' contrast')
+        assert_close(cpu(m1).reshape(1), cpu(m2).reshape(1), 2e-5, what + ' mutual')
+        assert [p.grad is None for _, p in unique_named_params(native)] == \
+            [p.grad is None for _, p in unique_named_params(ref)], what
+        check_grads({k: grad_of(p) for k, p in unique_named_params(native)},
+                    {k: grad_of(p) for k, p in unique_named_params(ref)}, what)
+    native._trainer.check_errors()
+
+
+@pytest.mark.parametrize('K,restarter,hist_len', [(40, 'static', 8), (10, 'seq', 70)])
+def test_models_past_the_native_limits_train_through_the_torch_op_route(K, restarter, hist_len):
+    """More than 32 neighbors, or a seq restarter history longer than 64: the drop-in trains such a model through the
+    torch-op route instead of failing inside the native step."""
+    from www2023tiger_b200.train import NativeTrainer
+    torch.manual_seed(0)
+    make, batch = synthetic_setup(K, 2, restarter, hist_len=hist_len)
+    model = make()
+    model.reset()
+    with pytest.raises(NotImplementedError):
+        NativeTrainer(model, 80)
+    assert not model._native_training()
+    model.zero_grad(set_to_none=True)
+    c, m = model.contrast_and_mutual_learning(*batch(1200, 80))
+    assert c.grad_fn is not None and not type(c.grad_fn).__name__.startswith('_NativeStep')
+    (c + m).backward()
+    assert getattr(model, '_trainer', None) is None
+    grads = [p.grad for p in model.parameters() if p.grad is not None]
+    assert grads and all(bool(torch.isfinite(g).all()) for g in grads)
+    assert model.time_encoder.basis_freq.grad is not None and float(model.time_encoder.basis_freq.grad.abs().max()) > 0

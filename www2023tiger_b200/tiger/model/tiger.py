@@ -388,11 +388,14 @@ class TIGER(TIGE):
     # ---- native training step (www2023tiger_b200/train.py) ----
     def _native_training(self) -> bool:
         """The hand-written training step covers the reference's default operator variants; anything else (and
-        TIGER_AUTOGRAD_ROUTE=1, the comparison route of the tests) trains through the torch-op route below."""
+        TIGER_AUTOGRAD_ROUTE=1, the comparison route of the tests) trains through the torch-op route below, and so do
+        models past the native step's sizes (more than 32 neighbors, a seq restarter history longer than 64)."""
         import os
+        from www2023tiger_b200.train import native_limit_error
         from .restarters import SeqRestarter, StaticRestarter
         return (torch.is_grad_enabled() and self.training and self._fusable()
                 and isinstance(self.restarter_fn, (SeqRestarter, StaticRestarter))
+                and native_limit_error(self) is None
                 and os.environ.get('TIGER_AUTOGRAD_ROUTE') != '1')
 
     def native_trainer(self, batch_size: int, **kw):

@@ -126,6 +126,25 @@ def _seed_step_word(device) -> Tensor:
     return _SEED_WORDS[idx]
 
 
+# Largest neighborhood and seq-restarter history the training kernels take: the attention core keeps one dropout bit
+# per slot in a 32-bit word (ATT_MAXK, csrc/train.cu), the seq pool stages at most 64 positions (SP_MAXL,
+# csrc/train_seq.cu).  Larger models train through the torch-op route, which has neither limit.
+MAX_NEIGHBORS = 32
+MAX_HIST_LEN = 64
+
+
+def native_limit_error(model) -> Optional[str]:
+    """Why the native step cannot train `model` at its sizes, or None when it can."""
+    if model.n_neighbors > MAX_NEIGHBORS:
+        return (f'native training takes at most {MAX_NEIGHBORS} neighbors per query (the attention core keeps one '
+                f'dropout bit per slot in a 32-bit word); this model has n_neighbors={model.n_neighbors}')
+    r = model.restarter_fn
+    if type(r).__name__ == 'SeqRestarter' and r.hist_len > MAX_HIST_LEN:
+        return (f'native training takes a seq restarter history of at most {MAX_HIST_LEN} events; this model has '
+                f'hist_len={r.hist_len}')
+    return None
+
+
 def _param_group(name: str) -> int:
     if name.startswith('right_mem_updater.'):
         return 1
@@ -172,6 +191,9 @@ class NativeTrainer:
                 and model.n_layers in (1, 2) and model.hit_type in ('bin', 'none')):
             raise NotImplementedError('native training covers the default operator variants '
                                       '(tsfm_fn id, upd_fn gru, n_layers 1|2, hit_type bin|none)')
+        limit = native_limit_error(model)
+        if limit is not None:
+            raise NotImplementedError(limit)
         self.model = model
         # a static restarter owns a time encoder it never uses (restarters.py:17-33,254-277): never stepped (group 3)
         static = type(model.restarter_fn).__name__ == 'StaticRestarter'
