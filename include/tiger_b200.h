@@ -176,20 +176,6 @@ int tiger_left_writeback(const int64_t* pos_ids, int64_t n_pos, int64_t batch, c
                          uint8_t* left_active, uint32_t* err_flags, void* stream);
 
 /* ---------------------------------------------------------------------------------------
- * Parameter packing: kernels read weights from k-major ("transposed") copies so that
- * consecutive threads read consecutive addresses.  Re-run whenever the weights change.
- * ------------------------------------------------------------------------------------- */
-
-/* out[k*ld_out + n] = w[n*ld_in + k] for k<cols, n<rows; columns n in [rows, pad_rows) are zeroed;
- * columns >= pad_rows are left untouched (several blocks can share one packed row). */
-int tiger_transpose_pad(const float* w, int64_t rows, int64_t cols, int64_t ld_in, float* out,
-                        int64_t ld_out, int64_t pad_rows, void* stream);
-
-/* out[r*ld_out + c] = w[r*ld_in + c] for c<cols, zero for c in [cols, ld_out). */
-int tiger_copy_pad(const float* w, int64_t rows, int64_t cols, int64_t ld_in, float* out,
-                   int64_t ld_out, void* stream);
-
-/* ---------------------------------------------------------------------------------------
  * Dense operators
  * ------------------------------------------------------------------------------------- */
 
@@ -217,8 +203,8 @@ int tiger_gru_update(const int64_t* node_ids, const int32_t* count, int64_t n_ro
 /* temporal-attention parameters (device pointers): the reference's tensors as stored
  * (temporal_embedding_fn.fns.0.*), plus one caller-allocated buffer for the folded weights.
  * E = 2d, C = 2d + de, hd = E / n_head. */
-/* Optional fusion of update_left_memory (tiger.py:408-420, tiger_left_writeback below) into the last product of
- * tiger_temporal_attention: the rows p < n_pos of the result whose winner[p] != 0 are also written to
+/* Fusion of update_left_memory (tiger.py:408-420, tiger_left_writeback below) into the last product of
+ * tiger_temporal_attention_ex: the rows p < n_pos of the result whose winner[p] != 0 are also written to
  * left_vals[pos_ids[p]], with left_ts[...] = ts[p % batch] (error flag if the stored clock is later) and
  * left_active[...] = 1 - the embeddings are persisted by the kernel that produces them.  ready_event (a
  * cudaEvent_t, may be NULL) is waited for on the stream in front of that product: it must cover the producer of
@@ -250,9 +236,11 @@ typedef struct {
   const float* time_w;   /* [d] time_encoder.basis_freq                                     */
   const float* time_b;   /* [d] time_encoder.phase                                          */
   float* folded;         /* tiger_attn_fold_bytes() bytes, 16-byte aligned, filled by tiger_attn_fold */
-  float* score_folded;   /* optional: tiger_score_fold blob - the last GEMM then also emits the scorer terms  */
-  float* pq_out;         /* optional per-call output [n_query][2d]: P = W1a z | Q = W1b z (with score_folded) */
-  const tiger_left_writeback_fused* left_wb;   /* optional, see above (gather form only) */
+  /* The fused last product of the batch-node depth: either all three of the following are set, and only for
+   * tiger_temporal_attention_ex, or all three are NULL (TIGER_EINVAL otherwise). */
+  float* score_folded;   /* tiger_score_fold blob - the last GEMM then also emits the scorer terms              */
+  float* pq_out;         /* per-call output [n_query][2d]: P = W1a z | Q = W1b z                               */
+  const tiger_left_writeback_fused* left_wb;   /* see above                                                   */
 } tiger_attn_params;
 
 /* Folds the projections that are linear in the per-query vectors (exact by linearity, accumulated in
@@ -280,19 +268,10 @@ int64_t tiger_temporal_attention_work_bytes(int64_t n_query, int k, int d, int d
  * Wqk, masked softmax, pooled keys) -> folded value / out projection + merger MLP on the tensor
  * cores, as the launch sequence described in csrc/attention.cu.
  * Node representations: row(u) = sel[u] >= 0 ? rows_b[sel[u]] : rows_a[u]
- *   fused engine : rows_a = right memory, rows_b = GRU output, sel = gru_row
+ *   fused routes : rows_a = right memory, rows_b = GRU output, sel = gru_row
  *   class surface: rows_a = NULL, rows_b = involved_node_reprs, sel = local_index
- * sel is int32 when sel_is_i64==0, int64 otherwise.  q_ts has ts_period entries (ts.repeat(3)).
- * out [n_query, d]. */
-int tiger_temporal_attention(const int64_t* center_nids, const float* q_ts, int64_t n_query,
-                             int64_t ts_period, const int64_t* neigh_nids, const int64_t* neigh_eids,
-                             const float* neigh_ts, int k, const float* rows_a, const float* rows_b,
-                             const void* sel, int sel_is_i64, const float* nfeats,
-                             const float* efeats, int d, int de, int n_head,
-                             const tiger_attn_params* params, float* out, void* work, void* stream);
-
-/* The same layer for any depth of a multi-layer embedding (tiger_temporal_attention is this entry point with
- * ts_group = 1 and key_rows = NULL):
+ * sel is int32 when sel_is_i64==0, int64 otherwise.  out [n_query, d].  Any depth of a multi-layer embedding
+ * (one layer: ts_group = 1, key_rows = NULL):
  *   query q reads q_ts[(q / ts_group) % ts_period]: the depth-1 queries of n_layers = 2 are the K neighbors
  *     of each of the 3B batch nodes at the parent event's time, ts_group = K, ts_period = B
  *     (repeat_interleave(ts.repeat(3), K)).
@@ -315,17 +294,10 @@ int tiger_temporal_attention_dense(const float* qx, const float* qt, const float
                                    int d, int de, int n_head, const tiger_attn_params* params, float* out,
                                    void* work, void* stream);
 
-/* step 7 of TIGE.contrast_learning (tiger.py:259-288), hit_type 'bin' or 'none': hit flags
- * from the neighbor table, hit embedding, score_fn MergeLayer on positive / negative pairs,
- * BCE-with-logits mean.  h [3B,d] = embeddings of [src;dst;neg]; neigh_nids [3B,K] (may be
- * NULL when hit_emb is NULL).  fc1T [2d][ldD] k-major (ldD = d rounded up to 4), fc2_w [d].  scores [2B] = pos then neg. */
-int tiger_link_score(const float* h, int64_t batch, int d, const int64_t* src, const int64_t* dst,
-                     const int64_t* neg, const int64_t* neigh_nids, int k, const float* hit_emb,
-                     const float* fc1T, const float* fc1_b, const float* fc2_w, const float* fc2_b,
-                     float* scores, float* loss, uint32_t* done_counter, void* stream);
-
-/* Folded form of the same step (see tiger_score_fold): pq [3B][2d] = [W1a z | W1b z] rows of [src ; dst ; neg]
- * from tiger_temporal_attention, cab = blob + tiger_score_fold_cab_offset(d); neigh_nids NULL = hit_type 'none'. */
+/* step 7 of TIGE.contrast_learning (tiger.py:259-288), hit_type 'bin' or 'none': hit flags from the neighbor table
+ * [3B][K], hit embedding, score_fn MergeLayer on positive / negative pairs, BCE-with-logits mean; scores [2B] = pos
+ * then neg.  Folded form (see tiger_score_fold): pq [3B][2d] = [W1a z | W1b z] rows of [src ; dst ; neg]
+ * from tiger_temporal_attention_ex, cab = blob + tiger_score_fold_cab_offset(d); neigh_nids NULL = hit_type 'none'. */
 int tiger_link_score_folded(const float* pq, int64_t batch, int d, const int64_t* src, const int64_t* dst,
                             const int64_t* neg, const int64_t* neigh_nids, int k, const float* cab,
                             const float* fc2_w, const float* fc2_b, float* scores, float* loss,
@@ -419,14 +391,6 @@ int tiger_sgemm_nt_packed(const float* A, int64_t lda, const float* wpack, int b
                           int64_t ldc, int64_t m_rows, const int32_t* count, int64_t rows_per_count, int n_cols,
                           int k_dim, float alpha, int relu, void* stream);
 
-/* Same with a split output: the pack has ceil((n_split + n_cols1) / bn) tiles; result columns [0, n_cols0)
- * go to C, columns [n_split, n_split + n_cols1) to C2 (n_split a multiple of 16 >= n_cols0; bias is indexed
- * in the padded column space). */
-int tiger_sgemm_nt_packed_split(const float* A, int64_t lda, const float* wpack, int bn, const float* bias,
-                                float* C, int64_t ldc, int n_cols0, float* C2, int64_t ldc2, int n_split,
-                                int n_cols1, int64_t m_rows, const int32_t* count, int64_t rows_per_count,
-                                int k_dim, float alpha, int relu, void* stream);
-
 /* Same with a gathered A operand: row m of A is row sel[ids[m]] of rows_b when that index is >= 0 (or rows_a
  * is NULL), else row ids[m] of rows_a, plus row ids[m] of add_rows when given - the "latest representation of
  * node u" lookup of compute_embedding_with_computation_graph (temporal_agg_modules.py:210-235: memory row or
@@ -438,8 +402,10 @@ int tiger_sgemm_nt_packed_gather(const int64_t* ids, const void* sel, int sel_is
                                  const int32_t* count, int64_t rows_per_count, int n_cols, int k_dim, float alpha,
                                  int relu, void* stream);
 
-/* tiger_sgemm_nt_packed / _packed_split (C2 may be NULL here) with the fused row scatter described at
- * tiger_left_writeback_fused: result rows are additionally stored into a node-indexed table. */
+/* tiger_sgemm_nt_packed with the fused row scatter described at tiger_left_writeback_fused: result rows are
+ * additionally stored into a node-indexed table.  With C2 (may be NULL) the output is split: the pack has
+ * ceil((n_split + n_cols1) / bn) tiles; result columns [0, n_cols0) go to C, columns [n_split, n_split + n_cols1) to
+ * C2 (n_split a multiple of 16 >= n_cols0; bias is indexed in the padded column space). */
 int tiger_sgemm_nt_packed_scatter(const float* A, int64_t lda, const float* wpack, int bn, const float* bias, float* C,
                                   int64_t ldc, int n_cols0, float* C2, int64_t ldc2, int n_split, int n_cols1,
                                   int64_t m_rows, int k_dim, const tiger_left_writeback_fused* wb, void* stream);
@@ -479,7 +445,7 @@ int tiger_pipe_join(void* pipe, void* stream);
  * train_self_supervised.py:165-171 and train_self_supervised_ddp.py:203-208 run through autograd.  Dense products
  * go through tiger_sgemm_ex; gradients accumulate into caller-owned buffers that tiger_train_adam zeroes.
  *   gather_pending / gru_gates[_bwd]   compute_messages + GRUUpdater (tiger.py:292-356, update_modules.py:30-37)
- *   attn_build[_bwd][_ex] / attn_core[_bwd] compute_embedding_with_computation_graph + TemporalAttention with
+ *   attn_build[_bwd]_ex / attn_core[_bwd]   compute_embedding_with_computation_graph + TemporalAttention with
  *                                      dropout (temporal_agg_modules.py:29-104,210-235), either depth of n_layers = 2,
  *                                      TimeEncode gradients
  *   score_build[_bwd] / score_head[_bwd] hit embedding + score_fn + BCE (tiger.py:259-288)
@@ -490,9 +456,8 @@ int tiger_pipe_join(void* pipe, void* stream);
 int tiger_train_gather_pending(const int64_t* ids, const int32_t* count, int64_t cap, const float* msg_vals, int m_dim, const float* msg_ts, const float* upd_vals, int d, const float* check_mem_ts, int check_equal, float* X, float* H, float* dh_zero, uint32_t* err_flags, float* n_rows_out, void* stream);
 int tiger_train_gru_gates(const float* Gi, const float* Gh, const float* H, const int32_t* count, int64_t cap, int d, float* h_new, float* r_out, float* z_out, float* n_out, void* stream);
 int tiger_train_gru_gates_bwd(const float* dh, const float* r_in, const float* z_in, const float* n_in, const float* Gh, const float* H, const int32_t* count, int64_t cap, int d, float* dGi, float* dGh, void* stream);
-int tiger_train_attn_build(const int64_t* center, int64_t n_q, const float* ts, int64_t batch, const int64_t* neigh_nids, const int64_t* neigh_eids, const float* neigh_ts, int k, const float* rows_a, const float* rows_b, const int32_t* sel, const float* nfeats, const float* efeats, int d, int de, const float* time_w, const float* time_b, float* q_in, float* kv_in, float* cat, int64_t ld_cat, int cat_off, void* stream);
-/* attn_build[_bwd]_ex: the same builders for either depth of n_layers = 2 (attn_build[_bwd] are these with ts_group = 1
- * and key_rows / d_key_rows = NULL), the training twins of tiger_temporal_attention_ex:
+/* attn_build[_bwd]_ex: the builders for either depth of n_layers = 2 (one layer: ts_group = 1 and key_rows / d_key_rows
+ * = NULL), the training twins of tiger_temporal_attention_ex:
  *   query i's time is ts[(i / ts_group) % batch] (depth 1: ts_group = K, repeat_interleave(ts.repeat(3), K));
  *   key_rows [n_q * K][d] (NULL: the rows above): slot r takes key_rows[r] as its node part, no node features added
  *     (depth 2: the depth-1 output);
@@ -502,7 +467,6 @@ int tiger_train_attn_build(const int64_t* center, int64_t n_q, const float* ts, 
 int tiger_train_attn_build_ex(const int64_t* center, int64_t n_q, const float* ts, int64_t batch, int64_t ts_group, const int64_t* neigh_nids, const int64_t* neigh_eids, const float* neigh_ts, int k, const float* rows_a, const float* rows_b, const float* key_rows, const int32_t* sel, const float* nfeats, const float* efeats, int d, int de, const float* time_w, const float* time_b, float* q_in, float* kv_in, float* cat, int64_t ld_cat, int cat_off, void* stream);
 int tiger_train_attn_core(const float* Q, int64_t ldq, const float* Kp, const float* Vp, int64_t ldkv, const int64_t* neigh_nids, int64_t n_q, int k, int n_head, int head_dim, float p_drop, int seed, float* attn, int64_t ld_attn, float* P, uint32_t* keep_bits, uint8_t* empty, void* stream);
 int tiger_train_attn_core_bwd(const float* dattn, int64_t ld_attn, const float* Q, int64_t ldq, const float* Kp, const float* Vp, int64_t ldkv, const float* P, const uint32_t* keep_bits, int64_t n_q, int k, int n_head, int head_dim, float p_drop, float* dQ, float* dKp, float* dVp, void* stream);
-int tiger_train_attn_build_bwd(const float* dkv_in, const float* dq_in, const float* dcat, int64_t ld_cat, int cat_off, const int64_t* center, int64_t n_q, const float* ts, int64_t batch, const int64_t* neigh_nids, const float* neigh_ts, int k, const int32_t* sel, int d, int de, const float* time_w, const float* time_b, float* dh_new, float* g_time_w, float* g_time_b, void* stream);
 int tiger_train_attn_build_bwd_ex(const float* dkv_in, const float* dq_in, const float* dcat, int64_t ld_cat, int cat_off, const int64_t* center, int64_t n_q, const float* ts, int64_t batch, int64_t ts_group, const int64_t* neigh_nids, const float* neigh_ts, int k, const int32_t* sel, int d, int de, const float* time_w, const float* time_b, float* dh_new, float* d_key_rows, float* g_time_w, float* g_time_b, void* stream);
 int tiger_train_zero_rows(float* buf, int64_t ld, int cols, int64_t n_rows, const uint8_t* flag, void* stream);
 int tiger_train_relu_bwd(float* dy, int64_t ld_dy, const float* y, int64_t ld_y, int cols, int64_t n_rows, const int32_t* count, int64_t rows_per_count, float scale, void* stream);

@@ -145,6 +145,31 @@ def test_dropin_replays_reference_golden(name):
         assert len(model.msg_store.nodes_with_messages) == 0
 
 
+def test_fused_route_detaches_the_score_fold_and_left_writeback():
+    """The fused route attaches the score fold and the left write-back to the pack of fns.0 for its last attention
+    product only.  The step-by-step route's graph-form call uses the same pack: afterwards it must write neither the
+    left memory nor pq."""
+    g = Golden('seq_left_right')
+    full, graph, coll, dl, model = setup(g)
+    assert g.n_layers == 1
+    src, dst, neg, ts, eids, cg = to_dev(next(iter(dl)))
+    model.eval()
+    model.reset()
+    with torch.no_grad():
+        model.contrast_learning(src, dst, neg, ts, eids, cg)
+        s = model.temporal_embedding_fn.fns[0].packed(model.time_encoder).struct
+        assert s.left_wb is None and s.score_folded is None and s.pq_out is None
+        left = model.left_memory
+        before = [t.clone() for t in (left.vals, left.update_ts, left.active_mask, model._ws.pq)]
+        # representations unlike the fused call's, so that a leaked attachment would change what it writes
+        reprs = model.right_memory.vals[cg.computation_graph_nodes] + 1.0
+        model.temporal_embedding_fn.compute_embedding_with_computation_graph(
+            reprs, torch.cat([src, dst, neg]), ts.repeat(3), cg)
+        after = (left.vals, left.update_ts, left.active_mask, model._ws.pq)
+        for a, b, what in zip(after, before, ('left vals', 'left ts', 'left active', 'pq')):
+            assert torch.equal(a, b), what
+
+
 @pytest.mark.parametrize('name', ['seq_left_right', 'static_right_right_dim10'])
 def test_autograd_route_equals_fused_route_and_trains(name):
     """Training-mode forward (torch autograd ops, dropout 0) must agree with the fused kernel route on the

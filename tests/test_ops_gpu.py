@@ -292,15 +292,28 @@ def test_temporal_attention_dense_at_k64_baseline_width_and_k65_refusal(gu):
 
 
 # ------------------------------------------------------------------ step 7: scorer
+@pytest.mark.parametrize('hit_type', ['bin', 'none'])
 @pytest.mark.parametrize('d,B,k', [(172, 200, 10), (100, 37, 10), (10, 25, 5)])
-def test_link_score_matches_oracle(gu, d, B, k):
+def test_link_score_folded_matches_oracle(gu, d, B, k, hit_type):
+    """The folded scorer: the batch nodes' attention (gather form) with the score fold and the left write-back
+    attached writes pq, tiger_link_score_folded scores the pairs from it."""
     W = perturb_biases(random_weights(d, d, seed=B))
     g = torch.Generator().manual_seed(B)
-    h = torch.randn(3 * B, d, generator=g)
-    src, dst, neg = (torch.randint(1, 40, (B,), generator=g) for _ in range(3))
-    neigh = torch.randint(0, 40, (3 * B, k), generator=g)
-    x, y, ny = h.reshape(3, B, d)
-    emb = W['hit_embedding.weight']
+    N, E, H = 40, 300, 2
+    rows, efeats = torch.randn(N, d, generator=g), torch.randn(E, d, generator=g)
+    src, dst, neg = (torch.randint(1, N, (B,), generator=g) for _ in range(3))
+    centers = torch.cat([src, dst, neg])
+    neigh = torch.randint(0, N, (3 * B, k), generator=g)            # id 0: padding slot
+    neigh[::9] = 0                                                  # rows without a live slot
+    neigh_e = torch.randint(0, E, (3 * B, k), generator=g)
+    ts = torch.rand(B, generator=g) * 100 + 100
+    neigh_ts = ts.repeat(3)[:, None] - torch.rand(3 * B, k, generator=g) * 100
+    p = 'temporal_embedding_fn.fns.0.'
+    tw, tb = W['time_encoder.basis_freq'], W['time_encoder.phase']
+    z = O.temporal_attention(W, p, H, rows[centers], O.time_encode(torch.zeros(3 * B), tw, tb), rows[neigh],
+                             efeats[neigh_e], O.time_encode(ts.repeat(3)[:, None] - neigh_ts, tw, tb), neigh == 0)
+    x, y, ny = z.reshape(3, B, d)
+    emb = W['hit_embedding.weight'] if hit_type == 'bin' else torch.zeros(2, d)
     flag = lambda c, rows: (c[:, None] == rows).any(1).long()
     xp, yp = x + emb[flag(src, neigh[B:2 * B])], y + emb[flag(dst, neigh[:B])]
     xn, yn = x + emb[flag(src, neigh[2 * B:])], ny + emb[flag(neg, neigh[:B])]
@@ -308,10 +321,31 @@ def test_link_score_matches_oracle(gu, d, B, k):
     ps, ns = O.merge_layer(xp, yp, *sw).squeeze(1), O.merge_layer(xn, yn, *sw).squeeze(1)
     loss = torch.nn.functional.binary_cross_entropy_with_logits(torch.cat([ps, ns]),
                                                                 torch.cat([torch.ones(B), torch.zeros(B)]))
-    pack = ops.ScorePack(d, 'cuda')
-    pack.refresh(*(gu.dev(t) for t in sw), gu.dev(emb))
+    pack = ops.AttnPack(d, d, 'cuda', H)
+    m = p + 'mha_fn.'
+    pack.refresh(*(gu.dev(W[n]) for n in (m + 'q_proj_weight', m + 'k_proj_weight', m + 'v_proj_weight',
+                                            m + 'in_proj_bias', m + 'out_proj.weight', m + 'out_proj.bias',
+                                            p + 'merger.fc1.weight', p + 'merger.fc1.bias', p + 'merger.fc2.weight',
+                                            p + 'merger.fc2.bias', 'time_encoder.basis_freq', 'time_encoder.phase')))
+    fold, pq = ops.ScoreFold(d, 'cuda'), torch.zeros(3 * B, 2 * d, device='cuda')
+    fold.refresh(*(gu.dev(t) for t in sw), gu.dev(W[p + 'merger.fc2.weight']), gu.dev(W[p + 'merger.fc2.bias']),
+                 gu.dev(emb) if hit_type == 'bin' else None)
+    d_centers, d_ts = gu.dev(centers), gu.dev(ts)
+    pos = d_centers[:2 * B]
+    winner = ops.select_latest(pos, d_ts, want_unique=False, want_count=False)[0]
+    left_vals, left_ts = torch.zeros(N, d, device='cuda'), torch.zeros(N, device='cuda')
+    left_active = torch.zeros(N, dtype=torch.uint8, device='cuda')
+    pack.attach_score_fold(fold, pq)
+    pack.attach_left_writeback(pos, winner, d_ts, left_vals, left_ts, left_active)
+    out = ops.temporal_attention(pack, H, d_centers, d_ts, gu.dev(neigh), gu.dev(neigh_e), gu.dev(neigh_ts),
+                                 rows_a=None, rows_b=gu.dev(rows), sel=torch.arange(N, dtype=torch.int32, device='cuda'),
+                                 nfeats=None, efeats=gu.dev(efeats))
+    assert_close(gu.cpu(out), z.numpy(), TOL, 'attention')
+    w = winner.bool()
+    assert torch.equal(left_vals[pos[w]], out[:2 * B][w]), 'fused left write-back'
     for _ in range(2):                    # twice: the done-counter must reset itself
-        scores, dl = ops.link_score(pack, gu.dev(h), gu.dev(src), gu.dev(dst), gu.dev(neg), gu.dev(neigh))
+        scores, dl = ops.link_score_folded(fold, pq, gu.dev(src), gu.dev(dst), gu.dev(neg),
+                                           gu.dev(neigh) if hit_type == 'bin' else None)
         assert_close(gu.cpu(scores), torch.cat([ps, ns]).numpy(), TOL, 'scores')
         assert_close(gu.cpu(dl), loss.reshape(1).numpy(), TOL, 'loss')
 

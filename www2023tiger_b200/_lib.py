@@ -32,15 +32,12 @@ _SIGNATURES: Dict[str, str] = {
     'tiger_store_messages_dense': 'ppppl' + 'p' + 'pppp' + 'ppii' + 'pppp' + 'pp' + 'p',
     'tiger_right_writeback': 'plp' + 'ppi' + 'pppp' + 'pppp' + 'p' + 'p',
     'tiger_left_writeback': 'pllp' + 'pip' + 'ppp' + 'p' + 'p',
-    'tiger_transpose_pad': 'plllpll' + 'p',
-    'tiger_copy_pad': 'plllpl' + 'p',
     'tiger_gru_pack_bytes': 'ii',
     'tiger_gru_pack': 'ppiip' + 'p',
     'tiger_gru_update': 'ppl' + 'plpl' + 'ii' + 'p' + 'ppp' + 'ppi' + 'p' + 'p',
     'tiger_attn_fold_bytes': 'iii',
     'tiger_attn_fold': 'piii' + 'p',
     'tiger_temporal_attention_work_bytes': 'liiii',
-    'tiger_temporal_attention': 'ppll' + 'pppi' + 'pppi' + 'pp' + 'iii' + 'ppp' + 'p',
     'tiger_temporal_attention_ex': 'pplll' + 'pppi' + 'ppppi' + 'pp' + 'iii' + 'ppp' + 'p',
     'tiger_temporal_attention_dense': 'pppppp' + 'li' + 'iii' + 'ppp' + 'p',
     'tiger_score_fold_bytes': 'i',
@@ -55,19 +52,15 @@ _SIGNATURES: Dict[str, str] = {
     'tiger_pipe_wait': 'pii',
     'tiger_pipe_join': 'pp',
     'tiger_sgemm_nt_packed_scatter': 'plpippli' + 'pliil' + 'ip' + 'p',
-    'tiger_sgemm_nt_packed_split': 'plpippli' + 'pliil' + 'pl' + 'ifi' + 'p',
-    'tiger_link_score': 'pli' + 'pppp' + 'i' + 'ppppp' + 'ppp' + 'p',
     'tiger_min_time': 'plp' + 'p',
     'tiger_seq_tokens': 'ppli' + 'ppppp' + 'ppii' + 'ppp' + 'ppp' + 'p',
     'tiger_sgemm_nt': 'plplp' + 'pl' + 'lpl' + 'iii' + 'p',
     'tiger_train_gather_pending': 'pplpippipipppppp',
     'tiger_train_gru_gates': 'pppplippppp',
     'tiger_train_gru_gates_bwd': 'ppppppplippp',
-    'tiger_train_attn_build': 'plplpppipppppiippppplip',
     'tiger_train_attn_build_ex': 'plpll' + 'pppi' + 'ppppp' + 'p' + 'ii' + 'pp' + 'ppp' + 'li' + 'p',
     'tiger_train_attn_core': 'plpplpliiifiplpppp',
     'tiger_train_attn_core_bwd': 'plplpplppliiifpppp',
-    'tiger_train_attn_build_bwd': 'pppliplplppipiipppppp',
     'tiger_train_attn_build_bwd_ex': 'pppli' + 'plpll' + 'ppi' + 'pii' + 'pp' + 'pppp' + 'p',
     'tiger_train_zero_rows': 'plilpp',
     'tiger_train_relu_bwd': 'plplilplfp',

@@ -684,22 +684,12 @@ static int attention_run(AttArgs& a, const tiger_attn_params* p, float* out, cud
   rc = tiger_sgemm_nt_packed_splitk_fused(a.w.kvc, m.ld_kvc, f.pk_w2f, ATT_BN_D, p->fc1_b, a.w.hid, m.ld_hid,
                                           ATT_KPARTS, n, nullptr, 1, m.d, m.off_live + 1, 1.0f, 1, s);
   if (rc != TIGER_OK) return rc;
-  const bool fold_scorer = p->score_folded != nullptr && p->pq_out != nullptr;
-  if (p->left_wb != nullptr && !a.dense) {
-    // last GEMM also persists the winners' embeddings into the left memory (waits for left_wb->ready_event first)
-    if (fold_scorer) {
-      const ScoreFold sf = score_fold(m.d, p->score_folded);
-      return tiger_sgemm_nt_packed_scatter(a.w.hid, m.ld_hid, sf.pack, ATT_BN_F3, sf.b3, out, m.d, m.d, p->pq_out, 2 * m.d,
-                                           sf.n_split, 2 * m.d, n, m.d, p->left_wb, s);
-    }
-    return tiger_sgemm_nt_packed_scatter(a.w.hid, m.ld_hid, f.pk_fc2, ATT_BN_F3, p->fc2_b, out, m.d, m.d, nullptr, 0, 0, 0, n,
-                                         m.d, p->left_wb, s);
-  }
-  if (fold_scorer) {
-    // last GEMM with the link-scorer fold: z -> out, [W1a z | W1b z] -> pq_out
+  if (p->left_wb != nullptr) {
+    // batch-node depth of the fused routes: the last GEMM writes z -> out and [W1a z | W1b z] -> pq_out (link-scorer
+    // fold) and persists the winners' embeddings into the left memory (waits for left_wb->ready_event first)
     const ScoreFold sf = score_fold(m.d, p->score_folded);
-    return tiger_sgemm_nt_packed_split(a.w.hid, m.ld_hid, sf.pack, ATT_BN_F3, sf.b3, out, m.d, m.d, p->pq_out, 2 * m.d,
-                                       sf.n_split, 2 * m.d, n, nullptr, 1, m.d, 1.0f, 0, s);
+    return tiger_sgemm_nt_packed_scatter(a.w.hid, m.ld_hid, sf.pack, ATT_BN_F3, sf.b3, out, m.d, m.d, p->pq_out, 2 * m.d,
+                                         sf.n_split, 2 * m.d, n, m.d, p->left_wb, s);
   }
   return tiger_sgemm_nt_packed(a.w.hid, m.ld_hid, f.pk_fc2, ATT_BN_F3, p->fc2_b, out, m.d, n, nullptr, 1, m.d, m.d, 1.0f,
                                0, s);
@@ -708,6 +698,10 @@ static int attention_run(AttArgs& a, const tiger_attn_params* p, float* out, cud
 static int attention_entry(AttArgs& a, int k, int d, int de, int n_head, const tiger_attn_params* params, float* out,
                            void* work, void* stream) {
   if (params == nullptr || params->folded == nullptr || work == nullptr) return TIGER_EINVAL;
+  // the fused last product comes whole (score fold, its pq output and the left write-back) and in the gather form only
+  const bool fused = params->left_wb != nullptr;
+  if ((fused && a.dense) || (params->score_folded != nullptr) != fused || (params->pq_out != nullptr) != fused)
+    return TIGER_EINVAL;
   if (a.n_query < 0 || k <= 0 || d <= 0 || de <= 0 || n_head <= 0 || n_head > ATT_MAXH) return TIGER_EINVAL;
   if ((2 * d) % n_head != 0 || (((uintptr_t)work) & 15) != 0) return TIGER_EINVAL;
   if (a.n_query == 0) return TIGER_OK;
@@ -731,17 +725,6 @@ extern "C" int tiger_temporal_attention_ex(const int64_t* center_nids, const flo
   a.nfeats = nfeats; a.efeats = efeats; a.dense = 0;
   a.n_query = n_query;
   return attention_entry(a, k, d, de, n_head, params, out, work, stream);
-}
-
-extern "C" int tiger_temporal_attention(const int64_t* center_nids, const float* q_ts, int64_t n_query,
-                                        int64_t ts_period, const int64_t* neigh_nids, const int64_t* neigh_eids,
-                                        const float* neigh_ts, int k, const float* rows_a, const float* rows_b,
-                                        const void* sel, int sel_is_i64, const float* nfeats, const float* efeats,
-                                        int d, int de, int n_head, const tiger_attn_params* params, float* out,
-                                        void* work, void* stream) {
-  return tiger_temporal_attention_ex(center_nids, q_ts, n_query, ts_period, 1, neigh_nids, neigh_eids, neigh_ts, k,
-                                     rows_a, rows_b, nullptr, sel, sel_is_i64, nfeats, efeats, d, de, n_head, params,
-                                     out, work, stream);
 }
 
 extern "C" int tiger_temporal_attention_dense(const float* qx, const float* qt, const float* kx, const float* ky,

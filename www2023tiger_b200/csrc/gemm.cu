@@ -874,18 +874,6 @@ extern "C" int tiger_sgemm_nt_packed(const float* A, int64_t lda, const float* w
                             stream);
 }
 
-extern "C" int tiger_sgemm_nt_packed_split(const float* A, int64_t lda, const float* wpack, int bn, const float* bias,
-                                           float* C, int64_t ldc, int n_cols0, float* C2, int64_t ldc2, int n_split,
-                                           int n_cols1, int64_t m_rows, const int32_t* count,
-                                           int64_t rows_per_count, int k_dim, float alpha, int relu, void* stream) {
-  if (C2 == nullptr) return TIGER_EINVAL;
-  return gemm_packed_launch({.A = A, .lda = lda, .wpack = wpack, .bn = bn, .bias = bias, .C = C, .ldc = ldc,
-                             .n_cols = n_cols0, .m_rows = m_rows, .count = count, .rows_per_count = rows_per_count,
-                             .k_dim = k_dim, .alpha = alpha, .relu = relu, .C2 = C2, .ldc2 = ldc2, .n_split = n_split,
-                             .n_cols1 = n_cols1},
-                            stream);
-}
-
 extern "C" int tiger_sgemm_nt_packed_scatter(const float* A, int64_t lda, const float* wpack, int bn, const float* bias,
                                              float* C, int64_t ldc, int n_cols0, float* C2, int64_t ldc2, int n_split,
                                              int n_cols1, int64_t m_rows, int k_dim, const tiger_left_writeback_fused* wb,

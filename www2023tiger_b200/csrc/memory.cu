@@ -425,43 +425,3 @@ extern "C" int tiger_left_writeback(const int64_t* pos_ids, int64_t n_pos, int64
       pos_ids, n_pos, batch, winner, h_left, d, ts, left_vals, left_ts, left_active, err_flags, rpw, tma ? 1 : 0);
   return tiger_launch_status();
 }
-
-// ---------------------------------------------------------------- parameter packing
-__global__ void transpose_pad_kernel(const float* __restrict__ w, int64_t rows, int64_t cols, int64_t ld_in,
-                                     float* __restrict__ out, int64_t ld_out, int64_t pad_rows) {
-  __shared__ float tile[32][33];
-  const int64_t n0 = (int64_t)blockIdx.x * 32, k0 = (int64_t)blockIdx.y * 32;
-  for (int i = threadIdx.y; i < 32; i += blockDim.y) {
-    const int64_t n = n0 + i, k = k0 + threadIdx.x;
-    tile[i][threadIdx.x] = (n < rows && k < cols) ? w[n * ld_in + k] : 0.f;
-  }
-  __syncthreads();
-  for (int i = threadIdx.y; i < 32; i += blockDim.y) {
-    const int64_t k = k0 + i, n = n0 + threadIdx.x;
-    if (k < cols && n < pad_rows) out[k * ld_out + n] = tile[threadIdx.x][i];
-  }
-}
-
-extern "C" int tiger_transpose_pad(const float* w, int64_t rows, int64_t cols, int64_t ld_in, float* out,
-                                   int64_t ld_out, int64_t pad_rows, void* stream) {
-  if (rows <= 0 || cols <= 0 || ld_in < cols || pad_rows < rows || ld_out < pad_rows) return TIGER_EINVAL;
-  dim3 grid((unsigned)((pad_rows + 31) / 32), (unsigned)((cols + 31) / 32));
-  transpose_pad_kernel<<<grid, dim3(32, 8), 0, as_stream(stream)>>>(w, rows, cols, ld_in, out, ld_out, pad_rows);
-  return tiger_launch_status();
-}
-
-__global__ void copy_pad_kernel(const float* __restrict__ w, int64_t rows, int64_t cols, int64_t ld_in,
-                                float* __restrict__ out, int64_t ld_out) {
-  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= rows * ld_out) return;
-  const int64_t r = i / ld_out, c = i % ld_out;
-  out[i] = c < cols ? w[r * ld_in + c] : 0.f;
-}
-
-extern "C" int tiger_copy_pad(const float* w, int64_t rows, int64_t cols, int64_t ld_in, float* out,
-                              int64_t ld_out, void* stream) {
-  if (rows <= 0 || cols <= 0 || ld_in < cols || ld_out < cols) return TIGER_EINVAL;
-  const int64_t total = rows * ld_out;
-  copy_pad_kernel<<<(unsigned)((total + 255) / 256), 256, 0, as_stream(stream)>>>(w, rows, cols, ld_in, out, ld_out);
-  return tiger_launch_status();
-}

@@ -2,181 +2,12 @@
 // hit flags ('bin': tiger.py:266-270, data_loader.py:61-75) -> hit embedding -> score_fn
 // MergeLayer (basic_modules.py:16-19) on positive and negative pairs -> BCE-with-logits mean.
 //
-// One CTA scores SCORE_GP pairs.  The fc1 weights (k-major, L2 resident) are streamed once per CTA with
-// coalesced loads; the reduction dimension (2d) is split over SCORE_KS thread groups so that
-// SCORE_KS * ceil32(d) threads are busy, each keeping SCORE_GP accumulators in registers and 8 weight
-// loads in flight (the kernel is bound by the L2 latency of that stream, not by bandwidth or FMAs).
+// Folded form (see tiger_score_fold in attention.cu): the first scorer layer was applied to every
+// embedding row by the last attention GEMM (PQ[row] = [W1a z | W1b z]); a pair (s, t) with hit flags (a, b)
+// scores  w2 . relu(P[s] + Q[t] + c_ab) + b2.  One warp per pair; the BCE mean is reduced by the last CTA
+// in a fixed order, so the loss does not depend on the order in which the CTAs finish.
 #include "common.cuh"
 
-#define SCORE_GP 8   // pairs per CTA
-#define SCORE_KS 4   // split of the reduction dimension over thread groups
-
-__global__ void __launch_bounds__(1024)
-link_score_kernel(const float* __restrict__ h, int64_t batch, int d, int dp, const int64_t* __restrict__ src,
-                  const int64_t* __restrict__ dst, const int64_t* __restrict__ neg,
-                  const int64_t* __restrict__ neigh, int k, const float* __restrict__ hit_emb,
-                  const float* __restrict__ fc1T, int ld, const float* __restrict__ fc1_b,
-                  const float* __restrict__ fc2_w, const float* __restrict__ fc2_b, float* __restrict__ scores,
-                  float* __restrict__ loss, uint32_t* __restrict__ done_counter) {
-  extern __shared__ __align__(16) float sm[];
-  float* xin = sm;                             // [2d][GP]
-  float* part = xin + 2 * d * SCORE_GP;        // [KS-1][dp][GP]  partial sums of the upper K parts
-  float* red = part + (SCORE_KS - 1) * dp * SCORE_GP;   // [warps][GP]
-  __shared__ int s_flag[SCORE_GP][2];
-  __shared__ bool s_last;
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, n_warps = blockDim.x >> 5;
-  const int64_t p0 = (int64_t)blockIdx.x * SCORE_GP;
-  const int64_t n_pairs = 2 * batch;
-  // hit flags: one warp per (pair, side)
-  for (int i = warp; i < SCORE_GP * 2; i += n_warps) {
-    const int g = i >> 1, side = i & 1;
-    const int64_t p = p0 + g;
-    int flag = 0;
-    if (p < n_pairs && hit_emb != nullptr) {
-      const bool is_neg = p >= batch;
-      const int64_t e = is_neg ? p - batch : p;
-      int64_t center, row;
-      if (!is_neg) {
-        center = side == 0 ? src[e] : dst[e];          // src_hits: src in N(dst) ; dst_hits: dst in N(src)
-        row = side == 0 ? batch + e : e;
-      } else {
-        center = side == 0 ? src[e] : neg[e];          // neg_src_hits: src in N(neg) ; neg_dst_hits: neg in N(src)
-        row = side == 0 ? 2 * batch + e : e;
-      }
-      for (int j = lane; j < k; j += 32) flag |= (neigh[row * k + j] == center);
-      flag = __any_sync(TIGER_FULL_MASK, flag);
-    }
-    if (lane == 0) s_flag[g][side] = flag;
-  }
-  __syncthreads();
-  // inputs [x + he | y + he] in [c][GP] layout
-  for (int i = tid; i < SCORE_GP * 2 * d; i += blockDim.x) {
-    const int g = i / (2 * d), c = i % (2 * d);
-    const int64_t p = p0 + g;
-    float v = 0.f;
-    if (p < n_pairs) {
-      const bool is_neg = p >= batch;
-      const int64_t e = is_neg ? p - batch : p;
-      const int side = c >= d;
-      const int cc = side ? c - d : c;
-      const int64_t row = side == 0 ? e : (is_neg ? 2 * batch + e : batch + e);
-      v = h[row * d + cc];
-      if (hit_emb != nullptr) v += hit_emb[s_flag[g][side] * d + cc];
-    }
-    xin[c * SCORE_GP + g] = v;
-  }
-  __syncthreads();
-  // hidden layer: thread (part, n) accumulates K range [part * kper, (part + 1) * kper) of output unit n
-  const int kpart = tid / dp, n = tid % dp;
-  const int kper = (2 * d + SCORE_KS - 1) / SCORE_KS;
-  float acc[SCORE_GP];
-#pragma unroll
-  for (int g = 0; g < SCORE_GP; ++g) acc[g] = 0.f;
-  if (n < d) {
-    const int c0 = kpart * kper;
-    const int c1 = (c0 + kper) < 2 * d ? (c0 + kper) : 2 * d;
-    const float* wcol = fc1T + n;
-#pragma unroll 8
-    for (int c = c0; c < c1; ++c) {
-      const float w = __ldg(wcol + (int64_t)c * ld);
-      const float4* x4 = reinterpret_cast<const float4*>(xin + c * SCORE_GP);
-#pragma unroll
-      for (int q = 0; q < SCORE_GP / 4; ++q) {
-        const float4 x = x4[q];
-        acc[4 * q + 0] = fmaf(w, x.x, acc[4 * q + 0]);
-        acc[4 * q + 1] = fmaf(w, x.y, acc[4 * q + 1]);
-        acc[4 * q + 2] = fmaf(w, x.z, acc[4 * q + 2]);
-        acc[4 * q + 3] = fmaf(w, x.w, acc[4 * q + 3]);
-      }
-    }
-    if (kpart > 0) {
-#pragma unroll
-      for (int g = 0; g < SCORE_GP; ++g) part[((kpart - 1) * dp + n) * SCORE_GP + g] = acc[g];
-    }
-  }
-  __syncthreads();
-  float out[SCORE_GP];
-#pragma unroll
-  for (int g = 0; g < SCORE_GP; ++g) out[g] = 0.f;
-  if (kpart == 0 && n < d) {
-    const float b = fc1_b[n], w2 = fc2_w[n];
-#pragma unroll
-    for (int g = 0; g < SCORE_GP; ++g) {
-      float a = acc[g];
-#pragma unroll
-      for (int q = 1; q < SCORE_KS; ++q) a += part[((q - 1) * dp + n) * SCORE_GP + g];
-      out[g] = fmaxf(a + b, 0.f) * w2;
-    }
-  }
-#pragma unroll
-  for (int g = 0; g < SCORE_GP; ++g) {
-    const float t = warp_sum(out[g]);
-    if (lane == 0) red[warp * SCORE_GP + g] = t;
-  }
-  __syncthreads();
-  if (tid < SCORE_GP && p0 + tid < n_pairs) {
-    float s = 0.f;
-    for (int w = 0; w < n_warps; ++w) s += red[w * SCORE_GP + tid];
-    scores[p0 + tid] = s + fc2_b[0];
-  }
-  if (loss == nullptr) return;
-  // last CTA reduces the BCE-with-logits mean in a fixed order
-  __threadfence();
-  __syncthreads();
-  if (tid == 0) s_last = (atomicAdd(done_counter, 1u) == gridDim.x - 1);
-  __syncthreads();
-  if (!s_last) return;
-  __threadfence();
-  float a = 0.f;
-  for (int64_t p = tid; p < n_pairs; p += blockDim.x) {
-    const float x = __ldcg(scores + p);
-    const float y = p < batch ? 1.f : 0.f;
-    a += fmaxf(x, 0.f) - x * y + log1pf(expf(-fabsf(x)));
-  }
-  a = warp_sum(a);
-  if (lane == 0) red[warp] = a;
-  __syncthreads();
-  if (tid == 0) {
-    float s = 0.f;
-    for (int w = 0; w < n_warps; ++w) s += red[w];
-    *loss = s / (float)n_pairs;
-    *done_counter = 0u;
-  }
-}
-
-extern "C" int tiger_link_score(const float* h, int64_t batch, int d, const int64_t* src, const int64_t* dst,
-                                const int64_t* neg, const int64_t* neigh_nids, int k, const float* hit_emb,
-                                const float* fc1T, const float* fc1_b, const float* fc2_w, const float* fc2_b,
-                                float* scores, float* loss, uint32_t* done_counter, void* stream) {
-  if (batch < 0 || d <= 0 || d > 256 || (hit_emb != nullptr && (neigh_nids == nullptr || k <= 0))) return TIGER_EINVAL;
-  if (loss != nullptr && done_counter == nullptr) return TIGER_EINVAL;
-  if (batch == 0) return TIGER_OK;
-  const int dp = (d + 31) / 32 * 32;
-  const int threads = SCORE_KS * dp;
-  if (threads > 1024) return TIGER_EINVAL;
-  const int ld = (d + 3) / 4 * 4;
-  const size_t smem = ((size_t)2 * d * SCORE_GP + (size_t)(SCORE_KS - 1) * dp * SCORE_GP +
-                       (size_t)(threads / 32) * SCORE_GP + 32) * sizeof(float);
-  static size_t configured = 48 * 1024;
-  if (smem > configured) {
-    if (smem > 200 * 1024 ||
-        cudaFuncSetAttribute(link_score_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
-      return TIGER_EINVAL;
-    configured = smem;
-  }
-  const unsigned grid = (unsigned)((2 * batch + SCORE_GP - 1) / SCORE_GP);
-  link_score_kernel<<<grid, threads, smem, as_stream(stream)>>>(h, batch, d, dp, src, dst, neg, neigh_nids, k,
-                                                               hit_emb, fc1T, ld, fc1_b, fc2_w, fc2_b, scores, loss,
-                                                               done_counter);
-  return tiger_launch_status();
-}
-
-// ------------------------------------------------------------------------------------------
-// Folded link scorer (see tiger_score_fold in attention.cu): the first scorer layer was applied to every
-// embedding row by the last attention GEMM (PQ[row] = [W1a z | W1b z]); a pair (s, t) with hit flags (a, b)
-// scores  w2 . relu(P[s] + Q[t] + c_ab) + b2.  One warp per pair, rows read as 16-byte vectors; the BCE mean
-// is reduced by the last CTA in a fixed order, as in link_score_kernel.
-// ------------------------------------------------------------------------------------------
 #define SCOREF_WARPS 8
 __global__ void __launch_bounds__(SCOREF_WARPS * 32)
 link_score_folded_kernel(const float* __restrict__ pq, int64_t batch, int d, const int64_t* __restrict__ src,

@@ -246,17 +246,6 @@ extern "C" int tiger_train_attn_build_ex(const int64_t* center, int64_t n_q, con
   return tiger_launch_status();
 }
 
-extern "C" int tiger_train_attn_build(const int64_t* center, int64_t n_q, const float* ts, int64_t batch,
-                                      const int64_t* neigh_nids, const int64_t* neigh_eids, const float* neigh_ts,
-                                      int k, const float* rows_a, const float* rows_b, const int32_t* sel,
-                                      const float* nfeats, const float* efeats, int d, int de, const float* time_w,
-                                      const float* time_b, float* q_in, float* kv_in, float* cat, int64_t ld_cat,
-                                      int cat_off, void* stream) {
-  return tiger_train_attn_build_ex(center, n_q, ts, batch, 1, neigh_nids, neigh_eids, neigh_ts, k, rows_a, rows_b,
-                                   nullptr, sel, nfeats, efeats, d, de, time_w, time_b, q_in, kv_in, cat, ld_cat,
-                                   cat_off, stream);
-}
-
 #define ATT_MAXK 32
 
 // One warp per (query, head).  s_j = (q_h * scale) . k_jh, padding (neighbor id 0) -> -inf, rows without any
@@ -525,16 +514,6 @@ extern "C" int tiger_train_attn_build_bwd_ex(const float* dkv_in, const float* d
       dkv_in, dq_in, dcat, ld_cat, cat_off, center, n_q, ts, batch, ts_group, neigh_nids, neigh_ts, k, sel, d, de,
       time_w, time_b, dh_new, d_key_rows, g_time_w, g_time_b);
   return tiger_launch_status();
-}
-
-extern "C" int tiger_train_attn_build_bwd(const float* dkv_in, const float* dq_in, const float* dcat, int64_t ld_cat,
-                                          int cat_off, const int64_t* center, int64_t n_q, const float* ts,
-                                          int64_t batch, const int64_t* neigh_nids, const float* neigh_ts, int k,
-                                          const int32_t* sel, int d, int de, const float* time_w, const float* time_b,
-                                          float* dh_new, float* g_time_w, float* g_time_b, void* stream) {
-  return tiger_train_attn_build_bwd_ex(dkv_in, dq_in, dcat, ld_cat, cat_off, center, n_q, ts, batch, 1, neigh_nids,
-                                       neigh_ts, k, sel, d, de, time_w, time_b, dh_new, nullptr, g_time_w, g_time_b,
-                                       stream);
 }
 
 // ------------------------------------------------------------------------------------------

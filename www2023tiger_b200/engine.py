@@ -12,20 +12,21 @@ Launch sequence of one batch (B events, K neighbors):
   2 tiger_compact_involved   involved / outdated / restart lists + gru_row map
   3 tiger_static_restart     (lazy-restart mode only) re-initialise not-yet-seen nodes
   4 tiger_gru_update         h(t'+) for the O outdated nodes      (steps 1-2 of the reference)
-  5 tiger_temporal_attention h(t-) for [src;dst;neg]              (step 3)
-  6 tiger_select_latest      argmax-by-timestamp winners of [src;dst]
-  7 tiger_right_writeback    persist h(t'+) of outdated positives (step 4) [+ restarter targets]
-  8 tiger_store_messages     build + store the new raw messages   (step 5)
-  9 tiger_left_writeback     persist h(t-) of positives           (step 6)
- 10 tiger_link_score         hit flags, scorer, BCE loss          (step 7)
+  5 tiger_select_latest      argmax-by-timestamp winners of [src;dst]
+  6 tiger_right_writeback    persist h(t'+) of outdated positives (step 4) [+ restarter targets]
+  7 tiger_store_messages     build + store the new raw messages   (step 5)
+  8 tiger_temporal_attention_ex  h(t-) for [src;dst;neg] (step 3); its last product also persists h(t-) of the
+                             positives (step 6, tiger_left_writeback_fused) and writes the scorer's first layer pq
+  9 tiger_link_score_folded  hit flags, scorer, BCE loss          (step 7)
+Under graph capture 5-7 run on a side stream beside 8.
 
 With n_layers = 2 (GraphEmbedding.compute_embedding_with_computation_graph, temporal_agg_modules.py:79-104):
   1  tiger_find_recent hop 1 as above, then the hop-1 times widened to float64 and tiger_find_recent hop 2: the K
      neighbors of each of the 3B*K hop-1 neighbors at that neighbor's own event time (the collator's two calls);
      both mark the involved bitmap, so U, O, R, the GRU and the lazy restart cover the 2-hop nodes
-  5a tiger_temporal_attention_ex, fns.1, 3B*K depth-1 queries (center = hop-1 neighbor, time = its parent event's)
+  8a tiger_temporal_attention_ex, fns.1, 3B*K depth-1 queries (center = hop-1 neighbor, time = its parent event's)
      over the hop-2 table -> emb1 [3B*K, d]
-  5b tiger_temporal_attention_ex, fns.0, the 3B batch nodes over the hop-1 table, slot (q, j) keyed by emb1[q*K + j]
+  8b tiger_temporal_attention_ex, fns.0, the 3B batch nodes over the hop-1 table, slot (q, j) keyed by emb1[q*K + j]
 """
 from typing import Dict, Optional
 
@@ -114,7 +115,6 @@ class TigerEngine:
         self.gru_pack = None
         self.attn_pack = ops.AttnPack(self.d, self.de, dev, n_head)
         self.attn_pack1 = ops.AttnPack(self.d, self.de, dev, n_head) if n_layers == 2 else None   # fns.1 (depth 1)
-        self.score_pack = ops.ScorePack(self.d, dev)
         self.score_fold = ops.ScoreFold(self.d, dev)
         self.pq = torch.zeros(3 * batch_size, 2 * self.d, dtype=f32, device=dev)   # [W1a z | W1b z] per query row
         self.hist_len = hist_len
@@ -142,8 +142,6 @@ class TigerEngine:
                              g(fa + 'merger.fc1.weight'), g(fa + 'merger.fc1.bias'),
                              g(fa + 'merger.fc2.weight'), g(fa + 'merger.fc2.bias'), self.time_w, self.time_b)
         s = 'score_fn.'
-        self.score_pack.refresh(g(s + 'fc1.weight'), g(s + 'fc1.bias'), g(s + 'fc2.weight'), g(s + 'fc2.bias'),
-                                g('hit_embedding.weight') if self.hit_type == 'bin' else None)
         self.score_fold.refresh(g(s + 'fc1.weight'), g(s + 'fc1.bias'), g(s + 'fc2.weight'), g(s + 'fc2.bias'),
                                 g(a + 'merger.fc2.weight'), g(a + 'merger.fc2.bias'),
                                 g('hit_embedding.weight') if self.hit_type == 'bin' else None)

@@ -208,24 +208,6 @@ def left_writeback(pos_ids, batch, winner, h_left, d, ts, left_vals, left_ts, le
 # ------------------------------------------------------------------------------------------
 # parameter packing
 # ------------------------------------------------------------------------------------------
-def round_up(x: int, m: int) -> int:
-    return (x + m - 1) // m * m
-
-
-def transpose_pad(w: Tensor, out: Tensor, ld_out: int, pad_rows: Optional[int] = None):
-    """out[k*ld_out + n] = w[n, k]; w is a (possibly row-sliced) contiguous 2-D parameter."""
-    check_cuda(w, out)
-    rows, cols = w.shape
-    call('tiger_transpose_pad', ptr(w), rows, cols, w.stride(0), ptr(out), ld_out,
-         pad_rows if pad_rows is not None else ld_out)
-
-
-def copy_pad(w: Tensor, out: Tensor, ld_out: int):
-    check_cuda(w, out)
-    rows, cols = w.shape
-    call('tiger_copy_pad', ptr(w), rows, cols, w.stride(0), ptr(out), ld_out)
-
-
 class GruPack:
     """nn.GRUCell parameters as the kernel reads them: the gate weights pre-split into tf32 head / tail
     planes in the stage layout of tiger_gru_update (tiger_gru_pack), biases as stored."""
@@ -278,7 +260,8 @@ class AttnPack:
     """TemporalAttention parameters for the kernels: the reference's tensors as stored plus the folded
     weights (tiger_attn_fold: Wqk, bqk, W2f), and a workspace that grows on demand.  A multi-layer embedding
     keeps one pack per layer (temporal_embedding_fn.fns.i); the score fold and the fused left write-back attach
-    only to the pack of the batch-node layer, whose result they read."""
+    together, only to the pack of the batch-node layer, whose result they read, and only for the gather form
+    (temporal_attention): the kernel refuses a call with one of them alone or with the dense form."""
 
     def __init__(self, d: int, de: int, device, n_head: int = 2):
         self.d, self.de, self.n_head = d, de, n_head
@@ -308,8 +291,8 @@ class AttnPack:
         return ctypes.addressof(self.struct)
 
     def attach_score_fold(self, fold: Optional['ScoreFold'], pq_out: Optional[Tensor]):
-        """With a ScoreFold attached the last attention GEMM also emits the link scorer's first layer
-        (pq_out [n_query, 2d]); detach with (None, None)."""
+        """With a ScoreFold (and the left write-back) attached the last attention GEMM also emits the link scorer's
+        first layer (pq_out [n_query, 2d]); detach with (None, None)."""
         self._score_fold, self._pq_out = fold, pq_out
         self.struct.score_folded = fold.blob.data_ptr() if fold is not None else None
         self.struct.pq_out = pq_out.data_ptr() if pq_out is not None else None
@@ -375,23 +358,6 @@ def temporal_attention_dense(pack: AttnPack, n_head: int, qx, qt, kx, ky, kt, pa
     return out
 
 
-class ScorePack:
-    """k-major pack of score_fn (MergeLayer(d, d, d, 1)) + optional hit embedding."""
-
-    def __init__(self, d: int, device):
-        self.d = d
-        self.ldD = round_up(d, 4)
-        self.fc1T = torch.zeros(2 * d * self.ldD, dtype=f32, device=device)
-        self.done = torch.zeros(1, dtype=i32, device=device)
-
-    def refresh(self, fc1_w, fc1_b, fc2_w, fc2_b, hit_emb: Optional[Tensor]):
-        transpose_pad(fc1_w.detach().contiguous(), self.fc1T, self.ldD)
-        self.fc1_b = fc1_b.detach().contiguous()
-        self.fc2_w = fc2_w.detach().reshape(-1).contiguous()
-        self.fc2_b = fc2_b.detach().contiguous()
-        self.hit_emb = None if hit_emb is None else hit_emb.detach().contiguous()
-
-
 class ScoreFold:
     """Link scorer folded into the attention's last GEMM (tiger_score_fold): refresh whenever score_fn,
     the embedding module's merger.fc2 or the hit embedding change."""
@@ -422,19 +388,6 @@ def link_score_folded(fold: ScoreFold, pq: Tensor, src: Tensor, dst: Tensor, neg
     k = neigh_nids.shape[1] if neigh_nids is not None else 0
     call('tiger_link_score_folded', ptr(pq), B, fold.d, ptr(src), ptr(dst), ptr(neg), ptr(neigh_nids), k, ptr(fold.cab),
          ptr(fold.fc2_w), ptr(fold.fc2_b), ptr(scores), ptr(loss), ptr(fold.done))
-    return scores, loss
-
-
-def link_score(pack: ScorePack, h: Tensor, src: Tensor, dst: Tensor, neg: Tensor, neigh_nids: Optional[Tensor],
-               scores: Optional[Tensor] = None, loss: Optional[Tensor] = None):
-    B = src.numel()
-    if scores is None:
-        scores = _empty(2 * B, f32, h)
-    if loss is None:
-        loss = _empty(1, f32, h)
-    k = neigh_nids.shape[1] if neigh_nids is not None else 0
-    call('tiger_link_score', ptr(h), B, pack.d, ptr(src), ptr(dst), ptr(neg), ptr(neigh_nids), k, ptr(pack.hit_emb),
-         ptr(pack.fc1T), ptr(pack.fc1_b), ptr(pack.fc2_w), ptr(pack.fc2_b), ptr(scores), ptr(loss), ptr(pack.done))
     return scores, loss
 
 

@@ -2,9 +2,10 @@
 (reference tiger/model/tiger.py:27-618; same constructor keywords, methods and state_dict layout).
 
 `contrast_learning` has two routes:
-* no-grad (evaluation, warm-up, `flush_msg`): the fused launch sequence of DESIGN.md §3 - compaction
-  of the pending-message set, gather+GRU, fused temporal attention, argmax-by-timestamp selection,
-  right write-back, message build+store, left write-back, link scorer - with every
+* no-grad (evaluation, warm-up, `flush_msg`): the fused launch sequence of DESIGN.md §3, in the order of
+  TigerEngine.launch_model on the caller's stream - compaction of the pending-message set, gather+GRU,
+  argmax-by-timestamp selection, right write-back, message build+store, fused temporal attention whose last
+  product also writes the left memory and the folded scorer's first layer, link scorer - with every
   data-dependent size kept on the device; one host poll of the error word per batch.
 * autograd (the training loops): the seven steps of the reference, differentiable operators through
   torch ops, index / memory operators through the kernels.
@@ -72,6 +73,7 @@ class _Workspace:
         self.h_new = z(self.cap, d)
         self.winner = z(2 * B, dt=torch.uint8)
         self.sel_count = z(1, dt=torch.int32)
+        self.pq = z(3 * B, 2 * d)          # [W1a z | W1b z] per batch-node row: the folded scorer's first layer
 
 
 class TIGE(nn.Module):
@@ -129,7 +131,7 @@ class TIGE(nn.Module):
             raise ValueError(f'Invalid upd_src={upd_src}')
         self._err = ErrFlags()
         self._ws: Optional[_Workspace] = None
-        self._score_pack, self._score_key = None, None
+        self._fold, self._fold_key = None, None
 
     def _bind_sources(self):
         self.msg_memory = self.left_memory if self.msg_src == 'left' else self.right_memory
@@ -160,19 +162,21 @@ class TIGE(nn.Module):
             ws = self._ws = _Workspace(self.n_nodes, self.memory_dim, B, K, dev, self.n_layers)
         return ws
 
-    def _scorer(self) -> ops.ScorePack:
-        s = self.score_fn
-        params = [s.fc1.weight, s.fc1.bias, s.fc2.weight, s.fc2.bias]
+    def _score_fold(self) -> ops.ScoreFold:
+        """The link scorer folded into the batch-node attention's last product (score_fn, the merger's fc2 of
+        fns.0, the hit embedding), refreshed when one of them changes."""
+        s, m = self.score_fn, self.temporal_embedding_fn.fns[0].merger
+        params = [s.fc1.weight, s.fc1.bias, s.fc2.weight, s.fc2.bias, m.fc2.weight, m.fc2.bias]
         if self.hit_type == 'bin':
             params.append(self.hit_embedding.weight)
         key = tuple((p.data_ptr(), p._version) for p in params)
-        if self._score_pack is None or key != self._score_key:
-            if self._score_pack is None or self._score_pack.fc1T.device != params[0].device:
-                self._score_pack = ops.ScorePack(self.nfeat_dim, params[0].device)
+        if self._fold is None or key != self._fold_key:
+            if self._fold is None or self._fold.blob.device != params[0].device:
+                self._fold = ops.ScoreFold(self.nfeat_dim, params[0].device)
             args = [f32c(p) for p in params] + ([None] if self.hit_type != 'bin' else [])
-            self._score_pack.refresh(*args)
-            self._score_key = key
-        return self._score_pack
+            self._fold.refresh(*args)
+            self._fold_key = key
+        return self._fold
 
     def _contrast_learning_fused(self, src_ids, dst_ids, neg_dst_ids, ts, eids, cg):
         B, d, N = len(src_ids), self.memory_dim, self.n_nodes
@@ -194,6 +198,20 @@ class TIGE(nn.Module):
                        h_table=self.upd_memory.vals, n_rows=ws.cap, out=ws.h_new, count=ws.counts[1:],
                        msg_ts=store.node_msg_ts, check_mem_ts=self.msg_memory.update_ts,
                        check_equal=(self.msg_src == 'left'), err_flags=err)
+        # steps 4-5 (tiger.py:230-255) ahead of step 3, in TigerEngine.launch_model's order: the right write-back
+        # writes only rows the attention reads from h_new, the message builder only the message store (DESIGN.md §3,
+        # "Why the post-GRU branches may overlap"), and both read the old left rows before the last attention
+        # product overwrites them
+        winner = ws.winner[:2 * B]
+        ops.select_latest(pos, ts, want_unique=False, winner=winner, want_count=False)
+        h_prev_left = torch.empty(2 * B, d, device=dev)
+        h_prev_right = torch.empty(2 * B, d, device=dev)
+        ops.right_writeback(pos, winner, ws.gru_row, ws.h_new, d, right.vals, right.update_ts, right.active_mask,
+                            store.node_msg_ts, store.has_msg, left.vals, h_prev_left, h_prev_right, err)
+        ops.store_messages(batch_nids[:B], batch_nids[B:2 * B], eids.contiguous(), ts, winner, self.msg_memory.vals,
+                           self.msg_memory.update_ts, fg.nfeats, fg.efeats, d, self.efeat_dim,
+                           f32c(self.time_encoder.basis_freq), f32c(self.time_encoder.phase), store.node_msg_vals,
+                           store.node_msg_ts, store.has_msg, err)
         # step 3: temporal attention over the sampled neighbors (tiger.py:225-227)
         fns = self.temporal_embedding_fn.fns
         key_rows = None
@@ -205,25 +223,25 @@ class TIGE(nn.Module):
                                               nn_.reshape(-1).contiguous(), ts, n2, e2, t2, rows_a=right.vals,
                                               rows_b=ws.h_new, sel=ws.gru_row, nfeats=fg.nfeats, efeats=fg.efeats,
                                               ts_group=K)
+        # the batch nodes' last product also persists the winners' embeddings into the left memory (step 6,
+        # tiger.py:255) and writes the link scorer's first layer for every row (pq).  The pack is the one the
+        # step-by-step route and TemporalAttention.forward use, so the attachments live for this call only.
+        fold = self._score_fold()
         fn = fns[0]
-        emb = ops.temporal_attention(fn.packed(self.time_encoder), fn.n_head, batch_nids, ts, nn_, ne_, nt_,
-                                     rows_a=right.vals, rows_b=ws.h_new, sel=ws.gru_row, nfeats=fg.nfeats,
-                                     efeats=fg.efeats, key_rows=key_rows)
-        # steps 4-6 (tiger.py:230-255)
-        winner = ws.winner[:2 * B]
-        ops.select_latest(pos, ts, want_unique=False, winner=winner, want_count=False)
-        h_prev_left = torch.empty(2 * B, d, device=dev)
-        h_prev_right = torch.empty(2 * B, d, device=dev)
-        ops.right_writeback(pos, winner, ws.gru_row, ws.h_new, d, right.vals, right.update_ts, right.active_mask,
-                            store.node_msg_ts, store.has_msg, left.vals, h_prev_left, h_prev_right, err)
-        ops.store_messages(batch_nids[:B], batch_nids[B:2 * B], eids.contiguous(), ts, winner, self.msg_memory.vals,
-                           self.msg_memory.update_ts, fg.nfeats, fg.efeats, d, self.efeat_dim,
-                           f32c(self.time_encoder.basis_freq), f32c(self.time_encoder.phase), store.node_msg_vals,
-                           store.node_msg_ts, store.has_msg, err)
-        ops.left_writeback(pos, B, winner, emb, d, ts, left.vals, left.update_ts, left.active_mask, err)
+        pack = fn.packed(self.time_encoder)
+        pq = ws.pq[:3 * B]
+        pack.attach_score_fold(fold, pq)
+        pack.attach_left_writeback(pos, winner, ts, left.vals, left.update_ts, left.active_mask, err)
+        try:
+            emb = ops.temporal_attention(pack, fn.n_head, batch_nids, ts, nn_, ne_, nt_, rows_a=right.vals,
+                                         rows_b=ws.h_new, sel=ws.gru_row, nfeats=fg.nfeats, efeats=fg.efeats,
+                                         key_rows=key_rows)
+        finally:
+            pack.attach_score_fold(None, None)
+            pack.attach_left_writeback(None)
         # step 7 (tiger.py:259-288)
-        scores, loss = ops.link_score(self._scorer(), emb, batch_nids[:B], batch_nids[B:2 * B], batch_nids[2 * B:],
-                                      nn_ if self.hit_type == 'bin' else None)
+        scores, loss = ops.link_score_folded(fold, pq, batch_nids[:B], batch_nids[B:2 * B], batch_nids[2 * B:],
+                                             nn_ if self.hit_type == 'bin' else None)
         self._err.check()
         return loss[0], emb[:2 * B], scores[:B], scores[B:], h_prev_left, h_prev_right
 
