@@ -200,6 +200,31 @@ int tiger_gru_update(const int64_t* node_ids, const int32_t* count, int64_t n_ro
                      const float* msg_ts, const float* check_mem_ts, int check_equal,
                      uint32_t* err_flags, void* stream);
 
+/* tiger_gru_update for MLPMessageFunction (message_modules.py:47-57, an MLP transform between the last-message
+ * gather and the GRUCell; reference message_modules.py:29-55): x row r is x_table[r] (row position, the hidden
+ * rows relu(W_1 msg + b_1) that a plain-row tiger_sgemm_nt_packed_gather wrote for the outdated rows) while h,
+ * msg_ts and the invariant checks read node_ids[r] (not NULL).  m_dim is the hidden width; the pack and b_ih are
+ * those of weight_ih W_2 and bias_ih + weight_ih b_2 (the second layer folded into the gates). */
+int tiger_gru_update_rows(const int64_t* node_ids, const int32_t* count, int64_t n_rows,
+                          const float* x_table, int64_t x_stride, const float* h_table, int64_t h_stride,
+                          int m_dim, int d, const float* wpack,
+                          const float* b_ih, const float* b_hh, float* h_new,
+                          const float* msg_ts, const float* check_mem_ts, int check_equal,
+                          uint32_t* err_flags, void* stream);
+
+/* First layer of MergeUpdater (update_modules.py:40-47: MergeLayer(msg_dim, d, d, d), basic_modules.py:8-20):
+ *   out[r,:] = relu(fc1 [x ; h] + b1)      fc1 [d][m_dim + d] as stored (message columns first)
+ * on the tensor cores of tiger_gru_update (tf32x3), with its row gather (x by node id, or by row position with
+ * x_by_row), its device row count and its message-invariant checks (tiger.py:319-327).  fc2 follows as a
+ * count-bounded tiger_sgemm_nt_packed.  wpack: tiger_merge_pack output, tiger_gru_pack_bytes(m_dim, d) bytes;
+ * re-run it whenever fc1 changes.  A linear / MLP message transform folds into the message columns of fc1. */
+int tiger_merge_pack(const float* fc1_w, int m_dim, int d, float* out, void* stream);
+int tiger_merge_update(const int64_t* node_ids, const int32_t* count, int64_t n_rows,
+                       const float* x_table, int64_t x_stride, int x_by_row, const float* h_table,
+                       int64_t h_stride, int m_dim, int d, const float* wpack, const float* b1, float* out,
+                       const float* msg_ts, const float* check_mem_ts, int check_equal,
+                       uint32_t* err_flags, void* stream);
+
 /* temporal-attention parameters (device pointers): the reference's tensors as stored
  * (temporal_embedding_fn.fns.0.*), plus one caller-allocated buffer for the folded weights.
  * E = 2d, C = 2d + de, hd = E / n_head. */
@@ -395,7 +420,8 @@ int tiger_sgemm_nt_packed(const float* A, int64_t lda, const float* wpack, int b
  * is NULL), else row ids[m] of rows_a, plus row ids[m] of add_rows when given - the "latest representation of
  * node u" lookup of compute_embedding_with_computation_graph (temporal_agg_modules.py:210-235: memory row or
  * the row the GRU just produced, + node features) done by the GEMM's producer warps.  sel is int32 or int64
- * (sel_is_i64); all three tables have row stride ld_rows. */
+ * (sel_is_i64); all three tables have row stride ld_rows.  sel == NULL: row m is row ids[m] of rows_a (rows_b
+ * unused) - the outdated nodes' pending messages for the first layer of MLPMessageFunction (message_modules.py:47-57). */
 int tiger_sgemm_nt_packed_gather(const int64_t* ids, const void* sel, int sel_is_i64, const float* rows_a,
                                  const float* rows_b, int64_t ld_rows, const float* add_rows, const float* wpack,
                                  int bn, const float* bias, float* C, int64_t ldc, int64_t m_rows,

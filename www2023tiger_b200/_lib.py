@@ -35,6 +35,9 @@ _SIGNATURES: Dict[str, str] = {
     'tiger_gru_pack_bytes': 'ii',
     'tiger_gru_pack': 'ppiip' + 'p',
     'tiger_gru_update': 'ppl' + 'plpl' + 'ii' + 'p' + 'ppp' + 'ppi' + 'p' + 'p',
+    'tiger_gru_update_rows': 'ppl' + 'plpl' + 'ii' + 'p' + 'ppp' + 'ppi' + 'p' + 'p',
+    'tiger_merge_pack': 'piipp',
+    'tiger_merge_update': 'ppl' + 'plipl' + 'ii' + 'ppp' + 'ppi' + 'p' + 'p',
     'tiger_attn_fold_bytes': 'iii',
     'tiger_attn_fold': 'piii' + 'p',
     'tiger_temporal_attention_work_bytes': 'liiii',

@@ -484,8 +484,9 @@ __global__ void __launch_bounds__(TS_THREADS, 1) gemm_tf32x3_ts_kernel(const Gem
     const float* addp = nullptr;
     if (g.a_ids != nullptr) {
       const int64_t u = g.a_ids[m];
-      const int64_t r = g.a_sel_i64 ? reinterpret_cast<const int64_t*>(g.a_sel)[u]
-                                    : (int64_t) reinterpret_cast<const int32_t*>(g.a_sel)[u];
+      const int64_t r = g.a_sel == nullptr ? -1
+                        : g.a_sel_i64 ? reinterpret_cast<const int64_t*>(g.a_sel)[u]
+                                      : (int64_t) reinterpret_cast<const int32_t*>(g.a_sel)[u];
       rowp = (A == nullptr || r >= 0) ? g.a_alt + r * g.lda : A + u * g.lda;
       if (g.a_add != nullptr) addp = g.a_add + u * g.lda;
     }
@@ -802,7 +803,8 @@ struct PackedGemm {
   int64_t ldc2;
   int n_split, n_cols1;
   int k_parts = 1;                // > 1: K split over a thread-block cluster of up to 8 CTAs per tile
-  // gathered A (GemmArgs::a_ids): row m is row sel[ids[m]] of alt when that is >= 0, else row ids[m] of A, + add
+  // gathered A (GemmArgs::a_ids): row m is row sel[ids[m]] of alt when that is >= 0, else row ids[m] of A, + add;
+  // without sel always row ids[m] of A
   const int64_t* ids;
   const void* sel;
   int sel_is_i64;
@@ -905,7 +907,7 @@ extern "C" int tiger_sgemm_nt_packed_gather(const int64_t* ids, const void* sel,
                                             const float* wpack, int bn, const float* bias, float* C, int64_t ldc,
                                             int64_t m_rows, const int32_t* count, int64_t rows_per_count,
                                             int n_cols, int k_dim, float alpha, int relu, void* stream) {
-  if (ids == nullptr || sel == nullptr || rows_b == nullptr) return TIGER_EINVAL;
+  if (ids == nullptr || (sel != nullptr ? rows_b == nullptr : rows_a == nullptr)) return TIGER_EINVAL;
   return gemm_packed_launch({.A = rows_a, .lda = ld_rows, .wpack = wpack, .bn = bn, .bias = bias, .C = C, .ldc = ldc,
                              .n_cols = n_cols, .m_rows = m_rows, .count = count, .rows_per_count = rows_per_count,
                              .k_dim = k_dim, .alpha = alpha, .relu = relu, .ids = ids, .sel = sel,

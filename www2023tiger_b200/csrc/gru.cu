@@ -30,6 +30,13 @@
 //                it accumulates, a bias that grows with the number of accumulation steps: the K split
 //                halves the steps per accumulator); 2 sets x 192 + 2 x 64 activation columns = 512 TMEM columns
 //   epilogue     the producer warps add the two sets out of TMEM into the shared-memory partial tile
+//
+// The same kernel runs the first layer of MergeUpdater (update_modules.py:40-47, MergeLayer, basic_modules.py:8-20):
+// relu(fc1 [x | h] + b1) is the n-gate column group without r and z - the x phase multiplies the message columns of
+// fc1 into [Win x], the h phase its state columns into [Whn h] (tiger_merge_pack puts them at the n rows of each
+// stage), the [r | z] MMAs are skipped and the epilogue is relu(Win x + Whn h + b1).  With x_by_row the message row
+// of result row r is x_table row r (the hidden rows of MLPMessageFunction, computed per outdated row upstream)
+// instead of x_table row node_ids[r]; h, the message timestamps and the invariant checks stay node-indexed.
 #include "common.cuh"
 #include "umma.cuh"
 
@@ -83,6 +90,8 @@ struct GruArgs {
   int check_equal;
   uint32_t* err_flags;
   int vec_x, vec_h;
+  int x_by_row;        // x row r is x_table[r] instead of x_table[node_ids[r]]
+  int merge;           // MergeLayer first layer: out = relu(fc1_x x + fc1_h h + b1), b1 in b_ih
 };
 
 __global__ void __launch_bounds__(GRU_THREADS, 1) gru_update_kernel(const GruArgs g) {
@@ -119,7 +128,11 @@ __global__ void __launch_bounds__(GRU_THREADS, 1) gru_update_kernel(const GruArg
     r = r < n ? r : n - 1;
     prod_u = g.node_ids != nullptr ? g.node_ids[r] : r;
   }
-  if (tid < GRU_U) {
+  if (tid < GRU_U && g.merge) {
+    const int j = j0 + tid;
+    bias_s[tid] = bias_s[GRU_U + tid] = bias_s[3 * GRU_U + tid] = 0.f;
+    bias_s[2 * GRU_U + tid] = j < d ? g.b_ih[j] : 0.f;
+  } else if (tid < GRU_U) {
     const int j = j0 + tid;
     const bool ok = j < d;
     bias_s[tid] = ok ? g.b_ih[j] + g.b_hh[j] : 0.f;
@@ -170,7 +183,7 @@ __global__ void __launch_bounds__(GRU_THREADS, 1) gru_update_kernel(const GruArg
       const int64_t r = row0 + rl;
       const int j = j0 + c;
       gate_h[it] = make_float4(0.f, 0.f, 0.f, 0.f);
-      if (i < GATE_RB * GATE_Q && r < n && j < d) {
+      if (!g.merge && i < GATE_RB * GATE_Q && r < n && j < d) {
         const int64_t u = g.node_ids != nullptr ? g.node_ids[r] : r;
         gate_h[it] = umma_load_chunk(g.h_table + u * g.h_stride, j, d, g.vec_h != 0);
       }
@@ -187,7 +200,7 @@ __global__ void __launch_bounds__(GRU_THREADS, 1) gru_update_kernel(const GruArg
     const bool live = r < n;
     r = live ? r : n - 1;
     const int64_t u = prod_u;
-    const float* xp = g.x_table + u * g.x_stride;
+    const float* xp = g.x_table + (g.x_by_row ? r : u) * g.x_stride;
     const float* hp = g.h_table + u * g.h_stride;
     if (live && warp < 4 && g.check_mem_ts != nullptr && blockIdx.x == 0 && part == 0 && g.err_flags != nullptr) {
       const float mt = g.msg_ts[u], pt = g.check_mem_ts[u];
@@ -245,7 +258,7 @@ __global__ void __launch_bounds__(GRU_THREADS, 1) gru_update_kernel(const GruArg
       tmem_ld16(tacc + (uint32_t)c0, a);
       tmem_ld16(tacc + (uint32_t)(GRU_ACC_COLS + c0), t);
       // column groups this CTA's stages never touched hold no sum (U is a multiple of 16: a chunk lies in one group)
-      const bool valid = c0 < GRU_U ? has_x : (c0 < 3 * GRU_U ? (has_x || has_h) : has_h);
+      const bool valid = c0 < GRU_U ? has_x : (c0 < 3 * GRU_U ? (has_x || has_h) && !g.merge : has_h);
 #pragma unroll
       for (int e = 0; e < 16; e += 4)
         *reinterpret_cast<float4*>(red + c0 + e) =
@@ -305,7 +318,16 @@ __global__ void __launch_bounds__(GRU_THREADS, 1) gru_update_kernel(const GruArg
           const uint32_t ah = a_hi + 8u * j, al = a_lo + 8u * j, bh = b_hi + b_kstep * j, bl = b_lo + b_kstep * j;
           const uint32_t fresh = (first && j == 0) ? 0u : 1u;
           const uint32_t fresh_rz = (first && j == 0 && !has_x) ? 0u : 1u;
-          if (is_x) {
+          if (g.merge) {
+            // [Win x] from the stage's n rows (x phase), [Whn h] likewise (h phase); no r / z products
+            const uint32_t acc_n = acc + (xph ? 0u : 3u * GRU_U), b_n = xph ? 0u : 2u * GRU_U;
+            if (is_x) {
+              umma_tf32_ts(acc_n, al, bh + b_n, id1, fresh);
+              umma_tf32_ts(acc_n, ah, bl + b_n, id1, 1u);
+            } else {
+              umma_tf32_ts(acc_n, ah, bh + b_n, id1, fresh);
+            }
+          } else if (is_x) {
             if (xph) {
               // weight tile rows [n | r | z] -> columns [0, 3U)
               umma_tf32_ts(acc, al, bh, id3, fresh);
@@ -383,6 +405,10 @@ __global__ void __launch_bounds__(GRU_THREADS, 1) gru_update_kernel(const GruArg
       float o[4];
 #pragma unroll
       for (int e = 0; e < 4; ++e) {
+        if (g.merge) {
+          o[e] = fmaxf(an[e] + ah[e] + bias_s[2 * GRU_U + c + e], 0.f);
+          continue;
+        }
         const float rg = sigmoidf_acc(ar[e] + bias_s[c + e]);
         const float zg = sigmoidf_acc(az[e] + bias_s[GRU_U + c + e]);
         const float nn = tanhf((an[e] + bias_s[2 * GRU_U + c + e]) + rg * (ah[e] + bias_s[3 * GRU_U + c + e]));
@@ -410,7 +436,9 @@ __global__ void __launch_bounds__(GRU_THREADS, 1) gru_update_kernel(const GruArg
 }
 
 // Gate-weight pack: for unit tile t and k-block kb (x phase: kb < nbx over weight_ih, rows [n | r | z]; h phase over
-// weight_hh, rows [r | z | n]) the stage image [head plane | tail plane][kc][3U rows][4 floats].
+// weight_hh, rows [r | z | n]) the stage image [head plane | tail plane][kc][3U rows][4 floats].  Merge pack (w_hh
+// NULL, w_ih = fc1 [d][m_dim + d]): the message columns of fc1 at the x stages' n rows, its state columns at the h
+// stages' n rows, zeros elsewhere.
 __global__ void gru_pack_kernel(const float* __restrict__ w_ih, const float* __restrict__ w_hh, int m_dim, int d,
                                 int tiles, int nbx, int nbh, float* __restrict__ out) {
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -425,9 +453,13 @@ __global__ void gru_pack_kernel(const float* __restrict__ w_ih, const float* __r
   const int gi = r / GRU_U, j = t * GRU_U + r % GRU_U;
   const int gate = xph ? (gi == 0 ? 2 : gi - 1) : gi;   // gate order in the weights: r, z, n
   const int kdim = xph ? m_dim : d;
-  const float* w = xph ? w_ih : w_hh;
   const int k = (xph ? kb : kb - nbx) * TS_BK + kc * 4;
-  const float4 v = umma_load_chunk(j < d ? w + (int64_t)(gate * d + j) * kdim : nullptr, k, kdim, false);
+  const float* row = nullptr;
+  if (j < d && w_hh != nullptr)
+    row = (xph ? w_ih : w_hh) + (int64_t)(gate * d + j) * kdim;
+  else if (j < d && gate == 2)
+    row = w_ih + (int64_t)j * (m_dim + d) + (xph ? 0 : m_dim);
+  const float4 v = umma_load_chunk(row, k, kdim, false);
   float4 h, l;
   tf32_split(v, h, l);
   float* stage = out + ((int64_t)t * n_kb + kb) * GRU_W_STAGE_FLOATS;
@@ -454,13 +486,22 @@ extern "C" int tiger_gru_pack(const float* w_ih, const float* w_hh, int m_dim, i
   return tiger_launch_status();
 }
 
-extern "C" int tiger_gru_update(const int64_t* node_ids, const int32_t* count, int64_t n_rows,
-                                const float* x_table, int64_t x_stride, const float* h_table, int64_t h_stride,
-                                int m_dim, int d, const float* wpack, const float* b_ih, const float* b_hh,
-                                float* h_new, const float* msg_ts, const float* check_mem_ts, int check_equal,
-                                uint32_t* err_flags, void* stream) {
-  if (n_rows < 0 || m_dim <= 0 || d <= 0 || wpack == nullptr || (((uintptr_t)wpack) & 15) != 0) return TIGER_EINVAL;
-  if (n_rows == 0) return TIGER_OK;
+extern "C" int tiger_merge_pack(const float* fc1_w, int m_dim, int d, float* out, void* stream) {
+  if (fc1_w == nullptr || out == nullptr || tiger_gru_pack_bytes(m_dim, d) < 0 || (((uintptr_t)out) & 15) != 0)
+    return TIGER_EINVAL;
+  const int tiles = (d + GRU_U - 1) / GRU_U;
+  const int nbx = (m_dim + TS_BK - 1) / TS_BK, nbh = (d + TS_BK - 1) / TS_BK;
+  const int64_t total = (int64_t)tiles * (nbx + nbh) * TS_KCH * GRU_WROWS;
+  gru_pack_kernel<<<(unsigned)((total + 255) / 256), 256, 0, as_stream(stream)>>>(fc1_w, nullptr, m_dim, d, tiles, nbx,
+                                                                                 nbh, out);
+  return tiger_launch_status();
+}
+
+static int gru_update_launch(const GruArgs& a, void* stream) {
+  if (a.n_rows < 0 || a.m_dim <= 0 || a.d <= 0 || a.wpack == nullptr || (((uintptr_t)a.wpack) & 15) != 0 ||
+      a.b_ih == nullptr || (!a.merge && a.b_hh == nullptr) || (a.x_by_row && a.node_ids == nullptr))
+    return TIGER_EINVAL;
+  if (a.n_rows == 0) return TIGER_OK;
   static bool configured = false;
   if (!configured) {
     if (cudaFuncSetAttribute(gru_update_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, GRU_SMEM_BYTES) !=
@@ -468,14 +509,52 @@ extern "C" int tiger_gru_update(const int64_t* node_ids, const int32_t* count, i
       return TIGER_ECUDA;
     configured = true;
   }
-  GruArgs g;
+  GruArgs g = a;
+  g.vec_x = ((((uintptr_t)g.x_table) & 15) == 0 && (g.x_stride & 3) == 0) ? 1 : 0;
+  g.vec_h = ((((uintptr_t)g.h_table) & 15) == 0 && (g.h_stride & 3) == 0) ? 1 : 0;
+  return tiger_launch_chain(gru_update_kernel,
+                            dim3((unsigned)((g.d + GRU_U - 1) / GRU_U), (unsigned)((g.n_rows + GRU_BM - 1) / GRU_BM),
+                                 GRU_KPARTS),
+                            dim3(GRU_THREADS), GRU_SMEM_BYTES, as_stream(stream), dim3(1, 1, GRU_KPARTS), g);
+}
+
+extern "C" int tiger_gru_update(const int64_t* node_ids, const int32_t* count, int64_t n_rows,
+                                const float* x_table, int64_t x_stride, const float* h_table, int64_t h_stride,
+                                int m_dim, int d, const float* wpack, const float* b_ih, const float* b_hh,
+                                float* h_new, const float* msg_ts, const float* check_mem_ts, int check_equal,
+                                uint32_t* err_flags, void* stream) {
+  GruArgs g{};
   g.node_ids = node_ids; g.count = count; g.n_rows = n_rows;
   g.x_table = x_table; g.x_stride = x_stride; g.h_table = h_table; g.h_stride = h_stride;
   g.m_dim = m_dim; g.d = d; g.wpack = wpack; g.b_ih = b_ih; g.b_hh = b_hh; g.h_new = h_new;
   g.msg_ts = msg_ts; g.check_mem_ts = check_mem_ts; g.check_equal = check_equal; g.err_flags = err_flags;
-  g.vec_x = ((((uintptr_t)x_table) & 15) == 0 && (x_stride & 3) == 0) ? 1 : 0;
-  g.vec_h = ((((uintptr_t)h_table) & 15) == 0 && (h_stride & 3) == 0) ? 1 : 0;
-  return tiger_launch_chain(gru_update_kernel,
-                            dim3((unsigned)((d + GRU_U - 1) / GRU_U), (unsigned)((n_rows + GRU_BM - 1) / GRU_BM), GRU_KPARTS),
-                            dim3(GRU_THREADS), GRU_SMEM_BYTES, as_stream(stream), dim3(1, 1, GRU_KPARTS), g);
+  return gru_update_launch(g, stream);
+}
+
+extern "C" int tiger_gru_update_rows(const int64_t* node_ids, const int32_t* count, int64_t n_rows,
+                                     const float* x_table, int64_t x_stride, const float* h_table, int64_t h_stride,
+                                     int m_dim, int d, const float* wpack, const float* b_ih, const float* b_hh,
+                                     float* h_new, const float* msg_ts, const float* check_mem_ts, int check_equal,
+                                     uint32_t* err_flags, void* stream) {
+  GruArgs g{};
+  g.node_ids = node_ids; g.count = count; g.n_rows = n_rows;
+  g.x_table = x_table; g.x_stride = x_stride; g.h_table = h_table; g.h_stride = h_stride;
+  g.m_dim = m_dim; g.d = d; g.wpack = wpack; g.b_ih = b_ih; g.b_hh = b_hh; g.h_new = h_new;
+  g.msg_ts = msg_ts; g.check_mem_ts = check_mem_ts; g.check_equal = check_equal; g.err_flags = err_flags;
+  g.x_by_row = 1;
+  return gru_update_launch(g, stream);
+}
+
+extern "C" int tiger_merge_update(const int64_t* node_ids, const int32_t* count, int64_t n_rows,
+                                  const float* x_table, int64_t x_stride, int x_by_row, const float* h_table,
+                                  int64_t h_stride, int m_dim, int d, const float* wpack, const float* b1, float* out,
+                                  const float* msg_ts, const float* check_mem_ts, int check_equal, uint32_t* err_flags,
+                                  void* stream) {
+  GruArgs g{};
+  g.node_ids = node_ids; g.count = count; g.n_rows = n_rows;
+  g.x_table = x_table; g.x_stride = x_stride; g.h_table = h_table; g.h_stride = h_stride;
+  g.m_dim = m_dim; g.d = d; g.wpack = wpack; g.b_ih = b1; g.h_new = out;
+  g.msg_ts = msg_ts; g.check_mem_ts = check_mem_ts; g.check_equal = check_equal; g.err_flags = err_flags;
+  g.x_by_row = x_by_row != 0; g.merge = 1;
+  return gru_update_launch(g, stream);
 }

@@ -11,7 +11,8 @@ Launch sequence of one batch (B events, K neighbors):
   1 tiger_find_recent        3B queries -> neighbor tables, involved bitmap, float32 batch times
   2 tiger_compact_involved   involved / outdated / restart lists + gru_row map
   3 tiger_static_restart     (lazy-restart mode only) re-initialise not-yet-seen nodes
-  4 tiger_gru_update         h(t'+) for the O outdated nodes      (steps 1-2 of the reference)
+  4 tiger_gru_update         h(t'+) for the O outdated nodes      (steps 1-2 of the reference; the message transform
+                             and memory updater variants are ops.MemoryUpdater's launches in this position)
   5 tiger_select_latest      argmax-by-timestamp winners of [src;dst]
   6 tiger_right_writeback    persist h(t'+) of outdated positives (step 4) [+ restarter targets]
   7 tiger_store_messages     build + store the new raw messages   (step 5)
@@ -51,13 +52,18 @@ class TigerEngine:
                  efeats: Optional[Tensor], nfeats: Optional[Tensor] = None, n_neighbors: int = 10,
                  n_head: int = 2, batch_size: int = 200, msg_src: str = 'left', upd_src: str = 'right',
                  restarter: Optional[str] = None, hist_len: int = 40, hit_type: str = 'bin',
-                 lazy_restart: bool = False, want_restarter_targets: bool = False, n_layers: int = 1, device='cuda'):
+                 lazy_restart: bool = False, want_restarter_targets: bool = False, n_layers: int = 1,
+                 msg_tsfm_type: str = 'id', mem_update_type: str = 'gru', device='cuda'):
         if n_layers not in (1, 2):
             raise NotImplementedError(f'n_layers={n_layers}: the engine runs one or two attention layers')
         if msg_src not in ('left', 'right') or upd_src not in ('left', 'right'):
             raise ValueError(f'Invalid msg_src={msg_src} / upd_src={upd_src}')   # tiger.py:156-160
         if hit_type not in ('bin', 'none'):
             raise NotImplementedError(f'hit_type={hit_type}')
+        if msg_tsfm_type not in ops.MemoryUpdater.TSFM:
+            raise NotImplementedError(f'msg_tsfm_type={msg_tsfm_type}')     # tiger.py:104-108
+        if mem_update_type not in ops.MemoryUpdater.UPD:
+            raise NotImplementedError(f'mem_update_type={mem_update_type}')   # tiger.py:110-113
         if lazy_restart and restarter not in ('static', 'seq'):
             raise NotImplementedError(f'lazy restart needs a seq or static restarter, got {restarter!r}')
         dev = torch.device(device)
@@ -112,7 +118,8 @@ class TigerEngine:
         self._serial = int(os.environ.get('TIGER_SERIAL', '0'))   # debug aid, bit mask: branches kept on the main stream
         self._ev_fork, self._ev_side = torch.cuda.Event(), torch.cuda.Event()
         self._ev_fork0, self._ev_rst = torch.cuda.Event(), torch.cuda.Event()
-        self.gru_pack = None
+        # steps 1-2: message transform (--tsfm_fn) + memory updater (--upd_fn), scratch sized for `cap` outdated rows
+        self.updater = ops.MemoryUpdater(msg_tsfm_type, mem_update_type, self.d, self.M, self.cap, dev)
         self.attn_pack = ops.AttnPack(self.d, self.de, dev, n_head)
         self.attn_pack1 = ops.AttnPack(self.d, self.de, dev, n_head) if n_layers == 2 else None   # fns.1 (depth 1)
         self.score_fold = ops.ScoreFold(self.d, dev)
@@ -125,12 +132,7 @@ class TigerEngine:
     def load_weights(self, W: Dict[str, Tensor]):
         """(Re)pack parameters given under the reference's state_dict names."""
         g = lambda k: W[k].detach().to(self.device, f32).contiguous()
-        c = 'right_mem_updater.cell.'
-        args = (g(c + 'weight_ih'), g(c + 'weight_hh'), g(c + 'bias_ih'), g(c + 'bias_hh'))
-        if self.gru_pack is None:
-            self.gru_pack = ops.GruPack(*args)
-        else:
-            self.gru_pack.refresh(*args)
+        self.updater.refresh(g)
         a = 'temporal_embedding_fn.fns.0.'
         self.time_w, self.time_b = g('time_encoder.basis_freq'), g('time_encoder.phase')
         # fns.0 embeds the batch nodes (depth n_layers), fns.1 their neighbors (depth 1); the time encoder is shared
@@ -236,9 +238,9 @@ class TigerEngine:
                     ops.scatter_rows(self.right_vals, self.restart_nodes, hr, ts_table=self.right_ts, ts=pt,
                                      active=self.right_active, count=R)
                 self._ev_rst.record(side0)
-        ops.gru_update(self.gru_pack, node_ids=self.outdated, x_table=self.msg_vals, h_table=upd_vals,
-                       n_rows=self.cap, out=self.h_new, count=self.counts[1:], msg_ts=self.msg_ts,
-                       check_mem_ts=msg_ts_mem, check_equal=(self.msg_src == 'left'), err_flags=self.err_flags)
+        self.updater.launch(node_ids=self.outdated, x_table=self.msg_vals, h_table=upd_vals, n_rows=self.cap,
+                            out=self.h_new, count=self.counts[1:], msg_ts=self.msg_ts, check_mem_ts=msg_ts_mem,
+                            check_equal=(self.msg_src == 'left'), err_flags=self.err_flags)
         # Fork: the write-back / message branch (argmax-by-timestamp selection -> right write-back -> message
         # build + store) only needs the GRU output and the batch, and touches rows the attention never reads
         # (right-memory rows of nodes WITH a pending message are read from h_new, csrc/attention.cu
@@ -327,7 +329,7 @@ class TigerEngine:
             self.neigh_ts64, self.neigh2_nids, self.neigh2_eids, self.neigh2_ts = bufs[5:]
 
     def launches_per_step(self) -> int:
-        n = sum(KERNELS_PER_STEP.values())
+        n = sum(KERNELS_PER_STEP.values()) + self.updater.launches - KERNELS_PER_STEP['gru_update']
         if self.n_layers == 2:
             # hop-2 finder + the float64 widening of the hop-1 times (a torch copy) + the depth-1 attention chain
             n += 2 + KERNELS_PER_STEP['temporal_attention']

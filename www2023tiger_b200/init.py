@@ -15,7 +15,13 @@ def time_basis(d: int) -> torch.Tensor:
 
 
 def random_weights(d: int, de: int, *, n_nodes: int = 0, restarter: Optional[str] = None, hist_len: int = 40,
-                   seed: int = 0, nonzero_static: bool = False, n_layers: int = 1) -> Dict[str, torch.Tensor]:
+                   seed: int = 0, nonzero_static: bool = False, n_layers: int = 1, msg_tsfm_type: str = 'id',
+                   mem_update_type: str = 'gru') -> Dict[str, torch.Tensor]:
+    """msg_tsfm_type / mem_update_type as in build_model: 'linear' adds msg_transform_fn.fn.1 (nn.Linear(M, M)),
+    'mlp' fn.1 / fn.4 (nn.Linear(M, M/2), nn.Linear(M/2, M)); 'merge' replaces right_mem_updater.cell by
+    right_mem_updater.fn (MergeLayer(M, d, d, d), message_modules.py:37-57, update_modules.py:50-56)."""
+    if msg_tsfm_type not in ('id', 'linear', 'mlp') or mem_update_type not in ('gru', 'merge'):
+        raise NotImplementedError(f'msg_tsfm_type={msg_tsfm_type}, mem_update_type={mem_update_type}')
     g = torch.Generator().manual_seed(seed)
     E, C, M = 2 * d, 2 * d + de, 3 * d + de
 
@@ -76,6 +82,16 @@ def random_weights(d: int, de: int, *, n_nodes: int = 0, restarter: Optional[str
     # the lower layers' attention (n_layers > 1) is drawn last, so the weights above do not depend on n_layers
     for i in range(1, n_layers):
         attention_layer(f'temporal_embedding_fn.fns.{i}.', W)
+    # the updater / message transform variants likewise (a merge model draws the GRU cell too, then drops it)
+    if msg_tsfm_type == 'linear':
+        linear(M, M, 'msg_transform_fn.fn.1.', W)
+    elif msg_tsfm_type == 'mlp':
+        linear(M // 2, M, 'msg_transform_fn.fn.1.', W)
+        linear(M, M // 2, 'msg_transform_fn.fn.4.', W)
+    if mem_update_type == 'merge':
+        for n in ('weight_ih', 'weight_hh', 'bias_ih', 'bias_hh'):
+            del W[c + n]
+        merge_layer(M, d, d, d, 'right_mem_updater.fn.', W)
     return W
 
 

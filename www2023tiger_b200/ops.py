@@ -231,15 +231,167 @@ class GruPack:
 def gru_update(pack: GruPack, *, node_ids: Optional[Tensor], x_table: Tensor, h_table: Tensor, n_rows: int,
                out: Optional[Tensor] = None, count: Optional[Tensor] = None, msg_ts: Optional[Tensor] = None,
                check_mem_ts: Optional[Tensor] = None, check_equal: bool = False,
-               err_flags: Optional[Tensor] = None) -> Tensor:
-    """a6+a13: h_new[r] = GRUCell(x_table[ids[r]], h_table[ids[r]]) (ids None => dense rows)."""
+               err_flags: Optional[Tensor] = None, x_by_row: bool = False) -> Tensor:
+    """a6+a13: h_new[r] = GRUCell(x_table[ids[r]], h_table[ids[r]]) (ids None => dense rows).  x_by_row: x is
+    x_table[r] (tiger_gru_update_rows), h and the checks still read node ids[r]."""
     check_cuda(node_ids, x_table, h_table)
     if out is None:
         out = _empty((n_rows, pack.d), f32, x_table)
-    call('tiger_gru_update', ptr(node_ids), ptr(count), n_rows, ptr(x_table), x_table.stride(0), ptr(h_table),
-         h_table.stride(0), pack.m_dim, pack.d, ptr(pack.wpack), ptr(pack.b_ih),
-         ptr(pack.b_hh), ptr(out), ptr(msg_ts), ptr(check_mem_ts), int(check_equal), ptr(err_flags))
+    call('tiger_gru_update_rows' if x_by_row else 'tiger_gru_update', ptr(node_ids), ptr(count), n_rows,
+         ptr(x_table), x_table.stride(0), ptr(h_table), h_table.stride(0), pack.m_dim, pack.d, ptr(pack.wpack),
+         ptr(pack.b_ih), ptr(pack.b_hh), ptr(out), ptr(msg_ts), ptr(check_mem_ts), int(check_equal), ptr(err_flags))
     return out
+
+
+def fold_linear(w: Tensor, b: Tensor, w_t: Tensor, b_t: Tensor) -> Tuple[Tensor, Tensor]:
+    """A layer (w [n, m], b [n]) that consumes the output of a linear map (w_t [m, k], b_t [m]) as one layer on the
+    map's input: (w w_t, b + w b_t), accumulated in float64 and rounded once to float32."""
+    w64 = w.detach().to(f64)
+    return ((w64 @ w_t.detach().to(f64)).to(f32).contiguous(),
+            (b.detach().to(f64) + w64 @ b_t.detach().to(f64)).to(f32).contiguous())
+
+
+class MergePack:
+    """MergeLayer(m, d, d, d) of MergeUpdater as tiger_merge_update reads it: fc1 [d, m + d] pre-split into the stage
+    layout of the GRU kernel (tiger_merge_pack), fc2 as a WeightPack for the count-bounded second product."""
+
+    def __init__(self, fc1_w: Tensor, fc1_b: Tensor, fc2_w: Tensor, fc2_b: Tensor, m_rows_hint: int = 600):
+        self.d = fc2_w.shape[0]
+        self.m_dim = fc1_w.shape[1] - self.d
+        nbytes = _lib.load().tiger_gru_pack_bytes(self.m_dim, self.d)
+        self.wpack = torch.empty(nbytes // 4, dtype=f32, device=fc1_w.device)
+        self.fc2 = WeightPack(fc2_w.detach().to(f32).contiguous(), m_rows_hint=m_rows_hint)
+        self.refresh(fc1_w, fc1_b, fc2_w, fc2_b)
+
+    def refresh(self, fc1_w, fc1_b, fc2_w, fc2_b):
+        w1 = fc1_w.detach().to(f32).contiguous()
+        check_cuda(w1)
+        assert w1.shape == (self.d, self.m_dim + self.d)
+        call('tiger_merge_pack', ptr(w1), self.m_dim, self.d, ptr(self.wpack))
+        self.fc2.refresh(fc2_w.detach().to(f32).contiguous())
+        self.b1 = fc1_b.detach().to(f32).contiguous()
+        self.b2 = fc2_b.detach().to(f32).contiguous()
+
+
+def merge_update(pack: MergePack, *, node_ids: Tensor, x_table: Tensor, h_table: Tensor, n_rows: int, mid: Tensor,
+                 out: Tensor, x_by_row: bool = False, count: Optional[Tensor] = None, msg_ts: Optional[Tensor] = None,
+                 check_mem_ts: Optional[Tensor] = None, check_equal: bool = False,
+                 err_flags: Optional[Tensor] = None) -> Tensor:
+    """MergeUpdater: out[r] = fc2(relu(fc1 [x ; h] + b1)) + b2 with x = x_table[ids[r]] (x_table[r] with x_by_row),
+    h = h_table[ids[r]]; mid [>= n_rows, d] holds the first layer."""
+    check_cuda(node_ids, x_table, h_table, mid, out)
+    call('tiger_merge_update', ptr(node_ids), ptr(count), n_rows, ptr(x_table), x_table.stride(0), int(x_by_row),
+         ptr(h_table), h_table.stride(0), pack.m_dim, pack.d, ptr(pack.wpack), ptr(pack.b1), ptr(mid), ptr(msg_ts),
+         ptr(check_mem_ts), int(check_equal), ptr(err_flags))
+    return sgemm_nt_packed(mid, pack.fc2, pack.b2, out, m_rows=n_rows, count=count)
+
+
+def gather_linear(ids: Tensor, table: Tensor, pack: 'WeightPack', bias: Optional[Tensor], out: Tensor, *,
+                  relu: bool = False, count: Optional[Tensor] = None) -> Tensor:
+    """out[m] = act(W table[ids[m]] + bias) for m < count (the plain-row case of tiger_sgemm_nt_packed_gather)."""
+    check_cuda(ids, table, bias, out)
+    assert ids.dtype == i64 and table.shape[1] == pack.k
+    call('tiger_sgemm_nt_packed_gather', ptr(ids), None, 0, ptr(table), None, table.stride(0), None, ptr(pack.data),
+         pack.bn, ptr(bias), ptr(out), out.stride(0), ids.numel(), ptr(count), 1, pack.n, pack.k, 1.0, int(relu))
+    return out
+
+
+class MemoryUpdater:
+    """Steps 1-2 of the reference (tiger.py:206-221) for every message transform / memory updater pair the reference
+    offers (--tsfm_fn id|linear|mlp, --upd_fn gru|merge): h_new[r] = upd(tsfm(msg_vals[ids[r]]), h[ids[r]]) for the
+    outdated rows r < count, with the message invariants checked.
+
+      id / linear + gru    one tiger_gru_update; a linear transform is folded into weight_ih / bias_ih
+      mlp + gru            the hidden rows relu(W_1 msg + b_1) by row position, then tiger_gru_update_rows on the
+                           fold of W_2 into weight_ih / bias_ih
+      * + merge            as above with tiger_merge_update (folds into fc1's message columns) + the fc2 product
+
+    Folds are computed in float64 whenever `refresh` runs; the device buffers keep their addresses (captured graphs
+    stay valid)."""
+
+    TSFM, UPD = ('id', 'linear', 'mlp'), ('gru', 'merge')
+
+    def __init__(self, tsfm: str, upd: str, d: int, m_dim: int, cap: int, device):
+        if tsfm not in self.TSFM:
+            raise NotImplementedError(f'msg_tsfm_type={tsfm!r}: expected one of {self.TSFM}')
+        if upd not in self.UPD:
+            raise NotImplementedError(f'mem_update_type={upd!r}: expected one of {self.UPD}')
+        self.tsfm, self.upd, self.d, self.m_dim, self.device = tsfm, upd, d, m_dim, device
+        self.cap = 0
+        self.gru = self.merge = self.w1 = self.b1 = None
+        self.hid = self.mid = None
+        self.reserve(cap)
+
+    def reserve(self, cap: int):
+        """Scratch for `cap` outdated rows (hidden rows of the MLP, first layer of the merge)."""
+        if cap <= self.cap:
+            return
+        self.cap = cap
+        z = lambda w: torch.zeros(cap, w, dtype=f32, device=self.device)
+        self.hid = z(self.m_dim // 2) if self.tsfm == 'mlp' else None
+        self.mid = z(self.d) if self.upd == 'merge' else None
+
+    @property
+    def launches(self) -> int:
+        return 1 + (self.tsfm == 'mlp') + (self.upd == 'merge')
+
+    def param_names(self):
+        """The parameters this updater reads, under the reference's state_dict names."""
+        t = {'id': (), 'linear': ('fn.1.weight', 'fn.1.bias'),
+             'mlp': ('fn.1.weight', 'fn.1.bias', 'fn.4.weight', 'fn.4.bias')}[self.tsfm]
+        u = (('cell.weight_ih', 'cell.weight_hh', 'cell.bias_ih', 'cell.bias_hh') if self.upd == 'gru' else
+             ('fn.fc1.weight', 'fn.fc1.bias', 'fn.fc2.weight', 'fn.fc2.bias'))
+        return ['msg_transform_fn.' + n for n in t] + ['right_mem_updater.' + n for n in u]
+
+    def refresh(self, get):
+        """Re-pack from get(name) -> float32 device tensor (names of param_names())."""
+        p = {n: get(n) for n in self.param_names()}
+        t, u = 'msg_transform_fn.fn.', 'right_mem_updater.'
+        fold = None                                      # the linear map in front of the updater's message input
+        if self.tsfm == 'linear':
+            fold = (p[t + '1.weight'], p[t + '1.bias'])
+        elif self.tsfm == 'mlp':
+            fold = (p[t + '4.weight'], p[t + '4.bias'])
+            w1 = p[t + '1.weight'].detach().to(f32).contiguous()
+            if self.w1 is None:
+                self.w1 = WeightPack(w1, m_rows_hint=self.cap)
+            else:
+                self.w1.refresh(w1)
+            self.b1 = p[t + '1.bias'].detach().to(f32).contiguous()
+        if self.upd == 'gru':
+            w_ih, b_ih = p[u + 'cell.weight_ih'], p[u + 'cell.bias_ih']
+            if fold is not None:
+                w_ih, b_ih = fold_linear(w_ih, b_ih, *fold)
+            args = (w_ih, p[u + 'cell.weight_hh'], b_ih, p[u + 'cell.bias_hh'])
+            if self.gru is None:
+                self.gru = GruPack(*args)
+            else:
+                self.gru.refresh(*args)
+        else:
+            fc1, b1 = p[u + 'fn.fc1.weight'], p[u + 'fn.fc1.bias']
+            if fold is not None:
+                wx, b1 = fold_linear(fc1[:, :self.m_dim], b1, *fold)
+                fc1 = torch.cat([wx, fc1[:, self.m_dim:].detach().to(f32)], 1)
+            args = (fc1, b1, p[u + 'fn.fc2.weight'], p[u + 'fn.fc2.bias'])
+            if self.merge is None:
+                self.merge = MergePack(*args, m_rows_hint=self.cap)
+            else:
+                self.merge.refresh(*args)
+
+    def launch(self, *, node_ids: Tensor, x_table: Tensor, h_table: Tensor, n_rows: int, out: Tensor,
+               count: Optional[Tensor], msg_ts: Tensor, check_mem_ts: Optional[Tensor], check_equal: bool,
+               err_flags: Optional[Tensor]):
+        assert n_rows <= self.cap
+        x_by_row = self.tsfm == 'mlp'
+        if x_by_row:
+            x_table = gather_linear(node_ids[:n_rows], x_table, self.w1, self.b1, self.hid[:n_rows], relu=True,
+                                    count=count)
+        kw = dict(node_ids=node_ids, x_table=x_table, h_table=h_table, n_rows=n_rows, out=out, count=count,
+                  msg_ts=msg_ts, check_mem_ts=check_mem_ts, check_equal=check_equal, err_flags=err_flags,
+                  x_by_row=x_by_row)
+        if self.upd == 'gru':
+            return gru_update(self.gru, **kw)
+        return merge_update(self.merge, mid=self.mid, **kw)
 
 
 class AttnParamsC(ctypes.Structure):

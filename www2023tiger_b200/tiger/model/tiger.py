@@ -3,7 +3,8 @@
 
 `contrast_learning` has two routes:
 * no-grad (evaluation, warm-up, `flush_msg`): the fused launch sequence of DESIGN.md §3, in the order of
-  TigerEngine.launch_model on the caller's stream - compaction of the pending-message set, gather+GRU,
+  TigerEngine.launch_model on the caller's stream - compaction of the pending-message set, gather + message
+  transform + memory updater (GRU or merge, ops.MemoryUpdater),
   argmax-by-timestamp selection, right write-back, message build+store, fused temporal attention whose last
   product also writes the left memory and the folded scorer's first layer, link scorer - with every
   data-dependent size kept on the device; one host poll of the error word per batch.
@@ -132,6 +133,7 @@ class TIGE(nn.Module):
         self._err = ErrFlags()
         self._ws: Optional[_Workspace] = None
         self._fold, self._fold_key = None, None
+        self._updater, self._updater_key = None, None
 
     def _bind_sources(self):
         self.msg_memory = self.left_memory if self.msg_src == 'left' else self.right_memory
@@ -151,9 +153,29 @@ class TIGE(nn.Module):
 
     # ------------------------------------------------------------------ fused no-grad route
     def _fusable(self) -> bool:
-        return (isinstance(self.msg_transform_fn, IdentityMessageFunction)
-                and isinstance(self.right_mem_updater, GRUUpdater) and self.n_layers in (1, 2)
+        return (isinstance(self.msg_transform_fn, (IdentityMessageFunction, LinearMessageFunction, MLPMessageFunction))
+                and isinstance(self.right_mem_updater, (GRUUpdater, MergeUpdater)) and self.n_layers in (1, 2)
                 and self.hit_type in ('bin', 'none') and self.left_memory.vals.is_cuda)
+
+    def _memory_updater(self, cap: int) -> ops.MemoryUpdater:
+        """Steps 1-2 of the fused route for this model's message transform and memory updater, with the transform
+        folded into the updater's message weights; re-packed when one of their parameters changes (optimizer steps,
+        load_state_dict)."""
+        tsfm = {IdentityMessageFunction: 'id', LinearMessageFunction: 'linear',
+                MLPMessageFunction: 'mlp'}[type(self.msg_transform_fn)]
+        upd = 'gru' if isinstance(self.right_mem_updater, GRUUpdater) else 'merge'
+        u = self._updater
+        if u is None or (u.tsfm, u.upd) != (tsfm, upd) or u.device != self.device:
+            u = self._updater = ops.MemoryUpdater(tsfm, upd, self.memory_dim, self.raw_msg_dim, cap, self.device)
+            self._updater_key = None
+        u.reserve(cap)
+        params = [self.get_parameter(n) for n in u.param_names()]
+        key = tuple((p.data_ptr(), p._version) for p in params)
+        if key != self._updater_key:
+            p = dict(zip(u.param_names(), params))
+            u.refresh(lambda n: f32c(p[n]))
+            self._updater_key = key
+        return u
 
     def _workspace(self, B: int, K: int) -> _Workspace:
         dev = self.device
@@ -190,14 +212,15 @@ class TIGE(nn.Module):
         pos = batch_nids[:2 * B]
         ts = f32c(ts)
         fg = self.raw_feat_getter
-        # steps 1-2: pending-message set of the involved nodes, gather + GRU (tiger.py:206-221)
+        # steps 1-2: pending-message set of the involved nodes, gather + message transform + updater (tiger.py:206-221)
         ops.mark_nodes(cg.computation_graph_nodes.contiguous(), ws.bitmap, N)
         ops.compact_involved(ws.bitmap, N, ws.involved, ws.counts, has_msg=store.has_msg, outdated=ws.outdated,
                              gru_row=ws.gru_row, err_flags=err)
-        ops.gru_update(self.right_mem_updater.packed(), node_ids=ws.outdated, x_table=store.node_msg_vals,
-                       h_table=self.upd_memory.vals, n_rows=ws.cap, out=ws.h_new, count=ws.counts[1:],
-                       msg_ts=store.node_msg_ts, check_mem_ts=self.msg_memory.update_ts,
-                       check_equal=(self.msg_src == 'left'), err_flags=err)
+        self._memory_updater(ws.cap).launch(node_ids=ws.outdated, x_table=store.node_msg_vals,
+                                            h_table=self.upd_memory.vals, n_rows=ws.cap, out=ws.h_new,
+                                            count=ws.counts[1:], msg_ts=store.node_msg_ts,
+                                            check_mem_ts=self.msg_memory.update_ts,
+                                            check_equal=(self.msg_src == 'left'), err_flags=err)
         # steps 4-5 (tiger.py:230-255) ahead of step 3, in TigerEngine.launch_model's order: the right write-back
         # writes only rows the attention reads from h_new, the message builder only the message store (DESIGN.md §3,
         # "Why the post-GRU branches may overlap"), and both read the old left rows before the last attention
@@ -412,6 +435,8 @@ class TIGER(TIGE):
         from www2023tiger_b200.train import native_limit_error
         from .restarters import SeqRestarter, StaticRestarter
         return (torch.is_grad_enabled() and self.training and self._fusable()
+                and isinstance(self.msg_transform_fn, IdentityMessageFunction)
+                and isinstance(self.right_mem_updater, GRUUpdater)
                 and isinstance(self.restarter_fn, (SeqRestarter, StaticRestarter))
                 and native_limit_error(self) is None
                 and os.environ.get('TIGER_AUTOGRAD_ROUTE') != '1')
