@@ -284,6 +284,27 @@ int64_t tiger_score_fold_cab_offset(int d);   /* float offset of the c_ab table 
 int tiger_score_fold(const float* score_fc1, const float* score_fc1_b, const float* merger_fc2,
                      const float* merger_fc2_b, const float* hit_emb, int d, float* blob, void* stream);
 
+/* the scorer's hit types (--hit_type, tiger.py:129-136,259-288) */
+#define TIGER_HIT_NONE 0
+#define TIGER_HIT_BIN 1
+#define TIGER_HIT_VEC 2
+#define TIGER_HIT_COUNT 3
+
+/* The same fold for every hit type, with K = n_neighbors (ignored for 'bin' / 'none', whose blob is exactly
+ * tiger_score_fold's).  The head of the blob (W3, b3, c_ab, pack) keeps its layout; 'count' and 'vec' append
+ * their hit tables behind it (c_ab stays zero):
+ *   count: hit_emb [K+1][d]; tables U [K+1][d] | V [K+1][d], U[c] = b1 + W1a he_c, V[c] = W1b he_c.
+ *   vec  : hit_emb NULL, score_fc1 [d][2(d+K)] = [W1a | Ha | W1b | Hb] (score_fn = MergeLayer(d+K, d+K, d, 1));
+ *          tables b1 [d] | Ha^T [K][d] | Hb^T [K][d].
+ * hit_emb [2][d] for 'bin', NULL for 'none'.  -1 / TIGER_EINVAL for an unknown hit type or K <= 0 ('vec',
+ * 'count'). */
+int64_t tiger_score_fold_hit_bytes(int d, int hit_type, int k);
+int64_t tiger_score_fold_hit_offset(int d, int hit_type, int k);   /* float offset of the scorer's table:
+                                                                      c_ab ('bin', 'none') or the hit tables */
+int tiger_score_fold_hit(const float* score_fc1, const float* score_fc1_b, const float* merger_fc2,
+                         const float* merger_fc2_b, const float* hit_emb, int d, int hit_type, int k, float* blob,
+                         void* stream);
+
 /* bytes of caller-provided, 16-byte aligned workspace for n_query queries */
 int64_t tiger_temporal_attention_work_bytes(int64_t n_query, int k, int d, int de, int n_head);
 
@@ -327,6 +348,17 @@ int tiger_link_score_folded(const float* pq, int64_t batch, int d, const int64_t
                             const int64_t* neg, const int64_t* neigh_nids, int k, const float* cab,
                             const float* fc2_w, const float* fc2_b, float* scores, float* loss,
                             uint32_t* done_counter, void* stream);
+
+/* The same scorer for every hit type (TIGER_HIT_*); tables = blob + tiger_score_fold_hit_offset(d, hit_type, k).
+ * With the hit flags a_j = [N(t)[j] == s], b_j = [N(s)[j] == t] of a pair (s, t) over the K slots of the
+ * neighbor table, the first layer is P[s] + Q[t] plus
+ *   bin  : c_ab[2 any(a) + any(b)]          count: U[sum a] + V[sum b]
+ *   none : c_ab[0] (neigh_nids ignored)     vec  : b1 + sum_{a_j} Ha^T[j] + sum_{b_j} Hb^T[j]
+ * One launch per batch, any K >= 1 (neigh_nids required except for 'none'). */
+int tiger_link_score_folded_hit(const float* pq, int64_t batch, int d, const int64_t* src, const int64_t* dst,
+                                const int64_t* neg, const int64_t* neigh_nids, int k, int hit_type,
+                                const float* tables, const float* fc2_w, const float* fc2_b, float* scores,
+                                float* loss, uint32_t* done_counter, void* stream);
 
 /* ---------------------------------------------------------------------------------------
  * Restarters (tiger/model/restarters.py, tiger.py:594-609)

@@ -47,6 +47,10 @@ _SIGNATURES: Dict[str, str] = {
     'tiger_score_fold_cab_offset': 'i',
     'tiger_score_fold': 'pppppip' + 'p',
     'tiger_link_score_folded': 'pli' + 'pppp' + 'i' + 'ppp' + 'ppp' + 'p',
+    'tiger_score_fold_hit_bytes': 'iii',
+    'tiger_score_fold_hit_offset': 'iii',
+    'tiger_score_fold_hit': 'pppppiii' + 'p' + 'p',
+    'tiger_link_score_folded_hit': 'pli' + 'pppp' + 'ii' + 'ppp' + 'ppp' + 'p',
     'tiger_sgemm_nt_packed_gather': 'ppi' + 'pplp' + 'pi' + 'ppl' + 'lpl' + 'iifi' + 'p',
     'tiger_sgemm_nt_packed_splitk_fused': 'plpi' + 'ppl' + 'i' + 'lpl' + 'iifi' + 'p',
     'tiger_pipe_capture_begin': 'p',

@@ -212,9 +212,13 @@ extern "C" int tiger_attn_fold(const tiger_attn_params* p, int d, int de, int n_
 // split output), and scoring a pair is an elementwise relu(P[s] + Q[t] + c_ab) . w2 - the 17 us weight-
 // streaming scorer kernel becomes a 2 x 688-byte row read per pair.
 //   blob: w3 [n_split + 2d][d] | b3 [n_split + 2d] | cab [4][d] (c_ab, index 2a + b) | tf32 pack of w3
+// The 'count' and 'vec' hit types (tiger_score_fold_hit) keep this head and append their tables [rows][d]:
+//   count: U [K+1][d] | V [K+1][d], U[c] = b1 + W1a he_c, V[c] = W1b he_c (pair term U[ca] + V[cb])
+//   vec  : b1 [d] | Ha^T [K][d] | Hb^T [K][d]; fc1 [d][2(d+K)] = [W1a | Ha | W1b | Hb] (pair term
+//          b1 + sum of the Ha^T / Hb^T rows of the hit slots)
 // ------------------------------------------------------------------------------------------
 struct ScoreFold {
-  float *w3, *b3, *cab, *pack;
+  float *w3, *b3, *cab, *pack, *hit;
   int n_split, tiles;
   int64_t total_floats;
 };
@@ -230,7 +234,25 @@ static ScoreFold score_fold(int d, float* base) {
   f.b3 = take(rows);
   f.cab = take(4 * d);
   f.pack = take(tiger_gemm_pack_bytes(f.tiles, d, ATT_BN_F3) / 4);
+  f.hit = nullptr;
   f.total_floats = off;
+  return f;
+}
+
+// rows [ ][d] of the hit tables behind the head; -1: not a hit type of tiger_score_fold_hit (or K out of range)
+static int score_hit_rows(int hit_type, int k) {
+  switch (hit_type) {
+    case TIGER_HIT_NONE: case TIGER_HIT_BIN: return 0;
+    case TIGER_HIT_VEC: return k > 0 ? 1 + 2 * k : -1;
+    case TIGER_HIT_COUNT: return k > 0 ? 2 * (k + 1) : -1;
+    default: return -1;
+  }
+}
+
+static ScoreFold score_fold_hit(int d, int hit_type, int k, float* base) {
+  ScoreFold f = score_fold(d, base);
+  f.hit = base ? base + f.total_floats : nullptr;
+  f.total_floats += ((int64_t)score_hit_rows(hit_type, k) * d + 3) & ~(int64_t)3;
   return f;
 }
 
@@ -247,39 +269,89 @@ extern "C" int64_t tiger_score_fold_cab_offset(int d) {
   return (int64_t)(f.cab - &dummy);
 }
 
-extern "C" int tiger_score_fold(const float* score_fc1, const float* score_fc1_b, const float* merger_fc2,
-                                const float* merger_fc2_b, const float* hit_emb, int d, float* blob, void* stream) {
+extern "C" int64_t tiger_score_fold_hit_bytes(int d, int hit_type, int k) {
+  if (d <= 0 || score_hit_rows(hit_type, k) < 0) return -1;
+  return score_fold_hit(d, hit_type, k, nullptr).total_floats * (int64_t)sizeof(float);
+}
+
+// float offset of the table tiger_link_score_folded_hit reads: c_ab for 'bin' / 'none', the hit tables otherwise
+extern "C" int64_t tiger_score_fold_hit_offset(int d, int hit_type, int k) {
+  if (d <= 0 || score_hit_rows(hit_type, k) < 0) return -1;
+  float dummy;
+  const ScoreFold f = score_fold_hit(d, hit_type, k, &dummy);
+  return (int64_t)((hit_type == TIGER_HIT_VEC || hit_type == TIGER_HIT_COUNT ? f.hit : f.cab) - &dummy);
+}
+
+// hit tables of the 'count' / 'vec' fold (layout above), one thread per (row r, output m), double accumulation
+__global__ void score_hit_fold_kernel(const float* __restrict__ fc1, int64_t ld1, const float* __restrict__ b1,
+                                      const float* __restrict__ hit_emb, int d, int k, int hit_type,
+                                      float* __restrict__ out) {
+  const int m = blockIdx.x * blockDim.x + threadIdx.x, r = blockIdx.y;
+  if (m >= d) return;
+  const float* w = fc1 + (int64_t)m * ld1;
+  double acc;
+  if (hit_type == TIGER_HIT_COUNT) {
+    const int side = r / (k + 1), c = r % (k + 1);        // rows [0, K] = U, [K+1, 2K+1] = V
+    const float* wc = w + side * d;                        // W1a / W1b
+    const float* e = hit_emb + (int64_t)c * d;
+    acc = side == 0 ? (double)b1[m] : 0.0;
+    for (int i = 0; i < d; ++i) acc += (double)wc[i] * (double)e[i];
+  } else {                                                  // row 0 = b1, 1 + j = Ha[:, j], 1 + K + j = Hb[:, j]
+    const int side = (r - 1) / k, j = (r - 1) % k;
+    acc = r == 0 ? (double)b1[m] : (double)w[side * (d + k) + d + j];
+  }
+  out[(int64_t)r * d + m] = (float)acc;
+}
+
+extern "C" int tiger_score_fold_hit(const float* score_fc1, const float* score_fc1_b, const float* merger_fc2,
+                                    const float* merger_fc2_b, const float* hit_emb, int d, int hit_type, int k,
+                                    float* blob, void* stream) {
+  const int hit_rows = score_hit_rows(hit_type, k);
   if (score_fc1 == nullptr || score_fc1_b == nullptr || merger_fc2 == nullptr || merger_fc2_b == nullptr ||
-      blob == nullptr || d <= 0 || (((uintptr_t)blob) & 15) != 0)
+      blob == nullptr || d <= 0 || hit_rows < 0 || (((uintptr_t)blob) & 15) != 0)
     return TIGER_EINVAL;
-  const ScoreFold f = score_fold(d, blob);
+  if ((hit_emb != nullptr) != (hit_type == TIGER_HIT_BIN || hit_type == TIGER_HIT_COUNT)) return TIGER_EINVAL;
+  const ScoreFold f = score_fold_hit(d, hit_type, k, blob);
   cudaStream_t st = as_stream(stream);
-  const int64_t ld1 = 2 * d;
+  // fc1 [d][ld1]: [W1a | W1b] for 'bin' / 'none' / 'count', [W1a | Ha | W1b | Hb] for 'vec'
+  const bool vec = hit_type == TIGER_HIT_VEC;
+  const int64_t ld1 = vec ? 2 * (d + k) : 2 * d, w1b_col = vec ? d + k : d;
   if (cudaMemsetAsync(blob, 0, (size_t)f.total_floats * sizeof(float), st) != cudaSuccess) return TIGER_ECUDA;
   // rows [0, d): W2 (copy) ; rows [n_split, n_split + d): W1a W2 ; rows [n_split + d, n_split + 2d): W1b W2
   if (cudaMemcpyAsync(f.w3, merger_fc2, (size_t)d * d * sizeof(float), cudaMemcpyDeviceToDevice, st) != cudaSuccess ||
       cudaMemcpyAsync(f.b3, merger_fc2_b, (size_t)d * sizeof(float), cudaMemcpyDeviceToDevice, st) != cudaSuccess)
     return TIGER_ECUDA;
   for (int half = 0; half < 2; ++half) {
-    const float* w1 = score_fc1 + half * d;   // W1a / W1b: columns [half*d, half*d + d) of fc1 [d][2d]
+    const float* w1 = score_fc1 + half * w1b_col;   // W1a / W1b
     fold_mm(st, w1, ld1, 1, merger_fc2, d, 1, f.w3 + (int64_t)(f.n_split + half * d) * d, d, d, d, d, 1.0f, nullptr);
     fold_mm(st, w1, ld1, 1, merger_fc2_b, 1, 0, f.b3 + f.n_split + half * d, 1, d, 1, d, 1.0f, nullptr);
   }
-  // c_ab = b1 + W1a he_a + W1b he_b
-  for (int a = 0; a < 2; ++a)
-    for (int b = 0; b < 2; ++b) {
-      float* c = f.cab + (2 * a + b) * d;
-      if (hit_emb == nullptr) {
-        if (cudaMemcpyAsync(c, score_fc1_b, (size_t)d * sizeof(float), cudaMemcpyDeviceToDevice, st) != cudaSuccess)
-          return TIGER_ECUDA;
-      } else {
-        fold_mm(st, score_fc1, ld1, 1, hit_emb + a * d, 1, 0, c, 1, d, 1, d, 1.0f, score_fc1_b);
-        // second half accumulates onto the first: add = c itself
-        fold_mm(st, score_fc1 + d, ld1, 1, hit_emb + b * d, 1, 0, c, 1, d, 1, d, 1.0f, c);
+  if (hit_rows > 0) {
+    score_hit_fold_kernel<<<dim3((unsigned)((d + 127) / 128), (unsigned)hit_rows), 128, 0, st>>>(
+        score_fc1, ld1, score_fc1_b, hit_emb, d, k, hit_type, f.hit);
+  } else {
+    // c_ab = b1 + W1a he_a + W1b he_b
+    for (int a = 0; a < 2; ++a)
+      for (int b = 0; b < 2; ++b) {
+        float* c = f.cab + (2 * a + b) * d;
+        if (hit_emb == nullptr) {
+          if (cudaMemcpyAsync(c, score_fc1_b, (size_t)d * sizeof(float), cudaMemcpyDeviceToDevice, st) != cudaSuccess)
+            return TIGER_ECUDA;
+        } else {
+          fold_mm(st, score_fc1, ld1, 1, hit_emb + a * d, 1, 0, c, 1, d, 1, d, 1.0f, score_fc1_b);
+          // second half accumulates onto the first: add = c itself
+          fold_mm(st, score_fc1 + d, ld1, 1, hit_emb + b * d, 1, 0, c, 1, d, 1, d, 1.0f, c);
+        }
       }
-    }
+  }
   if (tiger_launch_status() != TIGER_OK) return TIGER_ECUDA;
   return tiger_gemm_pack_weight(f.w3, d, nullptr, f.n_split + 2 * d, d, ATT_BN_F3, f.tiles, f.pack, stream);
+}
+
+extern "C" int tiger_score_fold(const float* score_fc1, const float* score_fc1_b, const float* merger_fc2,
+                                const float* merger_fc2_b, const float* hit_emb, int d, float* blob, void* stream) {
+  return tiger_score_fold_hit(score_fc1, score_fc1_b, merger_fc2, merger_fc2_b, hit_emb, d,
+                              hit_emb != nullptr ? TIGER_HIT_BIN : TIGER_HIT_NONE, 0, blob, stream);
 }
 
 // ------------------------------------------------------------------------------------------

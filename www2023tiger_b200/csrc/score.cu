@@ -1,14 +1,22 @@
 // Link scorer: step 7 of TIGE.contrast_learning (tiger/model/tiger.py:259-288), eval mode:
-// hit flags ('bin': tiger.py:266-270, data_loader.py:61-75) -> hit embedding -> score_fn
-// MergeLayer (basic_modules.py:16-19) on positive and negative pairs -> BCE-with-logits mean.
+// hit flags (tiger.py:266-270, data_loader.py:61-75) -> hit term -> score_fn MergeLayer (basic_modules.py:16-19)
+// on positive and negative pairs -> BCE-with-logits mean.
 //
-// Folded form (see tiger_score_fold in attention.cu): the first scorer layer was applied to every
-// embedding row by the last attention GEMM (PQ[row] = [W1a z | W1b z]); a pair (s, t) with hit flags (a, b)
-// scores  w2 . relu(P[s] + Q[t] + c_ab) + b2.  One warp per pair; the BCE mean is reduced by the last CTA
-// in a fixed order, so the loss does not depend on the order in which the CTAs finish.
+// Folded form (see tiger_score_fold_hit in attention.cu): the first scorer layer was applied to every
+// embedding row by the last attention GEMM (PQ[row] = [W1a z | W1b z]); a pair (s, t) with hit flags a_j = [N(t)[j] == s],
+// b_j = [N(s)[j] == t] scores  w2 . relu(P[s] + Q[t] + h(a, b)) + b2  with the hit term h of the hit type
+// (compile-time mode HIT):
+//   bin / none : c_ab[2 any(a) + any(b)]              (four pre-folded constants; none: c_00, no table read)
+//   count      : U[sum a] + V[sum b]                  (hit embedding of the counts folded through W1a / W1b)
+//   vec        : b1 + sum_{a_j} Ha^T[j] + sum_{b_j} Hb^T[j]   (the hit vectors' columns of fc1)
+// One warp per pair; the flags of 32 slots at a time come from one ballot per side.  The BCE mean is reduced by the
+// last CTA in a fixed order, so the loss does not depend on the order in which the CTAs finish.
 #include "common.cuh"
 
 #define SCOREF_WARPS 8
+// HIT = TIGER_HIT_BIN also serves 'none' (neigh == NULL); `cab` is the table of the hit type (c_ab, U | V or
+// b1 | Ha^T | Hb^T, tiger_score_fold_hit_offset)
+template <int HIT>
 __global__ void __launch_bounds__(SCOREF_WARPS * 32)
 link_score_folded_kernel(const float* __restrict__ pq, int64_t batch, int d, const int64_t* __restrict__ src,
                          const int64_t* __restrict__ dst, const int64_t* __restrict__ neg,
@@ -26,22 +34,67 @@ link_score_folded_kernel(const float* __restrict__ pq, int64_t batch, int d, con
     const bool is_neg = p >= batch;
     const int64_t e = is_neg ? p - batch : p;
     const int64_t row_s = e, row_t = is_neg ? 2 * batch + e : batch + e;     // rows of [src ; dst ; neg]
-    int fa = 0, fb = 0;
-    if (neigh != nullptr) {
-      // src_hits: src in N(target) ; dst_hits: target in N(src)   (tiger.py:266-270, data_loader.py:61-75)
-      const int64_t s_id = src[e], t_id = is_neg ? neg[e] : dst[e];
-      for (int j = lane; j < k; j += 32) {
-        fa |= (neigh[row_t * k + j] == s_id);
-        fb |= (neigh[row_s * k + j] == t_id);
-      }
-      fa = __any_sync(TIGER_FULL_MASK, fa);
-      fb = __any_sync(TIGER_FULL_MASK, fb);
-    }
-    const float* P = pq + row_s * 2 * d;
-    const float* Q = pq + row_t * 2 * d + d;
-    const float* c = cab + (2 * fa + fb) * d;
     float acc = 0.f;
-    for (int j = lane; j < d; j += 32) acc = fmaf(fmaxf(P[j] + Q[j] + c[j], 0.f), fc2_w[j], acc);
+    if constexpr (HIT == TIGER_HIT_BIN) {
+      int fa = 0, fb = 0;
+      if (neigh != nullptr) {
+        // src_hits: src in N(target) ; dst_hits: target in N(src)   (tiger.py:266-270, data_loader.py:61-75)
+        const int64_t s_id = src[e], t_id = is_neg ? neg[e] : dst[e];
+        for (int j = lane; j < k; j += 32) {
+          fa |= (neigh[row_t * k + j] == s_id);
+          fb |= (neigh[row_s * k + j] == t_id);
+        }
+        fa = __any_sync(TIGER_FULL_MASK, fa);
+        fb = __any_sync(TIGER_FULL_MASK, fb);
+      }
+      const float* P = pq + row_s * 2 * d;
+      const float* Q = pq + row_t * 2 * d + d;
+      const float* c = cab + (2 * fa + fb) * d;
+      for (int j = lane; j < d; j += 32) acc = fmaf(fmaxf(P[j] + Q[j] + c[j], 0.f), fc2_w[j], acc);
+    } else {
+      const float* P = pq + row_s * 2 * d;
+      const float* Q = pq + row_t * 2 * d + d;
+      // slot flags a_j (src in N(target)) / b_j (target in N(src)) of slots [c0, c0 + 32), one ballot per side;
+      // the loops around the ballots are warp-uniform
+      const int64_t s_id = src[e], t_id = is_neg ? neg[e] : dst[e];
+      const int64_t *na = neigh + row_t * k, *nb = neigh + row_s * k;
+      auto ballots = [&](int c0, uint32_t& ma, uint32_t& mb) {
+        const int j = c0 + lane;
+        ma = __ballot_sync(TIGER_FULL_MASK, j < k && na[j] == s_id);
+        mb = __ballot_sync(TIGER_FULL_MASK, j < k && nb[j] == t_id);
+      };
+      if constexpr (HIT == TIGER_HIT_COUNT) {
+        int ca = 0, cb = 0;
+        for (int c0 = 0; c0 < k; c0 += 32) {
+          uint32_t ma, mb;
+          ballots(c0, ma, mb);
+          ca += __popc(ma);
+          cb += __popc(mb);
+        }
+        const float* U = cab + (int64_t)ca * d;
+        const float* V = cab + (int64_t)(k + 1 + cb) * d;
+        for (int j = lane; j < d; j += 32) acc = fmaf(fmaxf(P[j] + Q[j] + U[j] + V[j], 0.f), fc2_w[j], acc);
+      } else {
+        static_assert(HIT == TIGER_HIT_VEC, "hit mode");
+        const float* Ha = cab + d;                        // Ha^T [K][d], then Hb^T [K][d]
+        const float* Hb = cab + (int64_t)(1 + k) * d;
+        uint32_t ma0, mb0;
+        ballots(0, ma0, mb0);
+        for (int j0 = 0; j0 < d; j0 += 32) {
+          const int j = j0 + lane;
+          float h = 0.f;
+          for (int c0 = 0; c0 < k; c0 += 32) {            // K > 32: the later chunks' ballots again per column block
+            uint32_t ma = ma0, mb = mb0;
+            if (c0 > 0) ballots(c0, ma, mb);
+            if (j < d) {
+              for (; ma != 0u; ma &= ma - 1u) h += Ha[(int64_t)(c0 + __ffs(ma) - 1) * d + j];
+              for (; mb != 0u; mb &= mb - 1u) h += Hb[(int64_t)(c0 + __ffs(mb) - 1) * d + j];
+            }
+          }
+          if (j < d) acc = fmaf(fmaxf(P[j] + Q[j] + cab[j] + h, 0.f), fc2_w[j], acc);
+        }
+      }
+    }
     acc = warp_sum(acc);
     if (lane == 0) scores[p] = acc + fc2_b[0];
   }
@@ -69,15 +122,30 @@ link_score_folded_kernel(const float* __restrict__ pq, int64_t batch, int d, con
   }
 }
 
+extern "C" int tiger_link_score_folded_hit(const float* pq, int64_t batch, int d, const int64_t* src,
+                                           const int64_t* dst, const int64_t* neg, const int64_t* neigh_nids, int k,
+                                           int hit_type, const float* tables, const float* fc2_w, const float* fc2_b,
+                                           float* scores, float* loss, uint32_t* done_counter, void* stream) {
+  if (hit_type == TIGER_HIT_NONE) neigh_nids = nullptr;
+  else if (hit_type != TIGER_HIT_BIN && hit_type != TIGER_HIT_VEC && hit_type != TIGER_HIT_COUNT) return TIGER_EINVAL;
+  else if (neigh_nids == nullptr || k <= 0) return TIGER_EINVAL;
+  if (pq == nullptr || tables == nullptr || batch < 0 || d <= 0) return TIGER_EINVAL;
+  if (loss != nullptr && done_counter == nullptr) return TIGER_EINVAL;
+  if (batch == 0) return TIGER_OK;
+  const unsigned grid = (unsigned)((2 * batch + SCOREF_WARPS - 1) / SCOREF_WARPS);
+  decltype(&link_score_folded_kernel<TIGER_HIT_BIN>) kernel =
+      hit_type == TIGER_HIT_VEC     ? link_score_folded_kernel<TIGER_HIT_VEC>
+      : hit_type == TIGER_HIT_COUNT ? link_score_folded_kernel<TIGER_HIT_COUNT>
+                                    : link_score_folded_kernel<TIGER_HIT_BIN>;
+  return tiger_launch_chain(kernel, dim3(grid), dim3(SCOREF_WARPS * 32), 0, as_stream(stream), dim3(1, 1, 1), pq, batch,
+                            d, src, dst, neg, neigh_nids, k, tables, fc2_w, fc2_b, scores, loss, done_counter);
+}
+
 extern "C" int tiger_link_score_folded(const float* pq, int64_t batch, int d, const int64_t* src, const int64_t* dst,
                                        const int64_t* neg, const int64_t* neigh_nids, int k, const float* cab,
                                        const float* fc2_w, const float* fc2_b, float* scores, float* loss,
                                        uint32_t* done_counter, void* stream) {
-  if (pq == nullptr || cab == nullptr || batch < 0 || d <= 0 || (neigh_nids != nullptr && k <= 0)) return TIGER_EINVAL;
-  if (loss != nullptr && done_counter == nullptr) return TIGER_EINVAL;
-  if (batch == 0) return TIGER_OK;
-  const unsigned grid = (unsigned)((2 * batch + SCOREF_WARPS - 1) / SCOREF_WARPS);
-  return tiger_launch_chain(link_score_folded_kernel, dim3(grid), dim3(SCOREF_WARPS * 32), 0, as_stream(stream),
-                            dim3(1, 1, 1), pq, batch, d, src, dst, neg, neigh_nids, k, cab, fc2_w, fc2_b, scores, loss,
-                            done_counter);
+  return tiger_link_score_folded_hit(pq, batch, d, src, dst, neg, neigh_nids, k,
+                                     neigh_nids != nullptr ? TIGER_HIT_BIN : TIGER_HIT_NONE, cab, fc2_w, fc2_b, scores,
+                                     loss, done_counter, stream);
 }

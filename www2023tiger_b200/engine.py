@@ -58,25 +58,27 @@ class TigerEngine:
             raise NotImplementedError(f'n_layers={n_layers}: the engine runs one or two attention layers')
         if msg_src not in ('left', 'right') or upd_src not in ('left', 'right'):
             raise ValueError(f'Invalid msg_src={msg_src} / upd_src={upd_src}')   # tiger.py:156-160
-        if hit_type not in ('bin', 'none'):
-            raise NotImplementedError(f'hit_type={hit_type}')
+        if hit_type not in ops.HIT_TYPES:
+            raise NotImplementedError(f'hit_type={hit_type}')                  # tiger.py:129-136
         if msg_tsfm_type not in ops.MemoryUpdater.TSFM:
             raise NotImplementedError(f'msg_tsfm_type={msg_tsfm_type}')     # tiger.py:104-108
         if mem_update_type not in ops.MemoryUpdater.UPD:
             raise NotImplementedError(f'mem_update_type={mem_update_type}')   # tiger.py:110-113
         if lazy_restart and restarter not in ('static', 'seq'):
             raise NotImplementedError(f'lazy restart needs a seq or static restarter, got {restarter!r}')
+        self.hit_type, self.K = hit_type, n_neighbors
+        self.d = nfeats.shape[1] if nfeats is not None else dim              # feature_getter.py:76-77
+        self._check_hit_weights(weights)
         dev = torch.device(device)
         self.device, self.csr = dev, csr
-        self.N, self.K, self.H, self.B = n_nodes, n_neighbors, n_head, batch_size
+        self.N, self.H, self.B = n_nodes, n_head, batch_size
         self.n_layers = n_layers
         self.efeats = efeats
         self.nfeats = nfeats
-        self.d = nfeats.shape[1] if nfeats is not None else dim              # feature_getter.py:76-77
         self.de = efeats.shape[1] if efeats is not None else dim
         self.M = 3 * self.d + self.de                                          # tiger.py:62
         self.msg_src, self.upd_src = msg_src, upd_src
-        self.restarter, self.hit_type, self.lazy_restart = restarter, hit_type, lazy_restart
+        self.restarter, self.lazy_restart = restarter, lazy_restart
         self.want_targets = want_restarter_targets
         N, d, B, K = self.N, self.d, self.B, self.K
         z = lambda *s, dt=f32: torch.zeros(*s, dtype=dt, device=dev)
@@ -122,15 +124,27 @@ class TigerEngine:
         self.updater = ops.MemoryUpdater(msg_tsfm_type, mem_update_type, self.d, self.M, self.cap, dev)
         self.attn_pack = ops.AttnPack(self.d, self.de, dev, n_head)
         self.attn_pack1 = ops.AttnPack(self.d, self.de, dev, n_head) if n_layers == 2 else None   # fns.1 (depth 1)
-        self.score_fold = ops.ScoreFold(self.d, dev)
+        self.score_fold = ops.ScoreFold(self.d, dev, hit_type, K)
         self.pq = torch.zeros(3 * batch_size, 2 * self.d, dtype=f32, device=dev)   # [W1a z | W1b z] per query row
         self.hist_len = hist_len
         self.seq = ops.SeqRestarterOp(self.d, self.de, hist_len, n_head, self.cap, dev) if restarter == 'seq' else None
         self.load_weights(weights)
 
     # ------------------------------------------------------------------ parameters
+    def _check_hit_weights(self, W: Dict[str, Tensor]):
+        """The scorer's hit parameters are sized by K (tiger.py:129-136); the fold reads them with this engine's K."""
+        d, K = self.d, self.K
+        want = {'count': ('hit_embedding.weight', (K + 1, d)), 'vec': ('score_fn.fc1.weight', (d, 2 * (d + K)))}
+        if self.hit_type in want:
+            name, shape = want[self.hit_type]
+            if name not in W or tuple(W[name].shape) != shape:
+                got = tuple(W[name].shape) if name in W else 'missing'
+                raise ValueError(f'hit_type={self.hit_type} with n_neighbors={K}, dim={d}: {name} must be {shape}, '
+                                 f'got {got}')
+
     def load_weights(self, W: Dict[str, Tensor]):
         """(Re)pack parameters given under the reference's state_dict names."""
+        self._check_hit_weights(W)
         g = lambda k: W[k].detach().to(self.device, f32).contiguous()
         self.updater.refresh(g)
         a = 'temporal_embedding_fn.fns.0.'
@@ -146,7 +160,7 @@ class TigerEngine:
         s = 'score_fn.'
         self.score_fold.refresh(g(s + 'fc1.weight'), g(s + 'fc1.bias'), g(s + 'fc2.weight'), g(s + 'fc2.bias'),
                                 g(a + 'merger.fc2.weight'), g(a + 'merger.fc2.bias'),
-                                g('hit_embedding.weight') if self.hit_type == 'bin' else None)
+                                g('hit_embedding.weight') if self.hit_type in ('bin', 'count') else None)
         self.attn_pack.attach_score_fold(self.score_fold, self.pq)
         if self.restarter == 'static':
             self.left_emb = g('restarter_fn.left_emb.weight')
@@ -287,7 +301,7 @@ class TigerEngine:
 
     def launch_scorer(self):
         ops.link_score_folded(self.score_fold, self.pq, self.src, self.dst, self.neg,
-                              self.neigh_nids if self.hit_type == 'bin' else None, self.scores, self.loss)
+                              self.neigh_nids if self.hit_type != 'none' else None, self.scores, self.loss)
 
     def bind_pq(self, pq: Tensor):
         """The [3B, 2d] first-layer projections of the link scorer, written by the last attention product and read

@@ -16,12 +16,17 @@ def time_basis(d: int) -> torch.Tensor:
 
 def random_weights(d: int, de: int, *, n_nodes: int = 0, restarter: Optional[str] = None, hist_len: int = 40,
                    seed: int = 0, nonzero_static: bool = False, n_layers: int = 1, msg_tsfm_type: str = 'id',
-                   mem_update_type: str = 'gru') -> Dict[str, torch.Tensor]:
+                   mem_update_type: str = 'gru', hit_type: str = 'bin',
+                   n_neighbors: int = 10) -> Dict[str, torch.Tensor]:
     """msg_tsfm_type / mem_update_type as in build_model: 'linear' adds msg_transform_fn.fn.1 (nn.Linear(M, M)),
     'mlp' fn.1 / fn.4 (nn.Linear(M, M/2), nn.Linear(M/2, M)); 'merge' replaces right_mem_updater.cell by
-    right_mem_updater.fn (MergeLayer(M, d, d, d), message_modules.py:37-57, update_modules.py:50-56)."""
+    right_mem_updater.fn (MergeLayer(M, d, d, d), message_modules.py:37-57, update_modules.py:50-56).
+    hit_type as in build_model (tiger.py:129-136), K = n_neighbors: 'count' has a hit_embedding [K+1, d], 'vec' none
+    and a score_fn.fc1 [d, 2(d+K)] (MergeLayer(d+K, d+K, d, 1)); 'none' has no hit_embedding."""
     if msg_tsfm_type not in ('id', 'linear', 'mlp') or mem_update_type not in ('gru', 'merge'):
         raise NotImplementedError(f'msg_tsfm_type={msg_tsfm_type}, mem_update_type={mem_update_type}')
+    if hit_type not in ('none', 'bin', 'vec', 'count'):
+        raise NotImplementedError(f'hit_type={hit_type}')
     g = torch.Generator().manual_seed(seed)
     E, C, M = 2 * d, 2 * d + de, 3 * d + de
 
@@ -92,6 +97,14 @@ def random_weights(d: int, de: int, *, n_nodes: int = 0, restarter: Optional[str
         for n in ('weight_ih', 'weight_hh', 'bias_ih', 'bias_hh'):
             del W[c + n]
         merge_layer(M, d, d, d, 'right_mem_updater.fn.', W)
+    # the hit types likewise (the default 'bin' tensors above are drawn for every hit type, then replaced)
+    if hit_type != 'bin':
+        del W['hit_embedding.weight']
+    if hit_type == 'count':
+        W['hit_embedding.weight'] = torch.randn((n_neighbors + 1, d), generator=g)
+    elif hit_type == 'vec':
+        o, i = d, 2 * (d + n_neighbors)
+        W['score_fn.fc1.weight'] = torch.randn((o, i), generator=g) * math.sqrt(2.0 / (o + i))
     return W
 
 

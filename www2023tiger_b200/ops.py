@@ -510,36 +510,58 @@ def temporal_attention_dense(pack: AttnPack, n_head: int, qx, qt, kx, ky, kt, pa
     return out
 
 
-class ScoreFold:
-    """Link scorer folded into the attention's last GEMM (tiger_score_fold): refresh whenever score_fn,
-    the embedding module's merger.fc2 or the hit embedding change."""
+HIT_TYPES = ('none', 'bin', 'vec', 'count')      # --hit_type, index = TIGER_HIT_* (include/tiger_b200.h)
 
-    def __init__(self, d: int, device):
-        self.d = d
+
+class ScoreFold:
+    """Link scorer folded into the attention's last GEMM (tiger_score_fold_hit): refresh whenever score_fn,
+    the embedding module's merger.fc2 or the hit embedding change.  'bin' also serves 'none' (hit_emb None);
+    'vec' and 'count' fold for k = n_neighbors slots (score_fn.fc1 [d, 2(d+k)], hit_embedding [k+1, d])."""
+
+    def __init__(self, d: int, device, hit_type: str = 'bin', k: int = 0):
+        if hit_type not in HIT_TYPES:
+            raise NotImplementedError(f'hit_type={hit_type}')
+        self.d, self.hit_type = d, hit_type
+        self.k = k if hit_type in ('vec', 'count') else 0
         lib = _lib.load()
-        self.blob = torch.zeros(lib.tiger_score_fold_bytes(d) // 4, dtype=f32, device=device)
-        self.cab = self.blob[lib.tiger_score_fold_cab_offset(d):]
+        code = HIT_TYPES.index(hit_type)
+        nbytes = lib.tiger_score_fold_hit_bytes(d, code, self.k)
+        if nbytes <= 0:
+            raise _lib.TigerLibraryError(f'invalid score fold d={d} hit_type={hit_type} k={k}')
+        self.blob = torch.zeros(nbytes // 4, dtype=f32, device=device)
+        self.cab = self.blob[lib.tiger_score_fold_hit_offset(d, code, self.k):]    # the table the scorer reads
         self.done = torch.zeros(1, dtype=i32, device=device)
+
+    def code(self, with_hits: bool) -> int:
+        """TIGER_HIT_* of a fold / score call; for 'bin' / 'none' whether hit data is given decides."""
+        if self.hit_type in ('vec', 'count'):
+            return HIT_TYPES.index(self.hit_type)
+        return HIT_TYPES.index('bin' if with_hits else 'none')
 
     def refresh(self, fc1_w, fc1_b, fc2_w, fc2_b, merger_fc2_w, merger_fc2_b, hit_emb: Optional[Tensor]):
         det = lambda t: None if t is None else t.detach().to(f32).contiguous()
         self._keep = [det(t) for t in (fc1_w, fc1_b, merger_fc2_w, merger_fc2_b, hit_emb)]
         check_cuda(*self._keep)
-        call('tiger_score_fold', *(ptr(t) for t in self._keep), self.d, ptr(self.blob))
+        call('tiger_score_fold_hit', *(ptr(t) for t in self._keep), self.d, self.code(hit_emb is not None), self.k,
+             ptr(self.blob))
         self.fc2_w = fc2_w.detach().to(f32).reshape(-1).contiguous()
         self.fc2_b = fc2_b.detach().to(f32).contiguous()
 
 
 def link_score_folded(fold: ScoreFold, pq: Tensor, src: Tensor, dst: Tensor, neg: Tensor,
                       neigh_nids: Optional[Tensor], scores: Optional[Tensor] = None, loss: Optional[Tensor] = None):
+    """neigh_nids [3B, K]: the batch nodes' neighbor table (hit flags); None for hit_type 'none'."""
     B = src.numel()
     if scores is None:
         scores = _empty(2 * B, f32, pq)
     if loss is None:
         loss = _empty(1, f32, pq)
     k = neigh_nids.shape[1] if neigh_nids is not None else 0
-    call('tiger_link_score_folded', ptr(pq), B, fold.d, ptr(src), ptr(dst), ptr(neg), ptr(neigh_nids), k, ptr(fold.cab),
-         ptr(fold.fc2_w), ptr(fold.fc2_b), ptr(scores), ptr(loss), ptr(fold.done))
+    if fold.hit_type in ('vec', 'count') and k != fold.k:
+        raise ValueError(f'hit_type {fold.hit_type}: the fold holds {fold.k} slots, the neighbor table has {k}')
+    call('tiger_link_score_folded_hit', ptr(pq), B, fold.d, ptr(src), ptr(dst), ptr(neg), ptr(neigh_nids), k,
+         fold.code(neigh_nids is not None), ptr(fold.cab), ptr(fold.fc2_w), ptr(fold.fc2_b), ptr(scores), ptr(loss),
+         ptr(fold.done))
     return scores, loss
 
 

@@ -155,7 +155,7 @@ class TIGE(nn.Module):
     def _fusable(self) -> bool:
         return (isinstance(self.msg_transform_fn, (IdentityMessageFunction, LinearMessageFunction, MLPMessageFunction))
                 and isinstance(self.right_mem_updater, (GRUUpdater, MergeUpdater)) and self.n_layers in (1, 2)
-                and self.hit_type in ('bin', 'none') and self.left_memory.vals.is_cuda)
+                and self.hit_type in ops.HIT_TYPES and self.left_memory.vals.is_cuda)
 
     def _memory_updater(self, cap: int) -> ops.MemoryUpdater:
         """Steps 1-2 of the fused route for this model's message transform and memory updater, with the transform
@@ -185,17 +185,19 @@ class TIGE(nn.Module):
         return ws
 
     def _score_fold(self) -> ops.ScoreFold:
-        """The link scorer folded into the batch-node attention's last product (score_fn, the merger's fc2 of
-        fns.0, the hit embedding), refreshed when one of them changes."""
+        """The link scorer folded into the batch-node attention's last product (score_fn - whose fc1 also holds the
+        hit vectors' columns for 'vec' -, the merger's fc2 of fns.0, the hit embedding of 'bin' / 'count'),
+        refreshed when one of them changes."""
         s, m = self.score_fn, self.temporal_embedding_fn.fns[0].merger
         params = [s.fc1.weight, s.fc1.bias, s.fc2.weight, s.fc2.bias, m.fc2.weight, m.fc2.bias]
-        if self.hit_type == 'bin':
+        has_emb = self.hit_type in ('bin', 'count')
+        if has_emb:
             params.append(self.hit_embedding.weight)
         key = tuple((p.data_ptr(), p._version) for p in params)
         if self._fold is None or key != self._fold_key:
             if self._fold is None or self._fold.blob.device != params[0].device:
-                self._fold = ops.ScoreFold(self.nfeat_dim, params[0].device)
-            args = [f32c(p) for p in params] + ([None] if self.hit_type != 'bin' else [])
+                self._fold = ops.ScoreFold(self.nfeat_dim, params[0].device, self.hit_type, self.n_neighbors)
+            args = [f32c(p) for p in params] + ([] if has_emb else [None])
             self._fold.refresh(*args)
             self._fold_key = key
         return self._fold
@@ -264,7 +266,7 @@ class TIGE(nn.Module):
             pack.attach_left_writeback(None)
         # step 7 (tiger.py:259-288)
         scores, loss = ops.link_score_folded(fold, pq, batch_nids[:B], batch_nids[B:2 * B], batch_nids[2 * B:],
-                                             nn_ if self.hit_type == 'bin' else None)
+                                             nn_ if self.hit_type != 'none' else None)
         self._err.check()
         return loss[0], emb[:2 * B], scores[:B], scores[B:], h_prev_left, h_prev_right
 
@@ -434,7 +436,7 @@ class TIGER(TIGE):
         import os
         from www2023tiger_b200.train import native_limit_error
         from .restarters import SeqRestarter, StaticRestarter
-        return (torch.is_grad_enabled() and self.training and self._fusable()
+        return (torch.is_grad_enabled() and self.training and self._fusable() and self.hit_type in ('bin', 'none')
                 and isinstance(self.msg_transform_fn, IdentityMessageFunction)
                 and isinstance(self.right_mem_updater, GRUUpdater)
                 and isinstance(self.restarter_fn, (SeqRestarter, StaticRestarter))
