@@ -305,7 +305,10 @@ int tiger_score_fold_hit(const float* score_fc1, const float* score_fc1_b, const
                          const float* merger_fc2_b, const float* hit_emb, int d, int hit_type, int k, float* blob,
                          void* stream);
 
-/* bytes of caller-provided, 16-byte aligned workspace for n_query queries */
+/* bytes of caller-provided, 16-byte aligned workspace for n_query queries; -1 for dimensions both attention entry
+ * points refuse: k > 64, n_head > 8, or a score-pool shared-memory footprint
+ * 4 (k ru4(2d + de) + ru4(n_head k) + n_head ru4(2d + de + 1)) bytes over 200 KiB (ru4: rounded up to a multiple
+ * of 4) */
 int64_t tiger_temporal_attention_work_bytes(int64_t n_query, int k, int d, int de, int n_head);
 
 /* a15 + a16  one layer of GraphEmbedding.compute_embedding_with_computation_graph +

@@ -33,6 +33,8 @@
 #endif
 
 #define ATT_MAXH 8
+#define ATT_MAXK 64                   // the masked softmax holds two slots per lane of one warp
+#define ATT_MAX_POOL_SMEM (200 * 1024)  // dynamic shared memory of attn_score_pool: its K key rows stay staged
 #ifndef ATT_THREADS
 #define ATT_THREADS 256
 #endif
@@ -82,8 +84,21 @@ static AttWork att_work(const AttDims& a, int64_t n, float* base) {
   return w;
 }
 
+// dynamic shared memory of attn_score_pool: kv [K][Cp] | scores [H][K] (rounded to 4) | score weights [H][Cq]
+static size_t att_pool_smem(const AttDims& a) {
+  return ((size_t)a.K * a.Cp + (size_t)((a.H * a.K + 3) & ~3) + (size_t)a.H * a.Cq) * sizeof(float);
+}
+
+// the dimensions the kernels take: K, heads and the score-pool footprint within their limits
+static bool att_dims_ok(int k, int d, int de, int n_head) {
+  if (k <= 0 || d <= 0 || de <= 0 || n_head <= 0 || k > ATT_MAXK || n_head > ATT_MAXH) return false;
+  return att_pool_smem(att_dims(d, de, k, n_head)) <= ATT_MAX_POOL_SMEM;
+}
+
+// -1 for dimensions the attention refuses (also past ATT_MAXK, ATT_MAXH and ATT_MAX_POOL_SMEM): callers test a model
+// against the kernel's limits with it
 extern "C" int64_t tiger_temporal_attention_work_bytes(int64_t n_query, int k, int d, int de, int n_head) {
-  if (n_query < 0 || k <= 0 || d <= 0 || de <= 0 || n_head <= 0) return -1;
+  if (n_query < 0 || !att_dims_ok(k, d, de, n_head)) return -1;
   const AttDims a = att_dims(d, de, k, n_head);
   return att_work(a, n_query, nullptr).total_floats * (int64_t)sizeof(float);
 }
@@ -432,7 +447,6 @@ __global__ void __launch_bounds__(256) attn_prepare_kernel(const AttArgs a) {
 // The gathers of all K slots are issued together (every thread keeps up to 8 independent 16-byte loads in
 // flight) - the kernel's time is the latency of those random-row reads, not their volume; the score
 // weights of the query are staged in shared memory once.
-#define ATT_MAXK 64
 // exact f / w for 0 <= f < 2^20 with a float reciprocal (the flattened (slot, column) loops below would
 // otherwise spend more instructions on integer division than on their loads)
 __device__ __forceinline__ int fast_div(int f, float inv_w) { return __float2int_rz(((float)f + 0.5f) * inv_w); }
@@ -744,8 +758,7 @@ static int attention_run(AttArgs& a, const tiger_attn_params* p, float* out, cud
                                       s);
   }
   if (rc != TIGER_OK) return rc;
-  const size_t smem = ((size_t)m.K * m.Cp + (size_t)((m.H * m.K + 3) & ~3) + (size_t)m.H * m.Cq) * sizeof(float);
-  if (smem > 200 * 1024 || m.K > ATT_MAXK) return TIGER_EINVAL;
+  const size_t smem = att_pool_smem(m);
   rc = m.H == 2 ? launch_score_pool<2>(a, smem, st)
        : m.H == 1 ? launch_score_pool<1>(a, smem, st)
        : m.H == 4 ? launch_score_pool<4>(a, smem, st)
@@ -769,14 +782,16 @@ static int attention_run(AttArgs& a, const tiger_attn_params* p, float* out, cud
 
 static int attention_entry(AttArgs& a, int k, int d, int de, int n_head, const tiger_attn_params* params, float* out,
                            void* work, void* stream) {
-  if (params == nullptr || params->folded == nullptr || work == nullptr) return TIGER_EINVAL;
+  if (params == nullptr || params->folded == nullptr) return TIGER_EINVAL;
   // the fused last product comes whole (score fold, its pq output and the left write-back) and in the gather form only
   const bool fused = params->left_wb != nullptr;
   if ((fused && a.dense) || (params->score_folded != nullptr) != fused || (params->pq_out != nullptr) != fused)
     return TIGER_EINVAL;
-  if (a.n_query < 0 || k <= 0 || d <= 0 || de <= 0 || n_head <= 0 || n_head > ATT_MAXH) return TIGER_EINVAL;
+  // limits checked before the first launch, so a refused call leaves its outputs and workspace untouched
+  if (a.n_query < 0 || !att_dims_ok(k, d, de, n_head)) return TIGER_EINVAL;
   if ((2 * d) % n_head != 0 || (((uintptr_t)work) & 15) != 0) return TIGER_EINVAL;
-  if (a.n_query == 0) return TIGER_OK;
+  if (a.n_query == 0) return TIGER_OK;   // no workspace needed: tiger_temporal_attention_work_bytes(0, ..) is 0
+  if (work == nullptr) return TIGER_EINVAL;
   a.dm = att_dims(d, de, k, n_head);
   a.w = att_work(a.dm, a.n_query, reinterpret_cast<float*>(work));
   return attention_run(a, params, out, as_stream(stream));

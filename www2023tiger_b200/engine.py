@@ -76,6 +76,11 @@ class TigerEngine:
         self.efeats = efeats
         self.nfeats = nfeats
         self.de = efeats.shape[1] if efeats is not None else dim
+        # every layer has the same widths, K and heads; models past the attention kernel's limits run on the drop-in's
+        # torch route
+        limit = ops.attention_limit_error(self.d, self.de, n_neighbors, n_head)
+        if limit is not None:
+            raise NotImplementedError(limit)
         self.M = 3 * self.d + self.de                                          # tiger.py:62
         self.msg_src, self.upd_src = msg_src, upd_src
         self.restarter, self.lazy_restart = restarter, lazy_restart

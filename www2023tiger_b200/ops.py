@@ -4,6 +4,7 @@ Every function takes CUDA tensors, allocates its outputs with torch (device memo
 only thing torch does here), launches on the current stream and never synchronises.
 """
 import ctypes
+import functools
 import os
 from typing import Optional, Tuple
 
@@ -394,6 +395,36 @@ class MemoryUpdater:
         return merge_update(self.merge, mid=self.mid, **kw)
 
 
+@functools.lru_cache(maxsize=None)
+def _attention_max(which: str) -> int:
+    """Largest K ('k', one head) or head count ('h', one slot) the attention kernels take, read off
+    tiger_temporal_attention_work_bytes at a width where the shared-memory footprint is far from its limit."""
+    fits = lambda v: _lib.load().tiger_temporal_attention_work_bytes(0, v if which == 'k' else 1, 4, 4,
+                                                                       v if which == 'h' else 1) >= 0
+    v = 1
+    while fits(v + 1):
+        v += 1
+    return v
+
+
+@functools.lru_cache(maxsize=None)
+def attention_limit_error(d: int, de: int, k: int, n_head: int) -> Optional[str]:
+    """Why the attention kernels (temporal_attention, temporal_attention_dense) cannot run a layer of node width d,
+    edge width de, k neighbor slots and n_head heads, or None when they can.  The limits are the kernels' own
+    (tiger_temporal_attention_work_bytes); the reference has none, so callers run such layers through torch."""
+    if _lib.load().tiger_temporal_attention_work_bytes(0, k, d, de, n_head) >= 0:
+        return None
+    if min(d, de, k, n_head) <= 0:
+        return f'invalid attention dimensions d={d} de={de} n_neighbors={k} n_head={n_head}'
+    max_k, max_h = _attention_max('k'), _attention_max('h')
+    if k > max_k:
+        return f'the attention kernel takes at most {max_k} neighbors per query; this layer has n_neighbors={k}'
+    if n_head > max_h:
+        return f'the attention kernel takes at most {max_h} heads; this layer has n_head={n_head}'
+    return (f'the attention kernel stages the {k} key rows of a query in shared memory, which does not hold them at '
+            f'd={d}, de={de}, n_neighbors={k}, n_head={n_head} (shared-memory footprint over its limit)')
+
+
 class AttnParamsC(ctypes.Structure):
     _fields_ = [(n, ctypes.c_void_p) for n in
                 ('wq', 'wk', 'wv', 'wo', 'fc1', 'fc2', 'in_bias', 'out_bias', 'fc1_b', 'fc2_b', 'time_w', 'time_b',
@@ -475,6 +506,10 @@ class AttnPack:
         key = (n_query, k)
         if self._work is None or self._work_key is None or self._work_key[0] < n_query or self._work_key[1] != k:
             nbytes = _lib.load().tiger_temporal_attention_work_bytes(n_query, k, self.d, self.de, self.n_head)
+            if nbytes < 0:
+                raise _lib.TigerLibraryError('temporal attention: invalid argument ('
+                                             + (attention_limit_error(self.d, self.de, k, self.n_head)
+                                                or f'n_query={n_query}') + ')')
             self._work = torch.empty(nbytes, dtype=u8, device=self.folded.device)
             self._work_key = key
         return self._work

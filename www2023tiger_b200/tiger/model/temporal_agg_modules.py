@@ -47,9 +47,14 @@ class TemporalAttention(nn.Module):
             self._pack_key = key
         return self._pack
 
+    def fits_kernel(self, k: int) -> bool:
+        """Whether the attention kernel takes this layer with k neighbor slots (ops.attention_limit_error); past its
+        limits the layer runs its torch code, which has none."""
+        return ops.attention_limit_error(self.nfeat_dim, self.efeat_dim, k, self.n_head) is None
+
     def forward(self, qx: Tensor, qt: Tensor, kx: Tensor, ky: Tensor, kt: Tensor, padding_mask: Tensor) -> Tensor:
         """qx [n,d] qt [n,d] kx [n,len,d] ky [n,len,de] kt [n,len,d]; padding_mask [n,len], True = padding."""
-        if use_kernel(self) and qx.is_cuda:
+        if use_kernel(self) and qx.is_cuda and self.fits_kernel(kx.shape[1]):
             return ops.temporal_attention_dense(self.packed(), self.n_head, f32c(qx), f32c(qt), f32c(kx), f32c(ky),
                                                 f32c(kt), padding_mask)
         query = torch.cat([qx, qt], 1).unsqueeze(0)
@@ -82,7 +87,8 @@ class GraphEmbedding(nn.Module):
         (`involved_node_reprs[computation_graph.local_index[u]]`)."""
         depth = self.n_layers if depth is None else depth
         cg = computation_graph
-        if depth == 1 and use_kernel(self) and involved_node_reprs.is_cuda and hasattr(self, 'fns'):
+        if (depth == 1 and use_kernel(self) and involved_node_reprs.is_cuda and hasattr(self, 'fns')
+                and self.fns[self.n_layers - 1].fits_kernel(cg.layers[1][0].shape[1])):
             nn_, ne_, nt_ = cg.layers[1]
             fn = self.fns[self.n_layers - 1]
             return ops.temporal_attention(fn.packed(self.time_encoder), fn.n_head, center_nids.contiguous(), f32c(ts),

@@ -153,9 +153,12 @@ class TIGE(nn.Module):
 
     # ------------------------------------------------------------------ fused no-grad route
     def _fusable(self) -> bool:
+        # a model past the attention kernel's limits (neighbors, heads, shared-memory footprint) takes the step-by-step
+        # route, whose attention layers then run their torch code
         return (isinstance(self.msg_transform_fn, (IdentityMessageFunction, LinearMessageFunction, MLPMessageFunction))
                 and isinstance(self.right_mem_updater, (GRUUpdater, MergeUpdater)) and self.n_layers in (1, 2)
-                and self.hit_type in ops.HIT_TYPES and self.left_memory.vals.is_cuda)
+                and self.hit_type in ops.HIT_TYPES and self.left_memory.vals.is_cuda
+                and all(fn.fits_kernel(self.n_neighbors) for fn in self.temporal_embedding_fn.fns))
 
     def _memory_updater(self, cap: int) -> ops.MemoryUpdater:
         """Steps 1-2 of the fused route for this model's message transform and memory updater, with the transform
