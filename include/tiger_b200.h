@@ -94,6 +94,18 @@ int tiger_compact_involved(uint32_t* bitmap, int64_t n_nodes, uint8_t* has_msg, 
                            int64_t* outdated, int32_t* gru_row, int64_t* restart_nodes,
                            int32_t* counts, uint32_t* err_flags, void* stream);
 
+/* The same compaction with read_only != 0, for a query that scores candidates against the state without advancing it:
+ * the lists and counts are those of read_only == 0, but uptodate and has_msg are only read, and restarted node
+ * restart_nodes[r] gets gru_row[u] = restart_base + r (r < cap_involved) instead of -1, so the attention reads its
+ * restart surrogate from that row of its rows_b (tiger_static_restart_rows / the seq restarter's h_right).  Restart
+ * nodes never have a pending message in the lists, so [0, O) and [restart_base, restart_base + R) do not overlap when
+ * restart_base >= cap_involved.  tiger_compact_involved is this call with read_only = 0. */
+int tiger_compact_involved_ex(uint32_t* bitmap, int64_t n_nodes, uint8_t* has_msg, uint8_t* uptodate,
+                              int64_t* involved, int64_t cap_involved, int64_t* local_index,
+                              int64_t* outdated, int32_t* gru_row, int64_t* restart_nodes,
+                              int32_t* counts, uint32_t* err_flags, int read_only, int restart_base,
+                              void* stream);
+
 /* ---------------------------------------------------------------------------------------
  * Index utilities (tiger/model/utils.py)
  * ------------------------------------------------------------------------------------- */
@@ -335,6 +347,16 @@ int tiger_temporal_attention_ex(const int64_t* center_nids, const float* q_ts, i
                                 const float* nfeats, const float* efeats, int d, int de, int n_head,
                                 const tiger_attn_params* params, float* out, void* work, void* stream);
 
+/* tiger_temporal_attention_ex for the batch-node depth of a read-only candidate query: params carries score_folded and
+ * pq_out and no left_wb (TIGER_EINVAL otherwise); the last product writes out and pq_out exactly as the fused route of
+ * tiger_temporal_attention_ex does and persists nothing. */
+int tiger_temporal_attention_query(const int64_t* center_nids, const float* q_ts, int64_t n_query,
+                                   int64_t ts_period, int64_t ts_group, const int64_t* neigh_nids,
+                                   const int64_t* neigh_eids, const float* neigh_ts, int k, const float* rows_a,
+                                   const float* rows_b, const float* key_rows, const void* sel, int sel_is_i64,
+                                   const float* nfeats, const float* efeats, int d, int de, int n_head,
+                                   const tiger_attn_params* params, float* out, void* work, void* stream);
+
 /* Same operator with the dense argument list of TemporalAttention.forward
  * (temporal_agg_modules.py:210-235): qx [n,d], qt [n,d], kx [n,K,d], ky [n,K,de], kt [n,K,d],
  * padding_mask [n,K] (1 = padding). */
@@ -363,6 +385,19 @@ int tiger_link_score_folded_hit(const float* pq, int64_t batch, int d, const int
                                 const float* tables, const float* fc2_w, const float* fc2_b, float* scores,
                                 float* loss, uint32_t* done_counter, void* stream);
 
+/* The scorer over C >= 1 candidate columns (tiger_link_score_folded_hit is this call with C = 2, pos = dst, negs = neg,
+ * ranks = NULL): pair (i, j), i < n_query, scores src[i] against column j's node - pos[i] for j = 0, negs[(j-1) n_query
+ * + i] for j >= 1 - from pq rows i and n_query + j n_query + i, i.e. pq and neigh_nids hold the rows of
+ * [src | column 0 | column 1 | ...].  scores [C][n_query] (candidate-major).  loss (may be NULL) is the BCE mean over
+ * the C n_query pairs with column 0 as the positive.  ranks (may be NULL) [n_query]:
+ * 1 + #{j >= 1 : s_ij > s_i0} + 0.5 #{j >= 1 : s_ij == s_i0}, column 0 the true candidate, ties counted half (the
+ * mean of the optimistic and the pessimistic rank), from integer counts (deterministic); a NaN s_i0 gives a NaN rank,
+ * a NaN s_ij neither beats nor ties s_i0, infinities compare as values.  One more launch when ranks are wanted. */
+int tiger_link_score_cands(const float* pq, int64_t n_query, int n_cands, int d, const int64_t* src,
+                           const int64_t* pos, const int64_t* negs, const int64_t* neigh_nids, int k, int hit_type,
+                           const float* tables, const float* fc2_w, const float* fc2_b, float* scores, float* ranks,
+                           float* loss, uint32_t* done_counter, void* stream);
+
 /* ---------------------------------------------------------------------------------------
  * Restarters (tiger/model/restarters.py, tiger.py:594-609)
  * ------------------------------------------------------------------------------------- */
@@ -378,6 +413,11 @@ int tiger_static_restart(const int64_t* nids, const int32_t* count, int64_t n,
                          const float* right_emb, int d, float* left_vals, float* left_ts,
                          uint8_t* left_active, float* right_vals, float* right_ts,
                          uint8_t* right_active, uint8_t* has_msg, float* out_prev_ts, void* stream);
+
+/* Restart surrogates of a read-only query: out_rows[i] = right_emb[nids[i]] (the right-memory row
+ * tiger_static_restart writes) for i < min(*count, n) (count may be NULL); writes nothing node-indexed. */
+int tiger_static_restart_rows(const int64_t* nids, const int32_t* count, int64_t n, const float* right_emb, int d,
+                              float* out_rows, void* stream);
 
 /* a21 + a24  SeqRestarter.forward (restarters.py:51-114) as a launch sequence; see restart_seq.cu.
  *
@@ -464,7 +504,8 @@ int tiger_sgemm_nt_packed_gather(const int64_t* ids, const void* sel, int sel_is
                                  int relu, void* stream);
 
 /* tiger_sgemm_nt_packed with the fused row scatter described at tiger_left_writeback_fused: result rows are
- * additionally stored into a node-indexed table.  With C2 (may be NULL) the output is split: the pack has
+ * additionally stored into a node-indexed table (wb may be NULL when C2 is given: the split output alone).  With C2
+ * (may be NULL) the output is split: the pack has
  * ceil((n_split + n_cols1) / bn) tiles; result columns [0, n_cols0) go to C, columns [n_split, n_split + n_cols1) to
  * C2 (n_split a multiple of 16 >= n_cols0; bias is indexed in the padded column space). */
 int tiger_sgemm_nt_packed_scatter(const float* A, int64_t lda, const float* wpack, int bn, const float* bias, float* C,

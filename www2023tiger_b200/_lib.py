@@ -23,6 +23,7 @@ _SIGNATURES: Dict[str, str] = {
     'tiger_hit_window': 'ppli' + 'p' + 'p',
     'tiger_mark_nodes': 'plpl' + 'p',
     'tiger_compact_involved': 'plpp' + 'plp' + 'ppp' + 'pp' + 'p',
+    'tiger_compact_involved_ex': 'plpp' + 'plp' + 'ppp' + 'pp' + 'ii' + 'p',
     'tiger_select_latest': 'ppil' + 'llppp' + 'pppp' + 'p',
     'tiger_anonymized_reindex': 'plip' + 'p' + 'p',
     'tiger_gather_rows': 'plplp' + 'pp' + 'p',
@@ -42,6 +43,7 @@ _SIGNATURES: Dict[str, str] = {
     'tiger_attn_fold': 'piii' + 'p',
     'tiger_temporal_attention_work_bytes': 'liiii',
     'tiger_temporal_attention_ex': 'pplll' + 'pppi' + 'ppppi' + 'pp' + 'iii' + 'ppp' + 'p',
+    'tiger_temporal_attention_query': 'pplll' + 'pppi' + 'ppppi' + 'pp' + 'iii' + 'ppp' + 'p',
     'tiger_temporal_attention_dense': 'pppppp' + 'li' + 'iii' + 'ppp' + 'p',
     'tiger_score_fold_bytes': 'i',
     'tiger_score_fold_cab_offset': 'i',
@@ -51,6 +53,7 @@ _SIGNATURES: Dict[str, str] = {
     'tiger_score_fold_hit_offset': 'iii',
     'tiger_score_fold_hit': 'pppppiii' + 'p' + 'p',
     'tiger_link_score_folded_hit': 'pli' + 'pppp' + 'ii' + 'ppp' + 'ppp' + 'p',
+    'tiger_link_score_cands': 'plii' + 'ppp' + 'pii' + 'ppp' + 'pppp' + 'p',
     'tiger_sgemm_nt_packed_gather': 'ppi' + 'pplp' + 'pi' + 'ppl' + 'lpl' + 'iifi' + 'p',
     'tiger_sgemm_nt_packed_splitk_fused': 'plpi' + 'ppl' + 'i' + 'lpl' + 'iifi' + 'p',
     'tiger_pipe_capture_begin': 'p',
@@ -98,6 +101,7 @@ _SIGNATURES: Dict[str, str] = {
     'tiger_gemm_pack_weight': 'plpiiiip' + 'p',
     'tiger_sgemm_nt_packed': 'plpippllpliifi' + 'p',
     'tiger_static_restart': 'ppl' + 'plp' + 'pp' + 'ppi' + 'ppp' + 'ppp' + 'pp' + 'p',
+    'tiger_static_restart_rows': 'pplpi' + 'p' + 'p',
 }
 _KIND = {'p': P, 'l': L, 'i': I, 'f': F}
 

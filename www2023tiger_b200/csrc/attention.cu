@@ -769,9 +769,10 @@ static int attention_run(AttArgs& a, const tiger_attn_params* p, float* out, cud
   rc = tiger_sgemm_nt_packed_splitk_fused(a.w.kvc, m.ld_kvc, f.pk_w2f, ATT_BN_D, p->fc1_b, a.w.hid, m.ld_hid,
                                           ATT_KPARTS, n, nullptr, 1, m.d, m.off_live + 1, 1.0f, 1, s);
   if (rc != TIGER_OK) return rc;
-  if (p->left_wb != nullptr) {
+  if (p->score_folded != nullptr) {
     // batch-node depth of the fused routes: the last GEMM writes z -> out and [W1a z | W1b z] -> pq_out (link-scorer
-    // fold) and persists the winners' embeddings into the left memory (waits for left_wb->ready_event first)
+    // fold) and, with left_wb, persists the winners' embeddings into the left memory (waits for left_wb->ready_event
+    // first); a read-only query (tiger_temporal_attention_query) has no left_wb and the same product otherwise
     const ScoreFold sf = score_fold(m.d, p->score_folded);
     return tiger_sgemm_nt_packed_scatter(a.w.hid, m.ld_hid, sf.pack, ATT_BN_F3, sf.b3, out, m.d, m.d, p->pq_out, 2 * m.d,
                                          sf.n_split, 2 * m.d, n, m.d, p->left_wb, s);
@@ -781,11 +782,13 @@ static int attention_run(AttArgs& a, const tiger_attn_params* p, float* out, cud
 }
 
 static int attention_entry(AttArgs& a, int k, int d, int de, int n_head, const tiger_attn_params* params, float* out,
-                           void* work, void* stream) {
+                           void* work, void* stream, bool query = false) {
   if (params == nullptr || params->folded == nullptr) return TIGER_EINVAL;
-  // the fused last product comes whole (score fold, its pq output and the left write-back) and in the gather form only
-  const bool fused = params->left_wb != nullptr;
-  if ((fused && a.dense) || (params->score_folded != nullptr) != fused || (params->pq_out != nullptr) != fused)
+  // the fused last product comes whole (score fold, its pq output and the left write-back) and in the gather form only;
+  // a query takes the score fold and its pq output without the write-back
+  const bool fused = query || params->left_wb != nullptr;
+  if ((fused && a.dense) || (params->score_folded != nullptr) != fused || (params->pq_out != nullptr) != fused ||
+      (query && params->left_wb != nullptr))
     return TIGER_EINVAL;
   // limits checked before the first launch, so a refused call leaves its outputs and workspace untouched
   if (a.n_query < 0 || !att_dims_ok(k, d, de, n_head)) return TIGER_EINVAL;
@@ -797,12 +800,11 @@ static int attention_entry(AttArgs& a, int k, int d, int de, int n_head, const t
   return attention_run(a, params, out, as_stream(stream));
 }
 
-extern "C" int tiger_temporal_attention_ex(const int64_t* center_nids, const float* q_ts, int64_t n_query,
-                                           int64_t ts_period, int64_t ts_group, const int64_t* neigh_nids,
-                                           const int64_t* neigh_eids, const float* neigh_ts, int k, const float* rows_a,
-                                           const float* rows_b, const float* key_rows, const void* sel, int sel_is_i64,
-                                           const float* nfeats, const float* efeats, int d, int de, int n_head,
-                                           const tiger_attn_params* params, float* out, void* work, void* stream) {
+static int attention_gather(const int64_t* center_nids, const float* q_ts, int64_t n_query, int64_t ts_period,
+                            int64_t ts_group, const int64_t* neigh_nids, const int64_t* neigh_eids, const float* neigh_ts,
+                            int k, const float* rows_a, const float* rows_b, const float* key_rows, const void* sel,
+                            int sel_is_i64, const float* nfeats, const float* efeats, int d, int de, int n_head,
+                            const tiger_attn_params* params, float* out, void* work, void* stream, bool query) {
   if (rows_b == nullptr || sel == nullptr || ts_group <= 0) return TIGER_EINVAL;
   AttArgs a = {};
   a.center_nids = center_nids; a.q_ts = q_ts; a.ts_period = ts_period > 0 ? ts_period : n_query;
@@ -811,7 +813,30 @@ extern "C" int tiger_temporal_attention_ex(const int64_t* center_nids, const flo
   a.rows_a = rows_a; a.rows_b = rows_b; a.key_rows = key_rows; a.sel = sel; a.sel_is_i64 = sel_is_i64;
   a.nfeats = nfeats; a.efeats = efeats; a.dense = 0;
   a.n_query = n_query;
-  return attention_entry(a, k, d, de, n_head, params, out, work, stream);
+  return attention_entry(a, k, d, de, n_head, params, out, work, stream, query);
+}
+
+extern "C" int tiger_temporal_attention_ex(const int64_t* center_nids, const float* q_ts, int64_t n_query,
+                                           int64_t ts_period, int64_t ts_group, const int64_t* neigh_nids,
+                                           const int64_t* neigh_eids, const float* neigh_ts, int k, const float* rows_a,
+                                           const float* rows_b, const float* key_rows, const void* sel, int sel_is_i64,
+                                           const float* nfeats, const float* efeats, int d, int de, int n_head,
+                                           const tiger_attn_params* params, float* out, void* work, void* stream) {
+  return attention_gather(center_nids, q_ts, n_query, ts_period, ts_group, neigh_nids, neigh_eids, neigh_ts, k, rows_a,
+                          rows_b, key_rows, sel, sel_is_i64, nfeats, efeats, d, de, n_head, params, out, work, stream,
+                          false);
+}
+
+extern "C" int tiger_temporal_attention_query(const int64_t* center_nids, const float* q_ts, int64_t n_query,
+                                              int64_t ts_period, int64_t ts_group, const int64_t* neigh_nids,
+                                              const int64_t* neigh_eids, const float* neigh_ts, int k,
+                                              const float* rows_a, const float* rows_b, const float* key_rows,
+                                              const void* sel, int sel_is_i64, const float* nfeats, const float* efeats,
+                                              int d, int de, int n_head, const tiger_attn_params* params, float* out,
+                                              void* work, void* stream) {
+  return attention_gather(center_nids, q_ts, n_query, ts_period, ts_group, neigh_nids, neigh_eids, neigh_ts, k, rows_a,
+                          rows_b, key_rows, sel, sel_is_i64, nfeats, efeats, d, de, n_head, params, out, work, stream,
+                          true);
 }
 
 extern "C" int tiger_temporal_attention_dense(const float* qx, const float* qt, const float* kx, const float* ky,

@@ -880,8 +880,8 @@ extern "C" int tiger_sgemm_nt_packed_scatter(const float* A, int64_t lda, const 
                                              float* C, int64_t ldc, int n_cols0, float* C2, int64_t ldc2, int n_split,
                                              int n_cols1, int64_t m_rows, int k_dim, const tiger_left_writeback_fused* wb,
                                              void* stream) {
-  if (wpack == nullptr || wb == nullptr) return TIGER_EINVAL;
-  if (wb->ready_event != nullptr &&
+  if (wpack == nullptr || (wb == nullptr && C2 == nullptr)) return TIGER_EINVAL;
+  if (wb != nullptr && wb->ready_event != nullptr &&
       cudaStreamWaitEvent(as_stream(stream), reinterpret_cast<cudaEvent_t>(wb->ready_event), 0) != cudaSuccess)
     return TIGER_ECUDA;
   return gemm_packed_launch({.A = A, .lda = lda, .wpack = wpack, .bn = bn, .bias = bias, .C = C, .ldc = ldc,

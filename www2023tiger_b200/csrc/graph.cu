@@ -148,7 +148,8 @@ compact_involved_kernel(uint32_t* __restrict__ bitmap, int64_t n_words, uint8_t*
                         uint8_t* __restrict__ uptodate, int64_t* __restrict__ involved, int64_t cap,
                         int64_t* __restrict__ local_index, int64_t* __restrict__ outdated,
                         int32_t* __restrict__ gru_row, int64_t* __restrict__ restart_nodes,
-                        int32_t* __restrict__ counts, uint32_t* __restrict__ err_flags) {
+                        int32_t* __restrict__ counts, uint32_t* __restrict__ err_flags, int read_only,
+                        int restart_base) {
   __shared__ int sm[3][32];
   __shared__ int total[3];
   const int tid = threadIdx.x;
@@ -180,13 +181,18 @@ compact_involved_kernel(uint32_t* __restrict__ bitmap, int64_t n_words, uint8_t*
       ++o_inv;
       const bool rst = (uptodate != nullptr) && (uptodate[u] == 0);
       const bool pend = (has_msg != nullptr) && (has_msg[u] != 0) && !rst;
+      int32_t row = pend ? o_out : -1;
       if (rst) {
         if (o_rst < cap) restart_nodes[o_rst] = u;
+        if (read_only) {
+          if (o_rst < cap) row = restart_base + o_rst;
+        } else {
+          uptodate[u] = 1;
+          if (has_msg != nullptr) has_msg[u] = 0;  // msg_store.clear(nids): memory.py:136
+        }
         ++o_rst;
-        uptodate[u] = 1;
-        if (has_msg != nullptr) has_msg[u] = 0;  // msg_store.clear(nids): memory.py:136
       }
-      if (gru_row != nullptr) gru_row[u] = pend ? o_out : -1;
+      if (gru_row != nullptr) gru_row[u] = row;
       if (pend) {
         if (o_out < cap) outdated[o_out] = u;
         ++o_out;
@@ -217,7 +223,7 @@ compact_involved_cluster_kernel(uint32_t* __restrict__ bitmap, int n_words, int 
                                 int64_t* __restrict__ involved, int64_t cap, int64_t* __restrict__ local_index,
                                 int64_t* __restrict__ outdated, int32_t* __restrict__ gru_row,
                                 int64_t* __restrict__ restart_nodes, int32_t* __restrict__ counts,
-                                uint32_t* __restrict__ err_flags) {
+                                uint32_t* __restrict__ err_flags, int read_only, int restart_base) {
   extern __shared__ uint32_t cw[];           // [3][chunk] masks (member, restart, pending) then [3][chunk] offsets
   uint32_t* m_mem = cw;
   uint32_t* m_rst = cw + chunk;
@@ -315,14 +321,19 @@ compact_involved_cluster_kernel(uint32_t* __restrict__ bitmap, int n_words, int 
     if (r_inv < cap) involved[r_inv] = u;
     if (local_index != nullptr) local_index[u] = r_inv;
     const bool rst = (br >> lane) & 1u, pend = (bp >> lane) & 1u;
+    const int r_out = base[1] + off[2 * chunk + w] + __popc(bp & lt);
+    int32_t row = pend ? r_out : -1;
     if (rst) {
       const int r = base[2] + off[chunk + w] + __popc(br & lt);
       if (r < cap) restart_nodes[r] = u;
-      uptodate[u] = 1;
-      if (has_msg != nullptr) has_msg[u] = 0;  // msg_store.clear(nids): memory.py:136
+      if (read_only) {
+        if (r < cap) row = restart_base + r;
+      } else {
+        uptodate[u] = 1;
+        if (has_msg != nullptr) has_msg[u] = 0;  // msg_store.clear(nids): memory.py:136
+      }
     }
-    const int r_out = base[1] + off[2 * chunk + w] + __popc(bp & lt);
-    if (gru_row != nullptr) gru_row[u] = pend ? r_out : -1;
+    if (gru_row != nullptr) gru_row[u] = row;
     if (pend && r_out < cap) outdated[r_out] = u;
   }
   if (rank == 0 && tid == 0) {
@@ -333,13 +344,16 @@ compact_involved_cluster_kernel(uint32_t* __restrict__ bitmap, int n_words, int 
   }
 }
 
-extern "C" int tiger_compact_involved(uint32_t* bitmap, int64_t n_nodes, uint8_t* has_msg, uint8_t* uptodate,
-                                      int64_t* involved, int64_t cap_involved, int64_t* local_index,
-                                      int64_t* outdated, int32_t* gru_row, int64_t* restart_nodes,
-                                      int32_t* counts, uint32_t* err_flags, void* stream) {
+extern "C" int tiger_compact_involved_ex(uint32_t* bitmap, int64_t n_nodes, uint8_t* has_msg, uint8_t* uptodate,
+                                         int64_t* involved, int64_t cap_involved, int64_t* local_index,
+                                         int64_t* outdated, int32_t* gru_row, int64_t* restart_nodes,
+                                         int32_t* counts, uint32_t* err_flags, int read_only, int restart_base,
+                                         void* stream) {
   if (n_nodes <= 0 || cap_involved <= 0 || counts == nullptr || involved == nullptr) return TIGER_EINVAL;
   if (has_msg != nullptr && outdated == nullptr) return TIGER_EINVAL;
   if (uptodate != nullptr && restart_nodes == nullptr) return TIGER_EINVAL;
+  if (read_only && (restart_base < 0 || (int64_t)restart_base + cap_involved > (int64_t)INT32_MAX)) return TIGER_EINVAL;
+  read_only = read_only ? 1 : 0;
   const int64_t n_words = (n_nodes + 31) / 32;
   if (n_words <= (int64_t)COMPACT_CTAS * COMPACT_FAST_WORDS) {
     static bool configured = false;
@@ -353,10 +367,18 @@ extern "C" int tiger_compact_involved(uint32_t* bitmap, int64_t n_nodes, uint8_t
     return tiger_launch_chain(compact_involved_cluster_kernel, dim3(COMPACT_CTAS), dim3(1024),
                               (size_t)chunk * 6 * sizeof(uint32_t), as_stream(stream), dim3(COMPACT_CTAS, 1, 1), bitmap,
                               (int)n_words, chunk, n_nodes, has_msg, uptodate, involved, cap_involved, local_index, outdated,
-                              gru_row, restart_nodes, counts, err_flags);
+                              gru_row, restart_nodes, counts, err_flags, read_only, restart_base);
   }
   compact_involved_kernel<<<1, 1024, 0, as_stream(stream)>>>(bitmap, n_words, has_msg, uptodate, involved,
                                                             cap_involved, local_index, outdated, gru_row,
-                                                            restart_nodes, counts, err_flags);
+                                                            restart_nodes, counts, err_flags, read_only, restart_base);
   return tiger_launch_status();
+}
+
+extern "C" int tiger_compact_involved(uint32_t* bitmap, int64_t n_nodes, uint8_t* has_msg, uint8_t* uptodate,
+                                      int64_t* involved, int64_t cap_involved, int64_t* local_index,
+                                      int64_t* outdated, int32_t* gru_row, int64_t* restart_nodes,
+                                      int32_t* counts, uint32_t* err_flags, void* stream) {
+  return tiger_compact_involved_ex(bitmap, n_nodes, has_msg, uptodate, involved, cap_involved, local_index, outdated,
+                                   gru_row, restart_nodes, counts, err_flags, 0, 0, stream);
 }

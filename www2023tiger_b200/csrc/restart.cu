@@ -64,3 +64,30 @@ extern "C" int tiger_static_restart(const int64_t* nids, const int32_t* count, i
       left_active, right_vals, right_ts, right_active, has_msg, out_prev_ts);
   return tiger_launch_status();
 }
+
+// Restart surrogates of a read-only query (tiger_compact_involved_ex with read_only): row i of out_rows receives
+// right_emb[nids[i]] - the right-memory row tiger_static_restart would write for the i-th restarted node - for
+// i < min(*count, n); nothing node-indexed is written.
+__global__ void __launch_bounds__(RST_WARPS * 32)
+static_restart_rows_kernel(const int64_t* __restrict__ nids, const int32_t* __restrict__ count, int64_t n,
+                           const float* __restrict__ right_emb, int d, float* __restrict__ out_rows) {
+  int64_t total = n;
+  if (count != nullptr) {
+    const int64_t c = *count;
+    total = c < n ? c : n;
+  }
+  const int lane = lane_id();
+  for (int64_t i = (int64_t)blockIdx.x * RST_WARPS + warp_id_in_block(); i < total; i += (int64_t)gridDim.x * RST_WARPS)
+    warp_copy_row(out_rows + i * (int64_t)d, right_emb + nids[i] * (int64_t)d, d, lane);
+}
+
+extern "C" int tiger_static_restart_rows(const int64_t* nids, const int32_t* count, int64_t n, const float* right_emb,
+                                         int d, float* out_rows, void* stream) {
+  if (n < 0 || d <= 0 || nids == nullptr || right_emb == nullptr || out_rows == nullptr) return TIGER_EINVAL;
+  if (n == 0) return TIGER_OK;
+  int64_t grid = (n + RST_WARPS - 1) / RST_WARPS;
+  grid = grid > 148 ? 148 : grid;
+  static_restart_rows_kernel<<<(unsigned)grid, RST_WARPS * 32, 0, as_stream(stream)>>>(nids, count, n, right_emb, d,
+                                                                                       out_rows);
+  return tiger_launch_status();
+}

@@ -9,8 +9,11 @@
 //   bin / none : c_ab[2 any(a) + any(b)]              (four pre-folded constants; none: c_00, no table read)
 //   count      : U[sum a] + V[sum b]                  (hit embedding of the counts folded through W1a / W1b)
 //   vec        : b1 + sum_{a_j} Ha^T[j] + sum_{b_j} Hb^T[j]   (the hit vectors' columns of fc1)
-// One warp per pair; the flags of 32 slots at a time come from one ballot per side.  The BCE mean is reduced by the
-// last CTA in a fixed order, so the loss does not depend on the order in which the CTAs finish.
+// Pairs are candidate-major: pair p = j Q + i of candidate column j (0: the true candidate pos[i], j >= 1: negs[(j-1) Q + i])
+// scores row i of [src | column 0 | column 1 | ...] with row Q + p - the batch layout [src ; dst ; neg] at C = 2 and
+// the query layout of a one-vs-many candidate query at any C.
+// One warp per pair; the flags of 32 slots at a time come from one ballot per side.  The BCE mean (optional) is reduced
+// by the last CTA in a fixed order, so the loss does not depend on the order in which the CTAs finish.
 #include "common.cuh"
 
 #define SCOREF_WARPS 8
@@ -18,28 +21,29 @@
 // b1 | Ha^T | Hb^T, tiger_score_fold_hit_offset)
 template <int HIT>
 __global__ void __launch_bounds__(SCOREF_WARPS * 32)
-link_score_folded_kernel(const float* __restrict__ pq, int64_t batch, int d, const int64_t* __restrict__ src,
-                         const int64_t* __restrict__ dst, const int64_t* __restrict__ neg,
+link_score_folded_kernel(const float* __restrict__ pq, int64_t batch, int n_cands, int d,
+                         const int64_t* __restrict__ src, const int64_t* __restrict__ pos,
+                         const int64_t* __restrict__ negs,
                          const int64_t* __restrict__ neigh, int k, const float* __restrict__ cab,
                          const float* __restrict__ fc2_w, const float* __restrict__ fc2_b,
                          float* __restrict__ scores, float* __restrict__ loss, uint32_t* __restrict__ done_counter) {
   __shared__ float red[SCOREF_WARPS];
   __shared__ bool s_last;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int64_t n_pairs = 2 * batch;
+  const int64_t n_pairs = (int64_t)n_cands * batch;
   const int64_t p = (int64_t)blockIdx.x * SCOREF_WARPS + warp;
   pdl_trigger();
   pdl_wait();      // PQ comes from the last attention product
   if (p < n_pairs) {
     const bool is_neg = p >= batch;
-    const int64_t e = is_neg ? p - batch : p;
-    const int64_t row_s = e, row_t = is_neg ? 2 * batch + e : batch + e;     // rows of [src ; dst ; neg]
+    const int64_t e = is_neg ? p % batch : p;
+    const int64_t row_s = e, row_t = batch + p;     // rows of [src | column 0 | column 1 | ...]
     float acc = 0.f;
     if constexpr (HIT == TIGER_HIT_BIN) {
       int fa = 0, fb = 0;
       if (neigh != nullptr) {
         // src_hits: src in N(target) ; dst_hits: target in N(src)   (tiger.py:266-270, data_loader.py:61-75)
-        const int64_t s_id = src[e], t_id = is_neg ? neg[e] : dst[e];
+        const int64_t s_id = src[e], t_id = is_neg ? negs[p - batch] : pos[e];
         for (int j = lane; j < k; j += 32) {
           fa |= (neigh[row_t * k + j] == s_id);
           fb |= (neigh[row_s * k + j] == t_id);
@@ -56,7 +60,7 @@ link_score_folded_kernel(const float* __restrict__ pq, int64_t batch, int d, con
       const float* Q = pq + row_t * 2 * d + d;
       // slot flags a_j (src in N(target)) / b_j (target in N(src)) of slots [c0, c0 + 32), one ballot per side;
       // the loops around the ballots are warp-uniform
-      const int64_t s_id = src[e], t_id = is_neg ? neg[e] : dst[e];
+      const int64_t s_id = src[e], t_id = is_neg ? negs[p - batch] : pos[e];
       const int64_t *na = neigh + row_t * k, *nb = neigh + row_s * k;
       auto ballots = [&](int c0, uint32_t& ma, uint32_t& mb) {
         const int j = c0 + lane;
@@ -122,23 +126,65 @@ link_score_folded_kernel(const float* __restrict__ pq, int64_t batch, int d, con
   }
 }
 
-extern "C" int tiger_link_score_folded_hit(const float* pq, int64_t batch, int d, const int64_t* src,
-                                           const int64_t* dst, const int64_t* neg, const int64_t* neigh_nids, int k,
-                                           int hit_type, const float* tables, const float* fc2_w, const float* fc2_b,
-                                           float* scores, float* loss, uint32_t* done_counter, void* stream) {
+// ranks[i] = 1 + #{j >= 1 : s_ij > s_i0} + #{j >= 1 : s_ij == s_i0} / 2 over the candidate-major scores, one warp per
+// query row; integer counts, so the result does not depend on the order of the lanes.  A NaN true score gives a NaN
+// rank; a NaN candidate score neither beats nor ties the true one.
+__global__ void __launch_bounds__(SCOREF_WARPS * 32)
+link_rank_kernel(const float* __restrict__ scores, int64_t batch, int n_cands, float* __restrict__ ranks) {
+  const int lane = lane_id();
+  const int64_t i = (int64_t)blockIdx.x * SCOREF_WARPS + warp_id_in_block();
+  pdl_trigger();
+  pdl_wait();      // the scores come from the scorer
+  if (i >= batch) return;
+  const float s0 = scores[i];
+  int gt = 0, eq = 0;
+  for (int j = 1 + lane; j < n_cands; j += 32) {
+    const float s = scores[(int64_t)j * batch + i];
+    gt += s > s0;
+    eq += s == s0;
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    gt += __shfl_xor_sync(TIGER_FULL_MASK, gt, o);
+    eq += __shfl_xor_sync(TIGER_FULL_MASK, eq, o);
+  }
+  if (lane == 0) ranks[i] = s0 == s0 ? 1.0f + (float)gt + 0.5f * (float)eq : s0;
+}
+
+extern "C" int tiger_link_score_cands(const float* pq, int64_t n_query, int n_cands, int d, const int64_t* src,
+                                      const int64_t* pos, const int64_t* negs, const int64_t* neigh_nids, int k,
+                                      int hit_type, const float* tables, const float* fc2_w, const float* fc2_b,
+                                      float* scores, float* ranks, float* loss, uint32_t* done_counter, void* stream) {
   if (hit_type == TIGER_HIT_NONE) neigh_nids = nullptr;
   else if (hit_type != TIGER_HIT_BIN && hit_type != TIGER_HIT_VEC && hit_type != TIGER_HIT_COUNT) return TIGER_EINVAL;
   else if (neigh_nids == nullptr || k <= 0) return TIGER_EINVAL;
-  if (pq == nullptr || tables == nullptr || batch < 0 || d <= 0) return TIGER_EINVAL;
+  if (pq == nullptr || tables == nullptr || n_query < 0 || n_cands < 1 || d <= 0 || scores == nullptr) return TIGER_EINVAL;
+  if (n_cands > 1 && negs == nullptr) return TIGER_EINVAL;
   if (loss != nullptr && done_counter == nullptr) return TIGER_EINVAL;
-  if (batch == 0) return TIGER_OK;
-  const unsigned grid = (unsigned)((2 * batch + SCOREF_WARPS - 1) / SCOREF_WARPS);
+  if (n_query == 0) return TIGER_OK;
+  const int64_t n_pairs = (int64_t)n_cands * n_query;
+  if ((n_pairs + SCOREF_WARPS - 1) / SCOREF_WARPS > 0x7fffffffll) return TIGER_EINVAL;
+  const unsigned grid = (unsigned)((n_pairs + SCOREF_WARPS - 1) / SCOREF_WARPS);
   decltype(&link_score_folded_kernel<TIGER_HIT_BIN>) kernel =
       hit_type == TIGER_HIT_VEC     ? link_score_folded_kernel<TIGER_HIT_VEC>
       : hit_type == TIGER_HIT_COUNT ? link_score_folded_kernel<TIGER_HIT_COUNT>
                                     : link_score_folded_kernel<TIGER_HIT_BIN>;
-  return tiger_launch_chain(kernel, dim3(grid), dim3(SCOREF_WARPS * 32), 0, as_stream(stream), dim3(1, 1, 1), pq, batch,
-                            d, src, dst, neg, neigh_nids, k, tables, fc2_w, fc2_b, scores, loss, done_counter);
+  int rc = tiger_launch_chain(kernel, dim3(grid), dim3(SCOREF_WARPS * 32), 0, as_stream(stream), dim3(1, 1, 1), pq,
+                              n_query, n_cands, d, src, pos, negs, neigh_nids, k, tables, fc2_w, fc2_b, scores, loss,
+                              done_counter);
+  if (rc != TIGER_OK || ranks == nullptr) return rc;
+  return tiger_launch_chain(link_rank_kernel, dim3((unsigned)((n_query + SCOREF_WARPS - 1) / SCOREF_WARPS)),
+                            dim3(SCOREF_WARPS * 32), 0, as_stream(stream), dim3(1, 1, 1), (const float*)scores, n_query,
+                            n_cands, ranks);
+}
+
+extern "C" int tiger_link_score_folded_hit(const float* pq, int64_t batch, int d, const int64_t* src,
+                                           const int64_t* dst, const int64_t* neg, const int64_t* neigh_nids, int k,
+                                           int hit_type, const float* tables, const float* fc2_w, const float* fc2_b,
+                                           float* scores, float* loss, uint32_t* done_counter, void* stream) {
+  if (batch < 0) return TIGER_EINVAL;
+  return tiger_link_score_cands(pq, batch, 2, d, src, dst, neg, neigh_nids, k, hit_type, tables, fc2_w, fc2_b, scores,
+                                nullptr, loss, done_counter, stream);
 }
 
 extern "C" int tiger_link_score_folded(const float* pq, int64_t batch, int d, const int64_t* src, const int64_t* dst,

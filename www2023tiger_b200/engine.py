@@ -28,6 +28,9 @@ With n_layers = 2 (GraphEmbedding.compute_embedding_with_computation_graph, temp
   8a tiger_temporal_attention_ex, fns.1, 3B*K depth-1 queries (center = hop-1 neighbor, time = its parent event's)
      over the hop-2 table -> emb1 [3B*K, d]
   8b tiger_temporal_attention_ex, fns.0, the 3B batch nodes over the hop-1 table, slot (q, j) keyed by emb1[q*K + j]
+
+`CandidateQuery` (TigerEngine.candidate_query) scores one-vs-many candidate lists against the live state with the
+same launches, reading the state tables and writing none of them.
 """
 from typing import Dict, Optional
 
@@ -133,6 +136,7 @@ class TigerEngine:
         self.pq = torch.zeros(3 * batch_size, 2 * self.d, dtype=f32, device=dev)   # [W1a z | W1b z] per query row
         self.hist_len = hist_len
         self.seq = ops.SeqRestarterOp(self.d, self.de, hist_len, n_head, self.cap, dev) if restarter == 'seq' else None
+        self.weights_version = 0            # counts load_weights calls: a graph captured before one is stale
         self.load_weights(weights)
 
     # ------------------------------------------------------------------ parameters
@@ -172,6 +176,7 @@ class TigerEngine:
             self.right_emb = g('restarter_fn.right_emb.weight')
         elif self.restarter == 'seq':
             self.seq.set_weights(W)
+        self.weights_version += 1
 
     # ------------------------------------------------------------------ state
     def reset(self):
@@ -363,6 +368,161 @@ class TigerEngine:
         self.launch_finder()
         self.launch_model()
 
+    def candidate_query(self, max_queries: int, n_candidates: int) -> 'CandidateQuery':
+        """A read-only scorer of up to `max_queries` sources against `n_candidates` candidates each on this engine's
+        current state and weights (CandidateQuery)."""
+        return CandidateQuery(self, max_queries, n_candidates)
+
+
+class CandidateQuery:
+    """`scores, ranks = q.score(src [Q], cands [Q, C], ts [Q])`: scores[i, j] is the link-scorer logit the ingest step
+    would produce for the event (src[i], cands[i, j]) at ts[i] on the engine's current state - lazy restart of
+    not-yet-seen nodes at min(ts) as a surrogate, the updater overlay of nodes with a pending message, the attention
+    (one or two layers), the hit flags of cands[i, j] against src[i], the folded scorer - and ranks[i] =
+    1 + #{j >= 1: s_ij > s_i0} + 0.5 #{j >= 1: s_ij == s_i0} ranks column 0, the true candidate (ties count half; a
+    NaN s_i0 gives a NaN rank, a NaN s_ij neither beats nor ties s_i0).
+
+    Nothing persistent changes: the memories, the message store, `has_msg` and `uptodate` are only read, and the query
+    owns all its scratch (finder tables, bitmap, lists, `gru_row`, updater / attention / restarter workspaces, `pq`).
+    The weight packs are the engine's own, so `load_weights` reaches both paths; a graph captured before it would read
+    replaced weight tensors, so score() drops it and launches eagerly until capture() is called again.  The query's node list is [src | cands[:, 0] | cands[:, 1] | ...], the ingest step's batch layout
+    with 3 -> 1 + C rows per event: with C = 2 and cands = [dst, neg] it is that batch, and its scores are the step's.
+
+    Launches go to the current stream, behind the ingest steps issued there before; with a StreamRunner call
+    `runner.join()` first.  The results are views of this object's buffers (scores [Q, C] is the transpose of a
+    candidate-major [C, Q] buffer), valid until the next score()."""
+
+    def __init__(self, engine: TigerEngine, max_queries: int, n_candidates: int):
+        if not (isinstance(max_queries, int) and isinstance(n_candidates, int)) or max_queries < 1 or n_candidates < 1:
+            raise ValueError(f'max_queries and n_candidates must be positive ints, got {max_queries!r}, {n_candidates!r}')
+        e = self.e = engine
+        self.Q, self.C = max_queries, n_candidates
+        N, d, K, dev = e.N, e.d, e.K, e.device
+        n = (1 + n_candidates) * max_queries
+        full = n * (K + 1) if e.n_layers == 1 else (n + n * K) * (K + 1)
+        # the lists hold distinct nodes, so never more than N.  A query with at least as many rows as a batch gets at
+        # least the engine's own capacity, so that a query shaped like the batch (C = 2, max_queries = B) gets exactly
+        # that capacity and runs the step's launch shapes (the GEMMs pick their tiles by capacity)
+        self.cap = cap = min(full, max(N, e.cap))
+        z = lambda *sh, dt=f32: torch.zeros(*sh, dtype=dt, device=dev)
+        # inputs: [src | cands column-major] int64 [(1+C)Q], then the times as float64 bits [Q]
+        self.inp = z(n + max_queries, dt=i64)
+        self.nids, self.ts64 = self.inp[:n], self.inp[n:].view(f64)
+        self.ts32 = z(max_queries)
+        self.bitmap = z(ops.bitmap_words(N), dt=i32)
+        self.involved, self.outdated, self.restart_nodes = z(cap, dt=i64), z(cap, dt=i64), z(cap, dt=i64)
+        self.gru_row = torch.full((N,), -1, dtype=i32, device=dev)
+        self.counts, self.err_flags = z(4, dt=i32), z(1, dt=i32)
+        self.neigh_nids, self.neigh_eids, self.neigh_ts = z(n, K, dt=i64), z(n, K, dt=i64), z(n, K)
+        if e.n_layers == 2:
+            self.neigh_ts64 = z(n * K, dt=f64)
+            self.neigh2_nids, self.neigh2_eids, self.neigh2_ts = z(n * K, K, dt=i64), z(n * K, K, dt=i64), z(n * K, K)
+            self.emb1 = z(n * K, d)
+        # node rows the attention reads through gru_row: updater output [0, O), restart surrogates [cap, cap + R)
+        self.rows_b = z(2 * cap, d)
+        self.emb, self.pq = z(n, d), z(n, 2 * d)
+        self.scores, self.ranks = z(n_candidates * max_queries), z(max_queries)
+        self.upd_scratch = e.updater.scratch(cap)
+        self.attn = e.attn_pack.share()
+        self.attn.attach_score_fold(e.score_fold, self.pq)
+        self.attn1 = e.attn_pack1.share() if e.attn_pack1 is not None else None
+        # both attention workspaces sized once, for max_queries: a captured graph keeps their addresses whatever Q the
+        # eager calls in between use
+        self.attn.work(n, K)
+        if self.attn1 is not None:
+            self.attn1.work(n * K, K)
+        self.seq = None
+        if e.lazy_restart and e.restarter == 'seq':
+            self.seq = ops.SeqRestarterOp(d, e.de, e.hist_len, e.H, cap, dev)
+            self.seq.h_right = self.rows_b[cap:]        # the restarter writes the surrogates in place
+        self.graph = self._graph_key = None
+
+    # ------------------------------------------------------------------ inputs
+    def _upload(self, src, cands, ts, Q: int):
+        C = self.C
+        as_t = lambda x: x if isinstance(x, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(x))
+        src, cands, ts = as_t(src), as_t(cands), as_t(ts)
+        self.nids[:Q].copy_(src)
+        self.nids[Q:(1 + C) * Q].view(C, Q).copy_(cands.t())
+        self.ts64[:Q].copy_(ts)
+
+    # ------------------------------------------------------------------ the launch sequence
+    def launch(self, Q: int, ranks: bool = True):
+        """The query's launches for the first Q queries already in the input buffer (no host sync)."""
+        e, cap, K, C = self.e, self.cap, self.e.K, self.C
+        n = (1 + C) * Q
+        nids, ts64, ts32 = self.nids[:n], self.ts64[:Q], self.ts32[:Q]
+        nn, ne, nt = self.neigh_nids[:n], self.neigh_eids[:n], self.neigh_ts[:n]
+        ops.find_recent(e.csr, nids, ts64, K, ts_period=Q, want_dirs=False, ts32_out=ts32, bitmap=self.bitmap,
+                        out=(nn, ne, nt, None))
+        if e.n_layers == 2:
+            n2 = (self.neigh2_nids[:n * K], self.neigh2_eids[:n * K], self.neigh2_ts[:n * K])
+            ops.find_second_hop(e.csr, nn, nt, K, ts64=self.neigh_ts64[:n * K], bitmap=self.bitmap, out=n2)
+        ops.compact_involved(self.bitmap, e.N, self.involved, self.counts, has_msg=e.has_msg,
+                             uptodate=e.uptodate if e.lazy_restart else None, outdated=self.outdated,
+                             gru_row=self.gru_row, restart_nodes=self.restart_nodes if e.lazy_restart else None,
+                             err_flags=self.err_flags, read_only=True, restart_base=cap)
+        if e.lazy_restart:
+            R = self.counts[2:]
+            if e.restarter == 'static':
+                ops.static_restart_rows(self.restart_nodes, cap, e.right_emb, e.d, self.rows_b[cap:], count=R)
+            else:
+                self.seq.share_weights(e.seq)
+                ops.min_time(ts32, self.seq.tmin)
+                self.seq.history(e.csr, self.restart_nodes, self.seq.tmin, cap, ts_period=1, count=R)
+                self.seq.forward(self.restart_nodes, cap, e.nfeats, e.efeats, count=R)
+        msg_ts_mem = e._mem(e.msg_src)[1]
+        e.updater.launch(node_ids=self.outdated, x_table=e.msg_vals, h_table=e._mem(e.upd_src)[0], n_rows=cap,
+                         out=self.rows_b[:cap], count=self.counts[1:], msg_ts=e.msg_ts, check_mem_ts=msg_ts_mem,
+                         check_equal=(e.msg_src == 'left'), err_flags=self.err_flags, scratch=self.upd_scratch)
+        rows = dict(rows_a=e.right_vals, rows_b=self.rows_b, sel=self.gru_row, nfeats=e.nfeats, efeats=e.efeats)
+        key_rows = None
+        if e.n_layers == 2:
+            key_rows = self.emb1[:n * K]
+            ops.temporal_attention(self.attn1, e.H, nn.view(-1), ts32, *n2, out=key_rows, ts_group=K, **rows)
+        ops.temporal_attention(self.attn, e.H, nids, ts32, nn, ne, nt, out=self.emb[:n], key_rows=key_rows,
+                               read_only=True, **rows)
+        ops.link_score_cands(e.score_fold, self.pq[:n], nids[:Q], nids[Q:2 * Q], nids[2 * Q:],
+                             nn if e.hit_type != 'none' else None, self.scores[:C * Q],
+                             self.ranks[:Q] if ranks else None)
+
+    def capture(self, n_queries: Optional[int] = None, ranks: bool = True):
+        """Record launch(n_queries, ranks) as one CUDA graph; score() replays it for that many queries once it has
+        copied the inputs into the input buffer."""
+        Q = self.Q if n_queries is None else n_queries
+        if not 1 <= Q <= self.Q:
+            raise ValueError(f'n_queries={Q}: this CandidateQuery takes 1 to max_queries={self.Q}')
+        s = torch.cuda.Stream(device=self.e.device)
+        s.wait_stream(torch.cuda.current_stream())
+        with torch.cuda.stream(s):
+            self.launch(Q, ranks)               # warm-up: module loads and kernel attributes outside the capture
+        torch.cuda.current_stream().wait_stream(s)
+        torch.cuda.synchronize()
+        graph = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(graph):
+            self.launch(Q, ranks)
+        torch.cuda.synchronize()
+        self.graph, self._graph_key = graph, (Q, ranks, self.e.weights_version)
+
+    def score(self, src, cands, ts, ranks: bool = True):
+        """src int64 [Q], cands int64 [Q, C], ts float64 [Q] (numpy arrays or tensors) -> (scores [Q, C], ranks [Q] or
+        None), float32 views of this object's buffers.  ValueError before any launch for a wrong dtype, rank, shape,
+        node id or Q > max_queries."""
+        Q = check_query_inputs(src, cands, ts, max_queries=self.Q, n_candidates=self.C, n_nodes=self.e.N,
+                               device=self.e.device)
+        self._upload(src, cands, ts, Q)
+        if self.graph is not None and self._graph_key[2] != self.e.weights_version:
+            self.graph = self._graph_key = None          # captured on weight tensors load_weights has replaced
+        if self.graph is not None and self._graph_key[:2] == (Q, ranks):
+            self.graph.replay()
+        else:
+            self.launch(Q, ranks)
+        return self.scores[:self.C * Q].view(self.C, Q).t(), (self.ranks[:Q] if ranks else None)
+
+    def check_errors(self):
+        """Host sync: raise the reference's ValueError if an invariant flag of this object's launches is set."""
+        raise_on_err_flags(int(self.err_flags.item()) & 0xffffffff)
+
 
 class StreamRunner:
     """Replays an event stream through a TigerEngine.
@@ -519,3 +679,38 @@ class StreamRunner:
     @property
     def d2h_bytes_per_step(self) -> int:
         return self.h_out[0].numel() * 4
+
+
+def check_query_inputs(src, cands, ts, *, max_queries: int, n_candidates: int, n_nodes: int, device) -> int:
+    """The checks CandidateQuery.score runs before it launches anything: src int64 [Q], cands int64
+    [Q, n_candidates], ts float64 [Q], numpy arrays or tensors (CUDA tensors on `device`), 1 <= Q <= max_queries, node
+    ids in [0, n_nodes).  Raises ValueError; returns Q."""
+    def dtype_of(x, what):
+        if isinstance(x, torch.Tensor):
+            return str(x.dtype).replace('torch.', '')
+        if isinstance(x, np.ndarray):
+            return str(x.dtype)
+        raise ValueError(f'{what} must be a numpy array or a torch tensor, got {type(x).__name__}')
+    for x, what, dt, nd in ((src, 'src', 'int64', 1), (cands, 'cands', 'int64', 2), (ts, 'ts', 'float64', 1)):
+        if dtype_of(x, what) != dt:
+            raise ValueError(f'{what} must be {dt}, got {dtype_of(x, what)}')
+        if x.ndim != nd:
+            raise ValueError(f'{what} must have {nd} dimension(s), got shape {tuple(x.shape)}')
+        if isinstance(x, torch.Tensor) and x.is_cuda:
+            want = torch.device(device)
+            if want.index is None:
+                want = torch.device(want.type, torch.cuda.current_device())
+            if x.device != want:
+                raise ValueError(f'{what} is on {x.device}, the engine on {want}')
+    Q = src.shape[0]
+    if Q < 1 or Q > max_queries:
+        raise ValueError(f'{Q} queries: this CandidateQuery takes 1 to max_queries={max_queries}')
+    if tuple(cands.shape) != (Q, n_candidates):
+        raise ValueError(f'cands must be [{Q}, n_candidates={n_candidates}], got {tuple(cands.shape)}')
+    if tuple(ts.shape) != (Q,):
+        raise ValueError(f'ts must be [{Q}], got {tuple(ts.shape)}')
+    for x, what in ((src, 'src'), (cands, 'cands')):
+        lo, hi = (x.min(), x.max()) if isinstance(x, np.ndarray) else (int(v) for v in torch.aminmax(x))
+        if lo < 0 or hi >= n_nodes:
+            raise ValueError(f'{what} holds node ids outside [0, {n_nodes})')
+    return Q

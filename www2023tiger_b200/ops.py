@@ -104,10 +104,12 @@ def compact_involved(bitmap: Tensor, n_nodes: int, involved: Tensor, counts: Ten
                      has_msg: Optional[Tensor] = None, uptodate: Optional[Tensor] = None,
                      local_index: Optional[Tensor] = None, outdated: Optional[Tensor] = None,
                      gru_row: Optional[Tensor] = None, restart_nodes: Optional[Tensor] = None,
-                     err_flags: Optional[Tensor] = None):
-    call('tiger_compact_involved', ptr(bitmap), n_nodes, ptr(has_msg), ptr(uptodate), ptr(involved),
+                     err_flags: Optional[Tensor] = None, read_only: bool = False, restart_base: int = 0):
+    """read_only: uptodate / has_msg are only read, restart node r gets gru_row = restart_base + r (its restart
+    surrogate's row, tiger_compact_involved_ex)."""
+    call('tiger_compact_involved_ex', ptr(bitmap), n_nodes, ptr(has_msg), ptr(uptodate), ptr(involved),
          involved.numel(), ptr(local_index), ptr(outdated), ptr(gru_row), ptr(restart_nodes), ptr(counts),
-         ptr(err_flags))
+         ptr(err_flags), int(read_only), restart_base)
 
 
 # ------------------------------------------------------------------------------------------
@@ -323,14 +325,17 @@ class MemoryUpdater:
         self.hid = self.mid = None
         self.reserve(cap)
 
+    def scratch(self, cap: int):
+        """(hid, mid) for `cap` outdated rows: hidden rows of the MLP, first layer of the merge (None when unused)."""
+        z = lambda w: torch.zeros(cap, w, dtype=f32, device=self.device)
+        return (z(self.m_dim // 2) if self.tsfm == 'mlp' else None, z(self.d) if self.upd == 'merge' else None)
+
     def reserve(self, cap: int):
-        """Scratch for `cap` outdated rows (hidden rows of the MLP, first layer of the merge)."""
+        """Own scratch for `cap` outdated rows."""
         if cap <= self.cap:
             return
         self.cap = cap
-        z = lambda w: torch.zeros(cap, w, dtype=f32, device=self.device)
-        self.hid = z(self.m_dim // 2) if self.tsfm == 'mlp' else None
-        self.mid = z(self.d) if self.upd == 'merge' else None
+        self.hid, self.mid = self.scratch(cap)
 
     @property
     def launches(self) -> int:
@@ -381,18 +386,20 @@ class MemoryUpdater:
 
     def launch(self, *, node_ids: Tensor, x_table: Tensor, h_table: Tensor, n_rows: int, out: Tensor,
                count: Optional[Tensor], msg_ts: Tensor, check_mem_ts: Optional[Tensor], check_equal: bool,
-               err_flags: Optional[Tensor]):
-        assert n_rows <= self.cap
+               err_flags: Optional[Tensor], scratch=None):
+        """scratch: (hid, mid) of another caller (`scratch(cap)`), which then runs on these packs beside the owner."""
+        hid, mid = (self.hid, self.mid) if scratch is None else scratch
+        assert n_rows <= self.cap if scratch is None else all(t is None or n_rows <= t.shape[0] for t in scratch)
         x_by_row = self.tsfm == 'mlp'
         if x_by_row:
-            x_table = gather_linear(node_ids[:n_rows], x_table, self.w1, self.b1, self.hid[:n_rows], relu=True,
+            x_table = gather_linear(node_ids[:n_rows], x_table, self.w1, self.b1, hid[:n_rows], relu=True,
                                     count=count)
         kw = dict(node_ids=node_ids, x_table=x_table, h_table=h_table, n_rows=n_rows, out=out, count=count,
                   msg_ts=msg_ts, check_mem_ts=check_mem_ts, check_equal=check_equal, err_flags=err_flags,
                   x_by_row=x_by_row)
         if self.upd == 'gru':
             return gru_update(self.gru, **kw)
-        return merge_update(self.merge, mid=self.mid, **kw)
+        return merge_update(self.merge, mid=mid, **kw)
 
 
 @functools.lru_cache(maxsize=None)
@@ -439,6 +446,9 @@ class LeftWritebackFusedC(ctypes.Structure):
                 ('ready_event', ctypes.c_void_p)]
 
 
+_ATTN_WEIGHT_FIELDS = tuple(n for n, _ in AttnParamsC._fields_[:13])    # wq .. folded
+
+
 class AttnPack:
     """TemporalAttention parameters for the kernels: the reference's tensors as stored plus the folded
     weights (tiger_attn_fold: Wqk, bqk, W2f), and a workspace that grows on demand.  A multi-layer embedding
@@ -457,6 +467,16 @@ class AttnPack:
         self._keep = None
         self._work = None
         self._work_key = None
+        self._base = None
+
+    def share(self) -> 'AttnPack':
+        """A pack on this pack's weights and folds (no copy) with its own score-fold attachment and workspace: a
+        second caller of the same layer (a candidate query beside the engine's step).  It re-reads the weight pointers
+        of this pack at every launch, so refresh() here reaches it."""
+        v = AttnPack.__new__(AttnPack)
+        v.d, v.de, v.n_head, v.E, v.C = self.d, self.de, self.n_head, self.E, self.C
+        v.folded, v.struct, v._keep, v._work, v._work_key, v._base = self.folded, AttnParamsC(), None, None, None, self
+        return v
 
     def refresh(self, q_w, k_w, v_w, in_bias, out_w, out_b, fc1_w, fc1_b, fc2_w, fc2_b, time_w, time_b):
         det = lambda t: t.detach().to(f32).contiguous()
@@ -471,6 +491,9 @@ class AttnPack:
         call('tiger_attn_fold', self.byref(), self.d, self.de, self.n_head)
 
     def byref(self):
+        if self._base is not None:
+            for name in _ATTN_WEIGHT_FIELDS:
+                setattr(self.struct, name, getattr(self._base.struct, name))
         return ctypes.addressof(self.struct)
 
     def attach_score_fold(self, fold: Optional['ScoreFold'], pq_out: Optional[Tensor]):
@@ -518,17 +541,20 @@ class AttnPack:
 def temporal_attention(pack: AttnPack, n_head: int, center_nids: Tensor, q_ts: Tensor, neigh_nids: Tensor,
                        neigh_eids: Tensor, neigh_ts: Tensor, *, rows_a: Optional[Tensor], rows_b: Tensor,
                        sel: Tensor, nfeats: Optional[Tensor], efeats: Optional[Tensor],
-                       out: Optional[Tensor] = None, key_rows: Optional[Tensor] = None, ts_group: int = 1) -> Tensor:
+                       out: Optional[Tensor] = None, key_rows: Optional[Tensor] = None, ts_group: int = 1,
+                       read_only: bool = False) -> Tensor:
     """a15+a16 (gather form).  Query q uses q_ts[(q // ts_group) % len(q_ts)] (ts.repeat semantics; ts_group = K
     gives repeat_interleave(ts.repeat(3), K), the depth-1 queries of n_layers = 2).  key_rows [n * K, d]: slot
-    (q, j) takes the lower layer's output row q * K + j as its node representation, without node features."""
+    (q, j) takes the lower layer's output row q * K + j as its node representation, without node features.
+    read_only: the pack has a score fold attached and no left write-back (tiger_temporal_attention_query)."""
     check_cuda(center_nids, q_ts, neigh_nids, neigh_eids, neigh_ts, rows_a, rows_b, sel, nfeats, efeats, key_rows)
     n, k = neigh_nids.shape
     if out is None:
         out = _empty((n, pack.d), f32, rows_b)
     assert sel.dtype in (i32, i64) and n_head == pack.n_head
     assert key_rows is None or (key_rows.dtype == f32 and key_rows.numel() >= n * k * pack.d)
-    call('tiger_temporal_attention_ex', ptr(center_nids), ptr(q_ts), n, q_ts.numel(), ts_group, ptr(neigh_nids),
+    entry = 'tiger_temporal_attention_query' if read_only else 'tiger_temporal_attention_ex'
+    call(entry, ptr(center_nids), ptr(q_ts), n, q_ts.numel(), ts_group, ptr(neigh_nids),
          ptr(neigh_eids), ptr(neigh_ts), k, ptr(rows_a), ptr(rows_b), ptr(key_rows), ptr(sel), int(sel.dtype == i64),
          ptr(nfeats), ptr(efeats), pack.d, pack.de, n_head, pack.byref(), ptr(out), ptr(pack.work(n, k)))
     return out
@@ -598,6 +624,28 @@ def link_score_folded(fold: ScoreFold, pq: Tensor, src: Tensor, dst: Tensor, neg
          fold.code(neigh_nids is not None), ptr(fold.cab), ptr(fold.fc2_w), ptr(fold.fc2_b), ptr(scores), ptr(loss),
          ptr(fold.done))
     return scores, loss
+
+
+def link_score_cands(fold: ScoreFold, pq: Tensor, src: Tensor, pos: Tensor, negs: Tensor,
+                     neigh_nids: Optional[Tensor], scores: Tensor, ranks: Optional[Tensor] = None,
+                     loss: Optional[Tensor] = None):
+    """The scorer over C = scores.numel() / Q candidate columns (tiger_link_score_cands): pq / neigh_nids hold the rows
+    of [src | pos | negs], negs [(C-1) Q] candidate-major; scores [C Q] candidate-major, ranks [Q] of column 0."""
+    Q = src.numel()
+    C = scores.numel() // Q
+    k = neigh_nids.shape[1] if neigh_nids is not None else 0
+    if fold.hit_type in ('vec', 'count') and k != fold.k:
+        raise ValueError(f'hit_type {fold.hit_type}: the fold holds {fold.k} slots, the neighbor table has {k}')
+    call('tiger_link_score_cands', ptr(pq), Q, C, fold.d, ptr(src), ptr(pos), ptr(negs), ptr(neigh_nids), k,
+         fold.code(neigh_nids is not None), ptr(fold.cab), ptr(fold.fc2_w), ptr(fold.fc2_b), ptr(scores), ptr(ranks),
+         ptr(loss), ptr(fold.done) if loss is not None else None)
+    return scores, ranks
+
+
+def static_restart_rows(nids: Tensor, n: int, right_emb: Tensor, d: int, out_rows: Tensor, *, count=None):
+    """out_rows[i] = right_emb[nids[i]] for i < min(*count, n): the right-memory rows a static restart writes."""
+    check_cuda(nids, right_emb, out_rows, count)
+    call('tiger_static_restart_rows', ptr(nids), ptr(count), n, ptr(right_emb), d, ptr(out_rows))
 
 
 def static_restart(nids: Tensor, n: int, csr: DeviceCSR, left_emb: Tensor, right_emb: Tensor, d: int, *,
@@ -790,6 +838,12 @@ class SeqRestarterOp:
         self.fn_w, self.fn_b = g('out_fn.weight'), g('out_fn.bias')
         self.fc1_w, self.fc1_b = g('merger.fc1.weight'), g('merger.fc1.bias')
         self.fc2_w, self.fc2_b = g('merger.fc2.weight'), g('merger.fc2.bias')
+
+    def share_weights(self, other: 'SeqRestarterOp'):
+        """Read the weights of `other` (no copy): a second workspace for the same restarter."""
+        for n in ('time_w', 'time_b', 'anony_emb', 'in_w', 'in_b', 'out_w', 'out_b', 'fn_w', 'fn_b', 'fc1_w', 'fc1_b',
+                  'fc2_w', 'fc2_b'):
+            setattr(self, n, getattr(other, n))
 
     def history(self, csr: DeviceCSR, nids: Tensor, q_ts: Tensor, n: int, *, ts_period: int = 0,
                 count: Optional[Tensor] = None):
