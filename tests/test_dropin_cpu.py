@@ -100,3 +100,25 @@ def test_native_trainer_refuses_sizes_past_its_kernels(K, restarter, hist_len, m
     ok = build_model(None, torch.zeros(50, 6), None, 40, 49, torch.device('cpu'), dim=None, n_neighbors=32,
                      restarter_type=restarter, hist_len=64)
     assert native_limit_error(ok) is None
+
+
+@pytest.mark.parametrize('hist_len', [65, 100])
+def test_engine_refuses_seq_histories_past_the_pooling_kernel(hist_len):
+    """The seq pooling kernel stages at most 64 events: TigerEngine and SeqRestarterOp refuse a longer history at
+    construction, before any device work, instead of failing at the first restart; the drop-in restarter takes its
+    torch code for it."""
+    from www2023tiger_b200 import ops
+    from www2023tiger_b200.engine import TigerEngine
+    from www2023tiger_b200.init import build_model
+    with pytest.raises(NotImplementedError, match='at most 64 events'):
+        TigerEngine({}, None, n_nodes=10, dim=8, efeats=None, device='cpu', restarter='seq', hist_len=hist_len)
+    with pytest.raises(NotImplementedError, match='at most 64 events'):
+        ops.SeqRestarterOp(8, 8, hist_len, 2, 4, 'cpu')
+    assert ops.seq_restarter_limit_error(8, 8, 64, 2) is None
+    assert 'n_head=3' in ops.seq_restarter_limit_error(8, 8, 64, 3)
+    model = build_model(None, torch.zeros(50, 6), None, 40, 49, torch.device('cpu'), dim=None, restarter_type='seq',
+                        hist_len=hist_len)
+    assert not model.restarter_fn.fits_kernel()
+    ok = build_model(None, torch.zeros(50, 6), None, 40, 49, torch.device('cpu'), dim=None, restarter_type='seq',
+                     hist_len=64)
+    assert ok.restarter_fn.fits_kernel()

@@ -399,7 +399,8 @@ def test_seq_restarter_matches_reference_golden(gu, name):
         assert np.array_equal(gu.cpu(pt), g.b(ib, 'r_hist_ts')[:, -1])
 
 
-@pytest.mark.parametrize('n_pick', [70, 30, 1])       # > / <= SeqRestarterOp.tail_rows: tensor-core products / fused tail
+# n = n_pick + 1 rows: 70 and 64 take the tensor-core products, 63 (n = 64 = SeqRestarterOp.tail_rows), 30, 1 the tail
+@pytest.mark.parametrize('n_pick', [70, 64, 63, 30, 1])
 @pytest.mark.parametrize('d,de,L,with_nf', [(172, 172, 40, False), (100, 4, 40, False), (24, 10, 64, True)])
 def test_seq_restarter_matches_oracle(gu, d, de, L, with_nf, n_pick):
     """Restarter with computation_graph=None: history looked up on the device CSR (restart path)."""

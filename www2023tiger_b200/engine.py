@@ -84,6 +84,12 @@ class TigerEngine:
         limit = ops.attention_limit_error(self.d, self.de, n_neighbors, n_head)
         if limit is not None:
             raise NotImplementedError(limit)
+        # the seq restarter's pooling kernel holds at most 64 history events: a longer history would fail at the first
+        # restart, after compact_involved has already marked the restarted nodes up to date
+        if restarter == 'seq':
+            limit = ops.seq_restarter_limit_error(self.d, self.de, hist_len, n_head)
+            if limit is not None:
+                raise NotImplementedError(limit)
         self.M = 3 * self.d + self.de                                          # tiger.py:62
         self.msg_src, self.upd_src = msg_src, upd_src
         self.restarter, self.lazy_restart = restarter, lazy_restart

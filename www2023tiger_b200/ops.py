@@ -798,6 +798,23 @@ def min_time(ts: Tensor, out: Tensor):
     call('tiger_min_time', ptr(ts), ts.numel(), ptr(out))
 
 
+SEQ_MAX_HIST_LEN = 64     # the pooling kernel stages at most this many positions per node (SP_MAXL, csrc/train_seq.cu)
+
+
+def seq_restarter_limit_error(d: int, de: int, hist_len: int, n_head: int) -> Optional[str]:
+    """Why the seq restarter's kernels (SeqRestarterOp, the native training step) cannot run a restarter of node width
+    d, edge width de, hist_len events and n_head heads, or None when they can.  The reference has no history limit,
+    so callers run such a restarter through torch."""
+    if min(d, de, hist_len, n_head) <= 0:
+        return f'invalid seq restarter dimensions d={d} de={de} hist_len={hist_len} n_head={n_head}'
+    if hist_len > SEQ_MAX_HIST_LEN:
+        return (f'the seq restarter kernels take a history of at most {SEQ_MAX_HIST_LEN} events (the pooling kernel '
+                f'stages them in shared memory); this restarter has hist_len={hist_len}')
+    if (4 * d + de) % n_head != 0:
+        return f'd_model = 4 d + de = {4 * d + de} is not a multiple of n_head={n_head}'
+    return None
+
+
 class SeqRestarterOp:
     """SeqRestarter.forward (reference restarters.py:51-114) on device buffers of capacity `cap` rows.
 
@@ -805,6 +822,9 @@ class SeqRestarterOp:
     change; `set_weights` only keeps contiguous fp32 views."""
 
     def __init__(self, d: int, de: int, hist_len: int, n_head: int, cap: int, device):
+        limit = seq_restarter_limit_error(d, de, hist_len, n_head)
+        if limit is not None:
+            raise NotImplementedError(limit)
         self.d, self.de, self.L, self.H, self.cap = d, de, hist_len, n_head, cap
         self.dm = 4 * d + de
         z = lambda *shape, dt=f32: torch.zeros(*shape, dtype=dt, device=device)

@@ -64,6 +64,11 @@ class SeqRestarter(Restarter):
         hn, he, ht, hd = self.graph.find_recent_device(nids.contiguous(), ts.double().contiguous(), self.hist_len)
         return hn, he, ht, hd, ops.anonymized_reindex(hn)
 
+    def fits_kernel(self) -> bool:
+        """Whether the kernels take this restarter (ops.seq_restarter_limit_error); past their limits (a history of
+        more than 64 events) it runs its torch code, which has none."""
+        return ops.seq_restarter_limit_error(self.nfeat_dim, self.efeat_dim, self.hist_len, self.n_head) is None
+
     def forward(self, nids: Tensor, ts: Tensor, computation_graph=None) -> Tuple[Tensor, Tensor, Tensor]:
         if computation_graph is None:
             hn, he, ht, hd, an = self.history(nids, ts)
@@ -71,7 +76,7 @@ class SeqRestarter(Restarter):
             r = computation_graph.restart_data
             hn, he, ht, hd, an = r.hist_nids, r.hist_eids, r.hist_ts, r.hist_dirs, r.anonymized_ids
         n = nids.numel()
-        if use_kernel(self) and hn.is_cuda:
+        if use_kernel(self) and hn.is_cuda and self.fits_kernel():
             op = self._operator(n, hn.device)
             fg = self.raw_feat_getter
             hl, hr, pt = op.forward(nids.contiguous(), n, fg.nfeats, fg.efeats,

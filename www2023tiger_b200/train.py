@@ -126,11 +126,10 @@ def _seed_step_word(device) -> Tensor:
     return _SEED_WORDS[idx]
 
 
-# Largest neighborhood and seq-restarter history the training kernels take: the attention core keeps one dropout bit
-# per slot in a 32-bit word (ATT_MAXK, csrc/train.cu), the seq pool stages at most 64 positions (SP_MAXL,
-# csrc/train_seq.cu).  Larger models train through the torch-op route, which has neither limit.
+# Largest neighborhood the training kernels take: the attention core keeps one dropout bit per slot in a 32-bit word
+# (ATT_MAXK, csrc/train.cu).  The seq restarter's limits are the inference kernels' (ops.seq_restarter_limit_error).
+# Larger models train through the torch-op route, which has neither limit.
 MAX_NEIGHBORS = 32
-MAX_HIST_LEN = 64
 
 
 def native_limit_error(model) -> Optional[str]:
@@ -139,9 +138,10 @@ def native_limit_error(model) -> Optional[str]:
         return (f'native training takes at most {MAX_NEIGHBORS} neighbors per query (the attention core keeps one '
                 f'dropout bit per slot in a 32-bit word); this model has n_neighbors={model.n_neighbors}')
     r = model.restarter_fn
-    if type(r).__name__ == 'SeqRestarter' and r.hist_len > MAX_HIST_LEN:
-        return (f'native training takes a seq restarter history of at most {MAX_HIST_LEN} events; this model has '
-                f'hist_len={r.hist_len}')
+    if type(r).__name__ == 'SeqRestarter':
+        limit = ops.seq_restarter_limit_error(r.nfeat_dim, r.efeat_dim, r.hist_len, r.n_head)
+        if limit is not None:
+            return 'native training: ' + limit
     return None
 
 
