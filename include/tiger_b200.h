@@ -72,6 +72,30 @@ int tiger_find_recent(const int64_t* indptr, const int32_t* adj_nbr, const int32
                       int64_t* out_nids, int64_t* out_eids, float* out_ts, int64_t* out_dirs,
                       float* out_ts32, uint32_t* mark_bitmap, const int32_t* count, void* stream);
 
+/* tiger_find_recent over M chunks of the stream that share one CSR (ChunkSampler, data_loader.py:23-48: every DDP rank
+ * keeps its own memory over its own contiguous slice; here the M slices run as one call).  Node u of chunk c has the
+ * virtual id v = c * node_stride + u; q_nids hold virtual ids and each query reads the CSR segment of
+ * u = v mod node_stride.  mark_bitmap (ceil(M * node_stride / 32) words) is marked with virtual ids.
+ *   TIGER_FIND_CHUNK_NEIGHBORS  the neighbor tables of the batch nodes and the second hop
+ *       (sample_temporal_neighbor, graph.py:117-127; data_loader.py:105-131): query i at q_ts[i % ts_period] as in
+ *       tiger_find_recent, out_nids offset by c * node_stride except id 0: the padding stays 0 (the attention and the
+ *       seq restarter key their masks on id 0; node 0 is the padding node, the reference's ids start at 1) and marks
+ *       the chunk's own node 0, c * node_stride, as an unchunked call marks node 0.  A query with id 0 - the second
+ *       hop of a padding slot, whose chunk the id does not tell - marks nothing (its chunk's node 0 is marked by the
+ *       padding slot it comes from).
+ *   TIGER_FIND_CHUNK_HISTORY    the seq restarter's get_history (graph.py:150-155) at each chunk's own restart time:
+ *       query i at q_ts[v / node_stride] (M chunk times, tiger_min_time_ex), ts_period and out_ts32 unused, out_nids
+ *       the real neighbor ids (restarters.py:80-87 masks the padding id 0).
+ * mode 0 is tiger_find_recent. */
+#define TIGER_FIND_CHUNK_NEIGHBORS 1
+#define TIGER_FIND_CHUNK_HISTORY 2
+int tiger_find_recent_ex(const int64_t* indptr, const int32_t* adj_nbr, const int32_t* adj_eid,
+                         const double* adj_ts, const uint8_t* adj_flag, const int64_t* q_nids,
+                         const double* q_ts, int64_t n_query, int64_t ts_period, int k,
+                         int64_t* out_nids, int64_t* out_eids, float* out_ts, int64_t* out_dirs,
+                         float* out_ts32, uint32_t* mark_bitmap, const int32_t* count,
+                         int64_t node_stride, int mode, void* stream);
+
 /* a4  GraphCollator.check_in_window (data_loader.py:61-67): hit[i,k] = (center[i]==neigh[i,k]). */
 int tiger_hit_window(const int64_t* center, const int64_t* neigh, int64_t n, int k, float* hit,
                      void* stream);
@@ -414,6 +438,20 @@ int tiger_static_restart(const int64_t* nids, const int32_t* count, int64_t n,
                          uint8_t* left_active, float* right_vals, float* right_ts,
                          uint8_t* right_active, uint8_t* has_msg, float* out_prev_ts, void* stream);
 
+/* tiger_static_restart in chunk mode (node_stride > 0; virtual ids v = c * node_stride + u as in
+ * tiger_find_recent_ex): restart node v of chunk c cuts its history at chunk_ts[c] (the float32 minimum of that
+ * chunk's batch times, tiger_min_time_ex: TIGER.restart, tiger.py:594-609, receives the ts.min() of its own rank's
+ * batch) and reads its CSR segment and its left_emb / right_emb rows at u (StaticRestarter.forward,
+ * restarters.py:254-277); the memories, clocks, flags and has_msg are written at v.  batch_ts and q_ts are unused.
+ * node_stride == 0 is tiger_static_restart (chunk_ts unused). */
+int tiger_static_restart_ex(const int64_t* nids, const int32_t* count, int64_t n,
+                            const float* batch_ts, int64_t batch, const double* q_ts,
+                            const int64_t* indptr, const double* adj_ts, const float* left_emb,
+                            const float* right_emb, int d, float* left_vals, float* left_ts,
+                            uint8_t* left_active, float* right_vals, float* right_ts,
+                            uint8_t* right_active, uint8_t* has_msg, float* out_prev_ts,
+                            int64_t node_stride, const double* chunk_ts, void* stream);
+
 /* Restart surrogates of a read-only query: out_rows[i] = right_emb[nids[i]] (the right-memory row
  * tiger_static_restart writes) for i < min(*count, n) (count may be NULL); writes nothing node-indexed. */
 int tiger_static_restart_rows(const int64_t* nids, const int32_t* count, int64_t n, const float* right_emb, int d,
@@ -424,6 +462,11 @@ int tiger_static_restart_rows(const int64_t* nids, const int32_t* count, int64_t
  * tiger_min_time: out[0] = (double)min(ts[0..n)) - the float32 ts.min() that restart() receives
  * (train_self_supervised.py:161, eval_utils.py:40), widened for the float64 history search. */
 int tiger_min_time(const float* ts, int64_t n, double* out, void* stream);
+
+/* out[c] = (double)min(ts[c*n .. (c+1)*n)) for c < n_chunks: the restart time of each chunk of a chunked batch
+ * (chunk-major ts, tiger_find_recent_ex), each chunk's own ts.min() as its DDP rank would compute it
+ * (train_self_supervised.py:161).  n_chunks == 1 is tiger_min_time. */
+int tiger_min_time_ex(const float* ts, int64_t n_chunks, int64_t n, double* out, void* stream);
 
 /* Event tokens of SeqRestarter.forward (restarters.py:85-104): for node i and history position j
  *   x[i,j,:] = [nf(src) | nf(dst) | anony_emb[anony_ids] | ef(hist_eids) | cos((t_last - hist_ts)*w + b)]

@@ -20,6 +20,7 @@ _SIGNATURES: Dict[str, str] = {
     'tiger_csr_build_work_bytes': 'll',
     'tiger_csr_build': 'ppppll' + 'ppppp' + 'p' + 'p',
     'tiger_find_recent': 'ppppp' + 'pp' + 'lli' + 'pppp' + 'pp' + 'p' + 'p',
+    'tiger_find_recent_ex': 'ppppp' + 'pp' + 'lli' + 'pppp' + 'pp' + 'p' + 'li' + 'p',
     'tiger_hit_window': 'ppli' + 'p' + 'p',
     'tiger_mark_nodes': 'plpl' + 'p',
     'tiger_compact_involved': 'plpp' + 'plp' + 'ppp' + 'pp' + 'p',
@@ -63,6 +64,7 @@ _SIGNATURES: Dict[str, str] = {
     'tiger_pipe_join': 'pp',
     'tiger_sgemm_nt_packed_scatter': 'plpippli' + 'pliil' + 'ip' + 'p',
     'tiger_min_time': 'plp' + 'p',
+    'tiger_min_time_ex': 'pllp' + 'p',
     'tiger_seq_tokens': 'ppli' + 'ppppp' + 'ppii' + 'ppp' + 'ppp' + 'p',
     'tiger_sgemm_nt': 'plplp' + 'pl' + 'lpl' + 'iii' + 'p',
     'tiger_train_gather_pending': 'pplpippipipppppp',
@@ -101,6 +103,7 @@ _SIGNATURES: Dict[str, str] = {
     'tiger_gemm_pack_weight': 'plpiiiip' + 'p',
     'tiger_sgemm_nt_packed': 'plpippllpliifi' + 'p',
     'tiger_static_restart': 'ppl' + 'plp' + 'pp' + 'ppi' + 'ppp' + 'ppp' + 'pp' + 'p',
+    'tiger_static_restart_ex': 'ppl' + 'plp' + 'pp' + 'ppi' + 'ppp' + 'ppp' + 'pp' + 'lp' + 'p',
     'tiger_static_restart_rows': 'pplpi' + 'p' + 'p',
 }
 _KIND = {'p': P, 'l': L, 'i': I, 'f': F}

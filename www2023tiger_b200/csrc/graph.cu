@@ -15,7 +15,13 @@
 // of dependent loads (node id -> indptr -> probes -> entries); several queries per warp keep enough of
 // those chains in flight to use the memory system.
 // ------------------------------------------------------------------------------------------
+// Chunk modes (MODE != 0, tiger_find_recent_ex): query ids are virtual ids v = c * stride + u of chunk c; the search
+// reads the CSR segment of u.  TIGER_FIND_CHUNK_NEIGHBORS returns the neighbor ids offset by c * stride except the
+// padding id 0, which stays 0 (the attention masks slots by id 0) but marks the chunk's own node 0; a query with id 0
+// (the second hop of a padding slot) marks nothing.  TIGER_FIND_CHUNK_HISTORY takes the query time from q_ts[c] and
+// returns the real neighbor ids.  Both mark the bitmap with virtual ids.
 #define FIND_G 8
+template <int MODE>
 __global__ void __launch_bounds__(256)
 find_recent_kernel(const int64_t* __restrict__ indptr, const int32_t* __restrict__ adj_nbr,
                    const int32_t* __restrict__ adj_eid, const double* __restrict__ adj_ts,
@@ -23,22 +29,24 @@ find_recent_kernel(const int64_t* __restrict__ indptr, const int32_t* __restrict
                    const double* __restrict__ q_ts, int64_t n_query, const int32_t* __restrict__ count,
                    int64_t ts_period, int k, int64_t* __restrict__ out_nids, int64_t* __restrict__ out_eids,
                    float* __restrict__ out_ts, int64_t* __restrict__ out_dirs,
-                   float* __restrict__ out_ts32, uint32_t* __restrict__ bitmap) {
+                   float* __restrict__ out_ts32, uint32_t* __restrict__ bitmap, int64_t stride) {
   const int lane = lane_id(), l = lane & (FIND_G - 1);
   const int64_t q = ((int64_t)blockIdx.x * (blockDim.x >> 5) + warp_id_in_block()) * (32 / FIND_G) + lane / FIND_G;
   const bool live = q < n_query && (count == nullptr || q < *count);
-  int64_t nid = 0, beg = 0, end = 0;
+  int64_t nid = 0, beg = 0, end = 0, base = 0;
   double t = 0.0;
   if (live) {
     nid = q_nids[q];
-    t = q_ts[q % ts_period];
-    if (out_ts32 != nullptr && q < ts_period && l == 0) out_ts32[q] = (float)t;
-    beg = indptr[nid];
-    end = indptr[nid + 1];
+    if (MODE != 0) base = nid - nid % stride;
+    t = MODE == TIGER_FIND_CHUNK_HISTORY ? q_ts[nid / stride] : q_ts[q % ts_period];
+    if (MODE != TIGER_FIND_CHUNK_HISTORY && out_ts32 != nullptr && q < ts_period && l == 0) out_ts32[q] = (float)t;
+    beg = indptr[nid - base];
+    end = indptr[nid - base + 1];
   }
   const int64_t cut = group_lower_bound<FIND_G>(adj_ts, beg, end, t, lane);
   if (!live) return;
-  if (bitmap != nullptr && l == 0) atomicOr(bitmap + (nid >> 5), 1u << (nid & 31));
+  const bool mark = bitmap != nullptr && (MODE != TIGER_FIND_CHUNK_NEIGHBORS || nid != 0);
+  if (mark && l == 0) atomicOr(bitmap + (nid >> 5), 1u << (nid & 31));
   for (int kk = l; kk < k; kk += FIND_G) {
     const int64_t s = cut - k + kk;
     int64_t nb = 0, ei = 0, dr = 0;
@@ -50,11 +58,12 @@ find_recent_kernel(const int64_t* __restrict__ indptr, const int32_t* __restrict
       dr = adj_flag[s];
     }
     const int64_t o = q * k + kk;
-    out_nids[o] = nb;
+    out_nids[o] = MODE == TIGER_FIND_CHUNK_NEIGHBORS && nb != 0 ? nb + base : nb;
     out_eids[o] = ei;
     out_ts[o] = tv;
     if (out_dirs != nullptr) out_dirs[o] = dr;
-    if (bitmap != nullptr) atomicOr(bitmap + (nb >> 5), 1u << (nb & 31));
+    if (MODE != 0) nb += base;
+    if (mark) atomicOr(bitmap + (nb >> 5), 1u << (nb & 31));
   }
 }
 
@@ -68,9 +77,32 @@ extern "C" int tiger_find_recent(const int64_t* indptr, const int32_t* adj_nbr, 
   if (ts_period == 0) ts_period = n_query;
   const int warps = 8, per_cta = warps * (32 / FIND_G);
   const unsigned grid = (unsigned)((n_query + per_cta - 1) / per_cta);
-  find_recent_kernel<<<grid, warps * 32, 0, as_stream(stream)>>>(
+  find_recent_kernel<0><<<grid, warps * 32, 0, as_stream(stream)>>>(
       indptr, adj_nbr, adj_eid, adj_ts, adj_flag, q_nids, q_ts, n_query, count, ts_period, k, out_nids, out_eids,
-      out_ts, out_dirs, out_ts32, mark_bitmap);
+      out_ts, out_dirs, out_ts32, mark_bitmap, 0);
+  return tiger_launch_status();
+}
+
+extern "C" int tiger_find_recent_ex(const int64_t* indptr, const int32_t* adj_nbr, const int32_t* adj_eid,
+                                    const double* adj_ts, const uint8_t* adj_flag, const int64_t* q_nids,
+                                    const double* q_ts, int64_t n_query, int64_t ts_period, int k,
+                                    int64_t* out_nids, int64_t* out_eids, float* out_ts, int64_t* out_dirs,
+                                    float* out_ts32, uint32_t* mark_bitmap, const int32_t* count,
+                                    int64_t node_stride, int mode, void* stream) {
+  if (mode == 0)
+    return tiger_find_recent(indptr, adj_nbr, adj_eid, adj_ts, adj_flag, q_nids, q_ts, n_query, ts_period, k,
+                             out_nids, out_eids, out_ts, out_dirs, out_ts32, mark_bitmap, count, stream);
+  if (n_query < 0 || k <= 0 || ts_period < 0 || node_stride <= 0) return TIGER_EINVAL;
+  if (mode != TIGER_FIND_CHUNK_NEIGHBORS && mode != TIGER_FIND_CHUNK_HISTORY) return TIGER_EINVAL;
+  if (n_query == 0) return TIGER_OK;
+  if (ts_period == 0) ts_period = n_query;
+  const int warps = 8, per_cta = warps * (32 / FIND_G);
+  const unsigned grid = (unsigned)((n_query + per_cta - 1) / per_cta);
+  auto kernel = mode == TIGER_FIND_CHUNK_NEIGHBORS ? find_recent_kernel<TIGER_FIND_CHUNK_NEIGHBORS>
+                                                   : find_recent_kernel<TIGER_FIND_CHUNK_HISTORY>;
+  kernel<<<grid, warps * 32, 0, as_stream(stream)>>>(indptr, adj_nbr, adj_eid, adj_ts, adj_flag, q_nids, q_ts,
+                                                     n_query, count, ts_period, k, out_nids, out_eids, out_ts,
+                                                     out_dirs, out_ts32, mark_bitmap, node_stride);
   return tiger_launch_status();
 }
 

@@ -16,8 +16,11 @@
 #include "common.cuh"
 
 // ------------------------------------------------------------------------------------------
+// one CTA per chunk of n times
 __global__ void min_time_kernel(const float* __restrict__ ts, int64_t n, double* __restrict__ out) {
   __shared__ float red[32];
+  ts += blockIdx.x * n;
+  out += blockIdx.x;
   float m = INFINITY;
   for (int64_t i = threadIdx.x; i < n; i += blockDim.x) m = fminf(m, ts[i]);
   m = warp_min(m);
@@ -33,6 +36,12 @@ __global__ void min_time_kernel(const float* __restrict__ ts, int64_t n, double*
 extern "C" int tiger_min_time(const float* ts, int64_t n, double* out, void* stream) {
   if (n <= 0 || out == nullptr) return TIGER_EINVAL;
   min_time_kernel<<<1, 256, 0, as_stream(stream)>>>(ts, n, out);
+  return tiger_launch_status();
+}
+
+extern "C" int tiger_min_time_ex(const float* ts, int64_t n_chunks, int64_t n, double* out, void* stream) {
+  if (n_chunks <= 0 || n_chunks > 0x7fffffff || n <= 0 || out == nullptr) return TIGER_EINVAL;
+  min_time_kernel<<<(unsigned)n_chunks, 256, 0, as_stream(stream)>>>(ts, n, out);
   return tiger_launch_status();
 }
 

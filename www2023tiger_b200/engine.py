@@ -31,6 +31,12 @@ With n_layers = 2 (GraphEmbedding.compute_embedding_with_computation_graph, temp
 
 `CandidateQuery` (TigerEngine.candidate_query) scores one-vs-many candidate lists against the live state with the
 same launches, reading the state tables and writing none of them.
+
+With `n_chunks=M` one step ingests one batch of B events from each of M independent chunks of the stream (the DDP
+partition of the reference's ChunkSampler, data_loader.py:23-48, on one GPU).  Node u of chunk c has the virtual id
+c*N + u: every per-node state table has M*N rows, the launches above run on the M*B events of the step in that id
+space, and only the finder (tiger_find_recent_ex), the chunk restart times (tiger_min_time_ex) and the static restart
+(tiger_static_restart_ex) map a virtual id back to its real node for the shared CSR and restarter embeddings.
 """
 from typing import Dict, Optional
 
@@ -44,6 +50,7 @@ from . import _lib, ops
 from ._lib import raise_on_err_flags
 from .ops import f32, f64, i32, i64, u8
 
+SELECT_SMALL_N = 2048      # tiger_select_latest ranks at most this many positions without per-node scratch
 KERNELS_PER_STEP = {  # launches of our kernels per batch (for the bench `gpu_launches` field)
     'find_recent': 1, 'compact_involved': 1, 'gru_update': 1, 'temporal_attention': 4, 'select_latest': 1,
     'right_writeback': 1, 'store_messages': 2, 'left_writeback': 0, 'link_score': 1,
@@ -56,7 +63,21 @@ class TigerEngine:
                  n_head: int = 2, batch_size: int = 200, msg_src: str = 'left', upd_src: str = 'right',
                  restarter: Optional[str] = None, hist_len: int = 40, hit_type: str = 'bin',
                  lazy_restart: bool = False, want_restarter_targets: bool = False, n_layers: int = 1,
-                 msg_tsfm_type: str = 'id', mem_update_type: str = 'gru', device='cuda'):
+                 msg_tsfm_type: str = 'id', mem_update_type: str = 'gru', n_chunks: int = 1, device='cuda'):
+        """n_chunks = M: each step takes one batch of `batch_size` events from each of M chunks of the stream, and
+        each chunk evolves exactly as a separate engine fed only that chunk's batches from reset() would (its own
+        memories, message store, pending / up-to-date flags, lazy restart at its own batch minimum); the chunks share
+        the weights, the CSR and the feature tables.  Inputs are chunk-major [M, batch_size] arrays of real node ids
+        (set_batch, device_records), scores come back as [M, batch_size] (chunk_scores).  With M > 1 node 0 is the
+        padding node only (ids of events start at 1, as in the reference's data): the input helpers reject id 0.  M = 1
+        is the unchunked engine."""
+        if isinstance(n_chunks, bool) or not isinstance(n_chunks, int) or n_chunks < 1:
+            raise ValueError(f'n_chunks must be a positive int, got {n_chunks!r}')
+        if n_chunks * n_nodes > 2 ** 31 - 1:
+            raise ValueError(f'n_chunks * n_nodes = {n_chunks * n_nodes} virtual node ids do not fit the int32 index '
+                             f'range of the per-node tables and the CSR')
+        if n_chunks > 1 and want_restarter_targets:
+            raise NotImplementedError('restarter targets (a training input) on a chunked engine')
         if n_layers not in (1, 2):
             raise NotImplementedError(f'n_layers={n_layers}: the engine runs one or two attention layers')
         if msg_src not in ('left', 'right') or upd_src not in ('left', 'right'):
@@ -74,10 +95,14 @@ class TigerEngine:
         self._check_hit_weights(weights)
         dev = torch.device(device)
         self.device, self.csr = dev, csr
-        self.N, self.H, self.B = n_nodes, n_head, batch_size
+        # B: events per step over all chunks (what every launch is sized by); N: real nodes, NV: per-node table rows
+        self.n_chunks, self.chunk_batch = n_chunks, batch_size
+        self.N, self.H, self.B = n_nodes, n_head, n_chunks * batch_size
+        self.NV = n_chunks * n_nodes
         self.n_layers = n_layers
         self.efeats = efeats
-        self.nfeats = nfeats
+        # the attention, the message builder and the seq tokens read node features by (virtual) node id
+        self.nfeats = nfeats.repeat(n_chunks, 1) if nfeats is not None and n_chunks > 1 else nfeats
         self.de = efeats.shape[1] if efeats is not None else dim
         # every layer has the same widths, K and heads; models past the attention kernel's limits run on the drop-in's
         # torch route
@@ -94,7 +119,7 @@ class TigerEngine:
         self.msg_src, self.upd_src = msg_src, upd_src
         self.restarter, self.lazy_restart = restarter, lazy_restart
         self.want_targets = want_restarter_targets
-        N, d, B, K = self.N, self.d, self.B, self.K
+        N, d, B, K = self.NV, self.d, self.B, self.K
         z = lambda *s, dt=f32: torch.zeros(*s, dtype=dt, device=dev)
         # ---- persistent state (reference: Memory x2, MessageStoreNoGradLastOnly) ----
         self.left_vals, self.left_ts, self.left_active = z(N, d), z(N), z(N, dt=u8)
@@ -105,6 +130,8 @@ class TigerEngine:
         # involved-node capacity: every query node and its K neighbors (collate_memory_nodes); with the second hop
         # the 3B*K hop-1 neighbors are queries too, and no list can hold more than the N distinct nodes
         self.cap = 3 * B * (K + 1) if n_layers == 1 else min((3 * B + 3 * B * K) * (K + 1), N)
+        if n_chunks > 1:
+            self.cap = min(self.cap, N)
         self.bitmap = z(ops.bitmap_words(N), dt=i32)
         self.involved, self.outdated, self.restart_nodes = z(self.cap, dt=i64), z(self.cap, dt=i64), z(self.cap, dt=i64)
         self.gru_row = torch.full((N,), -1, dtype=i32, device=dev)
@@ -123,6 +150,10 @@ class TigerEngine:
         self.emb = z(3 * B, d)
         self.winner = z(2 * B, dt=u8)
         self.sel_count = z(1, dt=i32)
+        # M*B events can pass the all-pairs selection's 2,048 positions: the per-node slot route (same winners)
+        self.sel_scratch = ops.SelectScratch(N, dev) if n_chunks > 1 and 2 * B > SELECT_SMALL_N else None
+        self._stride = n_nodes if n_chunks > 1 else 0          # node stride of the chunk modes, 0: unchunked
+        self.chunk_tmin = z(n_chunks, dt=f64) if n_chunks > 1 else None     # restart time of each chunk
         self.out_buf = z(2 * B + 1)                    # [pos scores | neg scores | loss]
         self.hprev_left = z(2 * B, d) if want_restarter_targets else None
         self.hprev_right = z(2 * B, d) if want_restarter_targets else None
@@ -139,9 +170,15 @@ class TigerEngine:
         self.attn_pack = ops.AttnPack(self.d, self.de, dev, n_head)
         self.attn_pack1 = ops.AttnPack(self.d, self.de, dev, n_head) if n_layers == 2 else None   # fns.1 (depth 1)
         self.score_fold = ops.ScoreFold(self.d, dev, hit_type, K)
-        self.pq = torch.zeros(3 * batch_size, 2 * self.d, dtype=f32, device=dev)   # [W1a z | W1b z] per query row
+        self.pq = torch.zeros(3 * self.B, 2 * self.d, dtype=f32, device=dev)   # [W1a z | W1b z] per query row
         self.hist_len = hist_len
         self.seq = ops.SeqRestarterOp(self.d, self.de, hist_len, n_head, self.cap, dev) if restarter == 'seq' else None
+        if self.seq is not None and n_chunks > 1:
+            self.seq.tmin = self.chunk_tmin
+            # the restarted rows of all chunks share one launch sequence, and the restarter picks its arithmetic route
+            # (matrix-vector tail for few rows, tensor-core products otherwise) from their total count: a fixed route
+            # keeps a chunk's rounding independent of how many nodes the other chunks restart
+            self.seq.tail_rows = 0
         self.weights_version = 0            # counts load_weights calls: a graph captured before one is stale
         self.load_weights(weights)
 
@@ -207,22 +244,63 @@ class TigerEngine:
         raise_on_err_flags(int(self.err_flags.item()) & 0xffffffff)
 
     def set_batch(self, src, dst, neg, ts, eids):
-        """Copy one batch (numpy or tensors; ts float64) into the device input buffer."""
+        """Copy one batch (numpy or tensors; ts float64) into the device input buffer.  With n_chunks = M > 1 each
+        argument is chunk-major [M, batch_size] with real node ids (fill_record)."""
         B = self.B
         host = torch.empty(5 * B, dtype=i64)
         h = host.numpy()
-        h[:B], h[B:2 * B], h[2 * B:3 * B], h[3 * B:4 * B] = src, dst, neg, eids
-        h[4 * B:].view(np.float64)[:] = ts
+        if self.n_chunks > 1:
+            self.fill_record(h, src, dst, neg, ts, eids)
+        else:
+            h[:B], h[B:2 * B], h[2 * B:3 * B], h[3 * B:4 * B] = src, dst, neg, eids
+            h[4 * B:].view(np.float64)[:] = ts
         self.inp.copy_(host)
+
+    def fill_record(self, h: np.ndarray, src, dst, neg, ts, eids):
+        """Writes batches into int64 host records h [..., 5 * M * batch_size] (the layout of self.inp) from arrays
+        (numpy or CPU tensors) of shape [..., M, batch_size]: real node ids, edge ids, float64 times.  Chunk c's node ids
+        are stored as the virtual ids c * n_nodes + u, edge ids and times as given.  Node ids must lie in [0, n_nodes),
+        and with M > 1 in [1, n_nodes): a chunked engine keeps id 0 for the padding of the neighbor tables, as the
+        reference's data does (ids start at 1), so a real node 0 is rejected (ValueError)."""
+        M, Bc = self.n_chunks, self.chunk_batch
+        lo = 1 if M > 1 else 0
+        rec = h.reshape(-1, 5, M, Bc)
+        n = rec.shape[0]
+        for i, x in enumerate((src, dst, neg)):
+            x = np.asarray(x).reshape(n, M, Bc)
+            if x.size and (x.min() < lo or x.max() >= self.N):
+                raise ValueError(f'node ids outside [{lo}, {self.N})' + (' (node 0 is the padding node)' if lo else ''))
+            np.add(x, np.arange(M, dtype=np.int64)[:, None] * self.N, out=rec[:, i])
+        rec[:, 3] = np.asarray(eids).reshape(n, M, Bc)
+        rec[:, 4] = np.asarray(ts, dtype=np.float64).reshape(n, M, Bc).view(np.int64)
+
+    def device_records(self, src, dst, neg, ts, eids) -> Tensor:
+        """Batch records for StreamRunner.submit_device, resident on the engine's device: arrays of shape
+        [n, M, batch_size] give int64 [n, 5 * M * batch_size], arrays of shape [M, batch_size] one record [5 * M *
+        batch_size] (fill_record)."""
+        one = np.asarray(src).ndim <= 2
+        h = np.empty((np.asarray(src).size // self.B, 5 * self.B), dtype=np.int64)
+        self.fill_record(h, src, dst, neg, ts, eids)
+        out = torch.from_numpy(h).to(self.device)
+        return out[0] if one else out
+
+    def chunk_scores(self):
+        """(pos, neg) link-scorer logits of the latest step, float32 [M, batch_size] views of the result buffer.  The
+        step's loss (self.loss) is the mean BCE over all 2 M batch_size rows; with equal batches per chunk that is the
+        mean of the M per-chunk losses."""
+        M, Bc = self.n_chunks, self.chunk_batch
+        return self.scores[:self.B].view(M, Bc), self.scores[self.B:].view(M, Bc)
 
     # ------------------------------------------------------------------ the launch sequence
     def launch_finder(self):
         ops.find_recent(self.csr, self.batch_nids, self.ts64, self.K, ts_period=self.B, want_dirs=False,
                         ts32_out=self.ts32, bitmap=self.bitmap,
-                        out=(self.neigh_nids, self.neigh_eids, self.neigh_ts, None))
+                        out=(self.neigh_nids, self.neigh_eids, self.neigh_ts, None),
+                        chunk_mode=ops.FIND_CHUNK_NEIGHBORS if self._stride else 0, node_stride=self._stride)
         if self.n_layers == 2:
             ops.find_second_hop(self.csr, self.neigh_nids, self.neigh_ts, self.K, ts64=self.neigh_ts64,
-                                bitmap=self.bitmap, out=(self.neigh2_nids, self.neigh2_eids, self.neigh2_ts))
+                                bitmap=self.bitmap, out=(self.neigh2_nids, self.neigh2_eids, self.neigh2_ts),
+                                node_stride=self._stride)
 
     def launch_model(self, with_scorer: bool = True):
         d, B = self.d, self.B
@@ -237,7 +315,7 @@ class TigerEngine:
         side1 = cur if serial & 2 else self._side
         msg_vals_mem, msg_ts_mem = self._mem(self.msg_src)
         upd_vals, _ = self._mem(self.upd_src)
-        ops.compact_involved(self.bitmap, self.N, self.involved, self.counts, has_msg=self.has_msg,
+        ops.compact_involved(self.bitmap, self.NV, self.involved, self.counts, has_msg=self.has_msg,
                              uptodate=self.uptodate if self.lazy_restart else None, outdated=self.outdated,
                              gru_row=self.gru_row, restart_nodes=self.restart_nodes if self.lazy_restart else None,
                              err_flags=self.err_flags)
@@ -251,17 +329,22 @@ class TigerEngine:
             with torch.cuda.stream(side0):
                 side0.wait_event(self._ev_fork0)
                 if self.restarter == 'static':
+                    # chunked: each chunk cuts at the minimum of its own batch times
+                    if self._stride:
+                        ops.min_time(self.ts32, self.chunk_tmin, self.n_chunks)
                     ops.static_restart(self.restart_nodes, self.cap, self.csr, self.left_emb, self.right_emb, d,
                                        count=self.counts[2:], batch_ts=self.ts32, left_vals=self.left_vals,
                                        left_ts=self.left_ts, left_active=self.left_active, right_vals=self.right_vals,
-                                       right_ts=self.right_ts, right_active=self.right_active, has_msg=self.has_msg)
+                                       right_ts=self.right_ts, right_active=self.right_active, has_msg=self.has_msg,
+                                       node_stride=self._stride, chunk_ts=self.chunk_tmin)
                 else:
                     # TIGER.restart with the seq restarter (tiger.py:594-609, restarters.py:51-114): history at
                     # ts.min() of the batch, surrogate h(t'-) / h(t'+), both memories overwritten without checks
                     # (compact_involved has already dropped the pending-message flags of these nodes)
                     R = self.counts[2:]
-                    ops.min_time(self.ts32, self.seq.tmin)
-                    self.seq.history(self.csr, self.restart_nodes, self.seq.tmin, self.cap, ts_period=1, count=R)
+                    ops.min_time(self.ts32, self.seq.tmin, self.n_chunks)
+                    self.seq.history(self.csr, self.restart_nodes, self.seq.tmin, self.cap, ts_period=1, count=R,
+                                     node_stride=self._stride)
                     hl, hr, pt = self.seq.forward(self.restart_nodes, self.cap, self.nfeats, self.efeats, count=R)
                     ops.scatter_rows(self.left_vals, self.restart_nodes, hl, ts_table=self.left_ts, ts=pt,
                                      active=self.left_active, count=R)
@@ -281,7 +364,8 @@ class TigerEngine:
         self._ev_fork.record(main)
         with torch.cuda.stream(side1):
             side1.wait_event(self._ev_fork)
-            ops.select_latest(self.pos, self.ts32, want_unique=False, winner=self.winner, want_count=False)
+            ops.select_latest(self.pos, self.ts32, self.sel_scratch, want_unique=False, winner=self.winner,
+                              want_count=False)
             ops.right_writeback(self.pos, self.winner, self.gru_row, self.h_new, d, self.right_vals, self.right_ts,
                                 self.right_active, self.msg_ts, self.has_msg, self.left_vals, self.hprev_left,
                                 self.hprev_right, self.err_flags)
@@ -365,6 +449,11 @@ class TigerEngine:
             n += 2 + KERNELS_PER_STEP['temporal_attention']
         if self.lazy_restart:
             n += 1 if self.restarter == 'static' else ops.SeqRestarterOp.LAUNCHES + 2
+            if self.restarter == 'seq' and self.n_chunks > 1:
+                n -= ops.SeqRestarterOp.TAIL_LAUNCHES                             # products only
+            n += int(self.restarter == 'static' and self.n_chunks > 1)     # the chunk restart times
+        if self.sel_scratch is not None:
+            n += 3          # per-node slot selection: max-ts, min-position, flag and reset kernels
         if self.want_targets:
             n += 1
         return n
@@ -377,6 +466,8 @@ class TigerEngine:
     def candidate_query(self, max_queries: int, n_candidates: int) -> 'CandidateQuery':
         """A read-only scorer of up to `max_queries` sources against `n_candidates` candidates each on this engine's
         current state and weights (CandidateQuery)."""
+        if self.n_chunks > 1:
+            raise NotImplementedError('candidate_query on a chunked engine (n_chunks > 1)')
         return CandidateQuery(self, max_queries, n_candidates)
 
 
@@ -641,6 +732,9 @@ class StreamRunner:
         return slot
 
     def fill_host(self, slot: int, src, dst, neg, ts, eids):
+        if self.e.n_chunks > 1:
+            self.e.fill_record(self._h_in_np[slot], src, dst, neg, ts, eids)
+            return
         B = self.e.B
         h = self._h_in_np[slot]
         h[:B], h[B:2 * B], h[2 * B:3 * B], h[3 * B:4 * B] = src, dst, neg, eids
@@ -648,7 +742,8 @@ class StreamRunner:
 
     def submit_host(self, src, dst, neg, ts, eids) -> int:
         """Host-buffer step: H2D of the batch, the graphs, D2H of scores + loss.  Returns the slot whose
-        results become readable after `wait(slot)`."""
+        results become readable after `wait(slot)`.  A chunked engine takes chunk-major [M, batch_size] arrays of
+        real node ids (TigerEngine.fill_record)."""
         slot = self._next_slot()
         if self.slot_busy[slot]:
             raise RuntimeError(f'staging slot {slot} still holds unread results: call wait(slot) on every slot returned '
@@ -676,6 +771,11 @@ class StreamRunner:
             self.e.check_errors()          # attribute an invariant violation to (at most n_slots batches around) this one
         out = self.h_out[slot]
         B = self.e.B
+        if self.e.n_chunks > 1:
+            # [M, batch_size] scores; the loss is the mean over all 2 M batch_size rows, which with equal batches is
+            # the mean of the M per-chunk losses
+            shape = (self.e.n_chunks, self.e.chunk_batch)
+            return out[:B].view(shape), out[B:2 * B].view(shape), out[2 * B]
         return out[:B], out[B:2 * B], out[2 * B]
 
     @property
@@ -685,6 +785,20 @@ class StreamRunner:
     @property
     def d2h_bytes_per_step(self) -> int:
         return self.h_out[0].numel() * 4
+
+
+def chunk_bounds(n: int, n_chunks: int, batch_size: int, seed: int = 0, epoch: int = 0):
+    """The reference's DDP partition of n events into n_chunks contiguous chunks (ChunkSampler.bounds of every rank,
+    data_loader.py:23-48): [(lo_c, hi_c)] with hi_c - lo_c = n // (n_chunks * batch_size) * batch_size, all chunks
+    shifted by one draw from Generator(seed + epoch).  Batch i of a chunked engine is events
+    [lo_c + i * batch_size, lo_c + (i + 1) * batch_size) of every chunk c."""
+    from .tiger.data.data_loader import ChunkSampler
+    bounds = []
+    for rank in range(n_chunks):
+        s = ChunkSampler(n, rank, n_chunks, batch_size, seed=seed)
+        s.set_epoch(epoch)
+        bounds.append(s.bounds())
+    return bounds
 
 
 def check_query_inputs(src, cands, ts, *, max_queries: int, n_candidates: int, n_nodes: int, device) -> int:

@@ -53,11 +53,15 @@ def csr_build(src: Tensor, dst: Tensor, ts: Tensor, eids: Tensor, n_nodes: int) 
     return DeviceCSR(indptr, nbr, eid, ats, flag)
 
 
+FIND_CHUNK_NEIGHBORS, FIND_CHUNK_HISTORY = 1, 2     # chunk modes of tiger_find_recent_ex (include/tiger_b200.h)
+
+
 def find_recent(csr: DeviceCSR, q_nids: Tensor, q_ts: Tensor, k: int, *, ts_period: int = 0,
                 want_dirs: bool = True, ts32_out: Optional[Tensor] = None, bitmap: Optional[Tensor] = None,
                 out: Optional[Tuple[Tensor, Tensor, Tensor, Optional[Tensor]]] = None,
-                count: Optional[Tensor] = None):
-    """a2: K most recent events strictly before q_ts, right-aligned and zero-padded."""
+                count: Optional[Tensor] = None, chunk_mode: int = 0, node_stride: int = 0):
+    """a2: K most recent events strictly before q_ts, right-aligned and zero-padded.  chunk_mode (FIND_CHUNK_*):
+    q_nids are virtual ids c * node_stride + u of a chunked engine (tiger_find_recent_ex)."""
     check_cuda(q_nids, q_ts)
     assert q_nids.dtype == i64 and q_ts.dtype == f64
     n = q_nids.numel()
@@ -68,19 +72,24 @@ def find_recent(csr: DeviceCSR, q_nids: Tensor, q_ts: Tensor, k: int, *, ts_peri
         o_d = _empty((n, k), i64, q_nids) if want_dirs else None
     else:
         o_n, o_e, o_t, o_d = out
-    call('tiger_find_recent', ptr(csr.indptr), ptr(csr.nbr), ptr(csr.eid), ptr(csr.ts), ptr(csr.flag),
-         ptr(q_nids), ptr(q_ts), n, ts_period or q_ts.numel(), k, ptr(o_n), ptr(o_e), ptr(o_t), ptr(o_d),
-         ptr(ts32_out), ptr(bitmap), ptr(count))
+    args = (ptr(csr.indptr), ptr(csr.nbr), ptr(csr.eid), ptr(csr.ts), ptr(csr.flag), ptr(q_nids), ptr(q_ts), n,
+            ts_period or q_ts.numel(), k, ptr(o_n), ptr(o_e), ptr(o_t), ptr(o_d), ptr(ts32_out), ptr(bitmap),
+            ptr(count))
+    if chunk_mode:
+        call('tiger_find_recent_ex', *args, node_stride, chunk_mode)
+    else:
+        call('tiger_find_recent', *args)
     return o_n, o_e, o_t, o_d
 
 
 def find_second_hop(csr: DeviceCSR, nn1: Tensor, nt1: Tensor, k: int, *, ts64: Tensor, bitmap: Tensor,
-                    out: Tuple[Tensor, Tensor, Tensor]):
+                    out: Tuple[Tensor, Tensor, Tensor], node_stride: int = 0):
     """collate_memory_nodes' second neighbor call for n_layers = 2: the K most recent neighbors of each hop-1 neighbor
     nn1 [n, K] at its own float32 event time nt1, widened to float64 (an exact conversion) in `ts64` [n*K]; marks the
-    same involved-node bitmap as the first hop."""
+    same involved-node bitmap as the first hop.  node_stride > 0: nn1 holds virtual ids of a chunked engine."""
     ts64.copy_(nt1.view(-1))
-    find_recent(csr, nn1.view(-1), ts64, k, want_dirs=False, bitmap=bitmap, out=(*out, None))
+    find_recent(csr, nn1.view(-1), ts64, k, want_dirs=False, bitmap=bitmap, out=(*out, None),
+                chunk_mode=FIND_CHUNK_NEIGHBORS if node_stride else 0, node_stride=node_stride)
 
 
 def hit_window(center: Tensor, neigh: Tensor) -> Tensor:
@@ -650,10 +659,17 @@ def static_restart_rows(nids: Tensor, n: int, right_emb: Tensor, d: int, out_row
 
 def static_restart(nids: Tensor, n: int, csr: DeviceCSR, left_emb: Tensor, right_emb: Tensor, d: int, *,
                    count=None, batch_ts=None, q_ts=None, left_vals=None, left_ts=None, left_active=None,
-                   right_vals=None, right_ts=None, right_active=None, has_msg=None, out_prev_ts=None):
-    call('tiger_static_restart', ptr(nids), ptr(count), n, ptr(batch_ts), batch_ts.numel() if batch_ts is not None else 0,
-         ptr(q_ts), ptr(csr.indptr), ptr(csr.ts), ptr(left_emb), ptr(right_emb), d, ptr(left_vals), ptr(left_ts),
-         ptr(left_active), ptr(right_vals), ptr(right_ts), ptr(right_active), ptr(has_msg), ptr(out_prev_ts))
+                   right_vals=None, right_ts=None, right_active=None, has_msg=None, out_prev_ts=None,
+                   node_stride: int = 0, chunk_ts: Optional[Tensor] = None):
+    """node_stride > 0: nids are virtual ids of a chunked engine, cut at chunk_ts [M] float64
+    (tiger_static_restart_ex)."""
+    args = (ptr(nids), ptr(count), n, ptr(batch_ts), batch_ts.numel() if batch_ts is not None else 0, ptr(q_ts),
+            ptr(csr.indptr), ptr(csr.ts), ptr(left_emb), ptr(right_emb), d, ptr(left_vals), ptr(left_ts),
+            ptr(left_active), ptr(right_vals), ptr(right_ts), ptr(right_active), ptr(has_msg), ptr(out_prev_ts))
+    if node_stride:
+        call('tiger_static_restart_ex', *args, node_stride, ptr(chunk_ts))
+    else:
+        call('tiger_static_restart', *args)
 
 
 # ------------------------------------------------------------------------------------------
@@ -794,8 +810,12 @@ def check_cuda_strided(*tensors):
             raise _lib.TigerLibraryError('sgemm_nt needs 2-D float32 CUDA tensors with unit inner stride')
 
 
-def min_time(ts: Tensor, out: Tensor):
-    call('tiger_min_time', ptr(ts), ts.numel(), ptr(out))
+def min_time(ts: Tensor, out: Tensor, n_chunks: int = 1):
+    """out[c] = min of chunk c of the chunk-major ts (float64 [n_chunks]); one chunk: tiger_min_time."""
+    if n_chunks == 1:
+        call('tiger_min_time', ptr(ts), ts.numel(), ptr(out))
+    else:
+        call('tiger_min_time_ex', ptr(ts), n_chunks, ts.numel() // n_chunks, ptr(out))
 
 
 SEQ_MAX_HIST_LEN = 64     # the pooling kernel stages at most this many positions per node (SP_MAXL, csrc/train_seq.cu)
@@ -866,10 +886,12 @@ class SeqRestarterOp:
             setattr(self, n, getattr(other, n))
 
     def history(self, csr: DeviceCSR, nids: Tensor, q_ts: Tensor, n: int, *, ts_period: int = 0,
-                count: Optional[Tensor] = None):
-        """get_history (graph.py:150-155) + anonymized_reindex (utils.py:19-27) for n (or *count) nodes."""
+                count: Optional[Tensor] = None, node_stride: int = 0):
+        """get_history (graph.py:150-155) + anonymized_reindex (utils.py:19-27) for n (or *count) nodes.
+        node_stride > 0: nids are virtual ids of a chunked engine and q_ts holds one time per chunk."""
         find_recent(csr, nids[:n], q_ts, self.L, ts_period=ts_period, count=count,
-                    out=(self.hist_nids[:n], self.hist_eids[:n], self.hist_ts[:n], self.hist_dirs[:n]))
+                    out=(self.hist_nids[:n], self.hist_eids[:n], self.hist_ts[:n], self.hist_dirs[:n]),
+                    chunk_mode=FIND_CHUNK_HISTORY if node_stride else 0, node_stride=node_stride)
         anonymized_reindex(self.hist_nids[:n], out=self.anony[:n], count=count)
 
     def forward(self, nids: Tensor, n: int, nfeats: Optional[Tensor], efeats: Optional[Tensor], *,
@@ -938,6 +960,7 @@ class SeqRestarterOp:
         sgemm_nt(self.hid, self.fc2_w, self.fc2_b, self.h_right, m_rows=n, count=count)
 
     LAUNCHES = 5 + 7 + 6   # min_time, find_recent, reindex, tokens, pool + 7 GEMMs + gate_count, 5 tail layers
+    TAIL_LAUNCHES = 6      # gate_count + 5 tail layers: not launched when tail_rows == 0
 
 
 def store_messages_dense(src, dst, eids, ts, winner, src_vals, dst_vals, src_prev_ts, dst_prev_ts, nfeats, efeats,
